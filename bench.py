@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the render hot path on N B200s, BASELINE.json's metric (Mrays/s, ms/frame).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C3|C1|C2|C5] [--shard tiles|spp]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C3|C1|C2|C5] [--shard tiles|spp] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...      (one rank per GPU, NCCL)
 
 A "step" is one frame of the workload: render_init + render of the reference (main.cu:424-429), i.e. what its
@@ -40,6 +40,10 @@ CPU_STRIDE = {"C1": (4, 4), "C2": (2, 2), "C3": (16, 16), "C4": (96, 96), "C5": 
 # tests/golden/gen_ref_cuda_full.sh (tests/golden/ref_cuda/manifest_full.json: render time per sample count, clocks under load).
 REF_CUDA_BIN = {"C3": "ref_cuda_n100000_oct_spl300", "C4": "ref_cuda_n100000_oct_spl300_fp16"}
 REF_CUDA_LIVE_SPP = 4
+# --dump-outputs: frames up to this size are written whole, larger ones as a fixed, seeded sample of DUMP_SAMPLE_PIXELS pixels
+DUMP_FULL_FRAME_BYTES = 48 << 20
+DUMP_SAMPLE_PIXELS = 1 << 20
+DUMP_SAMPLE_SEED = 1984
 
 
 class ClockSampler(threading.Thread):
@@ -131,7 +135,7 @@ def ref_cuda_leg(cfg: str, rays_at_live_spp: float, rays_full: float, budget_s: 
         out["recorded"] = {"error": str(e)}
     exe = os.path.join(ROOT, "oracle", "_ref", REF_CUDA_BIN.get(cfg, "missing"))
     if not os.path.exists(exe):
-        out["live"] = {"error": "binary not built (make -C oracle ref_cuda needs /root/reference)"}
+        out["live"] = {"error": "binary not built (make -C oracle ref_cuda REF=<checkout of the reference>)"}
         return out
     if budget_s < 150:
         out["live"] = {"skipped": f"only {budget_s:.0f} s of the bench's time budget left; the run needs ~125 s (create_world alone ~115 s)"}
@@ -177,6 +181,25 @@ def run_reference_arm(args):
             "gpu_launches": 0}
     print(json.dumps(line), flush=True)
     return 0
+
+
+def dump_outputs(out_dir: str, fb, rays: float, paths: float):
+    """What the timed path handed its caller in the last timed step: the finished frame (float32 [ny, nx, 3] on the device) and
+    the ray and path counts.  A frame larger than DUMP_FULL_FRAME_BYTES is written as the same seeded pixel sample on every run
+    (frame_sample.npy [K, 3] float32, frame_sample_pixels.npy [K] float64: linear index j * nx + i)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    ny, nx, _ = fb.shape
+    if fb.numel() * 4 <= DUMP_FULL_FRAME_BYTES:
+        np.save(os.path.join(out_dir, "frame.npy"), fb.cpu().numpy())
+    else:
+        rng = np.random.default_rng(DUMP_SAMPLE_SEED)
+        pix = np.sort(rng.choice(nx * ny, size=min(DUMP_SAMPLE_PIXELS, nx * ny), replace=False))
+        sample = fb.reshape(-1, 3)[torch.from_numpy(pix).to(fb.device)].cpu().numpy()
+        np.save(os.path.join(out_dir, "frame_sample.npy"), sample)
+        np.save(os.path.join(out_dir, "frame_sample_pixels.npy"), pix.astype(np.float64))
+    np.save(os.path.join(out_dir, "ray_counts.npy"), np.array([rays, paths], dtype=np.float64))
 
 
 def measure_e2e(pkg, mg, rt, torch, dist, dev, rank, world, mode, prec, n, spl, octree, nx, ny, ns, frame, fb, steps):
@@ -271,7 +294,12 @@ def main():
     ap.add_argument("--no-ref-cuda", action="store_true", help="skip the live run of the reference's CUDA build (~130 s, N = 1 only)")
     ap.add_argument("--time-budget", type=float, default=330.0, help="seconds the whole bench may take; the reference-CUDA leg is skipped "
                                                                        "when less than 150 s of it are left")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed: use it with --impl ours")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -349,6 +377,16 @@ def main():
         total_ms, total_rays = float(tmax[0]), float(tsum[1])
     else:
         total_ms, total_rays = float(t[0]), float(t[1])
+    if args.dump_outputs:
+        last = torch.tensor([float(st["rays"]), float(st["paths"])], dtype=torch.float64, device=dev)
+        out = fb
+        if world > 1:                                  # every rank holds its finished slice of the flattened frame
+            dist.all_reduce(last, op=dist.ReduceOp.SUM)
+            whole = torch.empty(frame.S * world, dtype=torch.float32, device=dev)
+            dist.all_gather_into_tensor(whole, frame.slice)
+            out = whole[:frame.total].view(ny, nx, 3)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, out, float(last[0]), float(last[1]))
     e2e_result = measure_e2e(pkg, mg, rt, torch, dist, dev, rank, world, mode, prec, n, spl, octree, nx, ny, ns, frame, fb, args.steps)
     if rank != 0:
         if world > 1:

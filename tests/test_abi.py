@@ -82,7 +82,7 @@ def test_library_skip_ahead_matches_curand(pkg, golden_dir):
     """rt_xorwow_state (host side, no GPU): the product's own skip-ahead matrices against cuRAND's answers."""
     import json
     kat = json.load(open(os.path.join(golden_dir, "curand_subsequence_kat.json")))
-    for c in kat["cases"]:
+    for c in kat["cases"] + kat["random_cases"]:
         assert [int(x) for x in pkg.xorwow_state(c["seed"], c["subsequence"])] == c["state"], c
     with pytest.raises(pkg.RtError):
         pkg.xorwow_state(1984, 2 ** 40)
