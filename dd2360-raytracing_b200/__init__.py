@@ -39,7 +39,7 @@ ABI_SYMBOLS = [
     "rt_abi_version", "rt_create", "rt_destroy", "rt_last_error", "rt_set_stream", "rt_device_info",
     "rt_scene_generate", "rt_scene_generate_ex", "rt_scene_upload", "rt_scene_download", "rt_scene_size", "rt_camera_set", "rt_camera_get", "rt_camera_get_half",
     "rt_octree_build", "rt_octree_build_ex", "rt_octree_reference_bytes", "rt_octree_export_reference", "rt_octree_debug_read", "rt_xorwow_state", "rt_debug_counters", "rt_trace_rays", "rt_camera_get_rays", "rt_scatter_rays",
-    "rt_render_accumulate", "rt_last_render_stats", "rt_render_progressive", "rt_finalize", "rt_finalize_n", "rt_render", "rt_render_to_host", "rt_format_ppm",
+    "rt_render_accumulate", "rt_last_render_stats", "rt_render_progressive", "rt_finalize", "rt_finalize_n", "rt_finalize_ex", "rt_render", "rt_render_to_host", "rt_format_ppm",
     "rt_ppm_format", "rt_ppm_read", "rt_render_to_ppm",
     "rt_ffma_peak", "rt_hfma2_peak", "rt_malloc", "rt_free", "rt_memcpy_to_host", "rt_synchronize", "rt_kernel_name",
     "rt_comm_get_unique_id", "rt_comm_init_rank", "rt_comm_init_all", "rt_comm_attach", "rt_comm_destroy", "rt_comm_rank", "rt_comm_size",
@@ -126,6 +126,7 @@ def load_library(path: str | None = None) -> C.CDLL:
         "rt_render_progressive": (i32, [vp, C.POINTER(RenderArgs), vp, vp, i32, C.POINTER(RenderStats)]),
         "rt_finalize": (i32, [vp, vp, vp, i32, i32, i32]),
         "rt_finalize_n": (i32, [vp, vp, vp, sz, i32]),
+        "rt_finalize_ex": (i32, [vp, vp, vp, sz, i32, i32]),
         "rt_render": (i32, [vp, C.POINTER(RenderArgs), vp, C.POINTER(RenderStats)]),
         "rt_render_to_host": (i32, [vp, C.POINTER(RenderArgs), vp, C.POINTER(RenderStats)]),
         "rt_format_ppm": (sz, [vp, i32, i32, vp, sz]),
@@ -391,6 +392,11 @@ class RayTracer:
 
     def finalize_n(self, accum_dev_ptr: int, fb_dev_ptr: int, count: int, ns: int):
         self._ck(self.L.rt_finalize_n(self._ctx, C.c_void_p(accum_dev_ptr), C.c_void_p(fb_dev_ptr), count, ns), "rt_finalize_n")
+
+    def finalize_ex(self, accum_dev_ptr: int, fb_dev_ptr: int, count: int, ns: int, precision: int):
+        """/ns and sqrt on `count` linear sums in the given arithmetic (PREC_FP16: the sums are halves widened to float)."""
+        self._ck(self.L.rt_finalize_ex(self._ctx, C.c_void_p(accum_dev_ptr), C.c_void_p(fb_dev_ptr), count, ns, precision),
+                 "rt_finalize_ex")
 
     def hfma2_peak_tflops(self) -> float:
         """Measured dense packed-half HFMA2 rate (TFLOP/s, 4 flop per instruction): the USE_FP16 roofline denominator."""

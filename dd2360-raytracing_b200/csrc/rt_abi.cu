@@ -480,9 +480,10 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
     if (a->seed_mode != RT_SEED_HEAD && a->seed_mode != RT_SEED_UPSTREAM) return fail(ctx, RT_ERR_INVALID, "render: unknown seed_mode");
     if (a->precision != RT_PREC_FP32 && a->precision != RT_PREC_FP16) return fail(ctx, RT_ERR_INVALID, "render: unknown precision");
     const bool fp16 = a->precision == RT_PREC_FP16;
-    if (fp16 && prog) return fail(ctx, RT_ERR_UNSUPPORTED, "render: progressive rendering is FP32 only");
-    if (fp16 && a->shard_mode != RT_SHARD_NONE)
-        return fail(ctx, RT_ERR_UNSUPPORTED, "render: USE_FP16 frames are rendered whole (RT_SHARD_NONE): the half accumulator does not split");
+    // a tile shard holds whole pixels' half sums, exact in float, so shards add up to the 1-GPU frame; the half sum of ns/G
+    // samples per rank is a different image from any build of the reference
+    if (fp16 && a->shard_mode == RT_SHARD_SPP)
+        return fail(ctx, RT_ERR_UNSUPPORTED, "render: USE_FP16 frames shard by tiles only (RT_SHARD_TILES): spp shards' half sums do not add up to the 1-GPU frame");
     if (a->use_octree && ctx->octree->built && ctx->octree->fp16 != fp16)
         return fail(ctx, RT_ERR_STATE, "render: the octree was built for the other precision (rt_octree_build_ex)");
     CK(cudaSetDevice(ctx->device));
@@ -800,6 +801,16 @@ extern "C" int rt_finalize_n(rt_context *ctx, const float *accum_dev, float *fb_
     if (count == 0) return RT_OK;
     CK(cudaSetDevice(ctx->device));
     CK(launch_finalize_n(accum_dev, fb_dev, count, ns, ctx->stream));
+    return RT_OK;
+}
+
+extern "C" int rt_finalize_ex(rt_context *ctx, const float *accum_dev, float *fb_dev, size_t count, int ns, int precision) {
+    if (precision == RT_PREC_FP32) return rt_finalize_n(ctx, accum_dev, fb_dev, count, ns);
+    if (precision != RT_PREC_FP16) return fail(ctx, RT_ERR_INVALID, "rt_finalize_ex: unknown precision");
+    if (!ctx || !accum_dev || !fb_dev || ns < 1) return fail(ctx, RT_ERR_INVALID, "rt_finalize_ex: bad arguments");
+    if (count == 0) return RT_OK;
+    CK(cudaSetDevice(ctx->device));
+    CK(launch_finalize_half(accum_dev, fb_dev, count, ns, ctx->stream));
     return RT_OK;
 }
 

@@ -37,6 +37,9 @@ __device__ __forceinline__ hf hsub_(hf a, hf b) { return __hsub_rn(a, b); }
 __device__ __forceinline__ hf hdiv_(hf a, hf b) { return __hdiv(a, b); }                 // real_t::operator/ (precision_types.h:56-63)
 __device__ __forceinline__ hf hsqrtf_(hf a) { return f2h(__fsqrt_rn(h2f(a))); }          // sqrt(real_t) -> float sqrtf -> real_t
 __device__ __forceinline__ hf hneg_(hf a) { return __hneg(a); }
+// col /= real_t(ns): k = 1.0 / t in double, stored as real_t (vec3.h:137-144).  The one definition of the divisor of the final
+// average: k_render_h and k_finalize_h both use it, so a frame finalised from shards or progressive sums is the one-shot frame.
+__device__ __forceinline__ hf inv_ns_h(int ns) { return f2h((float)(1.0 / (double)h2f(f2h((float)ns)))); }
 
 struct vec3h {
     __half2 xy;

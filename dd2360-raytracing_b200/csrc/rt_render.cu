@@ -296,19 +296,31 @@ cudaError_t launch_camera_setup_half(const float lookfrom[3], const float lookat
                                            vfov, nx, ny, aspect_override, aperture, focus_dist, cam_h);
     return cudaGetLastError();
 }
+template <bool PROG>
+static cudaError_t launch_render_half_t(const RenderLaunch &p, bool octree, const uint2 *geom_h, const uint2 *matl_h, const __half *cam_h,
+                                        const h16::PairView &pv, const h16::NodeTab &nt, int sm_count, cudaStream_t st, int *blocks_out) {
+    if (p.variant == 30)        // A/B: root evaluation inside the scan loop (the first cooperative form); same image
+        return octree ? h16::launch_half<true, false, false, PROG>(p, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out)
+                      : h16::launch_half<false, false, false, PROG>(p, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out);
+    if (p.variant == 33 && octree)      // A/B: the octree line tests as a per-lane walk (walk_cells_h) instead of by the whole warp per ray;
+        return h16::launch_half<true, true, false, PROG>(p, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out);   // same image, 4 - 20 % slower
+    return octree ? h16::launch_half<true, true, true, PROG>(p, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out)
+                  : h16::launch_half<false, true, false, PROG>(p, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out);
+}
+
 cudaError_t launch_render_half(const RenderLaunch &p, bool octree, const uint2 *geom_h, const uint2 *matl_h, const __half *cam_h,
                                const HalfPairs &hp, int sm_count, cudaStream_t st, int *blocks_out) {
     h16::PairView pv;
     pv.geom = hp.geom; pv.idx = hp.idx; pv.start = hp.start;
     h16::NodeTab nt;
     nt.ent = hp.nodes; nt.count = hp.node_count;
-    if (p.variant == 30)        // A/B: root evaluation inside the scan loop (the first cooperative form); same image
-        return octree ? h16::launch_half<true, false>(p, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out)
-                      : h16::launch_half<false, false>(p, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out);
-    if (p.variant == 33 && octree)      // A/B: the octree line tests as a per-lane walk (walk_cells_h) instead of by the whole warp per ray;
-        return h16::launch_half<true, true, false>(p, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out);   // same image, 4 - 20 % slower
-    return octree ? h16::launch_half<true, true, true>(p, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out)
-                  : h16::launch_half<false, true>(p, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out);
+    return p.accumulate || p.state_out ? launch_render_half_t<true>(p, octree, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out)
+                                       : launch_render_half_t<false>(p, octree, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out);
+}
+
+cudaError_t launch_finalize_half(const float *accum, float *fb, size_t count, int ns, cudaStream_t st) {
+    h16::k_finalize_h<<<(unsigned)((count + 255) / 256), 256, 0, st>>>(accum, fb, count, ns);
+    return cudaGetLastError();
 }
 
 // (re)build the pair lists of the USE_FP16 path: lists = 1 (flat mode) or kCells (octree mode)

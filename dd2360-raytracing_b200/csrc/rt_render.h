@@ -70,6 +70,8 @@ struct HalfPairs {            // candidate lists as transposed sphere pairs (rt_
 cudaError_t build_half_pairs(HalfPairs &hp, const uint2 *geom_h, const int *tag, int n, bool octree, const TreeView &tv, cudaStream_t st);
 cudaError_t launch_render_half(const RenderLaunch &p, bool octree, const uint2 *geom_h, const uint2 *matl_h, const __half *cam_h,
                                const HalfPairs &hp, int sm_count, cudaStream_t st, int *blocks_out);
+// fb = the USE_FP16 build's sqrt(accum / ns) on `count` half sums widened to float
+cudaError_t launch_finalize_half(const float *accum, float *fb, size_t count, int ns, cudaStream_t st);
 // ---- output_to_stream on the device (rt_ppm.cu) ----
 struct PpmWorkspace {
     uint32_t *block_len = nullptr;

@@ -23,7 +23,7 @@ import os
 
 import numpy as np
 
-from . import SHARD_NONE, SHARD_SPP, SHARD_TILES, RayTracer
+from . import PREC_FP16, PREC_FP32, SHARD_NONE, SHARD_SPP, SHARD_TILES, RayTracer
 
 TILE_W, TILE_H = 8, 4
 
@@ -125,18 +125,22 @@ class ShardedFrame:
 
 
 def render_sharded(rt: RayTracer, frame: ShardedFrame, ns: int, use_octree: bool, mode: int = SHARD_TILES, dist=None,
-                   want_stats: bool = True, to_host: bool = False):
+                   want_stats: bool = True, to_host: bool = False, precision: int = PREC_FP32):
     """Render this rank's shard, reduce-scatter the linear sums, finalise this rank's slice (and copy it to the shared host
     frame when `to_host`).  Everything is queued on the RayTracer's stream / torch's current stream; the caller
-    synchronises.  Returns the per-rank render stats (None without want_stats)."""
+    synchronises.  Returns the per-rank render stats (None without want_stats).  PREC_FP16 frames shard by tiles only:
+    spp shards would each hold the half sum of ns/G samples, a different image from the 1-GPU one."""
+    if precision == PREC_FP16 and mode == SHARD_SPP:
+        raise ValueError("USE_FP16 frames shard by tiles only (SHARD_TILES): spp shards' half sums do not add up to the 1-GPU frame")
     world, rank = frame.world, frame.rank
-    args = rt.args(frame.nx, frame.ny, ns, use_octree, shard_mode=mode if world > 1 else SHARD_NONE, shard_rank=rank, shard_count=world)
+    args = rt.args(frame.nx, frame.ny, ns, use_octree, shard_mode=mode if world > 1 else SHARD_NONE, shard_rank=rank, shard_count=world,
+                   precision=precision)
     # the render is queued WITHOUT waiting for its statistics, so that the collective, the finalise kernel and the copy are
     # queued right behind it (no host round trip in the middle of the frame); the statistics are read at the end
     world_sharded = world > 1
     st = rt.render_accumulate(args, frame.accum.data_ptr(), want_stats=want_stats and not world_sharded)
     reduce_scatter_frame(frame.accum, frame.slice, dist)
-    rt.finalize_n(frame.slice.data_ptr(), frame.slice.data_ptr(), frame.S, ns)
+    rt.finalize_ex(frame.slice.data_ptr(), frame.slice.data_ptr(), frame.S, ns, precision)
     if to_host and frame.host is not None and frame.end > frame.begin:
         frame.host.tensor[frame.begin:frame.end].copy_(frame.slice[: frame.end - frame.begin], non_blocking=True)
     if want_stats and world_sharded:
