@@ -331,10 +331,9 @@ class RayTracer:
     # -- render (main.cu:424-429) --
     @staticmethod
     def args(nx, ny, ns, use_octree, max_depth=50, shard_mode=SHARD_NONE, shard_rank=0, shard_count=1,
-             seed_mode=SEED_HEAD, precision=PREC_FP32, variant=0, max_rounds=0, tune=(0, 0), test_min=0) -> RenderArgs:
+             seed_mode=SEED_HEAD, precision=PREC_FP32, variant=0) -> RenderArgs:
         a = RenderArgs(nx, ny, ns, max_depth, int(bool(use_octree)), seed_mode, shard_mode, shard_rank, shard_count, precision)
-        # kernel A/B and tuning knobs (0 = defaults); they never change the image
-        a.tune[1], a.tune[2], a.tune[3], a.tune[4], a.tune[5] = variant, max_rounds, tune[0], tune[1], test_min
+        a.tune[1] = variant          # kernel variant for A/B runs and tests (0 = automatic); it never changes the image
         return a
 
     def render(self, nx, ny, ns, use_octree=True, **kw):

@@ -15,7 +15,7 @@ LIB = os.path.join(HERE, "librt_b200.so")
 LIB_COUNTERS = os.path.join(HERE, "librt_b200_counters.so")   # same code with -DRT_COUNTERS: work counters for the roofline
 CLI = os.path.join(HERE, "RayTracing")
 SOURCES = ["rt_abi.cu", "rt_render.cu", "rt_octree.cu", "rt_ppm.cu"]
-HEADERS = ["rt_math.cuh", "rt_types.h", "rt_shade.cuh", "rt_trace.cuh", "rt_pool.cuh", "rt_coop.cuh", "rt_xorwow_skip.h", "rt_half.cuh", "rt_render_half.cuh", "rt_build.cuh", "rt_octree.h", "rt_render.h",
+HEADERS = ["rt_math.cuh", "rt_types.h", "rt_shade.cuh", "rt_trace.cuh", "rt_coop.cuh", "rt_xorwow_skip.h", "rt_half.cuh", "rt_render_half.cuh", "rt_build.cuh", "rt_octree.h", "rt_render.h",
            os.path.join("..", "..", "include", "rt_abi.h")]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "--extended-lambda",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-ffp-contract=off", "-Wno-deprecated-gpu-targets"]

@@ -171,7 +171,6 @@ extern "C" const char *rt_kernel_name(int kernel_id) {
     switch (kernel_id) {
         case kKernelLane: return "k_render<octree> (pixel per lane, grid walk)";
         case kKernelListSweep: return "k_render<list> (N-test sweep)";
-        case kKernelPool: return "k_render_pool<64,6>";
         case kKernelCoop: return "k_render_coop (warp-cooperative candidate tests)";
         case kKernelHalf: return "k_render_h (USE_FP16)";
         default: return "none";
@@ -550,12 +549,6 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
     p.total_items = (uint32_t)(owned * 32);
     p.finalize = finalize ? 1 : 0;
     p.variant = a->tune[1] ? a->tune[1] : ctx->default_variant;
-    if (p.variant == 22) p.tree.walk_single = 1;         // A/B: one candidate per loop trip in the pixel-per-lane walk
-    if (p.variant == 21) p.tree.check_visibility = 0;   // MEASUREMENT ONLY: cost of the visibility rule (same image only when nothing was dropped)
-    p.tune_sticky = a->tune[3] > 0 ? a->tune[3] : 8;              // re-swept after the tile stock (profiles/sweep_tune.py): 8 / 16
-    p.tune_sticky_min = a->tune[4] > 0 ? a->tune[4] : 16;
-    p.tune_test_min = a->tune[5] > 0 ? a->tune[5] : (a->tune[5] < 0 ? 0 : 24);     // measured: C3 +2 %, C5 +6 % over 0 (profiles/sweep_test_min.py)
-    p.max_rounds = a->tune[2] > 0 ? (uint32_t)a->tune[2] : 0x7fffffffu;            // A/B measurement knob; every variant renders the same image
     p.out = out_dev;
     p.work_counter = ctx->work_counter;
     p.counters = ctx->counters;
@@ -617,12 +610,8 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
                          &ctx->last_kernel));
     }
     CK(cudaEventRecord(ctx->ev1, ctx->stream));
-    rt_render_stats local_stats;
-    // the pooled kernel's watchdog (a scheduling bug must never hang the GPU) truncates the frame when it trips: such a frame
-    // must fail the call whether or not the caller asked for statistics, so pooled launches always read the counters back
-    if (!stats && ctx->last_kernel == kKernelPool) stats = &local_stats;
     if (stats) {
-        unsigned long long c[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+        unsigned long long c[4] = {0, 0, 0, 0};
         CK(cudaMemcpyAsync(c, ctx->counters, sizeof c, cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaEventSynchronize(ctx->ev1));
         CK(cudaStreamSynchronize(ctx->stream));
@@ -630,10 +619,6 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
         stats->rays = c[0]; stats->paths = c[1];
         stats->sphere_tests = c[2]; stats->node_tests = c[3];   // zero unless built with -DRT_COUNTERS
         stats->kernel_id = ctx->last_kernel;
-        if (c[7]) {
-            return fail(ctx, RT_ERR_STATE, "render: scheduler watchdog tripped in %llu warps (w0|w1 %016llx, w2|rounds %016llx)",
-                        c[7], c[5], c[6]);
-        }
         float ms = 0;
         cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
         stats->kernel_ms = ms;
@@ -657,7 +642,7 @@ extern "C" int rt_xorwow_state(unsigned long long seed, unsigned long long subse
 extern "C" int rt_last_render_stats(rt_context *ctx, rt_render_stats *stats) {
     if (!ctx || !stats) return fail(ctx, RT_ERR_INVALID, "rt_last_render_stats: null argument");
     CK(cudaSetDevice(ctx->device));
-    unsigned long long c[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    unsigned long long c[4] = {0, 0, 0, 0};
     CK(cudaMemcpyAsync(c, ctx->counters, sizeof c, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     memset(stats, 0, sizeof *stats);
@@ -667,11 +652,10 @@ extern "C" int rt_last_render_stats(rt_context *ctx, rt_render_stats *stats) {
     stats->launches = 1;
     float ms = 0;
     if (cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1) == cudaSuccess) stats->kernel_ms = ms;
-    if (c[7]) return fail(ctx, RT_ERR_STATE, "render: scheduler watchdog tripped in %llu warps", c[7]);
     return RT_OK;
 }
 
-// test hook: the raw device counters of the last render (instrumented builds fill [8..27] with per-state scheduling data)
+// test hook: the raw device counters of the last render
 extern "C" int rt_debug_counters(rt_context *ctx, uint64_t out[32]) {
     if (!ctx || !out) return fail(ctx, RT_ERR_INVALID, "rt_debug_counters: null argument");
     CK(cudaSetDevice(ctx->device));

@@ -302,12 +302,13 @@ __device__ __forceinline__ Hit coop_trace_tree(WarpShared &ws, const SceneView &
     return h;
 }
 
-// PARK: the pixel state a lane does not need while its warp traces (RNG stream, attenuation, colour sum, pixel bookkeeping:
-// 16 words) waits in shared memory during coop_trace instead of being spilled to local memory by the register allocator.
-template <int MINB, int ITEMS, bool PARK>
-__global__ void __launch_bounds__(kRenderThreads, MINB) k_render_coop(const __grid_constant__ RenderLaunch p) {
+// The pixel state a lane does not need while its warp traces (RNG stream, attenuation, colour sum, pixel bookkeeping: 21 words)
+// is parked in shared memory during coop_trace instead of being spilled to local memory by the register allocator; that is
+// what lets 8 blocks per SM be resident (-9 % frame time over 6 blocks without parking, profiles r02r-r02t).
+template <int ITEMS>
+__global__ void __launch_bounds__(kRenderThreads, 8) k_render_coop(const __grid_constant__ RenderLaunch p) {
     __shared__ WarpShared wsh[kRenderThreads / 32];
-    __shared__ uint32_t park[PARK ? 21 : 1][kRenderThreads];
+    __shared__ uint32_t park[21][kRenderThreads];
     WarpShared &ws = wsh[threadIdx.x >> 5];
     const SceneView sc = p.scene;
     const unsigned lane = threadIdx.x & 31u;
@@ -358,7 +359,7 @@ __global__ void __launch_bounds__(kRenderThreads, MINB) k_render_coop(const __gr
             npaths++;
         }
         if (has) nrays++;
-        if (PARK) {
+        {
             const unsigned t = threadIdx.x;
             park[0][t] = rng.d; park[1][t] = rng.v0; park[2][t] = rng.v1; park[3][t] = rng.v2; park[4][t] = rng.v3; park[5][t] = rng.v4;
             park[6][t] = __float_as_uint(att.x); park[7][t] = __float_as_uint(att.y); park[8][t] = __float_as_uint(att.z);
@@ -368,7 +369,7 @@ __global__ void __launch_bounds__(kRenderThreads, MINB) k_render_coop(const __gr
         }
         __syncwarp();
         const Hit h = coop_trace_tree<ITEMS>(ws, sc, p.tree, &p.tree.planes[0][0], lane, has, o, d, tc);
-        if (PARK) {
+        {
             const unsigned t = threadIdx.x;
             rng.d = park[0][t]; rng.v0 = park[1][t]; rng.v1 = park[2][t]; rng.v2 = park[3][t]; rng.v3 = park[4][t]; rng.v4 = park[5][t];
             att = mk(__uint_as_float(park[6][t]), __uint_as_float(park[7][t]), __uint_as_float(park[8][t]));
@@ -455,24 +456,6 @@ __global__ void __launch_bounds__(kRenderThreads) k_trace_rays_coop(const __grid
     tc.sphere_tests = tc.node_tests = tc.voxel_steps = 0;
     const Hit h = coop_trace_tree<2>(wsh[threadIdx.x >> 5], p.scene, p.tree, &p.tree.planes[0][0], threadIdx.x & 31u, has, o, d, tc);
     if (has) { out_idx[i] = h.idx; out_t[i] = h.t; }
-}
-
-template <int MINB, int ITEMS, bool PARK = false>
-static cudaError_t launch_coop(const RenderLaunch &p, int sm_count, cudaStream_t st, int *blocks_out) {
-    auto kern = k_render_coop<MINB, ITEMS, PARK>;
-    int per_sm = 0;
-    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kRenderThreads, 0);
-    if (e != cudaSuccess) return e;
-    if (per_sm < 1) return cudaErrorLaunchOutOfResources;
-    long long blocks = (long long)per_sm * sm_count;       // persistent grid: exactly what is resident
-    const long long need = ((long long)p.total_items + kRenderThreads - 1) / kRenderThreads;
-    if (blocks > need) blocks = need < 1 ? 1 : need;
-    const uint32_t head = (uint32_t)(blocks * kRenderThreads);
-    e = cudaMemcpyAsync(p.work_counter, &head, 4, cudaMemcpyHostToDevice, st);   // queue head starts past the grid
-    if (e != cudaSuccess) return e;
-    kern<<<(unsigned)blocks, kRenderThreads, 0, st>>>(p);
-    if (blocks_out) *blocks_out = (int)blocks;
-    return cudaGetLastError();
 }
 
 }  // namespace coop

@@ -277,13 +277,29 @@ __global__ void __launch_bounds__(kRenderThreads, 6) k_render(const __grid_const
 #endif
 }
 
-}  // namespace rt
-namespace rt {
-#include "rt_pool.cuh"
-#include "rt_coop.cuh"
-}  // namespace rt
-namespace rt {
+// Persistent grid of a queue-fed render kernel: exactly the blocks that are resident, never more than there is work; the queue
+// head starts past the grid (the first tile of every warp needs no atomic).  `args` are the kernel's arguments.
+template <typename... Params, typename... Args>
+static cudaError_t launch_persistent(void (*kern)(Params...), size_t smem, const RenderLaunch &p, int sm_count, cudaStream_t st,
+                                     int *blocks_out, Args... args) {
+    cudaError_t e;
+    if (smem && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
+    int per_sm = 0;
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kRenderThreads, smem);
+    if (e != cudaSuccess) return e;
+    if (per_sm < 1) return cudaErrorLaunchOutOfResources;
+    long long blocks = (long long)per_sm * sm_count;
+    const long long need = ((long long)p.total_items + kRenderThreads - 1) / kRenderThreads;
+    if (blocks > need) blocks = need < 1 ? 1 : need;
+    const uint32_t head = (uint32_t)(blocks * kRenderThreads);
+    e = cudaMemcpyAsync(p.work_counter, &head, 4, cudaMemcpyHostToDevice, st);
+    if (e != cudaSuccess) return e;
+    kern<<<(unsigned)blocks, kRenderThreads, smem, st>>>(args...);
+    if (blocks_out) *blocks_out = (int)blocks;
+    return cudaGetLastError();
+}
 
+#include "rt_coop.cuh"
 #include "rt_render_half.cuh"
 
 cudaError_t launch_scene_to_half(const float4 *geom, const float4 *matl, int n, uint2 *geom_h, uint2 *matl_h, cudaStream_t st) {
@@ -296,26 +312,16 @@ cudaError_t launch_camera_setup_half(const float lookfrom[3], const float lookat
                                            vfov, nx, ny, aspect_override, aperture, focus_dist, cam_h);
     return cudaGetLastError();
 }
-template <bool PROG>
-static cudaError_t launch_render_half_t(const RenderLaunch &p, bool octree, const uint2 *geom_h, const uint2 *matl_h, const __half *cam_h,
-                                        const h16::PairView &pv, const h16::NodeTab &nt, int sm_count, cudaStream_t st, int *blocks_out) {
-    if (p.variant == 30)        // A/B: root evaluation inside the scan loop (the first cooperative form); same image
-        return octree ? h16::launch_half<true, false, false, PROG>(p, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out)
-                      : h16::launch_half<false, false, false, PROG>(p, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out);
-    if (p.variant == 33 && octree)      // A/B: the octree line tests as a per-lane walk (walk_cells_h) instead of by the whole warp per ray;
-        return h16::launch_half<true, true, false, PROG>(p, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out);   // same image, 4 - 20 % slower
-    return octree ? h16::launch_half<true, true, true, PROG>(p, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out)
-                  : h16::launch_half<false, true, false, PROG>(p, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out);
-}
-
 cudaError_t launch_render_half(const RenderLaunch &p, bool octree, const uint2 *geom_h, const uint2 *matl_h, const __half *cam_h,
                                const HalfPairs &hp, int sm_count, cudaStream_t st, int *blocks_out) {
     h16::PairView pv;
     pv.geom = hp.geom; pv.idx = hp.idx; pv.start = hp.start;
     h16::NodeTab nt;
     nt.ent = hp.nodes; nt.count = hp.node_count;
-    return p.accumulate || p.state_out ? launch_render_half_t<true>(p, octree, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out)
-                                       : launch_render_half_t<false>(p, octree, geom_h, matl_h, cam_h, pv, nt, sm_count, st, blocks_out);
+    const bool prog = p.accumulate || p.state_out;
+    auto kern = octree ? (prog ? h16::k_render_h<true, true> : h16::k_render_h<true, false>)
+                       : (prog ? h16::k_render_h<false, true> : h16::k_render_h<false, false>);
+    return launch_persistent(kern, 0, p, sm_count, st, blocks_out, p, geom_h, matl_h, cam_h, pv, nt);
 }
 
 cudaError_t launch_finalize_half(const float *accum, float *fb, size_t count, int ns, cudaStream_t st) {
@@ -453,81 +459,26 @@ cudaError_t launch_finalize(const float *accum, float *fb, int nx, int ny, int n
     return launch_finalize_n(accum, fb, (size_t)nx * ny * 3, ns, st);
 }
 
-template <bool OCTREE, bool GEOM_SMEM>
-static cudaError_t launch_variant(const RenderLaunch &p, size_t smem, int sm_count, cudaStream_t st, int *blocks_out) {
-    auto kern = k_render<OCTREE, GEOM_SMEM>;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    int per_sm = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kRenderThreads, smem);
-    if (e != cudaSuccess) return e;
-    if (per_sm < 1) return cudaErrorLaunchOutOfResources;
-    // persistent grid: exactly what is resident, never more blocks than there is work
-    long long blocks = (long long)per_sm * sm_count;
-    const long long need = ((long long)p.total_items + kRenderThreads - 1) / kRenderThreads;
-    if (blocks > need) blocks = need < 1 ? 1 : need;
-    RenderLaunch q = p;
-    const uint32_t head = (uint32_t)(blocks * kRenderThreads);
-    e = cudaMemcpyAsync(q.work_counter, &head, 4, cudaMemcpyHostToDevice, st);   // queue head starts past the grid
-    if (e != cudaSuccess) return e;
-    kern<<<(unsigned)blocks, kRenderThreads, smem, st>>>(q);
-    if (blocks_out) *blocks_out = (int)blocks;
-    return cudaGetLastError();
-}
-
 cudaError_t launch_render(const RenderLaunch &p, bool octree, int sm_count, size_t smem_limit, cudaStream_t st,
                           int *blocks_out, int *kernel_out) {
     int dummy;
     int &which = kernel_out ? *kernel_out : dummy;
     if (octree) {
-        // the pooled kernel packs depth into 8 bits and the sample number into 24 (rt_pool.cuh F_SD): outside that range the
-        // other kernels render the frame
-        // ... and it has no progressive state carry (state_out / accumulate)
-        const bool pool_ok = p.max_depth <= 255 && p.ns_local < (1 << 24) && !p.state_out && !p.accumulate;
-        which = kKernelPool;
-        switch (pool_ok ? p.variant : -1) {          // A/B measurement variants; all produce the same image
-            case 10: return pool::launch_pool<96, 4>(p, sm_count, st, blocks_out);
-            case 11: return pool::launch_pool<64, 6>(p, sm_count, st, blocks_out);
-            case 12: return pool::launch_pool<128, 3>(p, sm_count, st, blocks_out);
-            case 13: return pool::launch_pool<32, 8>(p, sm_count, st, blocks_out);
-            case 14: return pool::launch_pool<64, 4>(p, sm_count, st, blocks_out);
-            case 15: return pool::launch_pool<64, 5>(p, sm_count, st, blocks_out);
-            default: break;
-        }
-        which = kKernelCoop;
-        switch (p.variant) {
-            case 40: return coop::launch_coop<6, 2>(p, sm_count, st, blocks_out);
-            case 41: return coop::launch_coop<5, 2>(p, sm_count, st, blocks_out);
-            case 42: return coop::launch_coop<4, 2>(p, sm_count, st, blocks_out);
-            case 43: return coop::launch_coop<8, 2>(p, sm_count, st, blocks_out);
-            case 44: return coop::launch_coop<6, 1>(p, sm_count, st, blocks_out);     // one candidate per lane and chunk step
-            case 45: return coop::launch_coop<6, 4>(p, sm_count, st, blocks_out);     // four
-            case 46: return coop::launch_coop<5, 4>(p, sm_count, st, blocks_out);
-            case 47: return coop::launch_coop<6, 2, true>(p, sm_count, st, blocks_out);      // A/B: idle pixel state parked in shared memory
-            case 48: return coop::launch_coop<7, 2, true>(p, sm_count, st, blocks_out);
-            case 49: return coop::launch_coop<8, 2, true>(p, sm_count, st, blocks_out);
-            case 50: return coop::launch_coop<6, 4, true>(p, sm_count, st, blocks_out);
-            case 51: return coop::launch_coop<7, 4, true>(p, sm_count, st, blocks_out);
-            case 52: return coop::launch_coop<8, 4, true>(p, sm_count, st, blocks_out);
-            default: break;
-        }
         // automatic choice by scene size (measured on B200, profiles/README.md r02f): the pixel-per-lane walk for small scenes
         // (short candidate lists, many empty voxels: C2 2.3 vs 3.4 ms), the warp-cooperative kernel from kCoopMinSpheres on
-        // (C3 +8 %, C5 +19 % over the pooled kernel, which stays available as variants 10-15); variant 1 forces the per-lane walk
-        if (p.variant != 1 && p.scene.n >= kCoopMinSpheres) {
+        // (C3 +8 %, C5 +19 % over the pooled kernel it replaced); variant 40 forces the cooperative kernel, variant 1 the per-lane walk
+        if (p.variant == 40 || (p.variant != 1 && p.scene.n >= kCoopMinSpheres)) {
             which = kKernelCoop;
             // four candidates per lane once voxel lists are long (C5: 71 references per voxel, +4 %; C3: 13 per voxel, -6 %)
-            // (8 / 7 blocks per SM with the idle pixel state parked in shared memory: -9 % over 6 blocks without, profiles r02r-r02t)
-            if (p.coop_items == 4) return coop::launch_coop<8, 4, true>(p, sm_count, st, blocks_out);
-            return coop::launch_coop<8, 2, true>(p, sm_count, st, blocks_out);
+            return launch_persistent(p.coop_items == 4 ? coop::k_render_coop<4> : coop::k_render_coop<2>, 0, p, sm_count, st, blocks_out, p);
         }
         which = kKernelLane;
-        return launch_variant<true, false>(p, 0, sm_count, st, blocks_out);
+        return launch_persistent(k_render<true, false>, 0, p, sm_count, st, blocks_out, p);
     }
     which = kKernelListSweep;
     const size_t geom_bytes = (size_t)p.scene.n * sizeof(float4);
-    if (geom_bytes + 1024 <= smem_limit) return launch_variant<false, true>(p, geom_bytes, sm_count, st, blocks_out);
-    return launch_variant<false, false>(p, 0, sm_count, st, blocks_out);
+    if (geom_bytes + 1024 <= smem_limit) return launch_persistent(k_render<false, true>, geom_bytes, p, sm_count, st, blocks_out, p);
+    return launch_persistent(k_render<false, false>, 0, p, sm_count, st, blocks_out, p);
 }
 
 }  // namespace rt

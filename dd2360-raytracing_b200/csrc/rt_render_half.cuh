@@ -3,7 +3,7 @@
 //
 // Same persistent, queue-fed kernel shape as k_render (one pixel chain per lane, ballot/popc-compacted claims), with the
 // per-lane state in half: ray, attenuation and — as in the reference, whose `vec3 col` is three halves (main.cu:101) —
-// the pixel accumulator.  Octree mode walks the reference's own cells (rt_half.cuh coop_trace_h2): the sub-grid of the
+// the pixel accumulator.  Octree mode walks the reference's own cells (rt_half.cuh coop_trace_h): the sub-grid of the
 // FP32 path is built on float error bounds that half arithmetic does not honour.
 #pragma once
 // (rt_half.cuh is included by rt_render.cu at file scope)
@@ -153,16 +153,15 @@ __global__ void k_camera_setup_h(const float lfx, const float lfy, const float l
     out[21] = lens_radius;
 }
 
-// COOP2: closest hit by coop_trace_h2 (filter and roots in separate converged phases); false keeps coop_trace_h for A/B runs.
 // PROG: progressive calls (p.accumulate, p.state_out) get instances of their own: compiled into the whole-frame instances, the
 // two per-pixel branches cost 1.6 % of a C4 frame (2 602 vs 2 559 ms, B200 at 1000 W)
-template <bool OCTREE, bool COOP2, bool COOPN = false, bool PROG = false>
+template <bool OCTREE, bool PROG>
 __global__ void __launch_bounds__(kRenderThreads, 5)
 k_render_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geom_h, const uint2 *__restrict__ matl_h,
            const __half *__restrict__ cam_h, const PairView pv, const NodeTab nt) {
-    __shared__ CoopSmem coop_sm[COOP2 ? kRenderThreads / 32 : 1];
+    __shared__ CoopSmem coop_sm[kRenderThreads / 32];
     __shared__ hf planes_h[3 * kPlanes];      // the slab planes of the octree boxes, rounded to half as AABB's real_t members are
-    if (COOP2 && OCTREE && threadIdx.x < 3 * kPlanes) planes_h[threadIdx.x] = f2h((&p.tree.planes[0][0])[threadIdx.x]);
+    if (OCTREE && threadIdx.x < 3 * kPlanes) planes_h[threadIdx.x] = f2h((&p.tree.planes[0][0])[threadIdx.x]);
     __syncthreads();
     CameraH cam;
     {
@@ -171,7 +170,7 @@ k_render_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geo
         cam.lens_radius = cam_h[21];
     }
     const unsigned lane = threadIdx.x & 31u;
-    if (COOP2 && lane == 0) {
+    if (lane == 0) {
         coop_sm[threadIdx.x >> 5].tail = 0u;
         coop_sm[threadIdx.x >> 5].pairs_lo = coop_sm[threadIdx.x >> 5].pairs_hi = 0u;
     }
@@ -185,9 +184,6 @@ k_render_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geo
     uint32_t nrays = 0, npaths = 0;
     bool exhausted = false;
     uint32_t stock_next = gwarp * 32u, stock_end = stock_next + 32u;
-    // single pixels from the frame-wide queue: here the warp traces its lanes' rays one after the other, each a scan of
-    // ~2 000 candidates, so balance between warps matters and the tile stock measured 3 - 14 % slower (variant 32 = tiles)
-    const uint32_t batch = p.variant == 32 ? 32u : 1u;
     const hf nxh = f2h((float)p.nx), nyh = f2h((float)p.ny);
     const hf inv_ns = inv_ns_h(p.ns_total);
 
@@ -196,7 +192,9 @@ k_render_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geo
             const bool need = pix < 0 && !exhausted;
             const unsigned m = __ballot_sync(0xffffffffu, need);
             if (!m) break;
-            const uint32_t item = claim_items(p, m, lane, stock_next, stock_end, batch);   // per-warp tile stock (rt_render.cu)
+            // single pixels from the frame-wide queue (batch 1): here the warp traces its lanes' rays one after the other, each a
+            // scan of ~2 000 candidates, so balance between warps matters and the per-warp tile stock measured 3 - 14 % slower
+            const uint32_t item = claim_items(p, m, lane, stock_next, stock_end, 1u);
             if (need) {
                 if (item >= p.total_items) {
                     exhausted = true;
@@ -226,8 +224,7 @@ k_render_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geo
             nrays++;
         }
         // closest hit of every lane's ray, one ray at a time by the whole warp (rt_half.cuh coop_trace_h)
-        const HitH h = COOP2 ? coop_trace_h2<OCTREE, COOPN>(coop_sm[threadIdx.x >> 5], planes_h, pv, nt, geom_h, have, o, d)
-                             : coop_trace_h<OCTREE>(pv, nt, geom_h, p.tree, have, o, d);
+        const HitH h = coop_trace_h<OCTREE>(coop_sm[threadIdx.x >> 5], planes_h, pv, nt, geom_h, have, o, d);
         if (have) {
             bool sample_done = false;
             vec3h contrib = mkh(zero, zero, zero);
@@ -278,10 +275,8 @@ k_render_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geo
         atomicAdd(p.counters + 0, r64);
         atomicAdd(p.counters + 1, p64);
 #ifdef RT_COUNTERS
-        if (COOP2) {     // two spheres per pair (NaN padding pairs included: they are scanned too)
-            const CoopSmem &cs = coop_sm[threadIdx.x >> 5];
-            atomicAdd(p.counters + 2, 2ull * ((unsigned long long)cs.pairs_hi << 32 | cs.pairs_lo));
-        }
+        const CoopSmem &cs = coop_sm[threadIdx.x >> 5];     // two spheres per pair (NaN padding pairs included: they are scanned too)
+        atomicAdd(p.counters + 2, 2ull * ((unsigned long long)cs.pairs_hi << 32 | cs.pairs_lo));
 #endif
     }
 }
@@ -291,25 +286,6 @@ k_render_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geo
 __global__ void k_finalize_h(const float *__restrict__ accum, float *__restrict__ fb, size_t count, int ns) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < count) fb[i] = h2f(hsqrtf_(hmul_(f2h(accum[i]), inv_ns_h(ns))));
-}
-
-template <bool OCTREE, bool COOP2, bool COOPN, bool PROG>
-static cudaError_t launch_half(const RenderLaunch &p, const uint2 *geom_h, const uint2 *matl_h, const __half *cam_h, const PairView pv,
-                               const NodeTab nt, int sm_count, cudaStream_t st, int *blocks_out) {
-    auto kern = k_render_h<OCTREE, COOP2, COOPN, PROG>;
-    int per_sm = 0;
-    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kRenderThreads, 0);
-    if (e != cudaSuccess) return e;
-    if (per_sm < 1) return cudaErrorLaunchOutOfResources;
-    long long blocks = (long long)per_sm * sm_count;
-    const long long need = ((long long)p.total_items + kRenderThreads - 1) / kRenderThreads;
-    if (blocks > need) blocks = need < 1 ? 1 : need;
-    const uint32_t head = (uint32_t)(blocks * kRenderThreads);
-    e = cudaMemcpyAsync(p.work_counter, &head, 4, cudaMemcpyHostToDevice, st);
-    if (e != cudaSuccess) return e;
-    kern<<<(unsigned)blocks, kRenderThreads, 0, st>>>(p, geom_h, matl_h, cam_h, pv, nt);
-    if (blocks_out) *blocks_out = (int)blocks;
-    return cudaGetLastError();
 }
 
 }  // namespace h16

@@ -370,7 +370,7 @@ RT_HD Hit trace_walk(const SceneView &sc, const TreeView &tv, const float *plane
             // fewer than 2 can be the closest hit.  Two candidates per trip: their loads and filters are independent
             // (the second filter sees the closest hit as it was before the first candidate — a larger bound, still
             // conservative); the exact tests run in list order against the up-to-date bound.
-            const bool two = !tv.walk_single && k + 1 < e;
+            const bool two = k + 1 < e;
 #if defined(__CUDA_ARCH__)
             const float4 s0 = RT_LDG(g.ref_geom + k), s1 = RT_LDG(g.ref_geom + (two ? k + 1 : k));
 #else

@@ -39,7 +39,7 @@ struct GridView {
     int nx, ny, nz;             // 0 = no grid
     const uint2 *vox;           // {first reference, reference count} per voxel
     const uint32_t *refs;       // sphere indices, ascending inside a voxel
-    const float4 *ref_geom;     // geom[refs[k]] copied into list order: the pooled kernel streams candidates with ONE
+    const float4 *ref_geom;     // geom[refs[k]] copied into list order: the render kernels stream candidates with ONE
                                 // dependent load instead of two (16 B per reference; 96 MB at C3, 4.9 GB at C5)
 };
 
@@ -74,7 +74,6 @@ struct TreeView {
     int no_drops;               // 1: the build dropped no entry ("Leaf nodes full" never happened), so a cell stores every sphere
                                 //    whose centre its r-expanded box contains
     float cell_inv[3];          // 8 / root box extent per axis: cell index guess from a coordinate
-    int walk_single;            // A/B knob: 1 = the pixel-per-lane walk tests one candidate per loop trip instead of two
 };
 
 }  // namespace rt

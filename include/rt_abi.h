@@ -76,14 +76,10 @@ typedef struct rt_render_args {
     int32_t shard_rank, shard_count;
     int32_t precision;       /* RT_PREC_* (USE_FP16, precision_types.h:8); FP16 shards by tiles only (RT_SHARD_TILES: the summed
                               * half sums are the 1-GPU sums exactly; finalise them with rt_finalize_ex(.., RT_PREC_FP16)) */
-    int32_t tune[6];         /* kernel A/B and tuning knobs for measurements; 0 = defaults; they never change the image
-                              * (one documented exception, variant 21).  [1] kernel variant: 1 pixel-per-lane kernel, 10-15 pooled
-                              * kernel shapes, 40-52 warp-cooperative kernel shapes (blocks per SM, candidates per lane, parked pixel
-                              * state), 20 flat list as an N-test sweep, 21 visibility rule off (MEASUREMENT ONLY: same image
-                              * only when the build dropped nothing), 30 first cooperative USE_FP16 form, 31 / 32 single-pixel /
-                              * tile queue, 33 per-lane USE_FP16 node walk; [2] pooled-kernel watchdog (scheduling rounds);
-                              * [3], [4] TEST chunks per round and the lane count that keeps a round going; [5] TEST hold-back
-                              * threshold (-1 = off); [0] unused */
+    int32_t tune[6];         /* kernel A/B knobs for measurements and tests; 0 = defaults; they never change the image.
+                              * [1] kernel variant: 0 automatic, 1 pixel-per-lane kernel (and per-lane rt_trace_rays), 20 flat
+                              * list as an N-test sweep, 31 single-pixel queue, 40 warp-cooperative kernel; other values select
+                              * the automatic choice.  [0], [2..5] reserved (ignored) */
 } rt_render_args;
 
 typedef struct rt_render_stats {
@@ -147,8 +143,7 @@ size_t rt_octree_debug_read(rt_context *ctx, int which, void *host, size_t cap);
 int rt_xorwow_state(unsigned long long seed, unsigned long long subsequence, uint32_t out6[6]);
 
 /* test hook: raw device counters of the last render call.  [0] rays, [1] paths; RT_COUNTERS builds add [2] sphere tests,
- * [3] visibility line tests, [4] voxel steps and, for the pooled kernel, [8+s] scheduling rounds and [18+s] contexts
- * processed per state s. */
+ * [3] visibility line tests and [4] voxel steps. */
 int rt_debug_counters(rt_context *ctx, uint64_t out[32]);
 
 /* test hook: closest hit (sphere index or -1, and t) of n caller-supplied rays — hitTree / hitable_list::hit per ray */

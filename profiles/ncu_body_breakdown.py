@@ -1,19 +1,18 @@
-r"""Attribute the SASS of the pooled render kernel to its bodies: walk the instructions in address order and assign each to
-the function of rt_pool.cuh whose source line was seen last (inlined rt_math/rt_shade/rt_trace code inherits it).
+r"""Attribute the SASS of a render kernel to its device functions: walk the instructions in address order and assign each to
+the function of the source file whose source line was seen last (inlined rt_math/rt_shade/rt_trace code inherits it).
 usage: python profiles/ncu_body_breakdown.py file.ncu-rep [source-file-in-csrc function-regex start-body]
-       (defaults: rt_pool.cuh and its body functions; for the USE_FP16 kernel:
-        rt_half.cuh 'coop_\w+|node_pass_h|ref_line_test_h|sphere_test_h|scatter_h|camera_ray_h|hit_point_h|sky_h|random_in_unit_sphere_h|best_update' k_render_h)"""
+       (defaults: the USE_FP16 kernel, rt_half.cuh and its device functions)"""
 import csv
 import re
 import subprocess
 import sys
 
 src = sys.argv[1]
-SRC_FILE = sys.argv[2] if len(sys.argv) > 2 else 'rt_pool.cuh'
-FUNCS = sys.argv[3] if len(sys.argv) > 3 else r'body_\w+|gen_sample|begin_walk|maybe_hit|load_voxel|end_walk|rewalk_checked|k_render_pool'
-START = sys.argv[4] if len(sys.argv) > 4 else 'k_render_pool'
+SRC_FILE = sys.argv[2] if len(sys.argv) > 2 else 'rt_half.cuh'
+FUNCS = sys.argv[3] if len(sys.argv) > 3 else r'coop_\w+|ref_line_test_h|sphere_test_h|scatter_h|camera_ray_h|hit_point_h|sky_h|random_in_unit_sphere_h|best_update'
+START = sys.argv[4] if len(sys.argv) > 4 else 'k_render_h'
 pool_src = open(__file__.rsplit('/', 2)[0] + '/dd2360-raytracing_b200/csrc/' + SRC_FILE).read().splitlines()
-# line -> enclosing function name in rt_pool.cuh
+# line -> enclosing function name in SRC_FILE
 func_of, cur = {}, 'header'
 for i, l in enumerate(pool_src, 1):
     m = re.search(r'\b(' + FUNCS + r')\b\s*\(', l)

@@ -32,12 +32,4 @@ if len(sys.argv) > 4 and sys.argv[4] == "counters":
     st = rti.render_device(rti.args(nx, ny, 1, octree, variant=variant), fb.data_ptr())
     print("counters (1 spp): sphere_tests/ray", round(st["sphere_tests"] / st["rays"], 2), "visibility line tests/ray",
           round(st["node_tests"] / st["rays"], 3), "rays/path", round(st["rays"] / st["paths"], 3))
-    dc = rti.debug_counters()
-    names = ["TEST", "CAND", "ENTER", "STEP", "END", "DIFF", "DIEL", "SAMPLE", "DONE", "-"]
-    if dc[8:18].sum():
-        print("pool scheduler, per state: rounds/kray, contexts/round, visits/ray")
-        for s_, nm in enumerate(names):
-            r_, c_ = int(dc[8 + s_]), int(dc[18 + s_])
-            if r_:
-                print(f"  {nm:7s} {1e3 * r_ / st['rays']:8.2f} {c_ / r_:6.2f} {c_ / st['rays']:7.3f}")
     rti.close()

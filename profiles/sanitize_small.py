@@ -5,7 +5,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import __graft_entry__ as entry
 pkg = entry.load_package()
 rt = pkg.RayTracer(0)
-for n, spl, nx, ny, ns, variants in ((8000, 30, 64, 40, 2, (0, 40, 45, 1, 11)), (100000, 300, 48, 27, 1, (0, 45))):
+for n, spl, nx, ny, ns, variants in ((8000, 30, 64, 40, 2, (0, 40, 1)), (100000, 300, 48, 27, 1, (0, 1))):
     rt.create_world(n, 0.1)
     rt.build_octree(spl)
     ref = None

@@ -1,4 +1,4 @@
-"""k_render (variant 1) against k_render_coop (variant 40) and k_render_pool (variant 11) over the sphere count.
+"""k_render (variant 1) against k_render_coop (variant 40) over the sphere count.
     python profiles/sweep_coop_threshold.py [nx ny spp]"""
 import os
 import sys
@@ -20,9 +20,8 @@ for n in (488, 2000, 8000, 20000, 50000, 100000, 300000, 1000000):
     rt.build_octree(spl)
     rt.set_camera(nx, ny)
     out = []
-    for v in (1, 40, 11):
+    for v in (1, 40):
         best = min(rt.render_device(rt.args(nx, ny, ns if n < 1000000 else 2, True, variant=v), fb.data_ptr())["kernel_ms"] for _ in range(2))
         out.append(best)
-    print(f"n={n}: k_render {out[0]:.2f} ms, k_render_coop {out[1]:.2f} ms, k_render_pool {out[2]:.2f} ms; coop/lane speed {out[0] / out[1]:.2f}x, "
-          f"coop/pool {out[2] / out[1]:.2f}x", flush=True)
+    print(f"n={n}: k_render {out[0]:.2f} ms, k_render_coop {out[1]:.2f} ms; coop/lane speed {out[0] / out[1]:.2f}x", flush=True)
 rt.close()

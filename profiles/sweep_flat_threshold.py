@@ -1,4 +1,4 @@
-"""From how many spheres do flat voxels and the cooperative kernel pay?  k_render (variant 1) and k_render_coop (variant 43) on
+"""From how many spheres do flat voxels and the cooperative kernel pay?  k_render (variant 1) and k_render_coop (variant 40) on
 cubic and flat voxels over the sphere count.
     python profiles/sweep_flat_threshold.py [nx ny spp]"""
 import os
@@ -23,8 +23,8 @@ for n in (2000, 5000, 10000, 20000, 30000, 50000, 100000):
         rt.create_world(n, 0.1)
         rt.build_octree(spl)
         rt.set_camera(nx, ny)
-        for v in (1, 43):
+        for v in (1, 40):
             out[(shape, v)] = min(rt.render_device(rt.args(nx, ny, ns, True, variant=v), fb.data_ptr())["kernel_ms"] for _ in range(3))
         rt.close()
-    print(f"n={n}: k_render cubic {out[('1:1:1', 1)]:.2f} flat {out[('1.5:0.75:1', 1)]:.2f} ms; k_render_coop cubic {out[('1:1:1', 43)]:.2f} "
-          f"flat {out[('1.5:0.75:1', 43)]:.2f} ms", flush=True)
+    print(f"n={n}: k_render cubic {out[('1:1:1', 1)]:.2f} flat {out[('1.5:0.75:1', 1)]:.2f} ms; k_render_coop cubic {out[('1:1:1', 40)]:.2f} "
+          f"flat {out[('1.5:0.75:1', 40)]:.2f} ms", flush=True)

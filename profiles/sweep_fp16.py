@@ -1,6 +1,6 @@
 """A/B of the USE_FP16 render kernel (k_render_h) on the C4 scene; every variant must reproduce the first one's frame.
     python profiles/sweep_fp16.py [nx] [ny] [spp] [v1,v2,...] [n_spheres] [octree]
-variant 0 = default (filter / root phases, coop_trace_h2), 30 = roots inside the scan loop (coop_trace_h)."""
+The USE_FP16 path has one kernel form (variant 0); an A/B partner gets a variant number of its own."""
 import os
 import sys
 
@@ -12,7 +12,7 @@ import __graft_entry__ as entry
 nx = int(sys.argv[1]) if len(sys.argv) > 1 else 960
 ny = int(sys.argv[2]) if len(sys.argv) > 2 else 540
 ns = int(sys.argv[3]) if len(sys.argv) > 3 else 4
-variants = [int(x) for x in sys.argv[4].split(",")] if len(sys.argv) > 4 else [0, 30]
+variants = [int(x) for x in sys.argv[4].split(",")] if len(sys.argv) > 4 else [0]
 n = int(sys.argv[5]) if len(sys.argv) > 5 else 100000
 octree = int(sys.argv[6]) if len(sys.argv) > 6 else 1
 spl = 300 if n > 10000 else 30

@@ -12,7 +12,7 @@ from bench import CONFIGS
 cfg = sys.argv[1] if len(sys.argv) > 1 else "C3"
 n, spl, octree, nx, ny, ns, desc = CONFIGS[cfg]
 ns = int(sys.argv[2]) if len(sys.argv) > 2 else 8
-variants = [int(x) for x in sys.argv[3].split(",")] if len(sys.argv) > 3 else [0, 10, 11, 12, 13, 14]
+variants = [int(x) for x in sys.argv[3].split(",")] if len(sys.argv) > 3 else [0, 1, 31, 40]
 pkg = entry.load_package()
 rt = pkg.RayTracer(0)
 rt.create_world(n, 0.1)
@@ -24,7 +24,7 @@ for v in variants:
     for k in range(3):
         fb.zero_()
         try:
-            st = rt.render_device(rt.args(nx, ny, ns, octree, variant=v, max_rounds=int(os.environ.get("RT_MAX_ROUNDS", "0"))), fb.data_ptr())
+            st = rt.render_device(rt.args(nx, ny, ns, octree, variant=v), fb.data_ptr())
         except Exception as ex:
             print("variant", v, "FAILED:", ex, flush=True)
             break

@@ -106,11 +106,11 @@ PROGRESSIVE_CASES = [   # n, spl, octree, nx, ny, seed_mode, variant
     (8000, 30, True, 120, 80, 0, 0),
     (100000, 300, True, 192, 108, 0, 0),
     (8000, 30, True, 120, 80, 1, 0),          # upstream seeding: the stored states continue the skip-ahead streams
-    (488, 30, True, 96, 64, 0, 30),           # the first cooperative USE_FP16 form
+    (488, 30, True, 96, 64, 0, 30),           # 30, 32, 33: retired USE_FP16 variant numbers, which select the automatic kernel
     (488, 30, False, 40, 24, 0, 30),
-    (8000, 30, True, 120, 80, 0, 32),         # the per-warp tile stock instead of the single-pixel queue
+    (8000, 30, True, 120, 80, 0, 32),
     (488, 30, False, 40, 24, 0, 32),
-    (8000, 30, True, 120, 80, 0, 33),         # the per-lane node walk (octree only)
+    (8000, 30, True, 120, 80, 0, 33),
 ]
 
 
@@ -149,7 +149,7 @@ SHARD_CASES = [   # n, spl, octree, nx, ny, variant, whether rank 1 renders its 
     (488, 30, False, 40, 24, 0, False),
     (8000, 30, True, 120, 80, 0, False),
     (100000, 300, True, 192, 108, 0, True),
-    (8000, 30, True, 120, 80, 32, False),
+    (8000, 30, True, 120, 80, 32, False),     # 32: a retired variant number, which selects the automatic kernel
     (488, 30, False, 44, 26, 32, False),      # not a multiple of the 8x4 tile
 ]
 

@@ -149,7 +149,7 @@ def test_render_matches_reference_cuda_goldens(rt, pkg, golden_dir):
 @pytest.mark.parametrize("n,spl,octree,nx,ny,ns", [
     (488, 30, True, 240, 160, 4),
     (488, 30, False, 96, 64, 2),
-    (100000, 300, True, 192, 108, 2),    # pooled kernel
+    (100000, 300, True, 192, 108, 2),    # cooperative kernel
 ])
 def test_upstream_seeding_matches_oracle(rt, pkg, O, golden_dir, n, spl, octree, nx, ny, ns):
     """RT_SEED_UPSTREAM = curand_init(1984, pixel_index, 0) (main.cu:90): per-pixel states from the library's own
@@ -480,26 +480,27 @@ def test_cli_modes_write_the_reference_image(pkg, golden_dir, tmp_path):
     (488, 30, 37, 23, 5),                # big spheres in the prolog list, image not a multiple of the tile
 ])
 def test_pooled_kernel_matches_oracle(rt, O, n, spl, nx, ny, ns):
-    """k_render_pool forced (variant 11; the automatic choice keeps it for scenes from 200 k spheres on big frames) against the oracle."""
+    """The scenes that held the retired pooled kernel to the oracle, rendered by k_render_coop forced (variant 40; the automatic
+    choice takes it from 40 k spheres on)."""
     rt.create_world(n, 0.1)
     rt.build_octree(spl)
     sph, _ = O.create_world(n)
     blob, _ = O.build_octree(sph, spl)
-    fb, s = rt.render(nx, ny, ns, use_octree=True, variant=11)
+    fb, s = rt.render(nx, ny, ns, use_octree=True, variant=40)
     ref, _, ctr = O.render(sph, O.camera(nx, ny, O.ARITH_DEVICE), O.make_params(nx, ny, ns, True, spl, O.ARITH_DEVICE), blob)
     assert _frac_identical(fb, ref) >= 1 - POWF_ALLOWANCE
     assert abs(int(s["rays"]) - ctr["rays"]) <= max(2, int(POWF_ALLOWANCE * ctr["rays"])) and s["paths"] == nx * ny * ns
 
 
 def test_pooled_and_plain_kernels_agree_at_4k(rt):
-    """Config 3 scene at 3840x2160 (two-tile claims per warp in the pooled kernel, tile claims in the plain one, single-pixel
-    claims with variant 31): the same frame from k_render_pool (variant 11), k_render (variant 1) and the pixel queue."""
+    """Config 3 scene at 3840x2160 (tile claims per warp, single-pixel claims with variant 31): the same frame from
+    k_render_coop (variant 40, in place of the retired pooled kernel), k_render (variant 1) and the pixel queue."""
     import torch
     nx, ny = 3840, 2160
     rt.create_world(100000, 0.1)
     rt.build_octree(300)
     fbs = []
-    for v in (11, 1, 31):
+    for v in (40, 1, 31):
         fb = torch.empty((ny, nx, 3), dtype=torch.float32, device="cuda")
         st = rt.render_device(rt.args(nx, ny, 1, True, variant=v), fb.data_ptr())
         fbs.append((fb, st["rays"]))

@@ -20,7 +20,7 @@ def rt(pkg):
     (488, 30, False, 40, 24, 0, 0),
     (8000, 30, True, 120, 80, 0, 1),        # the pixel-per-lane kernel
     (8000, 30, True, 120, 80, 1, 0),        # upstream seeding: the stored states continue the skip-ahead streams
-    (100000, 300, True, 192, 108, 0, 11),   # the pooled kernel has no state carry: progressive calls take the other kernels
+    (100000, 300, True, 192, 108, 0, 11),   # 11 (the retired pooled kernel) selects the automatic choice: the cooperative kernel
 ])
 def test_progressive_calls_equal_one_shot(rt, pkg, n, spl, octree, nx, ny, seed_mode, variant):
     """k calls of m samples == one k*m-sample render: linear sums, final frame and stream states, bit for bit —
@@ -81,12 +81,10 @@ def test_stats_name_the_kernel_that_ran(rt, pkg):
     rt.build_octree(30)
     _, s = rt.render(64, 40, 1, use_octree=True, variant=1)
     assert s["kernel"].startswith("k_render<octree>")
-    _, s = rt.render(64, 40, 1, use_octree=True, variant=11)
-    assert s["kernel"].startswith("k_render_pool")
     _, s = rt.render(64, 40, 1, use_octree=True, variant=40)
     assert s["kernel"].startswith("k_render_coop")
-    _, s = rt.render(64, 40, 1, use_octree=True, variant=11, max_depth=300)      # outside the pooled kernel's packed depth field
-    assert not s["kernel"].startswith("k_render_pool")
+    _, s = rt.render(64, 40, 1, use_octree=True, variant=11)      # a retired variant number: the automatic choice for 488 spheres
+    assert s["kernel"].startswith("k_render<octree>")
 
 
 def test_cooperative_and_per_lane_kernels_agree(rt):
