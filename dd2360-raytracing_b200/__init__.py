@@ -38,7 +38,8 @@ SPHERE_DTYPE = np.dtype(
 ABI_SYMBOLS = [
     "rt_abi_version", "rt_create", "rt_destroy", "rt_last_error", "rt_set_stream", "rt_device_info",
     "rt_scene_generate", "rt_scene_generate_ex", "rt_scene_upload", "rt_scene_download", "rt_scene_size", "rt_camera_set", "rt_camera_get", "rt_camera_get_half",
-    "rt_octree_build", "rt_octree_build_ex", "rt_octree_reference_bytes", "rt_octree_export_reference", "rt_octree_debug_read", "rt_xorwow_state", "rt_debug_counters", "rt_trace_rays", "rt_camera_get_rays", "rt_scatter_rays",
+    "rt_octree_build", "rt_octree_build_ex", "rt_octree_reference_bytes", "rt_octree_reference_bytes_ex", "rt_octree_export_reference", "rt_octree_debug_read", "rt_xorwow_state", "rt_debug_counters", "rt_trace_rays", "rt_camera_get_rays", "rt_scatter_rays",
+    "rt_trace_rays_ex", "rt_camera_get_rays_ex", "rt_scatter_rays_ex",
     "rt_render_accumulate", "rt_last_render_stats", "rt_render_progressive", "rt_finalize", "rt_finalize_n", "rt_finalize_ex", "rt_render", "rt_render_to_host", "rt_format_ppm",
     "rt_ppm_format", "rt_ppm_read", "rt_render_to_ppm",
     "rt_ffma_peak", "rt_hfma2_peak", "rt_malloc", "rt_free", "rt_memcpy_to_host", "rt_synchronize", "rt_kernel_name",
@@ -114,6 +115,7 @@ def load_library(path: str | None = None) -> C.CDLL:
         "rt_octree_build": (i32, [vp, i32, C.POINTER(OctreeStats)]),
         "rt_octree_build_ex": (i32, [vp, i32, i32, C.POINTER(OctreeStats)]),
         "rt_octree_reference_bytes": (sz, [i32]),
+        "rt_octree_reference_bytes_ex": (sz, [i32, i32]),
         "rt_octree_export_reference": (i32, [vp, vp, sz]),
         "rt_octree_debug_read": (sz, [vp, i32, vp, sz]),
         "rt_xorwow_state": (i32, [C.c_uint64, C.c_uint64, vp]),
@@ -121,6 +123,9 @@ def load_library(path: str | None = None) -> C.CDLL:
         "rt_trace_rays": (i32, [vp, i32, i32, vp, vp, vp, vp]),
         "rt_camera_get_rays": (i32, [vp, i32, vp, vp, vp, vp, vp]),
         "rt_scatter_rays": (i32, [vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
+        "rt_trace_rays_ex": (i32, [vp, i32, i32, i32, vp, vp, vp, vp]),
+        "rt_camera_get_rays_ex": (i32, [vp, i32, i32, vp, vp, vp, vp, vp]),
+        "rt_scatter_rays_ex": (i32, [vp, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
         "rt_render_accumulate": (i32, [vp, C.POINTER(RenderArgs), vp, C.POINTER(RenderStats)]),
         "rt_last_render_stats": (i32, [vp, C.POINTER(RenderStats)]),
         "rt_render_progressive": (i32, [vp, C.POINTER(RenderArgs), vp, vp, i32, C.POINTER(RenderStats)]),
@@ -200,6 +205,7 @@ class RayTracer:
         self.device = device
         self.n = 0
         self.spl = None
+        self.octree_precision = PREC_FP32
 
     # -- plumbing --
     def _ck(self, rc: int, what: str):
@@ -268,10 +274,12 @@ class RayTracer:
         st = OctreeStats()
         self._ck(self.L.rt_octree_build_ex(self._ctx, spheres_per_leaf, precision, C.byref(st)), "rt_octree_build_ex")
         self.spl = spheres_per_leaf
+        self.octree_precision = precision
         return st.as_dict()
 
     def export_octree(self) -> np.ndarray:
-        n = self.L.rt_octree_reference_bytes(self.spl)
+        """The tree in the reference's Octree layout; a tree built with PREC_FP16 in the USE_FP16 one (48-byte nodes)."""
+        n = self.L.rt_octree_reference_bytes_ex(self.spl, self.octree_precision)
         blob = np.zeros(n, dtype=np.uint8)
         self._ck(self.L.rt_octree_export_reference(self._ctx, blob.ctypes.data, n), "rt_octree_export_reference")
         return blob
@@ -295,37 +303,41 @@ class RayTracer:
         self._ck(self.L.rt_debug_counters(self._ctx, out.ctypes.data), "rt_debug_counters")
         return out
 
-    def trace_rays(self, origins: np.ndarray, dirs: np.ndarray, use_octree: bool):
-        """Test hook: closest hit per ray -> (idx[n] int32, t[n] float32)."""
+    def trace_rays(self, origins: np.ndarray, dirs: np.ndarray, use_octree: bool, precision: int = PREC_FP32):
+        """Test hook: closest hit per ray -> (idx[n] int32, t[n] float32).  PREC_FP16: the USE_FP16 build's hitTree /
+        hitable_list::hit (inputs rounded to half, t a half widened to float, +inf on a miss)."""
         o = np.ascontiguousarray(origins, dtype=np.float32)
         d = np.ascontiguousarray(dirs, dtype=np.float32)
         n = len(o)
         idx = np.zeros(n, dtype=np.int32)
         t = np.zeros(n, dtype=np.float32)
-        self._ck(self.L.rt_trace_rays(self._ctx, int(use_octree), n, o.ctypes.data, d.ctypes.data, idx.ctypes.data, t.ctypes.data),
-                 "rt_trace_rays")
+        self._ck(self.L.rt_trace_rays_ex(self._ctx, int(use_octree), precision, n, o.ctypes.data, d.ctypes.data, idx.ctypes.data,
+                                         t.ctypes.data), "rt_trace_rays_ex")
         return idx, t
 
-    def camera_rays(self, s: np.ndarray, t: np.ndarray, states: np.ndarray):
-        """camera::get_ray for n (s, t) pairs; `states` [n, 6] uint32 is advanced in place.  Returns (org[n,3], dir[n,3])."""
+    def camera_rays(self, s: np.ndarray, t: np.ndarray, states: np.ndarray, precision: int = PREC_FP32):
+        """camera::get_ray for n (s, t) pairs; `states` [n, 6] uint32 is advanced in place.  Returns (org[n,3], dir[n,3]).
+        PREC_FP16: with the USE_FP16 build's camera, s and t rounded to half, rays as halves widened to float."""
         s = np.ascontiguousarray(s, dtype=np.float32); t = np.ascontiguousarray(t, dtype=np.float32)
         assert states.dtype == np.uint32 and states.flags.c_contiguous and states.shape == (len(s), 6)
         org = np.zeros((len(s), 3), np.float32); d = np.zeros((len(s), 3), np.float32)
-        self._ck(self.L.rt_camera_get_rays(self._ctx, len(s), s.ctypes.data, t.ctypes.data, states.ctypes.data, org.ctypes.data, d.ctypes.data),
-                 "rt_camera_get_rays")
+        self._ck(self.L.rt_camera_get_rays_ex(self._ctx, precision, len(s), s.ctypes.data, t.ctypes.data, states.ctypes.data, org.ctypes.data,
+                                              d.ctypes.data), "rt_camera_get_rays_ex")
         return org, d
 
-    def scatter_rays(self, idx: np.ndarray, org: np.ndarray, dirs: np.ndarray, t_hit: np.ndarray, states: np.ndarray):
-        """material::scatter for n hits; returns dict(p, normal, dir, atten, scattered); `states` advanced in place."""
+    def scatter_rays(self, idx: np.ndarray, org: np.ndarray, dirs: np.ndarray, t_hit: np.ndarray, states: np.ndarray,
+                     precision: int = PREC_FP32):
+        """material::scatter for n hits; returns dict(p, normal, dir, atten, scattered); `states` advanced in place.
+        PREC_FP16: the USE_FP16 build's hit record and scatter (inputs rounded to half, outputs halves widened to float)."""
         idx = np.ascontiguousarray(idx, dtype=np.int32); org = np.ascontiguousarray(org, dtype=np.float32)
         dirs = np.ascontiguousarray(dirs, dtype=np.float32); t_hit = np.ascontiguousarray(t_hit, dtype=np.float32)
         n = len(idx)
         assert states.dtype == np.uint32 and states.flags.c_contiguous and states.shape == (n, 6)
         out = {k: np.zeros((n, 3), np.float32) for k in ("p", "normal", "dir", "atten")}
         out["scattered"] = np.zeros(n, np.int32)
-        self._ck(self.L.rt_scatter_rays(self._ctx, n, idx.ctypes.data, org.ctypes.data, dirs.ctypes.data, t_hit.ctypes.data, states.ctypes.data,
-                                        out["p"].ctypes.data, out["normal"].ctypes.data, out["dir"].ctypes.data, out["atten"].ctypes.data,
-                                        out["scattered"].ctypes.data), "rt_scatter_rays")
+        self._ck(self.L.rt_scatter_rays_ex(self._ctx, precision, n, idx.ctypes.data, org.ctypes.data, dirs.ctypes.data, t_hit.ctypes.data,
+                                           states.ctypes.data, out["p"].ctypes.data, out["normal"].ctypes.data, out["dir"].ctypes.data,
+                                           out["atten"].ctypes.data, out["scattered"].ctypes.data), "rt_scatter_rays_ex")
         return out
 
     # -- render (main.cu:424-429) --

@@ -449,11 +449,20 @@ extern "C" int rt_octree_build_ex(rt_context *ctx, int spl, int precision, rt_oc
 
 extern "C" size_t rt_octree_reference_bytes(int spl) { return OctreeBuilder::reference_bytes(spl); }
 
+extern "C" size_t rt_octree_reference_bytes_ex(int spl, int precision) {
+    if (spl < 1 || (precision != RT_PREC_FP32 && precision != RT_PREC_FP16)) return 0;
+    return OctreeBuilder::reference_bytes(spl, precision == RT_PREC_FP16);
+}
+
 extern "C" int rt_octree_export_reference(rt_context *ctx, void *host_blob, size_t bytes) {
     if (!ctx || !host_blob) return RT_ERR_INVALID;
     if (!ctx->octree->built) return fail(ctx, RT_ERR_STATE, "rt_octree_export_reference: build the octree first");
-    if (ctx->octree->fp16)
-        return fail(ctx, RT_ERR_UNSUPPORTED, "rt_octree_export_reference: the USE_FP16 Octree layout (48-byte nodes) is not exported");
+    if (ctx->octree->fp16) {      // the USE_FP16 AABB holds the planes as halves: they must be exact there (k_blob_nodes)
+        const float *pl = &ctx->octree->planes.p[0][0];
+        for (int k = 0; k < 3 * kPlanes; k++)
+            if (__half2float(__float2half_rn(pl[k])) != pl[k])
+                return fail(ctx, RT_ERR_UNSUPPORTED, "rt_octree_export_reference: box plane %g is not exact in half", (double)pl[k]);
+    }
     CK(cudaSetDevice(ctx->device));
     CK(ctx->octree->export_reference(ctx->stream, host_blob, bytes));
     return RT_OK;
@@ -463,6 +472,31 @@ extern "C" size_t rt_octree_debug_read(rt_context *ctx, int which, void *host, s
     if (!ctx) return 0;
     cudaSetDevice(ctx->device);
     return ctx->octree->debug_read(ctx->stream, which, host, cap);
+}
+
+// ---- USE_FP16 state -------------------------------------------------------------------------------------------------
+// What the half kernels read, derived on demand and kept until the scene, the tree or the frame size changes: always the scene
+// rounded to half; with kHalfPairs the pair lists of one mode (octree: the cells of `tv`; flat: all spheres); with kHalfCamera
+// the half camera of an nx x ny frame.  The render and the per-ray entry points share it.
+enum { kHalfPairs = 1, kHalfCamera = 2 };
+static int ensure_half(rt_context *ctx, unsigned what, bool octree, const TreeView &tv, int nx, int ny) {
+    if (ctx->half_cap < (size_t)ctx->n) {
+        cudaFree(ctx->geom_h); cudaFree(ctx->matl_h);
+        ctx->geom_h = ctx->matl_h = nullptr; ctx->half_cap = 0;
+        CK(cudaMalloc(&ctx->geom_h, (size_t)ctx->n * sizeof(uint2)));
+        CK(cudaMalloc(&ctx->matl_h, (size_t)ctx->n * sizeof(uint2)));
+        ctx->half_cap = (size_t)ctx->n;
+        ctx->half_valid = false;
+    }
+    if (!ctx->half_valid) {
+        CK(launch_scene_to_half(ctx->geom, ctx->matl, ctx->n, ctx->geom_h, ctx->matl_h, ctx->stream));
+        ctx->half_valid = true;
+        ctx->half_pairs.valid = false;
+    }
+    if ((what & kHalfPairs) && (!ctx->half_pairs.valid || ctx->half_pairs.octree != octree))
+        CK(build_half_pairs(ctx->half_pairs, ctx->geom_h, ctx->tag, ctx->n, octree, tv, ctx->stream));
+    if (what & kHalfCamera) return ensure_half_camera(ctx, nx, ny);
+    return RT_OK;
 }
 
 // ---- render -----------------------------------------------------------------------------------------------------
@@ -583,23 +617,8 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
         launches = 2;
     }
     if (fp16) {
-        if (ctx->half_cap < (size_t)ctx->n) {
-            cudaFree(ctx->geom_h); cudaFree(ctx->matl_h);
-            ctx->geom_h = ctx->matl_h = nullptr; ctx->half_cap = 0;
-            CK(cudaMalloc(&ctx->geom_h, (size_t)ctx->n * sizeof(uint2)));
-            CK(cudaMalloc(&ctx->matl_h, (size_t)ctx->n * sizeof(uint2)));
-            ctx->half_cap = (size_t)ctx->n;
-            ctx->half_valid = false;
-        }
-        if (!ctx->half_valid) {
-            CK(launch_scene_to_half(ctx->geom, ctx->matl, ctx->n, ctx->geom_h, ctx->matl_h, ctx->stream));
-            ctx->half_valid = true;
-            ctx->half_pairs.valid = false;
-        }
-        if (!ctx->half_pairs.valid || ctx->half_pairs.octree != (a->use_octree != 0))
-            CK(build_half_pairs(ctx->half_pairs, ctx->geom_h, ctx->tag, ctx->n, a->use_octree != 0, p.tree, ctx->stream));
         {
-            const int rc = ensure_half_camera(ctx, a->nx, a->ny);
+            const int rc = ensure_half(ctx, kHalfPairs | kHalfCamera, a->use_octree != 0, p.tree, a->nx, a->ny);
             if (rc) return rc;
         }
         CK(launch_render_half(p, a->use_octree != 0, ctx->geom_h, ctx->matl_h, ctx->cam_h, ctx->half_pairs, ctx->prop.multiProcessorCount,
@@ -746,6 +765,108 @@ extern "C" int rt_scatter_rays(rt_context *ctx, int n, const int *sphere_idx, co
     SceneView sv;
     sv.geom = ctx->geom; sv.matl = ctx->matl; sv.tag = ctx->tag; sv.n = ctx->n;
     CK(launch_scatter_rays(sv, n, d_i, d_o, d_d, d_t, d_st, d_p, d_n, d_od, d_a, d_sc, ctx->stream));
+    CK(cudaMemcpyAsync(out_p, d_p, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(out_normal, d_n, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(out_dir, d_od, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(out_atten, d_a, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(scattered, d_sc, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(states6, d_st, (size_t)n * 24, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return RT_OK;
+}
+
+// ---- the same three queries under a given arithmetic ----------------------------------------------------------------------
+// RT_PREC_FP16: the USE_FP16 build's hitTree / hitable_list::hit, camera::get_ray and material::scatter (rt_render_half.cuh):
+// float inputs are rounded to half on entry, outputs are halves widened to float.
+extern "C" int rt_trace_rays_ex(rt_context *ctx, int use_octree, int precision, int n, const float *org, const float *dir, int *out_idx,
+                                float *out_t) {
+    if (precision != RT_PREC_FP32 && precision != RT_PREC_FP16) return fail(ctx, RT_ERR_INVALID, "rt_trace_rays_ex: unknown precision");
+    if (!ctx || n < 1 || !org || !dir || !out_idx || !out_t) return fail(ctx, RT_ERR_INVALID, "rt_trace_rays_ex: bad arguments");
+    if (ctx->n < 1) return fail(ctx, RT_ERR_STATE, "rt_trace_rays_ex: no scene");
+    if (use_octree && !ctx->octree->built) return fail(ctx, RT_ERR_STATE, "rt_trace_rays_ex: no octree built");
+    if (use_octree && ctx->octree->fp16 != (precision == RT_PREC_FP16))
+        return fail(ctx, RT_ERR_STATE, "rt_trace_rays_ex: the octree was built for the other precision (rt_octree_build_ex)");
+    if (precision == RT_PREC_FP32) return rt_trace_rays(ctx, use_octree, n, org, dir, out_idx, out_t);
+    CK(cudaSetDevice(ctx->device));
+    RenderLaunch p;
+    memset(&p, 0, sizeof p);
+    p.scene.geom = ctx->geom; p.scene.matl = ctx->matl; p.scene.tag = ctx->tag; p.scene.n = ctx->n;
+    if (use_octree) p.tree = ctx->octree->view();
+    {
+        const int rc = ensure_half(ctx, kHalfPairs, use_octree != 0, p.tree, 0, 0);
+        if (rc) return rc;
+    }
+    Scratch sc;
+    float *d_o = nullptr, *d_d = nullptr, *d_t = nullptr;
+    int *d_i = nullptr;
+    CK(sc.get(d_o, (size_t)n * 3)); CK(sc.get(d_d, (size_t)n * 3));
+    CK(sc.get(d_t, (size_t)n)); CK(sc.get(d_i, (size_t)n));
+    CK(cudaMemcpyAsync(d_o, org, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_d, dir, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
+    CK(launch_trace_rays_half(p, use_octree != 0, ctx->geom_h, ctx->half_pairs, d_o, d_d, n, d_i, d_t, ctx->stream));
+    CK(cudaMemcpyAsync(out_idx, d_i, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(out_t, d_t, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return RT_OK;
+}
+
+extern "C" int rt_camera_get_rays_ex(rt_context *ctx, int precision, int n, const float *s, const float *t, uint32_t *states6, float *org,
+                                     float *dir) {
+    if (precision == RT_PREC_FP32) return rt_camera_get_rays(ctx, n, s, t, states6, org, dir);
+    if (precision != RT_PREC_FP16) return fail(ctx, RT_ERR_INVALID, "rt_camera_get_rays_ex: unknown precision");
+    if (!ctx || n < 1 || !s || !t || !states6 || !org || !dir) return fail(ctx, RT_ERR_INVALID, "rt_camera_get_rays_ex: bad arguments");
+    if (!ctx->have_camera) return fail(ctx, RT_ERR_STATE, "rt_camera_get_rays_ex: no camera set (rt_camera_set)");
+    CK(cudaSetDevice(ctx->device));
+    {
+        const int rc = ensure_half_camera(ctx, ctx->cam_nx, ctx->cam_ny);      // the camera the FP16 render of this frame size uses
+        if (rc) return rc;
+    }
+    Scratch sc;
+    float *d_s = nullptr, *d_t = nullptr, *d_o = nullptr, *d_d = nullptr;
+    uint32_t *d_st = nullptr;
+    CK(sc.get(d_s, (size_t)n)); CK(sc.get(d_t, (size_t)n)); CK(sc.get(d_o, (size_t)n * 3)); CK(sc.get(d_d, (size_t)n * 3)); CK(sc.get(d_st, (size_t)n * 6));
+    CK(cudaMemcpyAsync(d_s, s, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_t, t, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_st, states6, (size_t)n * 24, cudaMemcpyHostToDevice, ctx->stream));
+    CK(launch_camera_rays_half(ctx->cam_h, n, d_s, d_t, d_st, d_o, d_d, ctx->stream));
+    CK(cudaMemcpyAsync(org, d_o, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(dir, d_d, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(states6, d_st, (size_t)n * 24, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return RT_OK;
+}
+
+extern "C" int rt_scatter_rays_ex(rt_context *ctx, int precision, int n, const int *sphere_idx, const float *org, const float *dir,
+                                  const float *t_hit, uint32_t *states6, float *out_p, float *out_normal, float *out_dir, float *out_atten,
+                                  int *scattered) {
+    if (precision == RT_PREC_FP32)
+        return rt_scatter_rays(ctx, n, sphere_idx, org, dir, t_hit, states6, out_p, out_normal, out_dir, out_atten, scattered);
+    if (precision != RT_PREC_FP16) return fail(ctx, RT_ERR_INVALID, "rt_scatter_rays_ex: unknown precision");
+    if (!ctx || n < 1 || !sphere_idx || !org || !dir || !t_hit || !states6 || !out_p || !out_normal || !out_dir || !out_atten || !scattered)
+        return fail(ctx, RT_ERR_INVALID, "rt_scatter_rays_ex: bad arguments");
+    if (ctx->n < 1) return fail(ctx, RT_ERR_STATE, "rt_scatter_rays_ex: no scene");
+    CK(cudaSetDevice(ctx->device));
+    {
+        const TreeView none{};
+        const int rc = ensure_half(ctx, 0u, false, none, 0, 0);
+        if (rc) return rc;
+    }
+    Scratch sc;
+    int *d_i = nullptr, *d_sc = nullptr;
+    float *d_o = nullptr, *d_d = nullptr, *d_t = nullptr, *d_p = nullptr, *d_n = nullptr, *d_od = nullptr, *d_a = nullptr;
+    uint32_t *d_st = nullptr;
+    CK(sc.get(d_i, (size_t)n)); CK(sc.get(d_sc, (size_t)n)); CK(sc.get(d_o, (size_t)n * 3)); CK(sc.get(d_d, (size_t)n * 3)); CK(sc.get(d_t, (size_t)n));
+    CK(sc.get(d_p, (size_t)n * 3)); CK(sc.get(d_n, (size_t)n * 3)); CK(sc.get(d_od, (size_t)n * 3)); CK(sc.get(d_a, (size_t)n * 3)); CK(sc.get(d_st, (size_t)n * 6));
+    CK(cudaMemcpyAsync(d_i, sphere_idx, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_o, org, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_d, dir, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_t, t_hit, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(d_st, states6, (size_t)n * 24, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemsetAsync(d_p, 0, (size_t)n * 12, ctx->stream)); CK(cudaMemsetAsync(d_n, 0, (size_t)n * 12, ctx->stream));
+    CK(cudaMemsetAsync(d_od, 0, (size_t)n * 12, ctx->stream)); CK(cudaMemsetAsync(d_a, 0, (size_t)n * 12, ctx->stream));
+    SceneView sv;
+    sv.geom = ctx->geom; sv.matl = ctx->matl; sv.tag = ctx->tag; sv.n = ctx->n;
+    CK(launch_scatter_rays_half(sv, ctx->geom_h, ctx->matl_h, n, d_i, d_o, d_d, d_t, d_st, d_p, d_n, d_od, d_a, d_sc, ctx->stream));
     CK(cudaMemcpyAsync(out_p, d_p, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(out_normal, d_n, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(out_dir, d_od, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));

@@ -310,8 +310,13 @@ __global__ void k_leaf_number(const uint32_t *__restrict__ vals, const uint32_t 
     leaf_index[id] = rank >= 0 ? rank + 1 : 0;   // leaves[0] is never used (:58)
 }
 
+// OctNode (acceleration_structure.h:34-38) = {int level, AABB, int children[8]}.  AABB is six real_t: floats (60-byte nodes), or
+// under USE_FP16 halves (48-byte nodes: level at 0, the box at 4, children at 16).  The box planes are multiples of 2.75 (x, z)
+// and 0.25 (y) in [-11, 11], exact in half, and so is the reference's half subdivision low + (high - low) / 2 of exact values:
+// the half AABB is the float plane rounded to half.  rt_octree_export_reference checks that every plane round-trips.
+template <bool HALF>
 __global__ void k_blob_nodes(const int *__restrict__ node_of_potential, const int *__restrict__ leaf_index,
-                             BuildPlanes P, int32_t *__restrict__ blob_nodes) {
+                             BuildPlanes P, uint8_t *__restrict__ blob_nodes) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= kNumberNodes) return;
     const int ni = node_of_potential[t];
@@ -324,16 +329,23 @@ __global__ void k_blob_nodes(const int *__restrict__ node_of_potential, const in
         ix = (ix << 1) | (c >> 2); iy = (iy << 1) | ((c >> 1) & 1); iz = (iz << 1) | (c & 1);
     }
     const int sh = 3 - lv;
-    int32_t *nd = blob_nodes + ni * kNodeInts;
-    nd[0] = lv;
-    float *bx = reinterpret_cast<float *>(nd + 1);
-    bx[0] = P.p[0][ix << sh]; bx[1] = P.p[1][iy << sh]; bx[2] = P.p[2][iz << sh];
-    bx[3] = P.p[0][(ix + 1) << sh]; bx[4] = P.p[1][(iy + 1) << sh]; bx[5] = P.p[2][(iz + 1) << sh];
+    uint8_t *nd = blob_nodes + (size_t)ni * (HALF ? kNodeBytesHalf : kNodeInts * 4);
+    *reinterpret_cast<int32_t *>(nd) = lv;
+    const float box[6] = {P.p[0][ix << sh], P.p[1][iy << sh], P.p[2][iz << sh],
+                          P.p[0][(ix + 1) << sh], P.p[1][(iy + 1) << sh], P.p[2][(iz + 1) << sh]};
+    if (HALF) {
+        __half *bx = reinterpret_cast<__half *>(nd + 4);
+        for (int k = 0; k < 6; k++) bx[k] = __float2half_rn(box[k]);
+    } else {
+        float *bx = reinterpret_cast<float *>(nd + 4);
+        for (int k = 0; k < 6; k++) bx[k] = box[k];
+    }
+    int32_t *children = reinterpret_cast<int32_t *>(nd + 4 + 6 * (HALF ? 2 : 4));
     for (int c = 0; c < 8; c++) {
         int v;
         if (lv < 3) { const int ch = node_of_potential[level_base(lv + 1) + path * 8 + c]; v = ch >= 0 ? ch : 0; }
         else v = leaf_index[path * 8 + c];
-        nd[7 + c] = v;
+        children[c] = v;
     }
 }
 
@@ -524,22 +536,23 @@ cudaError_t OctreeBuilder::build(cudaStream_t st, const float4 *geom, const int 
     return cudaSuccess;
 }
 
-size_t OctreeBuilder::reference_bytes(int spl_) {
-    return (size_t)kNumberNodes * kNodeInts * 4 + (size_t)(kNumberLeafs + 1) * (size_t)(spl_ + 1) * 4 + 8;
+size_t OctreeBuilder::reference_bytes(int spl_, bool fp16_) {
+    return (size_t)kNumberNodes * (fp16_ ? kNodeBytesHalf : kNodeInts * 4) + (size_t)(kNumberLeafs + 1) * (size_t)(spl_ + 1) * 4 + 8;
 }
 
 cudaError_t OctreeBuilder::export_reference(cudaStream_t st, void *host_blob, size_t bytes) {
     if (!built) return cudaErrorNotReady;
-    const size_t need = reference_bytes(spl);
+    const size_t need = reference_bytes(spl, fp16);
     if (bytes < need) return cudaErrorInvalidValue;
     RT_CUDA(ensure(d.blob, cap.blob, need));
     RT_CUDA(cudaMemsetAsync(d.blob, 0, need, st));          // `new Octree()` value-initialises
     int *leaf_count = d.leaf_index + kCells * 8;
     RT_CUDA(cudaMemsetAsync(leaf_count, 0, 4, st));
     k_leaf_number<<<(kCells * 8 + 255) / 256, 256, 0, st>>>(d.vals_sorted, d.cell_start, spl, d.leaf_index, leaf_count);
-    int32_t *nodes = reinterpret_cast<int32_t *>(d.blob);
-    int32_t *leaves = nodes + kNumberNodes * kNodeInts;
-    k_blob_nodes<<<(kNumberNodes + 255) / 256, 256, 0, st>>>(d.node_of_potential, d.leaf_index, planes, nodes);
+    // the leaves follow the nodes: OctLeaf is all ints in both layouts, and the buckets of an FP16 build are its own memberships
+    int32_t *leaves = reinterpret_cast<int32_t *>(d.blob + (size_t)kNumberNodes * (fp16 ? kNodeBytesHalf : kNodeInts * 4));
+    if (fp16) k_blob_nodes<true><<<(kNumberNodes + 255) / 256, 256, 0, st>>>(d.node_of_potential, d.leaf_index, planes, d.blob);
+    else k_blob_nodes<false><<<(kNumberNodes + 255) / 256, 256, 0, st>>>(d.node_of_potential, d.leaf_index, planes, d.blob);
     if (E > 0)
         k_blob_leaves<<<(E + 255) / 256, 256, 0, st>>>(d.keys_sorted, d.vals_sorted, d.cell_start, E, spl, d.leaf_index, leaves);
     int lc = 0;

@@ -329,6 +329,31 @@ cudaError_t launch_finalize_half(const float *accum, float *fb, size_t count, in
     return cudaGetLastError();
 }
 
+cudaError_t launch_trace_rays_half(const RenderLaunch &p, bool octree, const uint2 *geom_h, const HalfPairs &hp, const float *org, const float *dir,
+                                   int n, int *out_idx, float *out_t, cudaStream_t st) {
+    h16::PairView pv;
+    pv.geom = hp.geom; pv.idx = hp.idx; pv.start = hp.start;
+    h16::NodeTab nt;
+    nt.ent = hp.nodes; nt.count = hp.node_count;
+    // whole blocks of whole warps: coop_trace_h is a full-warp collective
+    const unsigned blocks = (unsigned)((n + kRenderThreads - 1) / kRenderThreads);
+    if (octree) h16::k_trace_rays_h<true><<<blocks, kRenderThreads, 0, st>>>(p, geom_h, pv, nt, org, dir, n, out_idx, out_t);
+    else h16::k_trace_rays_h<false><<<blocks, kRenderThreads, 0, st>>>(p, geom_h, pv, nt, org, dir, n, out_idx, out_t);
+    return cudaGetLastError();
+}
+cudaError_t launch_camera_rays_half(const __half *cam_h, int n, const float *s, const float *t, uint32_t *states, float *org, float *dir,
+                                    cudaStream_t st) {
+    h16::k_camera_rays_h<<<(n + 127) / 128, 128, 0, st>>>(cam_h, n, s, t, states, org, dir);
+    return cudaGetLastError();
+}
+cudaError_t launch_scatter_rays_half(const SceneView &sc, const uint2 *geom_h, const uint2 *matl_h, int n, const int *sphere_idx, const float *org,
+                                     const float *dir, const float *t_hit, uint32_t *states, float *out_p, float *out_n, float *out_dir,
+                                     float *out_att, int *scattered, cudaStream_t st) {
+    h16::k_scatter_rays_h<<<(n + 127) / 128, 128, 0, st>>>(geom_h, matl_h, sc.tag, sc.n, n, sphere_idx, org, dir, t_hit, states, out_p, out_n,
+                                                            out_dir, out_att, scattered);
+    return cudaGetLastError();
+}
+
 // (re)build the pair lists of the USE_FP16 path: lists = 1 (flat mode) or kCells (octree mode)
 cudaError_t build_half_pairs(HalfPairs &hp, const uint2 *geom_h, const int *tag, int n, bool octree, const TreeView &tv, cudaStream_t st) {
     const int lists = octree ? kCells : 1;

@@ -70,6 +70,15 @@ cudaError_t launch_render_half(const RenderLaunch &p, bool octree, const uint2 *
                                const HalfPairs &hp, int sm_count, cudaStream_t st, int *blocks_out);
 // fb = the USE_FP16 build's sqrt(accum / ns) on `count` half sums widened to float
 cudaError_t launch_finalize_half(const float *accum, float *fb, size_t count, int ns, cudaStream_t st);
+// per-ray queries of the USE_FP16 build (hitTree / hitable_list::hit, camera::get_ray, material::scatter): float inputs are
+// rounded to half, outputs are halves widened to float
+cudaError_t launch_trace_rays_half(const RenderLaunch &p, bool octree, const uint2 *geom_h, const HalfPairs &hp, const float *org, const float *dir,
+                                   int n, int *out_idx, float *out_t, cudaStream_t st);
+cudaError_t launch_camera_rays_half(const __half *cam_h, int n, const float *s, const float *t, uint32_t *states, float *org, float *dir,
+                                    cudaStream_t st);
+cudaError_t launch_scatter_rays_half(const SceneView &sc, const uint2 *geom_h, const uint2 *matl_h, int n, const int *sphere_idx, const float *org,
+                                     const float *dir, const float *t_hit, uint32_t *states, float *out_p, float *out_n, float *out_dir,
+                                     float *out_att, int *scattered, cudaStream_t st);
 // ---- output_to_stream on the device (rt_ppm.cu) ----
 struct PpmWorkspace {
     uint32_t *block_len = nullptr;

@@ -288,4 +288,89 @@ __global__ void k_finalize_h(const float *__restrict__ accum, float *__restrict_
     if (i < count) fb[i] = h2f(hsqrtf_(hmul_(f2h(accum[i]), inv_ns_h(ns))));
 }
 
+// ---- per-ray queries of the USE_FP16 build: hitTree / hitable_list::hit, camera::get_ray, material::scatter -------------------
+// The device functions k_render_h composes, one call per caller-supplied input.  Every float input is rounded to half on entry
+// and every output is a half widened to float, so values that came out of one of these kernels go back in exactly.
+
+// Closest hit of n rays: coop_trace_h over the same pair lists, node tables and half slab planes as k_render_h, so the answer is
+// the one the render computes.  The warp traces its lanes' rays together (ballots, shuffles, REDUX over the full warp): lanes
+// past n stay in the kernel with no ray.  out_t is the hit's half t (+inf on a miss: FLT_MAX rounded to half).  The launch bounds
+// are k_render_h's: with kRenderThreads alone ptxas held the octree instance to 56 registers and spilled 46 bytes.
+template <bool OCTREE>
+__global__ void __launch_bounds__(kRenderThreads, 5)
+k_trace_rays_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geom_h, const PairView pv, const NodeTab nt,
+               const float *__restrict__ org, const float *__restrict__ dir, int n, int *__restrict__ out_idx, float *__restrict__ out_t) {
+    __shared__ CoopSmem coop_sm[kRenderThreads / 32];
+    __shared__ hf planes_h[3 * kPlanes];
+    if (OCTREE && threadIdx.x < 3 * kPlanes) planes_h[threadIdx.x] = f2h((&p.tree.planes[0][0])[threadIdx.x]);
+    __syncthreads();
+    const unsigned lane = threadIdx.x & 31u;
+    if (lane == 0) {
+        coop_sm[threadIdx.x >> 5].tail = 0u;
+        coop_sm[threadIdx.x >> 5].pairs_lo = coop_sm[threadIdx.x >> 5].pairs_hi = 0u;
+    }
+    __syncwarp();
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool have = i < n;
+    const hf zero = f2h(0.0f), one = f2h(1.0f);
+    vec3h o = mkh(zero, zero, zero), d = mkh(zero, zero, one);
+    if (have) {
+        o = mkh_f(org[3 * i], org[3 * i + 1], org[3 * i + 2]);
+        d = mkh_f(dir[3 * i], dir[3 * i + 1], dir[3 * i + 2]);
+    }
+    const HitH h = coop_trace_h<OCTREE>(coop_sm[threadIdx.x >> 5], planes_h, pv, nt, geom_h, have, o, d);
+    if (have) {
+        out_idx[i] = h.idx;
+        out_t[i] = h2f(h.t);
+    }
+}
+
+// camera::get_ray (camera.h:45-49) with the context's half camera (22 halves, k_camera_setup_h); each ray draws its lens sample
+// from its own XORWOW state (6 words, in and out)
+__global__ void k_camera_rays_h(const __half *__restrict__ cam_h, int n, const float *__restrict__ s, const float *__restrict__ t,
+                                uint32_t *__restrict__ states, float *__restrict__ org, float *__restrict__ dir) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    CameraH cam;
+    {
+        vec3h *v[7] = {&cam.origin, &cam.lower_left_corner, &cam.horizontal, &cam.vertical, &cam.u, &cam.v, &cam.w};
+        for (int k = 0; k < 7; k++) *v[k] = mkh(cam_h[3 * k], cam_h[3 * k + 1], cam_h[3 * k + 2]);
+        cam.lens_radius = cam_h[21];
+    }
+    xorwow rng;
+    uint32_t *st = states + (size_t)i * 6;
+    rng.d = st[0]; rng.v0 = st[1]; rng.v1 = st[2]; rng.v2 = st[3]; rng.v3 = st[4]; rng.v4 = st[5];
+    vec3h o, d;
+    camera_ray_h(cam, f2h(s[i]), f2h(t[i]), rng, o, d);
+    org[3 * i] = h2f(vx(o)); org[3 * i + 1] = h2f(vy(o)); org[3 * i + 2] = h2f(o.z);
+    dir[3 * i] = h2f(vx(d)); dir[3 * i + 1] = h2f(vy(d)); dir[3 * i + 2] = h2f(d.z);
+    st[0] = rng.d; st[1] = rng.v0; st[2] = rng.v1; st[3] = rng.v2; st[4] = rng.v3; st[5] = rng.v4;
+}
+
+// sphere.h:30-33 + material.h:55-113 for (ray, sphere, t): hit point, normal, scattered direction, attenuation, and
+// scattered = 1 / 0 (metal absorbs, material.h:72) / -1 (not a defined sphere); the state is advanced in place
+__global__ void k_scatter_rays_h(const uint2 *__restrict__ geom_h, const uint2 *__restrict__ matl_h, const int *__restrict__ tag, int nsph,
+                                 int n, const int *__restrict__ sphere_idx, const float *__restrict__ org, const float *__restrict__ dir,
+                                 const float *__restrict__ t_hit, uint32_t *__restrict__ states, float *__restrict__ out_p,
+                                 float *__restrict__ out_n, float *__restrict__ out_dir, float *__restrict__ out_att, int *__restrict__ scattered) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int idx = sphere_idx[i];
+    if (idx < 0 || idx >= nsph || tag[idx] < 0) { scattered[i] = -1; return; }
+    xorwow rng;
+    uint32_t *st = states + (size_t)i * 6;
+    rng.d = st[0]; rng.v0 = st[1]; rng.v1 = st[2]; rng.v2 = st[3]; rng.v3 = st[4]; rng.v4 = st[5];
+    const vec3h o = mkh_f(org[3 * i], org[3 * i + 1], org[3 * i + 2]), d = mkh_f(dir[3 * i], dir[3 * i + 1], dir[3 * i + 2]);
+    const hf zero = f2h(0.0f);
+    vec3h hp, hn, att, dn = mkh(zero, zero, zero);
+    hit_point_h(load_sphere_h(geom_h, idx), o, d, f2h(t_hit[i]), hp, hn);
+    const bool go = scatter_h(tag[idx], load_mat_h(matl_h, idx), d, hp, hn, att, dn, rng);
+    out_p[3 * i] = h2f(vx(hp)); out_p[3 * i + 1] = h2f(vy(hp)); out_p[3 * i + 2] = h2f(hp.z);
+    out_n[3 * i] = h2f(vx(hn)); out_n[3 * i + 1] = h2f(vy(hn)); out_n[3 * i + 2] = h2f(hn.z);
+    out_dir[3 * i] = h2f(vx(dn)); out_dir[3 * i + 1] = h2f(vy(dn)); out_dir[3 * i + 2] = h2f(dn.z);
+    out_att[3 * i] = h2f(vx(att)); out_att[3 * i + 1] = h2f(vy(att)); out_att[3 * i + 2] = h2f(att.z);
+    scattered[i] = go ? 1 : 0;
+    st[0] = rng.d; st[1] = rng.v0; st[2] = rng.v1; st[3] = rng.v2; st[4] = rng.v3; st[5] = rng.v4;
+}
+
 }  // namespace h16

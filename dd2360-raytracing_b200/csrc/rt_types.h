@@ -10,6 +10,7 @@ constexpr int kTreeHeight = 3;
 constexpr int kNumberNodes = 585;         // 1 + 8 + 64 + 512
 constexpr int kNumberLeafs = 4096;
 constexpr int kNodeInts = 15;             // OctNode: level, AABB (6 floats), children[8]
+constexpr int kNodeBytesHalf = 48;        // OctNode under USE_FP16: level, AABB (6 halves), children[8]
 constexpr int kCells = 512;               // level-3 cells of the fixed 8x8x8 subdivision
 constexpr int kPlanes = 9;                // slab planes per axis at level 3
 

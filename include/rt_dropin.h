@@ -18,6 +18,14 @@
  * rt_octree_export_reference, rt_trace_rays), so the arithmetic is the GPU's and the results are the ones the render
  * kernels compute.  The context they talk to is the one bound with rt_dropin_bind().  `curandState` is the XORWOW state
  * {d, v[5]} and `curand_init` / `curand_uniform` follow cuRAND (subsequence < 2^40, offset 0).
+ *
+ * Compiled with -DUSE_FP16 (the reference's precision switch, precision_types.h:8) those members answer as the reference's
+ * USE_FP16 build does: hitTree, camera::get_ray and material::scatter forward with RT_PREC_FP16 (rt_trace_rays_ex,
+ * rt_camera_get_rays_ex, rt_scatter_rays_ex), buildOctree builds with rt_octree_build_ex(.., RT_PREC_FP16, ..) and returns
+ * that build's layout (AABB of six halves, 48-byte nodes), and hitTree's rec.t, rec.p and rec.normal are the half values the
+ * library computes.  The host real_t stays float: every value crossing into the library is rounded to half there, every
+ * value coming back is a half widened to float (so it goes back in exactly), and arithmetic the caller does between member
+ * calls is the caller's own, in float — it is not the reference's half arithmetic.
  */
 #ifndef RT_DROPIN_H
 #define RT_DROPIN_H
@@ -146,7 +154,11 @@ inline bool material::scatter(const ray &r_in, const hit_record &rec, vec3 &atte
     uint32_t w[6] = {st->d, st->v[0], st->v[1], st->v[2], st->v[3], st->v[4]};
     float p[3], nrm[3], od[3], att[3];
     int go = 0;
+#ifdef USE_FP16
+    if (rt_scatter_rays_ex(ctx, RT_PREC_FP16, 1, &rec.sphere_index, o, d, &rec.t, w, p, nrm, od, att, &go) != 0 || go < 0) return false;
+#else
     if (rt_scatter_rays(ctx, 1, &rec.sphere_index, o, d, &rec.t, w, p, nrm, od, att, &go) != 0 || go < 0) return false;
+#endif
     st->d = w[0];
     for (int k = 0; k < 5; k++) st->v[k] = w[1 + k];
     attenuation = vec3(att[0], att[1], att[2]);
@@ -222,7 +234,11 @@ public:
         uint32_t w[6] = {local_rand_state->d, local_rand_state->v[0], local_rand_state->v[1], local_rand_state->v[2], local_rand_state->v[3],
                          local_rand_state->v[4]};
         float o[3] = {0, 0, 0}, d[3] = {0, 0, 0};
+#ifdef USE_FP16
+        if (ctx && rt_camera_get_rays_ex(ctx, RT_PREC_FP16, 1, &s, &t, w, o, d) == 0) {
+#else
         if (ctx && rt_camera_get_rays(ctx, 1, &s, &t, w, o, d) == 0) {
+#endif
             local_rand_state->d = w[0];
             for (int k = 0; k < 5; k++) local_rand_state->v[k] = w[1 + k];
         }
@@ -248,10 +264,37 @@ inline int rt_apply_camera(rt_context *ctx, const camera &cam, int nx, int ny) {
 #ifndef SPHERES_PER_LEAF
 #define SPHERES_PER_LEAF 30          /* acceleration_structure.h:15; -D overrides it, as the CLI does */
 #endif
+#ifdef USE_FP16
+/* one real_t member of the USE_FP16 layout: the 2 bytes of an IEEE half, read as float */
+struct rt_half_storage {
+    uint16_t bits;
+    operator float() const {
+        const uint32_t sign = (uint32_t)(bits & 0x8000u) << 16, e = (bits >> 10) & 0x1fu, m = bits & 0x3ffu;
+        uint32_t b;
+        if (e == 0) {                                   /* zero or subnormal: m * 2^-24, exact in float */
+            const float f = ldexpf((float)m, -24);
+            memcpy(&b, &f, 4);
+            b |= sign;
+        } else if (e == 31) {
+            b = sign | 0x7f800000u | (m << 13);         /* inf, NaN */
+        } else {
+            b = sign | ((e + 112u) << 23) | (m << 13);
+        }
+        float f;
+        memcpy(&f, &b, 4);
+        return f;
+    }
+};
+struct AABB {                        /* acceleration_structure.h:26-29 with real_t = half: 12 bytes */
+    rt_half_storage x_low, y_low, z_low;
+    rt_half_storage x_high, y_high, z_high;
+};
+#else
 struct AABB {
     real_t x_low, y_low, z_low;
     real_t x_high, y_high, z_high;
 };
+#endif
 struct OctNode {
     int level;
     AABB aabb;
@@ -270,15 +313,21 @@ struct Octree {
 
 /* acceleration_structure.h:195: the spheres become the bound context's world, the tree is built on the GPU (rt_octree_build)
  * and comes back in the reference layout, byte for byte what the serial host build produces.  nullptr on failure
- * (rt_last_error tells why).  The context keeps its own traversal structure for rendering and hitTree. */
+ * (rt_last_error tells why).  The context keeps its own traversal structure for rendering and hitTree.  Under USE_FP16: the
+ * tree of the FP16 build (half-rounded memberships, rt_octree_build_ex) in its layout. */
 inline Octree *buildOctree(sphere *d_list, const int num_hitables) {
     rt_context *ctx = rt_dropin_context();
     if (!ctx || !d_list || num_hitables < 1) return nullptr;
     std::vector<rt_sphere_desc> flat;
     for (int i = 0; i < num_hitables; i++) d_list[i].flatten(flat);
     if (rt_scene_upload(ctx, flat.data(), num_hitables) != 0) return nullptr;
+#ifdef USE_FP16
+    if (rt_octree_build_ex(ctx, SPHERES_PER_LEAF, RT_PREC_FP16, nullptr) != 0) return nullptr;
+    if (rt_octree_reference_bytes_ex(SPHERES_PER_LEAF, RT_PREC_FP16) != sizeof(Octree)) return nullptr;
+#else
     if (rt_octree_build(ctx, SPHERES_PER_LEAF, nullptr) != 0) return nullptr;
     if (rt_octree_reference_bytes(SPHERES_PER_LEAF) != sizeof(Octree)) return nullptr;
+#endif
     Octree *octree = new Octree();
     if (rt_octree_export_reference(ctx, octree, sizeof(Octree)) != 0) { delete octree; return nullptr; }
     return octree;
@@ -286,13 +335,31 @@ inline Octree *buildOctree(sphere *d_list, const int num_hitables) {
 
 /* acceleration_structure.h:319: closest hit through the octree built by buildOctree (the `octree` argument names it; the
  * query runs on the context's own traversal structure, which returns the reference's answer).  `world` is the hitable_list
- * the spheres were uploaded from: it supplies mat_ptr for the record. */
+ * the spheres were uploaded from: it supplies mat_ptr for the record.  Under USE_FP16 the query is the FP16 build's and rec.t,
+ * rec.p and rec.normal are its half values (sphere.h:30-33 as the library evaluates them, through rt_scatter_rays_ex with a
+ * scratch state whose scattered ray is dropped). */
 inline bool hitTree(Octree *octree, const ray &r, hit_record &rec, hitable **world) {
     rt_context *ctx = rt_dropin_context();
     if (!ctx || !octree) return false;
     const float o[3] = {r.A[0], r.A[1], r.A[2]}, d[3] = {r.B[0], r.B[1], r.B[2]};
     int idx = -1;
     float t = 0;
+#ifdef USE_FP16
+    if (rt_trace_rays_ex(ctx, 1, RT_PREC_FP16, 1, o, d, &idx, &t) != 0 || idx < 0) return false;
+    uint32_t w[6] = {6615241u, 123456789u, 362436069u, 521288629u, 88675123u, 5783321u};    /* any non-zero XORWOW state */
+    float p[3], nrm[3], od[3], att[3];
+    int go = 0;
+    if (rt_scatter_rays_ex(ctx, RT_PREC_FP16, 1, &idx, o, d, &t, w, p, nrm, od, att, &go) != 0 || go < 0) return false;
+    rec.t = t;
+    rec.sphere_index = idx;
+    rec.p = vec3(p[0], p[1], p[2]);
+    rec.normal = vec3(nrm[0], nrm[1], nrm[2]);
+    rec.mat_ptr = nullptr;
+    const hitable_list *wl = world ? dynamic_cast<const hitable_list *>(*world) : nullptr;
+    const sphere *sp = (wl && idx < wl->list_size) ? dynamic_cast<const sphere *>(wl->list[idx]) : nullptr;
+    if (sp) rec.mat_ptr = sp->mat_ptr;
+    return true;
+#else
     if (rt_trace_rays(ctx, 1, 1, o, d, &idx, &t) != 0 || idx < 0) return false;
     rec.t = t;
     rec.sphere_index = idx;
@@ -302,6 +369,7 @@ inline bool hitTree(Octree *octree, const ray &r, hit_record &rec, hitable **wor
     const sphere *sp = (wl && idx < wl->list_size) ? dynamic_cast<const sphere *>(wl->list[idx]) : nullptr;
     if (sp) { rec.mat_ptr = sp->mat_ptr; rec.normal = (rec.p - sp->center) / sp->radius; }
     return true;
+#endif
 }
 
 #endif
