@@ -40,7 +40,7 @@ ABI_SYMBOLS = [
     "rt_scene_generate", "rt_scene_generate_ex", "rt_scene_upload", "rt_scene_download", "rt_scene_size", "rt_camera_set", "rt_camera_get", "rt_camera_get_half",
     "rt_octree_build", "rt_octree_build_ex", "rt_octree_reference_bytes", "rt_octree_reference_bytes_ex", "rt_octree_export_reference", "rt_octree_debug_read", "rt_xorwow_state", "rt_debug_counters", "rt_trace_rays", "rt_camera_get_rays", "rt_scatter_rays",
     "rt_trace_rays_ex", "rt_camera_get_rays_ex", "rt_scatter_rays_ex",
-    "rt_render_accumulate", "rt_last_render_stats", "rt_render_progressive", "rt_finalize", "rt_finalize_n", "rt_finalize_ex", "rt_render", "rt_render_to_host", "rt_format_ppm",
+    "rt_render_accumulate", "rt_last_render_stats", "rt_render_progressive", "rt_finalize", "rt_finalize_n", "rt_finalize_ex", "rt_render", "rt_render_to_host", "rt_render_pixels", "rt_format_ppm",
     "rt_ppm_format", "rt_ppm_read", "rt_render_to_ppm",
     "rt_ffma_peak", "rt_hfma2_peak", "rt_malloc", "rt_free", "rt_memcpy_to_host", "rt_synchronize", "rt_kernel_name",
     "rt_comm_get_unique_id", "rt_comm_init_rank", "rt_comm_init_all", "rt_comm_attach", "rt_comm_destroy", "rt_comm_rank", "rt_comm_size",
@@ -134,6 +134,7 @@ def load_library(path: str | None = None) -> C.CDLL:
         "rt_finalize_ex": (i32, [vp, vp, vp, sz, i32, i32]),
         "rt_render": (i32, [vp, C.POINTER(RenderArgs), vp, C.POINTER(RenderStats)]),
         "rt_render_to_host": (i32, [vp, C.POINTER(RenderArgs), vp, C.POINTER(RenderStats)]),
+        "rt_render_pixels": (i32, [vp, C.POINTER(RenderArgs), vp, i32, vp, i32, C.POINTER(RenderStats)]),
         "rt_format_ppm": (sz, [vp, i32, i32, vp, sz]),
         "rt_ppm_format": (i32, [vp, vp, i32, i32, C.POINTER(sz)]),
         "rt_ppm_read": (i32, [vp, vp, sz]),
@@ -184,6 +185,19 @@ def xorwow_state(seed: int, subsequence: int) -> np.ndarray:
     if rc != 0:
         raise RtError(f"rt_xorwow_state failed ({rc})")
     return out
+
+
+def window_pixels(nx: int, ny: int, i0: int, i1: int, j0: int, j1: int) -> np.ndarray:
+    """Pixel indices j*nx + i of the rectangle i0 <= i < i1, j0 <= j < j1 (the frame region fb[j0:j1, i0:i1]) for
+    RayTracer.render_pixels: every pixel once, in 8x4 tiles laid from the rectangle's corner (tiles row by row, pixels row by
+    row inside a tile), so that a warp's 32 entries are neighbours in the image as they are in the frame's queue."""
+    if not (0 <= i0 < i1 <= nx and 0 <= j0 < j1 <= ny):
+        raise ValueError(f"window ({i0}, {i1}, {j0}, {j1}) is empty or outside the {nx}x{ny} frame")
+    tx, ty = (i1 - i0 + 7) // 8, (j1 - j0 + 3) // 4
+    t_y, t_x, y, x = np.meshgrid(np.arange(ty), np.arange(tx), np.arange(4), np.arange(8), indexing="ij")
+    i, j = i0 + t_x * 8 + x, j0 + t_y * 4 + y
+    keep = (i < i1) & (j < j1)
+    return (j[keep].astype(np.int64) * nx + i[keep]).astype(np.uint32)
 
 
 def quantise(fb: np.ndarray) -> np.ndarray:
@@ -355,6 +369,26 @@ class RayTracer:
         st = RenderStats()
         self._ck(self.L.rt_render_to_host(self._ctx, C.byref(a), fb.ctypes.data, C.byref(st)), "rt_render_to_host")
         return fb, st.as_dict()
+
+    def render_pixels(self, nx, ny, ns, pixels, use_octree=True, finalize=True, **kw):
+        """The listed pixels (host array of indices j*nx + i, any order, duplicates allowed) of the nx x ny frame, exactly as
+        render() (finalize) or render_accumulate() (linear sums) computes them.  Returns (values[count, 3] float32, stats);
+        an index >= nx*ny comes back as (0, 0, 0).  window_pixels() lists a rectangle."""
+        import torch
+        pix = np.ascontiguousarray(pixels, dtype=np.uint32).reshape(-1)
+        dev = torch.device("cuda", self.device)
+        pix_dev = torch.from_numpy(pix.view(np.int32)).to(dev)          # the same 32-bit patterns
+        out = torch.empty((len(pix), 3), dtype=torch.float32, device=dev)
+        st = self.render_pixels_device(self.args(nx, ny, ns, use_octree, **kw), pix_dev.data_ptr(), len(pix), out.data_ptr(), finalize)
+        return out.cpu().numpy(), st
+
+    def render_pixels_device(self, args: RenderArgs, pixels_ptr: int, count: int, out_ptr: int, finalize=True, want_stats=True):
+        """rt_render_pixels on device pointers: `count` uint32 pixel indices at pixels_ptr, count*3 floats to out_ptr (list order).
+        want_stats=False keeps the call asynchronous (last_render_stats() reads them later)."""
+        st = RenderStats()
+        self._ck(self.L.rt_render_pixels(self._ctx, C.byref(args), C.c_void_p(pixels_ptr), count, C.c_void_p(out_ptr), int(bool(finalize)),
+                                         C.byref(st) if want_stats else None), "rt_render_pixels")
+        return st.as_dict() if want_stats else None
 
     def format_ppm_device(self, fb_dev_ptr: int, nx: int, ny: int) -> bytes:
         """output_to_stream (main.cu:321-333) on the device: P3 text of a DEVICE frame; only the text is copied back."""

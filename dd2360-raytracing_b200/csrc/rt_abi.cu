@@ -504,10 +504,29 @@ struct ProgressiveIO {
     uint32_t *state = nullptr;     // 6 words per pixel, device
     bool first = true;
 };
+struct PixelList {                 // rt_render_pixels: render these pixels of the frame, results in list order
+    const uint32_t *pixels = nullptr;      // device
+    int count = 0;
+};
+// device (or managed) memory of the context's GPU: a kernel may dereference it
+static bool on_device(const rt_context *ctx, const void *ptr) {
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, ptr) != cudaSuccess) {
+        cudaGetLastError();
+        return false;
+    }
+    return (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) && at.device == ctx->device;
+}
 static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, bool finalize, rt_render_stats *stats,
-                     const ProgressiveIO *prog = nullptr) {
+                     const ProgressiveIO *prog = nullptr, const PixelList *list = nullptr) {
     if (!ctx || !a || !out_dev) return fail(ctx, RT_ERR_INVALID, "render: null argument");
     if (a->nx < 1 || a->ny < 1 || a->ns < 1) return fail(ctx, RT_ERR_INVALID, "render: bad nx/ny/ns");
+    if (list) {
+        if (!list->pixels || list->count < 1) return fail(ctx, RT_ERR_INVALID, "rt_render_pixels: null pixel list or count < 1");
+        if (a->shard_mode != RT_SHARD_NONE) return fail(ctx, RT_ERR_INVALID, "rt_render_pixels: pixel lists are not sharded (give each GPU its own list)");
+        if (!on_device(ctx, list->pixels) || !on_device(ctx, out_dev))
+            return fail(ctx, RT_ERR_INVALID, "rt_render_pixels: pixels_dev and out_dev must be device memory of the context's GPU");
+    }
     if (ctx->n < 1) return fail(ctx, RT_ERR_STATE, "render: no scene (rt_scene_generate / rt_scene_upload first)");
     if (a->use_octree && !ctx->octree->built) return fail(ctx, RT_ERR_STATE, "render: USE_OCTREE set but no octree built");
     if (a->seed_mode != RT_SEED_HEAD && a->seed_mode != RT_SEED_UPSTREAM) return fail(ctx, RT_ERR_INVALID, "render: unknown seed_mode");
@@ -580,7 +599,8 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
         }
     }
     if (owned * 32 > 0xfffffff0ll) return fail(ctx, RT_ERR_INVALID, "render: image too large for the 32-bit work queue");
-    p.total_items = (uint32_t)(owned * 32);
+    p.total_items = list ? (uint32_t)list->count : (uint32_t)(owned * 32);
+    if (list) p.pixels = list->pixels;
     p.finalize = finalize ? 1 : 0;
     p.variant = a->tune[1] ? a->tune[1] : ctx->default_variant;
     p.out = out_dev;
@@ -590,7 +610,7 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
     int blocks = 0;
     int launches = 1;
     if (a->seed_mode == RT_SEED_UPSTREAM && !continuing) {
-        const size_t npix = (size_t)a->nx * a->ny;
+        const size_t npix = list ? (size_t)list->count : (size_t)a->nx * a->ny;      // stream states to seed
         if (!ctx->skip_tables) {
             const std::vector<uint32_t> &t = host_skip_tables();
             CK(cudaMalloc(&ctx->skip_tables, t.size() * 4));
@@ -612,8 +632,11 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
     if (continuing) {
         p.seed_states = prog->state;                  // every pixel resumes its own stream
     } else if (p.seed_states) {   // render_init (main.cu:424): inside the timed region, as in the reference
-        // spp shard g draws from subsequences pixel_index + g * num_pixels (g = 0: the reference's streams)
-        CK(launch_seed_upstream(ctx->seed_states, (size_t)a->nx * a->ny, 1984ull, p.seed_offset, ctx->skip_tables, ctx->stream));
+        if (list)                 // only the listed pixels' streams
+            CK(launch_seed_upstream_list(ctx->seed_states, list->pixels, list->count, (size_t)a->nx * a->ny, 1984ull, ctx->skip_tables,
+                                         ctx->stream));
+        else                      // spp shard g draws from subsequences pixel_index + g * num_pixels (g = 0: the reference's streams)
+            CK(launch_seed_upstream(ctx->seed_states, (size_t)a->nx * a->ny, 1984ull, p.seed_offset, ctx->skip_tables, ctx->stream));
         launches = 2;
     }
     if (fp16) {
@@ -622,11 +645,11 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
             if (rc) return rc;
         }
         CK(launch_render_half(p, a->use_octree != 0, ctx->geom_h, ctx->matl_h, ctx->cam_h, ctx->half_pairs, ctx->prop.multiProcessorCount,
-                              ctx->stream, &blocks));
+                              ctx->stream, &blocks, list != nullptr));
         ctx->last_kernel = kKernelHalf;
     } else {
         CK(launch_render(p, a->use_octree != 0 || list_grid, ctx->prop.multiProcessorCount, ctx->prop.sharedMemPerBlockOptin, ctx->stream, &blocks,
-                         &ctx->last_kernel));
+                         &ctx->last_kernel, list != nullptr));
     }
     CK(cudaEventRecord(ctx->ev1, ctx->stream));
     if (stats) {
@@ -883,6 +906,14 @@ extern "C" int rt_render_accumulate(rt_context *ctx, const rt_render_args *args,
 
 extern "C" int rt_render(rt_context *ctx, const rt_render_args *args, float *fb_dev, rt_render_stats *stats) {
     return do_render(ctx, args, fb_dev, true, stats);
+}
+
+extern "C" int rt_render_pixels(rt_context *ctx, const rt_render_args *args, const uint32_t *pixels_dev, int count, float *out_dev,
+                                int finalize, rt_render_stats *stats) {
+    PixelList list;
+    list.pixels = pixels_dev;
+    list.count = count;
+    return do_render(ctx, args, out_dev, finalize != 0, stats, nullptr, &list);
 }
 
 extern "C" int rt_render_progressive(rt_context *ctx, const rt_render_args *args, float *accum_dev, uint32_t *rng_state_dev, int first,

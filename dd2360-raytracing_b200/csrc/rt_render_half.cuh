@@ -154,8 +154,9 @@ __global__ void k_camera_setup_h(const float lfx, const float lfy, const float l
 }
 
 // PROG: progressive calls (p.accumulate, p.state_out) get instances of their own: compiled into the whole-frame instances, the
-// two per-pixel branches cost 1.6 % of a C4 frame (2 602 vs 2 559 ms, B200 at 1000 W)
-template <bool OCTREE, bool PROG>
+// two per-pixel branches cost 1.6 % of a C4 frame (2 602 vs 2 559 ms, B200 at 1000 W).
+// LIST: pixel-list instances (with PROG = false), as k_render's (`pix` is the lane's list slot).
+template <bool OCTREE, bool PROG, bool LIST = false>
 __global__ void __launch_bounds__(kRenderThreads, 5)
 k_render_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geom_h, const uint2 *__restrict__ matl_h,
            const __half *__restrict__ cam_h, const PairView pv, const NodeTab nt) {
@@ -198,15 +199,15 @@ k_render_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geo
             if (need) {
                 if (item >= p.total_items) {
                     exhausted = true;
-                } else if (item_to_pixel(p, item, pi, pj)) {
-                    pix = pj * p.nx + pi;
+                } else if (LIST ? list_to_pixel(p, item, pi, pj) : item_to_pixel(p, item, pi, pj)) {
+                    pix = LIST ? (int)item : pj * p.nx + pi;
                     s = 0; depth = 0;
                     col = mkh(zero, zero, zero);
                     if (PROG && p.accumulate) {  // progressive: the stored sums are halves widened to float, so this is exact
                         const float *acc = p.out + (size_t)pix * 3;
                         col = mkh_f(acc[0], acc[1], acc[2]);
                     }
-                    pixel_stream(p, pix, rng);
+                    pixel_stream(p, LIST && !p.seed_states ? pj * p.nx + pi : pix, rng);
                 }
             }
         }

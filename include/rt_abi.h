@@ -208,6 +208,19 @@ int rt_finalize_ex(rt_context *ctx, const float *accum_dev, float *fb_dev, size_
 int rt_render(rt_context *ctx, const rt_render_args *args, float *fb_dev, rt_render_stats *stats);
 /* Same with a HOST destination: render + device->host copy (what the reference does through managed memory). */
 int rt_render_to_host(rt_context *ctx, const rt_render_args *args, float *fb_host, rt_render_stats *stats);
+/* Render only the pixels listed in pixels_dev (device memory: count uint32 pixel indices j*nx + i of the args->nx x args->ny
+ * frame, any order, duplicates allowed).  out_dev (device memory) receives count*3 floats in LIST order: entry k holds exactly
+ * what rt_render (finalize != 0) or rt_render_accumulate (finalize == 0) writes for pixel pixels_dev[k] of the same frame with
+ * the same args, bit for bit, in either precision and seeding.  An entry >= nx*ny yields (0, 0, 0) and traces nothing.
+ * Every pixel's result depends only on its own stream and sample chain, so a crop, a region or a few pixels of interest cost
+ * what their own rays cost.  The kernel is chosen as for the frame (from the scene and args->tune[1], not from count);
+ * RT_SEED_UPSTREAM seeds the listed pixels only (count x 24 bytes).  Stats as for frames: rays summed over the entries,
+ * paths = ns x the in-range entries.  A null pointer, count < 1, args->shard_mode != RT_SHARD_NONE, or a pixels_dev / out_dev
+ * that is not device (or managed) memory of the context's GPU -> RT_ERR_INVALID; no scene, or an octree built for the other
+ * precision -> RT_ERR_STATE; nothing is written on an error.  The list is rendered in the order given: list neighbouring
+ * pixels next to each other (e.g. in 8x4 tiles, as the frame queue does) for coherent warps. */
+int rt_render_pixels(rt_context *ctx, const rt_render_args *args, const uint32_t *pixels_dev, int count, float *out_dev,
+                     int finalize, rt_render_stats *stats);
 
 /* ---- output: replaces output_to_stream (main.cu:321-333) -------------------------------------------------- */
 /* P3 text, byte-identical to the reference writer.  Returns bytes needed when buf == NULL. */
