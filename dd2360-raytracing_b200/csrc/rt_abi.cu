@@ -29,7 +29,6 @@ struct rt_context {
     std::string err;
     // scene
     int n = 0;
-    bool slot0_defined = true;
     float4 *geom = nullptr, *matl = nullptr;
     int *tag = nullptr;
     size_t scene_cap = 0;
@@ -279,7 +278,6 @@ static int upload_scene(rt_context *ctx, const rt_sphere_desc *src, bool clamp_f
     if (clamp_fuzz)
         for (int i = 0; i < n; i++)
             if (host[i].mat == RT_MAT_METAL && !(host[i].param < 1.0f)) host[i].param = 1.0f;   // metal::metal clamps fuzz (material.h:67)
-    ctx->slot0_defined = host[0].mat != RT_MAT_NONE;
     CK(cudaMemcpyAsync(ctx->desc_dev, ctx->pinned, bytes, cudaMemcpyHostToDevice, ctx->stream));
     k_split_scene<<<(n + 255) / 256, 256, 0, ctx->stream>>>(static_cast<const rt_sphere_desc *>(ctx->desc_dev), n, ctx->geom, ctx->matl, ctx->tag);
     CK(cudaGetLastError());
@@ -558,8 +556,8 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
     // flat-list mode: hitable_list::hit is "closest over all spheres"; above a few hundred spheres the grid answers it
     // with a few dozen tests instead of N (the result is the same minimum; variant 20 forces the N-test sweep)
     bool list_grid = false;
-    if (!a->use_octree && a->precision == RT_PREC_FP32 && ctx->n >= kListGridMinSpheres && a->tune[1] != 20 &&
-        ctx->slot0_defined) {      // (the prolog tests sphere 0 unconditionally; an undefined slot 0 must stay unhittable)
+    // (an undefined slot 0 stays unhittable there too: the build sees its tag, TreeView::slot0_none)
+    if (!a->use_octree && a->precision == RT_PREC_FP32 && ctx->n >= kListGridMinSpheres && a->tune[1] != 20) {
         if (!ctx->list_accel_valid) {
             CK(ctx->list_accel->build(ctx->stream, ctx->geom, ctx->tag, ctx->n, 30, ctx->grid_density, false, true));
             ctx->list_accel_valid = true;

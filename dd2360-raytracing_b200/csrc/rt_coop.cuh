@@ -142,10 +142,10 @@ __device__ __forceinline__ Hit coop_trace(WarpShared &ws, const SceneView &sc, c
     ws.rd[lane] = make_float4(d.x, d.y, d.z, ia);
     ws.slot[lane] = lane;                   // (entries past this round's owners are read by lanes without an item: keep them lane ids)
     float best_t = kTMax;
-    {   // ground sphere first, unconditionally (acceleration_structure.h:322-332)
+    {   // ground sphere first, unconditionally (acceleration_structure.h:322-332) — unless slot 0 is undefined (never hit)
         uint32_t idx = 0xffffffffu;
         float t;
-        if (has) {
+        if (has && !tv.slot0_none) {
             RT_COUNT(sphere_tests);
             if (sphere_test(__ldg(sc.geom), o, d, a, kTMax, t)) { best_t = t; idx = 0u; }
         }

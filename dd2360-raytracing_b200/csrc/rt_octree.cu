@@ -65,6 +65,8 @@ __global__ void k_classify(const float4 *__restrict__ geom, int n, BuildPlanes P
         uint32_t packed = 0, cnt = 0;
         if (i >= 1) {   // ground sphere (index 0) is never inserted (acceleration_structure.h:208)
             const float4 s = geom[i];
+            // the SIGNED radius, as `intersects` has it: a cell shrinks by |r| for a hollow sphere (r < 0), so one with |r| >= 0.125
+            // (half a cell's height) is stored nowhere and smaller ones only where the centre lies.  The grid lists surfaces: |r|.
             // USE_FP16: AABB, centre and radius are real_t, so `low - radius` / `high + radius` round to half
             // (acceleration_structure.h:83-88); the planes themselves are exact in half
             const AxisRange rx = fp16 ? axis_range_h(P.p[0], s.x, s.w, true) : axis_range(P.p[0], s.x, s.w, true);
@@ -205,16 +207,18 @@ __global__ void k_grid_prep(const float4 *__restrict__ geom, const int *__restri
     float lo[3] = {3e38f, 3e38f, 3e38f}, hi[3] = {-3e38f, -3e38f, -3e38f};
     uint32_t live = 0;
     if (i < n) {
+        if (i == 0) out->slot0_none = tag[0] < 0 ? 1u : 0u;
         uint8_t f = sph_flag[i];
         if (f && tag[i] < 0) f = 0;                       // undefined slots are never hit (SURVEY D3)
         if (f) {
             const float4 s = geom[i];
-            if (s.w > big_r) {
+            const float ar = fabsf(s.w);                  // a hollow sphere (r < 0) is hit where |r| puts its surface (r*r)
+            if (ar > big_r) {
                 const uint32_t slot = atomicAdd(&out->nbig, 1u);
                 if (slot < (uint32_t)kMaxBig) { out->big[slot] = (uint32_t)i; f = 2; }
             }
             if (f == 1) {
-                const float r = s.w + sphere_pad(s.w);
+                const float r = ar + sphere_pad(ar);
                 lo[0] = s.x - r; hi[0] = s.x + r; lo[1] = s.y - r; hi[1] = s.y + r; lo[2] = s.z - r; hi[2] = s.z + r;
                 live = 1;
             }
@@ -234,9 +238,10 @@ __global__ void k_grid_prep(const float4 *__restrict__ geom, const int *__restri
     }
 }
 
-// enumerate the voxels crossed by the (padded) surface of sphere s
+// enumerate the voxels crossed by the (padded) surface of sphere s; a hollow sphere (r < 0) by |r|
 template <typename F>
-__device__ __forceinline__ void for_each_voxel(const GridView &g, const float4 s, F f) {
+__device__ __forceinline__ void for_each_voxel(const GridView &g, float4 s, F f) {
+    s.w = fabsf(s.w);
     const float pad = sphere_pad(s.w);
     int v0[3], v1[3];
     voxel_range(g, s, pad, v0, v1);
@@ -491,6 +496,7 @@ cudaError_t OctreeBuilder::build(cudaStream_t st, const float4 *geom, const int 
     RT_CUDA(cudaStreamSynchronize(st));
     trace.mark("sync 2 (counts, grid box)");
     nbig = (int)(prep.nbig < (uint32_t)kMaxBig ? prep.nbig : (uint32_t)kMaxBig);
+    slot0_none = prep.slot0_none != 0u ? 1 : 0;
     std::sort(prep.big, prep.big + nbig);       // ascending: deterministic traversal order
     prolog_h[0] = 0;
     memcpy(prolog_h + 1, prep.big, kMaxBig * 4);
@@ -608,6 +614,7 @@ TreeView OctreeBuilder::view() const {
     v.prolog = d.big_refs;
     v.prolog_geom = d.prolog_geom;
     v.nprolog = 1 + nbig;
+    v.slot0_none = slot0_none;
     for (int a = 0; a < 3; a++) for (int i = 0; i < kPlanes; i++) v.planes[a][i] = planes.p[a][i];
     v.no_drops = stats_h[1] == 0 ? 1 : 0;
     for (int a = 0; a < 3; a++) v.cell_inv[a] = 8.0f / (planes.p[a][kPlanes - 1] - planes.p[a][0]);

@@ -17,6 +17,7 @@ struct BuildCounts {
 struct GridPrep {                 // k_grid_prep output: bounding box (order-preserving uint encoding), counts, big list
     uint32_t lo[3], hi[3];
     uint32_t live, nbig;
+    uint32_t slot0_none;          // slot 0 is undefined (TreeView::slot0_none)
     uint32_t big[kMaxBig];
 };
 
@@ -48,6 +49,7 @@ public:
     uint32_t grid_flat_min;
     int spl = 0, n_spheres = 0, leaf_count_h = 0;
     int nbig = 0;
+    int slot0_none = 0;               // TreeView::slot0_none of the last build
     uint32_t prolog_h[kMaxBig + 1];   // staging for the async upload (must outlive build())
     uint32_t E = 0, total_refs = 0, total_voxels = 0;
     GridView grid;

@@ -303,10 +303,10 @@ RT_HD Hit trace_walk(const SceneView &sc, const TreeView &tv, const float *plane
     r.o = o; r.d = d;
     r.a = dot3(d, d);
     const float ia = rcp_trav(r.a);
-    {   // ground sphere first, unconditionally (:322-332)
+    {   // ground sphere first, unconditionally (:322-332) — unless slot 0 is undefined (RT_MAT_NONE: never hit)
         float t;
         RT_COUNT(sphere_tests);
-        if (sphere_test(RT_LDG(sc.geom), o, d, r.a, kTMax, t)) {
+        if (!tv.slot0_none && sphere_test(RT_LDG(sc.geom), o, d, r.a, kTMax, t)) {
             if (MODE != kWalkTies) { h.t = t; h.idx = 0; }
             else if (t == t_tie) { h.idx = 0; key_h = 0u; }
         }

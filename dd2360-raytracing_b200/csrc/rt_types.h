@@ -62,6 +62,8 @@ struct TreeView {
     const uint32_t *prolog;     // first candidate list of every ray: the ground sphere (index 0, tested unconditionally by
     int nprolog;                // hitTree :322-332), then the big spheres in ascending order; nprolog = 1 + nbig
     const float4 *prolog_geom;  // their geometry in list order
+    int slot0_none;             // 0: every ray tests slot 0 first, as hitTree does; 1: slot 0 is RT_MAT_NONE and never hit
+                                // (decided at build time, so the render kernels read no tag per ray; a zeroed view tests it)
     float planes[3][kPlanes];   // slab plane coordinates per axis (exact floats of the reference subdivision)
     // the reference's own cell lists (USE_FP16 path walks these): cell m (9-bit Morton id) was offered
     // cell_list[cell_start[m] .. cell_start[m+1]) in ascending sphere order and stored the first cell_cap = 8*SPL of them

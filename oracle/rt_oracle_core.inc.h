@@ -120,11 +120,12 @@ static void SUF(traverse)(const oct_view *ov, const rto_sphere *sph, v3 o, v3 d,
         if (children[i] != 0) SUF(traverse)(ov, sph, o, d, children[i], res, ctr);
 }
 
-/* acceleration_structure.h:319-342 hitTree: ground sphere (index 0) first, then the tree */
+/* acceleration_structure.h:319-342 hitTree: ground sphere (index 0) first, then the tree.  The reference's slot 0 is always the
+ * ground; a caller's world may leave it undefined, and an undefined slot is never hit (SURVEY D3), here as in the flat list. */
 static int SUF(hit_tree)(const oct_view *ov, const rto_sphere *sph, v3 o, v3 d, float *t_hit, rto_counters *ctr) {
     SUF(phit) res = {-1, FLT_MAX};
     float t;
-    if (SUF(sphere_hit)(&sph[0], o, d, 0.001f, FLT_MAX, &t, ctr)) { res.best = 0; res.closest = t; }
+    if (sph[0].mat != RTO_MAT_NONE && SUF(sphere_hit)(&sph[0], o, d, 0.001f, FLT_MAX, &t, ctr)) { res.best = 0; res.closest = t; }
     SUF(traverse)(ov, sph, o, d, 0, &res, ctr);
     *t_hit = res.closest;
     return res.best;

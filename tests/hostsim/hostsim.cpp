@@ -48,6 +48,53 @@ static void make_planes(float P[3][kPlanes]) {
 // voxel shape of slab-shaped scenes: the product's defaults; profiles/warp_model.py moves them (hs_set_grid_shape)
 static float g_grid_flat = kGridFlat, g_grid_wide = kGridWide, g_pad_reach = kSceneReach;
 
+// k_grid_prep + k_vox_pass: the big spheres (ascending index, up to kMaxBig) and the surface x voxel lists of the others, over
+// the defined spheres i >= 1 that `take(i)`.  A hollow sphere (r < 0) is hit where |r| puts its surface: gridded by |r|.
+template <typename Take>
+static void build_grid(const std::vector<float4> &geom, const std::vector<int> &tag, Take take, float density, HostTree &T) {
+    const int n = (int)geom.size();
+    const float big_r = kBigRadiusFrac * 2.75f;
+    std::vector<uint32_t> small;
+    float lo[3] = {3e38f, 3e38f, 3e38f}, hi[3] = {-3e38f, -3e38f, -3e38f};
+    for (int i = 1; i < n; i++) {
+        if (tag[(size_t)i] < 0 || !take(i)) continue;
+        const float4 s = geom[(size_t)i];
+        const float ar = fabsf(s.w);
+        if (ar > big_r && (int)T.big_refs.size() < kMaxBig) { T.big_refs.push_back((uint32_t)i); continue; }
+        small.push_back((uint32_t)i);
+        const float r = ar + sphere_pad(ar, g_pad_reach);
+        lo[0] = fminf(lo[0], s.x - r); hi[0] = fmaxf(hi[0], s.x + r);
+        lo[1] = fminf(lo[1], s.y - r); hi[1] = fmaxf(hi[1], s.y + r);
+        lo[2] = fminf(lo[2], s.z - r); hi[2] = fmaxf(hi[2], s.z + r);
+    }
+    memset(&T.grid, 0, sizeof T.grid);
+    const uint32_t voxels = choose_grid(lo, hi, (uint32_t)small.size(), density, T.grid, g_grid_flat, g_grid_wide);
+    if (voxels) {
+        std::vector<std::vector<uint32_t>> lists(voxels);
+        for (uint32_t idx : small) {
+            float4 s = geom[idx];
+            s.w = fabsf(s.w);
+            const float pad = sphere_pad(s.w, g_pad_reach);
+            int v0[3], v1[3];
+            voxel_range(T.grid, s, pad, v0, v1);
+            for (int z = v0[2]; z <= v1[2]; z++)
+                for (int y = v0[1]; y <= v1[1]; y++)
+                    for (int x = v0[0]; x <= v1[0]; x++) {
+                        float blo[3], bhi[3];
+                        voxel_box(T.grid, x, y, z, blo, bhi);
+                        if (shell_hits_box(s, pad, blo, bhi)) lists[((size_t)z * T.grid.ny + y) * T.grid.nx + x].push_back(idx);
+                    }
+        }
+        T.vox.resize(voxels);
+        for (uint32_t v = 0; v < voxels; v++) {
+            std::sort(lists[v].begin(), lists[v].end());
+            T.vox[v].x = (uint32_t)T.refs.size();
+            T.vox[v].y = (uint32_t)lists[v].size();
+            T.refs.insert(T.refs.end(), lists[v].begin(), lists[v].end());
+        }
+    }
+}
+
 // Rebuild the traversal structure on the host from a reference-layout Octree blob: the per-sphere lists of cells that
 // STORE the sphere come straight from the reference's leaf buckets.
 static void build_host_tree(const std::vector<float4> &geom, const std::vector<int> &tag, const int32_t *blob, int spl,
@@ -93,47 +140,17 @@ static void build_host_tree(const std::vector<float4> &geom, const std::vector<i
         T.ent_cell.insert(T.ent_cell.end(), cells_of[(size_t)i].begin(), cells_of[(size_t)i].end());
     }
     T.ent_off[(size_t)n] = (uint32_t)T.ent_cell.size();
-    const float big_r = kBigRadiusFrac * 2.75f;
-    std::vector<uint32_t> small;
-    float lo[3] = {3e38f, 3e38f, 3e38f}, hi[3] = {-3e38f, -3e38f, -3e38f};
-    for (int i = 1; i < n; i++) {
-        if (tag[(size_t)i] < 0 || cells_of[(size_t)i].empty()) continue;
-        const float4 s = geom[(size_t)i];
-        if (s.w > big_r && (int)T.big_refs.size() < kMaxBig) { T.big_refs.push_back((uint32_t)i); continue; }
-        small.push_back((uint32_t)i);
-        const float r = s.w + sphere_pad(s.w, g_pad_reach);
-        lo[0] = fminf(lo[0], s.x - r); hi[0] = fmaxf(hi[0], s.x + r);
-        lo[1] = fminf(lo[1], s.y - r); hi[1] = fmaxf(hi[1], s.y + r);
-        lo[2] = fminf(lo[2], s.z - r); hi[2] = fmaxf(hi[2], s.z + r);
-    }
-    memset(&T.grid, 0, sizeof T.grid);
-    const uint32_t voxels = choose_grid(lo, hi, (uint32_t)small.size(), density, T.grid, g_grid_flat, g_grid_wide);
-    if (voxels) {
-        std::vector<std::vector<uint32_t>> lists(voxels);
-        for (uint32_t idx : small) {
-            const float4 s = geom[idx];
-            const float pad = sphere_pad(s.w, g_pad_reach);
-            int v0[3], v1[3];
-            voxel_range(T.grid, s, pad, v0, v1);
-            for (int z = v0[2]; z <= v1[2]; z++)
-                for (int y = v0[1]; y <= v1[1]; y++)
-                    for (int x = v0[0]; x <= v1[0]; x++) {
-                        float blo[3], bhi[3];
-                        voxel_box(T.grid, x, y, z, blo, bhi);
-                        if (shell_hits_box(s, pad, blo, bhi)) lists[((size_t)z * T.grid.ny + y) * T.grid.nx + x].push_back(idx);
-                    }
-        }
-        T.vox.resize(voxels);
-        for (uint32_t v = 0; v < voxels; v++) {
-            std::sort(lists[v].begin(), lists[v].end());
-            T.vox[v].x = (uint32_t)T.refs.size();
-            T.vox[v].y = (uint32_t)lists[v].size();
-            T.refs.insert(T.refs.end(), lists[v].begin(), lists[v].end());
-        }
-    }
+    build_grid(geom, tag, [&](int i) { return !cells_of[(size_t)i].empty(); }, density, T);
 }
 
-static void view_of(HostTree &T, TreeView &tv) {
+// The flat-list mode's grid (OctreeBuilder::build with all_spheres): every defined sphere but slot 0, wherever it lies.
+static void build_list_grid(const std::vector<float4> &geom, const std::vector<int> &tag, float density, HostTree &T) {
+    make_planes(T.planes);
+    T.ent_off.assign(geom.size() + 1, 0u);
+    build_grid(geom, tag, [](int) { return true; }, density, T);
+}
+
+static void view_of(HostTree &T, TreeView &tv, bool slot0_none, bool check_visibility = true) {
     T.prolog.assign(1, 0u);
     T.prolog.insert(T.prolog.end(), T.big_refs.begin(), T.big_refs.end());
     memset(&tv, 0, sizeof tv);
@@ -141,7 +158,8 @@ static void view_of(HostTree &T, TreeView &tv) {
     tv.grid.vox = T.vox.data(); tv.grid.refs = T.refs.data();
     tv.vis.ent_off = T.ent_off.data(); tv.vis.ent_cell = T.ent_cell.data();
     tv.prolog = T.prolog.data(); tv.nprolog = (int)T.prolog.size();
-    tv.check_visibility = 1;
+    tv.check_visibility = check_visibility ? 1 : 0;
+    tv.slot0_none = slot0_none ? 1 : 0;
     memcpy(tv.planes, T.planes, sizeof tv.planes);
     tv.no_drops = T.no_drops ? 1 : 0;
     for (int a = 0; a < 3; a++) tv.cell_inv[a] = 8.0f / (T.planes[a][kPlanes - 1] - T.planes[a][0]);
@@ -173,7 +191,7 @@ static CoopHit coop_walk_host(const SceneView &sc, const TreeView &tv, const vec
         ring.clear();
         bound = fminf(bound, h.t);
     };
-    { float t; if (sphere_test(sc.geom[0], o, d, a, kTMax, t)) { h.t = t; h.idx = 0; bound = t; } }
+    { float t; if (!tv.slot0_none && sphere_test(sc.geom[0], o, d, a, kTMax, t)) { h.t = t; h.idx = 0; bound = t; } }
     for (int k = 1; k < tv.nprolog; k++) {
         const int idx = (int)tv.prolog[k];
         float ub;
@@ -221,14 +239,17 @@ static CoopHit coop_walk_host(const SceneView &sc, const TreeView &tv, const vec
     drain();
     return h;
 }
-static bool g_coop_check = false;
+static bool g_coop_check = false, g_list_grid = false;
 static unsigned long long g_coop_rays = 0, g_coop_bad = 0;
 
 extern "C" {
 
 void hs_set_grid_shape(float flat, float wide) { g_grid_flat = flat; g_grid_wide = wide; }
 void hs_set_pad_reach(float reach) { g_pad_reach = reach; }
-// every octree ray of the following renders is also traced by coop_walk_host (both schedules) and compared with trace_walk's minimum
+// every octree (or list-grid) ray of the following renders is also traced by coop_walk_host (both schedules) and compared with trace_walk's minimum
+// use_octree = 0 renders go through the flat-list mode's grid (hitable_list::hit answered by trace_tree without the visibility
+// rule), as the library does from kListGridMinSpheres spheres on; off: the plain list sweep (trace_list)
+void hs_set_list_grid(int on) { g_list_grid = on != 0; }
 void hs_coop_check(int on) { g_coop_check = on != 0; g_coop_rays = g_coop_bad = 0; }
 void hs_coop_check_result(unsigned long long *rays, unsigned long long *mismatches) { *rays = g_coop_rays; *mismatches = g_coop_bad; }
 // choose_grid as the build calls it (the product's default voxel shape): dims[3]; returns the voxel count
@@ -264,9 +285,14 @@ static int render_core(const hs_sphere *sph, int n, const float *camera22, const
         for (int a = 0; a < 3; a++) tv.cell_inv[a] = 8.0f / (T.planes[a][kPlanes - 1] - T.planes[a][0]);
     } else if (p->use_octree) {
         build_host_tree(geom, tag, static_cast<const int32_t *>(blob), p->spl, density, T);
-        view_of(T, tv);
+        view_of(T, tv, tag[0] < 0);
+        if (build_stats) { build_stats[0] = T.vox.size(); build_stats[1] = T.refs.size(); }
+    } else if (g_list_grid) {
+        build_list_grid(geom, tag, density, T);
+        view_of(T, tv, tag[0] < 0, false);
         if (build_stats) { build_stats[0] = T.vox.size(); build_stats[1] = T.refs.size(); }
     }
+    const bool tree = p->use_octree || g_list_grid;
     CameraData cam;
     memcpy(&cam, camera22, sizeof cam);
     hs_counters total;
@@ -293,9 +319,9 @@ static int render_core(const hs_sphere *sph, int n, const float *camera22, const
                     for (int depth = 0; depth < p->max_depth; depth++) {
                         c.rays++;
                         TraceCounters tcn{};
-                        Hit h = p->use_octree ? trace_tree(sc, tv, &tv.planes[0][0], o, d, tcn)
-                                              : trace_list(sc.geom, sc.tag, sc.n, o, d, tcn);
-                        if (g_coop_check && p->use_octree) {
+                        Hit h = tree ? trace_tree(sc, tv, &tv.planes[0][0], o, d, tcn)
+                                     : trace_list(sc.geom, sc.tag, sc.n, o, d, tcn);
+                        if (g_coop_check && tree) {
                             bool tie = false;
                             const Hit m = trace_walk<kWalkMin>(sc, tv, &tv.planes[0][0], o, d, tcn, 0.0f, &tie);
                             unsigned long long bad = 0;
@@ -361,6 +387,7 @@ int hs_render_with_tree(const hs_sphere *sph, int n, const float *camera22, cons
     prolog.insert(prolog.end(), static_cast<const uint32_t *>(big_refs), static_cast<const uint32_t *>(big_refs) + nbig);
     tv.prolog = prolog.data(); tv.nprolog = (int)prolog.size();
     tv.check_visibility = 1;
+    tv.slot0_none = sph[0].mat < 0;
     tv.no_drops = 1;
     for (uint32_t k = 0, e = tv.vis.ent_off[n]; k < e; k++) if (tv.vis.ent_cell[k] & kEntDropped) tv.no_drops = 0;
     return render_core(sph, n, camera22, nullptr, p, 0.f, fb_gamma, nullptr, ctr_out, nullptr, &tv);
@@ -377,7 +404,7 @@ int hs_visible_soundness(const hs_sphere *sph, int n, const void *blob, int spl,
     HostTree T;
     TreeView tv;
     build_host_tree(geom, tag, static_cast<const int32_t *>(blob), spl, 4.0f, T);
-    view_of(T, tv);
+    view_of(T, tv, tag[0] < 0);
     const float *planes = &tv.planes[0][0];
     uint64_t st = seed * 6364136223846793005ull + 1442695040888963407ull;
     auto rnd = [&]() { st = st * 6364136223846793005ull + 1442695040888963407ull; return (float)((st >> 40) & 0xffffff) / 16777216.0f; };
