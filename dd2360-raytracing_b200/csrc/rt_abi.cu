@@ -44,6 +44,7 @@ struct rt_context {
     float grid_density = 4.0f;
     int default_variant = 0;       // RT_RENDER_VARIANT: kernel A/B override for whole test runs (0 = automatic)
     int last_kernel = 0;           // KernelId of the last render launch
+    int last_launches = 0;         // kernels the last render call launched (upstream seeding + render)
     // render scratch
     uint32_t *work_counter = nullptr;
     unsigned long long *counters = nullptr;
@@ -515,6 +516,21 @@ static bool on_device(const rt_context *ctx, const void *ptr) {
     }
     return (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) && at.device == ctx->device;
 }
+// Statistics of the context's last render: its counters, kernel, launch count and the device time between its events.  Waits
+// for the context's stream.
+static int read_render_stats(rt_context *ctx, rt_render_stats *stats) {
+    unsigned long long c[4] = {0, 0, 0, 0};
+    CK(cudaMemcpyAsync(c, ctx->counters, sizeof c, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    memset(stats, 0, sizeof *stats);
+    stats->rays = c[0]; stats->paths = c[1];
+    stats->sphere_tests = c[2]; stats->node_tests = c[3];   // zero unless built with -DRT_COUNTERS
+    stats->kernel_id = ctx->last_kernel;
+    stats->launches = ctx->last_launches;
+    float ms = 0;
+    if (cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1) == cudaSuccess) stats->kernel_ms = ms;
+    return RT_OK;
+}
 static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, bool finalize, rt_render_stats *stats,
                      const ProgressiveIO *prog = nullptr, const PixelList *list = nullptr) {
     if (!ctx || !a || !out_dev) return fail(ctx, RT_ERR_INVALID, "render: null argument");
@@ -650,21 +666,8 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
                          &ctx->last_kernel, list != nullptr));
     }
     CK(cudaEventRecord(ctx->ev1, ctx->stream));
-    if (stats) {
-        unsigned long long c[4] = {0, 0, 0, 0};
-        CK(cudaMemcpyAsync(c, ctx->counters, sizeof c, cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaEventSynchronize(ctx->ev1));
-        CK(cudaStreamSynchronize(ctx->stream));
-        memset(stats, 0, sizeof *stats);
-        stats->rays = c[0]; stats->paths = c[1];
-        stats->sphere_tests = c[2]; stats->node_tests = c[3];   // zero unless built with -DRT_COUNTERS
-        stats->kernel_id = ctx->last_kernel;
-        float ms = 0;
-        cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
-        stats->kernel_ms = ms;
-        stats->launches = launches;
-    }
-    return RT_OK;
+    ctx->last_launches = launches;
+    return stats ? read_render_stats(ctx, stats) : RT_OK;
 }
 
 // curand_init(seed, subsequence, 0) -> {d, v0..v4}: host-side evaluation with the library's own skip matrices (no GPU needed)
@@ -682,17 +685,7 @@ extern "C" int rt_xorwow_state(unsigned long long seed, unsigned long long subse
 extern "C" int rt_last_render_stats(rt_context *ctx, rt_render_stats *stats) {
     if (!ctx || !stats) return fail(ctx, RT_ERR_INVALID, "rt_last_render_stats: null argument");
     CK(cudaSetDevice(ctx->device));
-    unsigned long long c[4] = {0, 0, 0, 0};
-    CK(cudaMemcpyAsync(c, ctx->counters, sizeof c, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    memset(stats, 0, sizeof *stats);
-    stats->rays = c[0]; stats->paths = c[1];
-    stats->sphere_tests = c[2]; stats->node_tests = c[3];
-    stats->kernel_id = ctx->last_kernel;
-    stats->launches = 1;
-    float ms = 0;
-    if (cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1) == cudaSuccess) stats->kernel_ms = ms;
-    return RT_OK;
+    return read_render_stats(ctx, stats);
 }
 
 // test hook: the raw device counters of the last render
@@ -704,96 +697,67 @@ extern "C" int rt_debug_counters(rt_context *ctx, uint64_t out[32]) {
     return RT_OK;
 }
 
-// device scratch of one API call, released on every exit path
-struct Scratch {
-    std::vector<void *> ptrs;
-    ~Scratch() { for (void *p : ptrs) cudaFree(p); }
-    template <typename T>
-    cudaError_t get(T *&out, size_t count) {
-        void *p = nullptr;
-        const cudaError_t e = cudaMalloc(&p, count * sizeof(T) + 16);
-        if (e == cudaSuccess) ptrs.push_back(p);
-        out = static_cast<T *>(p);
-        return e;
-    }
+// One host array of a per-ray query.  `in`: copied to the device before the launch; `out`: copied back after it (zero-filled
+// before, so what the kernel leaves unwritten comes back as zeros); both: copied in and back (the XORWOW states).
+struct HostArray {
+    const void *in;
+    void *out;
+    size_t bytes;
+};
+template <typename T> static HostArray stage_in(const T *h, size_t count) { return HostArray{h, nullptr, count * sizeof(T)}; }
+template <typename T> static HostArray stage_out(T *h, size_t count) { return HostArray{nullptr, h, count * sizeof(T)}; }
+template <typename T> static HostArray stage_inout(T *h, size_t count) { return HostArray{h, h, count * sizeof(T)}; }
+struct DevPtr {                    // a staged array's device address, handed to a launcher as the pointer type it takes
+    void *p;
+    template <typename T> operator T *() const { return static_cast<T *>(p); }
 };
 
-// test hook: closest hit of caller-supplied rays (host arrays of 3 floats per ray)
-extern "C" int rt_trace_rays(rt_context *ctx, int use_octree, int n, const float *org, const float *dir, int *out_idx, float *out_t) {
-    if (!ctx || n < 1 || !org || !dir || !out_idx || !out_t) return fail(ctx, RT_ERR_INVALID, "rt_trace_rays: bad arguments");
-    if (ctx->n < 1) return fail(ctx, RT_ERR_STATE, "rt_trace_rays: no scene");
-    if (use_octree && !ctx->octree->built) return fail(ctx, RT_ERR_STATE, "rt_trace_rays: no octree built");
-    CK(cudaSetDevice(ctx->device));
-    Scratch sc;
-    float *d_o = nullptr, *d_d = nullptr, *d_t = nullptr;
-    int *d_i = nullptr;
-    CK(sc.get(d_o, (size_t)n * 3)); CK(sc.get(d_d, (size_t)n * 3));
-    CK(sc.get(d_t, (size_t)n)); CK(sc.get(d_i, (size_t)n));
-    CK(cudaMemcpyAsync(d_o, org, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_d, dir, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
-    RenderLaunch p;
-    memset(&p, 0, sizeof p);
-    p.scene.geom = ctx->geom; p.scene.matl = ctx->matl; p.scene.tag = ctx->tag; p.scene.n = ctx->n;
-    if (use_octree) p.tree = ctx->octree->view();
-    p.variant = ctx->default_variant;
-    CK(launch_trace_rays(p, use_octree != 0, d_o, d_d, n, d_i, d_t, ctx->stream));
-    CK(cudaMemcpyAsync(out_idx, d_i, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(out_t, d_t, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+// Runs one per-ray query on the context's stream: stages `arrays` in one device allocation (each at a 16-byte aligned offset:
+// the states are read as uint2), calls launch(dev) with their device addresses in the order given, copies the results back and
+// synchronises once.  The allocation is released on every exit path.
+template <typename Launch>
+static int run_staged(rt_context *ctx, std::initializer_list<HostArray> arrays, Launch launch) {
+    auto padded = [](size_t bytes) { return (bytes + 15) & ~(size_t)15; };
+    size_t total = 0;
+    for (const HostArray &a : arrays) total += padded(a.bytes);
+    char *base = nullptr;
+    CK(cudaMalloc(&base, total));
+    struct Release {
+        void *p;
+        ~Release() { cudaFree(p); }
+    } release{base};
+    std::vector<DevPtr> dev;
+    size_t off = 0;
+    for (const HostArray &a : arrays) {
+        if (a.in) CK(cudaMemcpyAsync(base + off, a.in, a.bytes, cudaMemcpyHostToDevice, ctx->stream));
+        else CK(cudaMemsetAsync(base + off, 0, a.bytes, ctx->stream));
+        dev.push_back(DevPtr{base + off});
+        off += padded(a.bytes);
+    }
+    CK(launch(dev.data()));
+    off = 0;
+    for (const HostArray &a : arrays) {
+        if (a.out) CK(cudaMemcpyAsync(a.out, base + off, a.bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        off += padded(a.bytes);
+    }
     CK(cudaStreamSynchronize(ctx->stream));
     return RT_OK;
 }
 
+// test hook: closest hit of caller-supplied rays (host arrays of 3 floats per ray)
+extern "C" int rt_trace_rays(rt_context *ctx, int use_octree, int n, const float *org, const float *dir, int *out_idx, float *out_t) {
+    return rt_trace_rays_ex(ctx, use_octree, RT_PREC_FP32, n, org, dir, out_idx, out_t);
+}
+
 // camera::get_ray (camera.h:45-49) for n (s, t) pairs: each draws its lens sample from ITS OWN XORWOW state (6 words, in/out)
 extern "C" int rt_camera_get_rays(rt_context *ctx, int n, const float *s, const float *t, uint32_t *states6, float *org, float *dir) {
-    if (!ctx || n < 1 || !s || !t || !states6 || !org || !dir) return fail(ctx, RT_ERR_INVALID, "rt_camera_get_rays: bad arguments");
-    if (!ctx->have_camera) return fail(ctx, RT_ERR_STATE, "rt_camera_get_rays: no camera set (rt_camera_set)");
-    CK(cudaSetDevice(ctx->device));
-    Scratch sc;
-    float *d_s = nullptr, *d_t = nullptr, *d_o = nullptr, *d_d = nullptr;
-    uint32_t *d_st = nullptr;
-    CK(sc.get(d_s, (size_t)n)); CK(sc.get(d_t, (size_t)n)); CK(sc.get(d_o, (size_t)n * 3)); CK(sc.get(d_d, (size_t)n * 3)); CK(sc.get(d_st, (size_t)n * 6));
-    CK(cudaMemcpyAsync(d_s, s, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_t, t, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_st, states6, (size_t)n * 24, cudaMemcpyHostToDevice, ctx->stream));
-    CK(launch_camera_rays(ctx->cam_host, n, d_s, d_t, d_st, d_o, d_d, ctx->stream));
-    CK(cudaMemcpyAsync(org, d_o, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(dir, d_d, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(states6, d_st, (size_t)n * 24, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    return RT_OK;
+    return rt_camera_get_rays_ex(ctx, RT_PREC_FP32, n, s, t, states6, org, dir);
 }
 
 // material::scatter (material.h:55-113) + the hit record of sphere::hit (sphere.h:30-33) for n (ray, sphere, t) triples
 extern "C" int rt_scatter_rays(rt_context *ctx, int n, const int *sphere_idx, const float *org, const float *dir, const float *t_hit,
                                uint32_t *states6, float *out_p, float *out_normal, float *out_dir, float *out_atten, int *scattered) {
-    if (!ctx || n < 1 || !sphere_idx || !org || !dir || !t_hit || !states6 || !out_p || !out_normal || !out_dir || !out_atten || !scattered)
-        return fail(ctx, RT_ERR_INVALID, "rt_scatter_rays: bad arguments");
-    if (ctx->n < 1) return fail(ctx, RT_ERR_STATE, "rt_scatter_rays: no scene");
-    CK(cudaSetDevice(ctx->device));
-    Scratch sc;
-    int *d_i = nullptr, *d_sc = nullptr;
-    float *d_o = nullptr, *d_d = nullptr, *d_t = nullptr, *d_p = nullptr, *d_n = nullptr, *d_od = nullptr, *d_a = nullptr;
-    uint32_t *d_st = nullptr;
-    CK(sc.get(d_i, (size_t)n)); CK(sc.get(d_sc, (size_t)n)); CK(sc.get(d_o, (size_t)n * 3)); CK(sc.get(d_d, (size_t)n * 3)); CK(sc.get(d_t, (size_t)n));
-    CK(sc.get(d_p, (size_t)n * 3)); CK(sc.get(d_n, (size_t)n * 3)); CK(sc.get(d_od, (size_t)n * 3)); CK(sc.get(d_a, (size_t)n * 3)); CK(sc.get(d_st, (size_t)n * 6));
-    CK(cudaMemcpyAsync(d_i, sphere_idx, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_o, org, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_d, dir, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_t, t_hit, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_st, states6, (size_t)n * 24, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemsetAsync(d_p, 0, (size_t)n * 12, ctx->stream)); CK(cudaMemsetAsync(d_n, 0, (size_t)n * 12, ctx->stream));
-    CK(cudaMemsetAsync(d_od, 0, (size_t)n * 12, ctx->stream)); CK(cudaMemsetAsync(d_a, 0, (size_t)n * 12, ctx->stream));
-    SceneView sv;
-    sv.geom = ctx->geom; sv.matl = ctx->matl; sv.tag = ctx->tag; sv.n = ctx->n;
-    CK(launch_scatter_rays(sv, n, d_i, d_o, d_d, d_t, d_st, d_p, d_n, d_od, d_a, d_sc, ctx->stream));
-    CK(cudaMemcpyAsync(out_p, d_p, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(out_normal, d_n, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(out_dir, d_od, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(out_atten, d_a, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(scattered, d_sc, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(states6, d_st, (size_t)n * 24, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    return RT_OK;
+    return rt_scatter_rays_ex(ctx, RT_PREC_FP32, n, sphere_idx, org, dir, t_hit, states6, out_p, out_normal, out_dir, out_atten, scattered);
 }
 
 // ---- the same three queries under a given arithmetic ----------------------------------------------------------------------
@@ -805,97 +769,71 @@ extern "C" int rt_trace_rays_ex(rt_context *ctx, int use_octree, int precision, 
     if (!ctx || n < 1 || !org || !dir || !out_idx || !out_t) return fail(ctx, RT_ERR_INVALID, "rt_trace_rays_ex: bad arguments");
     if (ctx->n < 1) return fail(ctx, RT_ERR_STATE, "rt_trace_rays_ex: no scene");
     if (use_octree && !ctx->octree->built) return fail(ctx, RT_ERR_STATE, "rt_trace_rays_ex: no octree built");
-    if (use_octree && ctx->octree->fp16 != (precision == RT_PREC_FP16))
+    const bool fp16 = precision == RT_PREC_FP16;
+    if (use_octree && ctx->octree->fp16 != fp16)
         return fail(ctx, RT_ERR_STATE, "rt_trace_rays_ex: the octree was built for the other precision (rt_octree_build_ex)");
-    if (precision == RT_PREC_FP32) return rt_trace_rays(ctx, use_octree, n, org, dir, out_idx, out_t);
     CK(cudaSetDevice(ctx->device));
     RenderLaunch p;
     memset(&p, 0, sizeof p);
     p.scene.geom = ctx->geom; p.scene.matl = ctx->matl; p.scene.tag = ctx->tag; p.scene.n = ctx->n;
     if (use_octree) p.tree = ctx->octree->view();
-    {
+    if (fp16) {
         const int rc = ensure_half(ctx, kHalfPairs, use_octree != 0, p.tree, 0, 0);
         if (rc) return rc;
+    } else {
+        p.variant = ctx->default_variant;          // RT_RENDER_VARIANT=1: the per-lane walk
     }
-    Scratch sc;
-    float *d_o = nullptr, *d_d = nullptr, *d_t = nullptr;
-    int *d_i = nullptr;
-    CK(sc.get(d_o, (size_t)n * 3)); CK(sc.get(d_d, (size_t)n * 3));
-    CK(sc.get(d_t, (size_t)n)); CK(sc.get(d_i, (size_t)n));
-    CK(cudaMemcpyAsync(d_o, org, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_d, dir, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
-    CK(launch_trace_rays_half(p, use_octree != 0, ctx->geom_h, ctx->half_pairs, d_o, d_d, n, d_i, d_t, ctx->stream));
-    CK(cudaMemcpyAsync(out_idx, d_i, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(out_t, d_t, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    return RT_OK;
+    const size_t N = (size_t)n;
+    return run_staged(ctx, {stage_in(org, 3 * N), stage_in(dir, 3 * N), stage_out(out_idx, N), stage_out(out_t, N)}, [&](const DevPtr *d) {
+        return fp16 ? launch_trace_rays_half(p, use_octree != 0, ctx->geom_h, ctx->half_pairs, d[0], d[1], n, d[2], d[3], ctx->stream)
+                    : launch_trace_rays(p, use_octree != 0, d[0], d[1], n, d[2], d[3], ctx->stream);
+    });
 }
 
 extern "C" int rt_camera_get_rays_ex(rt_context *ctx, int precision, int n, const float *s, const float *t, uint32_t *states6, float *org,
                                      float *dir) {
-    if (precision == RT_PREC_FP32) return rt_camera_get_rays(ctx, n, s, t, states6, org, dir);
-    if (precision != RT_PREC_FP16) return fail(ctx, RT_ERR_INVALID, "rt_camera_get_rays_ex: unknown precision");
+    if (precision != RT_PREC_FP32 && precision != RT_PREC_FP16) return fail(ctx, RT_ERR_INVALID, "rt_camera_get_rays_ex: unknown precision");
     if (!ctx || n < 1 || !s || !t || !states6 || !org || !dir) return fail(ctx, RT_ERR_INVALID, "rt_camera_get_rays_ex: bad arguments");
     if (!ctx->have_camera) return fail(ctx, RT_ERR_STATE, "rt_camera_get_rays_ex: no camera set (rt_camera_set)");
     CK(cudaSetDevice(ctx->device));
-    {
+    const bool fp16 = precision == RT_PREC_FP16;
+    if (fp16) {
         const int rc = ensure_half_camera(ctx, ctx->cam_nx, ctx->cam_ny);      // the camera the FP16 render of this frame size uses
         if (rc) return rc;
     }
-    Scratch sc;
-    float *d_s = nullptr, *d_t = nullptr, *d_o = nullptr, *d_d = nullptr;
-    uint32_t *d_st = nullptr;
-    CK(sc.get(d_s, (size_t)n)); CK(sc.get(d_t, (size_t)n)); CK(sc.get(d_o, (size_t)n * 3)); CK(sc.get(d_d, (size_t)n * 3)); CK(sc.get(d_st, (size_t)n * 6));
-    CK(cudaMemcpyAsync(d_s, s, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_t, t, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_st, states6, (size_t)n * 24, cudaMemcpyHostToDevice, ctx->stream));
-    CK(launch_camera_rays_half(ctx->cam_h, n, d_s, d_t, d_st, d_o, d_d, ctx->stream));
-    CK(cudaMemcpyAsync(org, d_o, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(dir, d_d, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(states6, d_st, (size_t)n * 24, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    return RT_OK;
+    const size_t N = (size_t)n;
+    return run_staged(ctx, {stage_in(s, N), stage_in(t, N), stage_inout(states6, 6 * N), stage_out(org, 3 * N), stage_out(dir, 3 * N)},
+                      [&](const DevPtr *d) {
+                          return fp16 ? launch_camera_rays_half(ctx->cam_h, n, d[0], d[1], d[2], d[3], d[4], ctx->stream)
+                                      : launch_camera_rays(ctx->cam_host, n, d[0], d[1], d[2], d[3], d[4], ctx->stream);
+                      });
 }
 
 extern "C" int rt_scatter_rays_ex(rt_context *ctx, int precision, int n, const int *sphere_idx, const float *org, const float *dir,
                                   const float *t_hit, uint32_t *states6, float *out_p, float *out_normal, float *out_dir, float *out_atten,
                                   int *scattered) {
-    if (precision == RT_PREC_FP32)
-        return rt_scatter_rays(ctx, n, sphere_idx, org, dir, t_hit, states6, out_p, out_normal, out_dir, out_atten, scattered);
-    if (precision != RT_PREC_FP16) return fail(ctx, RT_ERR_INVALID, "rt_scatter_rays_ex: unknown precision");
+    if (precision != RT_PREC_FP32 && precision != RT_PREC_FP16) return fail(ctx, RT_ERR_INVALID, "rt_scatter_rays_ex: unknown precision");
     if (!ctx || n < 1 || !sphere_idx || !org || !dir || !t_hit || !states6 || !out_p || !out_normal || !out_dir || !out_atten || !scattered)
         return fail(ctx, RT_ERR_INVALID, "rt_scatter_rays_ex: bad arguments");
     if (ctx->n < 1) return fail(ctx, RT_ERR_STATE, "rt_scatter_rays_ex: no scene");
     CK(cudaSetDevice(ctx->device));
-    {
+    const bool fp16 = precision == RT_PREC_FP16;
+    if (fp16) {
         const TreeView none{};
         const int rc = ensure_half(ctx, 0u, false, none, 0, 0);
         if (rc) return rc;
     }
-    Scratch sc;
-    int *d_i = nullptr, *d_sc = nullptr;
-    float *d_o = nullptr, *d_d = nullptr, *d_t = nullptr, *d_p = nullptr, *d_n = nullptr, *d_od = nullptr, *d_a = nullptr;
-    uint32_t *d_st = nullptr;
-    CK(sc.get(d_i, (size_t)n)); CK(sc.get(d_sc, (size_t)n)); CK(sc.get(d_o, (size_t)n * 3)); CK(sc.get(d_d, (size_t)n * 3)); CK(sc.get(d_t, (size_t)n));
-    CK(sc.get(d_p, (size_t)n * 3)); CK(sc.get(d_n, (size_t)n * 3)); CK(sc.get(d_od, (size_t)n * 3)); CK(sc.get(d_a, (size_t)n * 3)); CK(sc.get(d_st, (size_t)n * 6));
-    CK(cudaMemcpyAsync(d_i, sphere_idx, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_o, org, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_d, dir, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_t, t_hit, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_st, states6, (size_t)n * 24, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemsetAsync(d_p, 0, (size_t)n * 12, ctx->stream)); CK(cudaMemsetAsync(d_n, 0, (size_t)n * 12, ctx->stream));
-    CK(cudaMemsetAsync(d_od, 0, (size_t)n * 12, ctx->stream)); CK(cudaMemsetAsync(d_a, 0, (size_t)n * 12, ctx->stream));
     SceneView sv;
     sv.geom = ctx->geom; sv.matl = ctx->matl; sv.tag = ctx->tag; sv.n = ctx->n;
-    CK(launch_scatter_rays_half(sv, ctx->geom_h, ctx->matl_h, n, d_i, d_o, d_d, d_t, d_st, d_p, d_n, d_od, d_a, d_sc, ctx->stream));
-    CK(cudaMemcpyAsync(out_p, d_p, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(out_normal, d_n, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(out_dir, d_od, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(out_atten, d_a, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(scattered, d_sc, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(states6, d_st, (size_t)n * 24, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    return RT_OK;
+    const size_t N = (size_t)n;
+    return run_staged(ctx, {stage_in(sphere_idx, N), stage_in(org, 3 * N), stage_in(dir, 3 * N), stage_in(t_hit, N), stage_inout(states6, 6 * N),
+                            stage_out(out_p, 3 * N), stage_out(out_normal, 3 * N), stage_out(out_dir, 3 * N), stage_out(out_atten, 3 * N),
+                            stage_out(scattered, N)},
+                      [&](const DevPtr *d) {
+                          return fp16 ? launch_scatter_rays_half(sv, ctx->geom_h, ctx->matl_h, n, d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7],
+                                                                 d[8], d[9], ctx->stream)
+                                      : launch_scatter_rays(sv, n, d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7], d[8], d[9], ctx->stream);
+                      });
 }
 
 extern "C" int rt_render_accumulate(rt_context *ctx, const rt_render_args *args, float *accum_dev, rt_render_stats *stats) {
@@ -924,32 +862,26 @@ extern "C" int rt_render_progressive(rt_context *ctx, const rt_render_args *args
 }
 
 extern "C" int rt_finalize(rt_context *ctx, const float *accum_dev, float *fb_dev, int nx, int ny, int ns) {
-    if (!ctx || !accum_dev || !fb_dev || nx < 1 || ny < 1 || ns < 1) return fail(ctx, RT_ERR_INVALID, "rt_finalize: bad arguments");
-    CK(cudaSetDevice(ctx->device));
-    CK(launch_finalize(accum_dev, fb_dev, nx, ny, ns, ctx->stream));
-    return RT_OK;
+    if (nx < 1 || ny < 1) return fail(ctx, RT_ERR_INVALID, "rt_finalize: bad arguments");
+    return rt_finalize_ex(ctx, accum_dev, fb_dev, (size_t)nx * ny * 3, ns, RT_PREC_FP32);
 }
 
 extern "C" int rt_finalize_n(rt_context *ctx, const float *accum_dev, float *fb_dev, size_t count, int ns) {
-    if (!ctx || !accum_dev || !fb_dev || ns < 1) return fail(ctx, RT_ERR_INVALID, "rt_finalize_n: bad arguments");
-    if (count == 0) return RT_OK;
-    CK(cudaSetDevice(ctx->device));
-    CK(launch_finalize_n(accum_dev, fb_dev, count, ns, ctx->stream));
-    return RT_OK;
+    return rt_finalize_ex(ctx, accum_dev, fb_dev, count, ns, RT_PREC_FP32);
 }
 
 extern "C" int rt_finalize_ex(rt_context *ctx, const float *accum_dev, float *fb_dev, size_t count, int ns, int precision) {
-    if (precision == RT_PREC_FP32) return rt_finalize_n(ctx, accum_dev, fb_dev, count, ns);
-    if (precision != RT_PREC_FP16) return fail(ctx, RT_ERR_INVALID, "rt_finalize_ex: unknown precision");
+    if (precision != RT_PREC_FP32 && precision != RT_PREC_FP16) return fail(ctx, RT_ERR_INVALID, "rt_finalize_ex: unknown precision");
     if (!ctx || !accum_dev || !fb_dev || ns < 1) return fail(ctx, RT_ERR_INVALID, "rt_finalize_ex: bad arguments");
     if (count == 0) return RT_OK;
     CK(cudaSetDevice(ctx->device));
-    CK(launch_finalize_half(accum_dev, fb_dev, count, ns, ctx->stream));
+    CK(precision == RT_PREC_FP16 ? launch_finalize_half(accum_dev, fb_dev, count, ns, ctx->stream)
+                                 : launch_finalize_n(accum_dev, fb_dev, count, ns, ctx->stream));
     return RT_OK;
 }
 
-extern "C" int rt_render_to_host(rt_context *ctx, const rt_render_args *args, float *fb_host, rt_render_stats *stats) {
-    if (!ctx || !args || !fb_host) return fail(ctx, RT_ERR_INVALID, "rt_render_to_host: null argument");
+// rt_render into the context's scratch frame, grown to the frame's size: the device frame of the host and PPM outputs
+static int render_to_scratch(rt_context *ctx, const rt_render_args *args, rt_render_stats *stats) {
     CK(cudaSetDevice(ctx->device));
     const size_t bytes = (size_t)args->nx * args->ny * 3 * sizeof(float);
     if (bytes > ctx->scratch_fb_bytes) {
@@ -958,9 +890,14 @@ extern "C" int rt_render_to_host(rt_context *ctx, const rt_render_args *args, fl
         CK(cudaMalloc(&ctx->scratch_fb, bytes));
         ctx->scratch_fb_bytes = bytes;
     }
-    const int rc = do_render(ctx, args, ctx->scratch_fb, true, stats);
+    return do_render(ctx, args, ctx->scratch_fb, true, stats);
+}
+
+extern "C" int rt_render_to_host(rt_context *ctx, const rt_render_args *args, float *fb_host, rt_render_stats *stats) {
+    if (!ctx || !args || !fb_host) return fail(ctx, RT_ERR_INVALID, "rt_render_to_host: null argument");
+    const int rc = render_to_scratch(ctx, args, stats);
     if (rc) return rc;
-    CK(cudaMemcpyAsync(fb_host, ctx->scratch_fb, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(fb_host, ctx->scratch_fb, (size_t)args->nx * args->ny * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return RT_OK;
 }
@@ -984,15 +921,7 @@ extern "C" int rt_ppm_read(rt_context *ctx, char *buf_host, size_t cap) {
 
 extern "C" int rt_render_to_ppm(rt_context *ctx, const rt_render_args *args, rt_render_stats *stats, size_t *len_out) {
     if (!ctx || !args) return fail(ctx, RT_ERR_INVALID, "rt_render_to_ppm: null argument");
-    CK(cudaSetDevice(ctx->device));
-    const size_t bytes = (size_t)args->nx * args->ny * 3 * sizeof(float);
-    if (bytes > ctx->scratch_fb_bytes) {
-        cudaFree(ctx->scratch_fb);
-        ctx->scratch_fb = nullptr; ctx->scratch_fb_bytes = 0;
-        CK(cudaMalloc(&ctx->scratch_fb, bytes));
-        ctx->scratch_fb_bytes = bytes;
-    }
-    const int rc = do_render(ctx, args, ctx->scratch_fb, true, stats);
+    const int rc = render_to_scratch(ctx, args, stats);
     if (rc) return rc;
     CK(ppm_format_device(ctx->ppm, ctx->scratch_fb, args->nx, args->ny, ctx->stream, len_out));
     return RT_OK;
@@ -1043,24 +972,32 @@ __global__ void __launch_bounds__(256) k_ffma_peak(float *out, int iters, float 
     if (s == 12345.678f) out[0] = s;   // keeps the chain alive, never true in practice
 }
 
-extern "C" int rt_ffma_peak(rt_context *ctx, float *tflops, float *ms_out) {
+// Rate of a peak probe kernel, launch(blocks, threads, iters): its best device time over three runs after a warm-up run, as
+// TFLOP/s for `iter_flops` per thread and iteration
+template <typename Launch>
+static int peak_rate(rt_context *ctx, double iter_flops, float *tflops, float *ms_out, Launch launch) {
     if (!ctx || !tflops) return RT_ERR_INVALID;
     CK(cudaSetDevice(ctx->device));
     const int blocks = ctx->prop.multiProcessorCount * 8, threads = 256, iters = 4096;
     float best = 1e30f;
     for (int rep = 0; rep < 4; rep++) {
         CK(cudaEventRecord(ctx->ev0, ctx->stream));
-        k_ffma_peak<<<blocks, threads, 0, ctx->stream>>>(reinterpret_cast<float *>(ctx->counters), iters, 1.000001f, 1e-7f);
+        launch(blocks, threads, iters);
         CK(cudaEventRecord(ctx->ev1, ctx->stream));
         CK(cudaEventSynchronize(ctx->ev1));
         float ms = 0;
         cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
         if (rep > 0 && ms < best) best = ms;
     }
-    const double flops = 2.0 * 8 * 16 * (double)iters * blocks * threads;
-    *tflops = (float)(flops / (best * 1e-3) / 1e12);
+    *tflops = (float)(iter_flops * (double)iters * blocks * threads / (best * 1e-3) / 1e12);
     if (ms_out) *ms_out = best;
     return RT_OK;
+}
+
+extern "C" int rt_ffma_peak(rt_context *ctx, float *tflops, float *ms_out) {
+    return peak_rate(ctx, 2.0 * 8 * 16, tflops, ms_out, [&](int blocks, int threads, int iters) {
+        k_ffma_peak<<<blocks, threads, 0, ctx->stream>>>(reinterpret_cast<float *>(ctx->counters), iters, 1.000001f, 1e-7f);
+    });
 }
 
 // the same for packed half arithmetic: dense HFMA2 rate (2 lanes x 2 flop per instruction), the roofline denominator of USE_FP16
@@ -1083,23 +1020,9 @@ __global__ void __launch_bounds__(256) k_hfma2_peak(float *out, int iters, float
 }
 
 extern "C" int rt_hfma2_peak(rt_context *ctx, float *tflops, float *ms_out) {
-    if (!ctx || !tflops) return RT_ERR_INVALID;
-    CK(cudaSetDevice(ctx->device));
-    const int blocks = ctx->prop.multiProcessorCount * 8, threads = 256, iters = 4096;
-    float best = 1e30f;
-    for (int rep = 0; rep < 4; rep++) {
-        CK(cudaEventRecord(ctx->ev0, ctx->stream));
+    return peak_rate(ctx, 4.0 * 8 * 16, tflops, ms_out, [&](int blocks, int threads, int iters) {
         k_hfma2_peak<<<blocks, threads, 0, ctx->stream>>>(reinterpret_cast<float *>(ctx->counters), iters, 0.999f, 1e-3f);
-        CK(cudaEventRecord(ctx->ev1, ctx->stream));
-        CK(cudaEventSynchronize(ctx->ev1));
-        float ms = 0;
-        cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
-        if (rep > 0 && ms < best) best = ms;
-    }
-    const double flops = 4.0 * 8 * 16 * (double)iters * blocks * threads;
-    *tflops = (float)(flops / (best * 1e-3) / 1e12);
-    if (ms_out) *ms_out = best;
-    return RT_OK;
+    });
 }
 
 // ---- device memory helpers -----------------------------------------------------------------------------------------

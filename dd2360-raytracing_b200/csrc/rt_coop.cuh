@@ -415,10 +415,8 @@ __global__ void __launch_bounds__(kRenderThreads, 8) k_render_coop(const __grid_
                     } else {
                         out[0] = col.x; out[1] = col.y; out[2] = col.z;
                     }
-                    if (!LIST && p.state_out) {           // main.cu:136: rand_state[pixel_index] = local_rand_state
-                        uint2 *so = reinterpret_cast<uint2 *>(p.state_out + (size_t)pix * 6);
-                        so[0] = make_uint2(rng.d, rng.v0); so[1] = make_uint2(rng.v1, rng.v2); so[2] = make_uint2(rng.v3, rng.v4);
-                    }
+                    // main.cu:136: rand_state[pixel_index] = local_rand_state
+                    if (!LIST && p.state_out) xorwow_store(p.state_out + (size_t)pix * 6, rng);
                     pix = -1;
                 }
             }

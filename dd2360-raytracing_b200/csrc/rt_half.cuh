@@ -205,6 +205,14 @@ struct CameraH {
     vec3h origin, lower_left_corner, horizontal, vertical, u, v, w;
     hf lens_radius;
 };
+// the 22 halves k_camera_setup_h writes, in CameraData order (origin, llc, horizontal, vertical, u, v, w, lens_radius)
+__device__ __forceinline__ CameraH load_camera_h(const __half *cam_h) {
+    CameraH cam;
+    vec3h *v[7] = {&cam.origin, &cam.lower_left_corner, &cam.horizontal, &cam.vertical, &cam.u, &cam.v, &cam.w};
+    for (int k = 0; k < 7; k++) *v[k] = mkh(cam_h[3 * k], cam_h[3 * k + 1], cam_h[3 * k + 2]);
+    cam.lens_radius = cam_h[21];
+    return cam;
+}
 
 // camera.h:12-18 + :45-49 under USE_FP16
 __device__ __forceinline__ void camera_ray_h(const CameraH &c, const hf s, const hf t, xorwow &rng, vec3h &o, vec3h &d) {

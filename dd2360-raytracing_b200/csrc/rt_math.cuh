@@ -83,4 +83,20 @@ RT_HD float xorwow_uniform(xorwow &s) {
     return fma_((float)xorwow_next(s), 2.3283064e-10f, 1.16415321826934814453125e-10f);
 }
 
+#if defined(__CUDACC__)
+// A stream state in device memory: 6 words {d, v0..v4}, moved as three uint2, so the buffer must be 8-byte aligned (upstream
+// seeds, progressive states, the per-ray queries' states).  The render kernels' start states are read by pixel_stream (__ldg).
+__device__ __forceinline__ xorwow xorwow_load(const uint32_t *st) {
+    const uint2 *s = reinterpret_cast<const uint2 *>(st);
+    const uint2 a = s[0], b = s[1], c = s[2];
+    xorwow rng;
+    rng.d = a.x; rng.v0 = a.y; rng.v1 = b.x; rng.v2 = b.y; rng.v3 = c.x; rng.v4 = c.y;
+    return rng;
+}
+__device__ __forceinline__ void xorwow_store(uint32_t *st, const xorwow &rng) {
+    uint2 *o = reinterpret_cast<uint2 *>(st);
+    o[0] = make_uint2(rng.d, rng.v0); o[1] = make_uint2(rng.v1, rng.v2); o[2] = make_uint2(rng.v3, rng.v4);
+}
+#endif
+
 }  // namespace rt

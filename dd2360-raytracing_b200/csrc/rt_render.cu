@@ -85,8 +85,7 @@ __global__ void k_seed_upstream(uint32_t *__restrict__ states, size_t npix, unsi
     if (pix >= npix) return;
     xorwow s;
     xorwow_seed_subsequence(s, seed, base + pix, tables);
-    uint2 *o = reinterpret_cast<uint2 *>(states + pix * 6);
-    o[0] = make_uint2(s.d, s.v0); o[1] = make_uint2(s.v1, s.v2); o[2] = make_uint2(s.v3, s.v4);
+    xorwow_store(states + pix * 6, s);
 }
 
 cudaError_t launch_seed_upstream(uint32_t *states, size_t npix, unsigned long long seed, unsigned long long subsequence_base,
@@ -104,8 +103,7 @@ __global__ void k_seed_upstream_list(uint32_t *__restrict__ states, const uint32
     if (pix >= npix) return;                  // out of the frame: never traced, its state is never read
     xorwow s;
     xorwow_seed_subsequence(s, seed, pix, tables);
-    uint2 *o = reinterpret_cast<uint2 *>(states + (size_t)k * 6);
-    o[0] = make_uint2(s.d, s.v0); o[1] = make_uint2(s.v1, s.v2); o[2] = make_uint2(s.v3, s.v4);
+    xorwow_store(states + (size_t)k * 6, s);
 }
 
 cudaError_t launch_seed_upstream_list(uint32_t *states, const uint32_t *pixels, int count, size_t npix, unsigned long long seed,
@@ -283,10 +281,8 @@ __global__ void __launch_bounds__(kRenderThreads, 6) k_render(const __grid_const
                     } else {
                         out[0] = col.x; out[1] = col.y; out[2] = col.z;
                     }
-                    if (!LIST && p.state_out) {           // main.cu:136: rand_state[pixel_index] = local_rand_state
-                        uint2 *so = reinterpret_cast<uint2 *>(p.state_out + (size_t)pix * 6);
-                        so[0] = make_uint2(rng.d, rng.v0); so[1] = make_uint2(rng.v1, rng.v2); so[2] = make_uint2(rng.v3, rng.v4);
-                    }
+                    // main.cu:136: rand_state[pixel_index] = local_rand_state
+                    if (!LIST && p.state_out) xorwow_store(p.state_out + (size_t)pix * 6, rng);
                     pix = -1;
                 }
             }
@@ -348,12 +344,16 @@ cudaError_t launch_camera_setup_half(const float lookfrom[3], const float lookat
                                            vfov, nx, ny, aspect_override, aperture, focus_dist, cam_h);
     return cudaGetLastError();
 }
+// the half kernels' views of the context's USE_FP16 pair lists and node tables
+static void half_views(const HalfPairs &hp, h16::PairView &pv, h16::NodeTab &nt) {
+    pv.geom = hp.geom; pv.idx = hp.idx; pv.start = hp.start;
+    nt.ent = hp.nodes; nt.count = hp.node_count;
+}
 cudaError_t launch_render_half(const RenderLaunch &p, bool octree, const uint2 *geom_h, const uint2 *matl_h, const __half *cam_h,
                                const HalfPairs &hp, int sm_count, cudaStream_t st, int *blocks_out, bool list) {
     h16::PairView pv;
-    pv.geom = hp.geom; pv.idx = hp.idx; pv.start = hp.start;
     h16::NodeTab nt;
-    nt.ent = hp.nodes; nt.count = hp.node_count;
+    half_views(hp, pv, nt);
     const bool prog = p.accumulate || p.state_out;
     auto kern = list ? (octree ? h16::k_render_h<true, false, true> : h16::k_render_h<false, false, true>)
               : octree ? (prog ? h16::k_render_h<true, true> : h16::k_render_h<true, false>)
@@ -369,9 +369,8 @@ cudaError_t launch_finalize_half(const float *accum, float *fb, size_t count, in
 cudaError_t launch_trace_rays_half(const RenderLaunch &p, bool octree, const uint2 *geom_h, const HalfPairs &hp, const float *org, const float *dir,
                                    int n, int *out_idx, float *out_t, cudaStream_t st) {
     h16::PairView pv;
-    pv.geom = hp.geom; pv.idx = hp.idx; pv.start = hp.start;
     h16::NodeTab nt;
-    nt.ent = hp.nodes; nt.count = hp.node_count;
+    half_views(hp, pv, nt);
     // whole blocks of whole warps: coop_trace_h is a full-warp collective
     const unsigned blocks = (unsigned)((n + kRenderThreads - 1) / kRenderThreads);
     if (octree) h16::k_trace_rays_h<true><<<blocks, kRenderThreads, 0, st>>>(p, geom_h, pv, nt, org, dir, n, out_idx, out_t);
@@ -461,14 +460,13 @@ __global__ void k_camera_rays(const CameraData cam, int n, const float *__restri
                               float *__restrict__ org, float *__restrict__ dir) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    xorwow rng;
     uint32_t *st = states + (size_t)i * 6;
-    rng.d = st[0]; rng.v0 = st[1]; rng.v1 = st[2]; rng.v2 = st[3]; rng.v3 = st[4]; rng.v4 = st[5];
+    xorwow rng = xorwow_load(st);
     vec3f o, d;
     camera_ray(cam, s[i], t[i], rng, o, d);
     org[3 * i] = o.x; org[3 * i + 1] = o.y; org[3 * i + 2] = o.z;
     dir[3 * i] = d.x; dir[3 * i + 1] = d.y; dir[3 * i + 2] = d.z;
-    st[0] = rng.d; st[1] = rng.v0; st[2] = rng.v1; st[3] = rng.v2; st[4] = rng.v3; st[5] = rng.v4;
+    xorwow_store(st, rng);
 }
 cudaError_t launch_camera_rays(const CameraData &cam, int n, const float *s, const float *t, uint32_t *states, float *org, float *dir,
                                cudaStream_t st) {
@@ -486,9 +484,8 @@ __global__ void k_scatter_rays(const SceneView sc, int n, const int *__restrict_
     if (i >= n) return;
     const int idx = sphere_idx[i];
     if (idx < 0 || idx >= sc.n || sc.tag[idx] < 0) { scattered[i] = -1; return; }
-    xorwow rng;
     uint32_t *st = states + (size_t)i * 6;
-    rng.d = st[0]; rng.v0 = st[1]; rng.v1 = st[2]; rng.v2 = st[3]; rng.v3 = st[4]; rng.v4 = st[5];
+    xorwow rng = xorwow_load(st);
     const vec3f o = mk(org[3 * i], org[3 * i + 1], org[3 * i + 2]), d = mk(dir[3 * i], dir[3 * i + 1], dir[3 * i + 2]);
     vec3f hp, hn, att, dn = mk(0.f, 0.f, 0.f);
     hit_point(sc.geom[idx], o, d, t_hit[i], hp, hn);
@@ -498,7 +495,7 @@ __global__ void k_scatter_rays(const SceneView sc, int n, const int *__restrict_
     out_dir[3 * i] = dn.x; out_dir[3 * i + 1] = dn.y; out_dir[3 * i + 2] = dn.z;
     out_att[3 * i] = att.x; out_att[3 * i + 1] = att.y; out_att[3 * i + 2] = att.z;
     scattered[i] = go ? 1 : 0;
-    st[0] = rng.d; st[1] = rng.v0; st[2] = rng.v1; st[3] = rng.v2; st[4] = rng.v3; st[5] = rng.v4;
+    xorwow_store(st, rng);
 }
 cudaError_t launch_scatter_rays(const SceneView &sc, int n, const int *sphere_idx, const float *org, const float *dir, const float *t_hit,
                                 uint32_t *states, float *out_p, float *out_n, float *out_dir, float *out_att, int *scattered, cudaStream_t st) {
@@ -516,9 +513,6 @@ cudaError_t launch_finalize_n(const float *accum, float *fb, size_t n3, int ns, 
     const float inv_ns = (float)(1.0 / (double)(float)ns);
     k_finalize<<<(unsigned)((n3 + 255) / 256), 256, 0, st>>>(accum, fb, n3, inv_ns);
     return cudaGetLastError();
-}
-cudaError_t launch_finalize(const float *accum, float *fb, int nx, int ny, int ns, cudaStream_t st) {
-    return launch_finalize_n(accum, fb, (size_t)nx * ny * 3, ns, st);
 }
 
 cudaError_t launch_render(const RenderLaunch &p, bool octree, int sm_count, size_t smem_limit, cudaStream_t st,

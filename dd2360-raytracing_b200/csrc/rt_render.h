@@ -98,7 +98,6 @@ struct PpmWorkspace {
 };
 cudaError_t ppm_format_device(PpmWorkspace &ws, const float *fb, int nx, int ny, cudaStream_t st, size_t *len_out);
 void ppm_free(PpmWorkspace &ws);
-cudaError_t launch_finalize(const float *accum, float *fb, int nx, int ny, int ns, cudaStream_t st);
 cudaError_t launch_finalize_n(const float *accum, float *fb, size_t count, int ns, cudaStream_t st);
 
 }  // namespace rt

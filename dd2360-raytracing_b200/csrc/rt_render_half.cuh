@@ -164,12 +164,7 @@ k_render_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geo
     __shared__ hf planes_h[3 * kPlanes];      // the slab planes of the octree boxes, rounded to half as AABB's real_t members are
     if (OCTREE && threadIdx.x < 3 * kPlanes) planes_h[threadIdx.x] = f2h((&p.tree.planes[0][0])[threadIdx.x]);
     __syncthreads();
-    CameraH cam;
-    {
-        vec3h *v[7] = {&cam.origin, &cam.lower_left_corner, &cam.horizontal, &cam.vertical, &cam.u, &cam.v, &cam.w};
-        for (int k = 0; k < 7; k++) *v[k] = mkh(cam_h[3 * k], cam_h[3 * k + 1], cam_h[3 * k + 2]);
-        cam.lens_radius = cam_h[21];
-    }
+    const CameraH cam = load_camera_h(cam_h);
     const unsigned lane = threadIdx.x & 31u;
     if (lane == 0) {
         coop_sm[threadIdx.x >> 5].tail = 0u;
@@ -257,10 +252,8 @@ k_render_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geo
                     } else {
                         out[0] = h2f(vx(col)); out[1] = h2f(vy(col)); out[2] = h2f(col.z);
                     }
-                    if (PROG && p.state_out) {   // main.cu:136: rand_state[pixel_index] = local_rand_state
-                        uint2 *so = reinterpret_cast<uint2 *>(p.state_out + (size_t)pix * 6);
-                        so[0] = make_uint2(rng.d, rng.v0); so[1] = make_uint2(rng.v1, rng.v2); so[2] = make_uint2(rng.v3, rng.v4);
-                    }
+                    // main.cu:136: rand_state[pixel_index] = local_rand_state
+                    if (PROG && p.state_out) xorwow_store(p.state_out + (size_t)pix * 6, rng);
                     pix = -1;
                 }
             }
@@ -332,20 +325,14 @@ __global__ void k_camera_rays_h(const __half *__restrict__ cam_h, int n, const f
                                 uint32_t *__restrict__ states, float *__restrict__ org, float *__restrict__ dir) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    CameraH cam;
-    {
-        vec3h *v[7] = {&cam.origin, &cam.lower_left_corner, &cam.horizontal, &cam.vertical, &cam.u, &cam.v, &cam.w};
-        for (int k = 0; k < 7; k++) *v[k] = mkh(cam_h[3 * k], cam_h[3 * k + 1], cam_h[3 * k + 2]);
-        cam.lens_radius = cam_h[21];
-    }
-    xorwow rng;
+    const CameraH cam = load_camera_h(cam_h);
     uint32_t *st = states + (size_t)i * 6;
-    rng.d = st[0]; rng.v0 = st[1]; rng.v1 = st[2]; rng.v2 = st[3]; rng.v3 = st[4]; rng.v4 = st[5];
+    xorwow rng = xorwow_load(st);
     vec3h o, d;
     camera_ray_h(cam, f2h(s[i]), f2h(t[i]), rng, o, d);
     org[3 * i] = h2f(vx(o)); org[3 * i + 1] = h2f(vy(o)); org[3 * i + 2] = h2f(o.z);
     dir[3 * i] = h2f(vx(d)); dir[3 * i + 1] = h2f(vy(d)); dir[3 * i + 2] = h2f(d.z);
-    st[0] = rng.d; st[1] = rng.v0; st[2] = rng.v1; st[3] = rng.v2; st[4] = rng.v3; st[5] = rng.v4;
+    xorwow_store(st, rng);
 }
 
 // sphere.h:30-33 + material.h:55-113 for (ray, sphere, t): hit point, normal, scattered direction, attenuation, and
@@ -358,9 +345,8 @@ __global__ void k_scatter_rays_h(const uint2 *__restrict__ geom_h, const uint2 *
     if (i >= n) return;
     const int idx = sphere_idx[i];
     if (idx < 0 || idx >= nsph || tag[idx] < 0) { scattered[i] = -1; return; }
-    xorwow rng;
     uint32_t *st = states + (size_t)i * 6;
-    rng.d = st[0]; rng.v0 = st[1]; rng.v1 = st[2]; rng.v2 = st[3]; rng.v3 = st[4]; rng.v4 = st[5];
+    xorwow rng = xorwow_load(st);
     const vec3h o = mkh_f(org[3 * i], org[3 * i + 1], org[3 * i + 2]), d = mkh_f(dir[3 * i], dir[3 * i + 1], dir[3 * i + 2]);
     const hf zero = f2h(0.0f);
     vec3h hp, hn, att, dn = mkh(zero, zero, zero);
@@ -371,7 +357,7 @@ __global__ void k_scatter_rays_h(const uint2 *__restrict__ geom_h, const uint2 *
     out_dir[3 * i] = h2f(vx(dn)); out_dir[3 * i + 1] = h2f(vy(dn)); out_dir[3 * i + 2] = h2f(dn.z);
     out_att[3 * i] = h2f(vx(att)); out_att[3 * i + 1] = h2f(vy(att)); out_att[3 * i + 2] = h2f(att.z);
     scattered[i] = go ? 1 : 0;
-    st[0] = rng.d; st[1] = rng.v0; st[2] = rng.v1; st[3] = rng.v2; st[4] = rng.v3; st[5] = rng.v4;
+    xorwow_store(st, rng);
 }
 
 }  // namespace h16

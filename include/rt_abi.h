@@ -152,7 +152,8 @@ int rt_xorwow_state(unsigned long long seed, unsigned long long subsequence, uin
  * [3] visibility line tests and [4] voxel steps. */
 int rt_debug_counters(rt_context *ctx, uint64_t out[32]);
 
-/* test hook: closest hit (sphere index or -1, and t) of n caller-supplied rays — hitTree / hitable_list::hit per ray */
+/* test hook: closest hit (sphere index or -1, and t) of n caller-supplied rays — hitTree / hitable_list::hit per ray.  An octree
+ * query on a tree built for RT_PREC_FP16 is RT_ERR_STATE ("other precision"), as in rt_trace_rays_ex. */
 int rt_trace_rays(rt_context *ctx, int use_octree, int n, const float *org, const float *dir, int *out_idx, float *out_t);
 
 /* camera::get_ray(s, t, &rand_state) (camera.h:45-49) for n (s, t) pairs, each drawing its lens sample from its own XORWOW

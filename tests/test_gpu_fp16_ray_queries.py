@@ -190,6 +190,7 @@ def test_fp16_queries_do_not_depend_on_the_batch(rt, pkg, n, spl, octree):
         return [r[::-1] for r in res] if rev else res
     base = scat(slice(0, H))
     assert (base[4][::97] == -1).all() and np.array_equal(base[5][::97], sst0[::97])
+    assert all((base[k][base[4] == -1] == 0).all() for k in range(4))        # p, normal, dir, atten of a non-sphere: zeros
     assert set(np.unique(base[4][base[4] >= 0])) <= {0, 1} and (base[4] == 1).sum() > H // 2
     for k in range(4):
         assert _same(base[k], _h(base[k]))
@@ -222,16 +223,22 @@ def test_fp32_ex_entry_points_are_the_fp32_ones(rt, pkg):
     assert _same(o_a, o_b) and _same(d_a, d_b) and np.array_equal(st_a, st_b)
     gi, gt = rt.trace_rays(org, dirs, True)
     hits = np.nonzero(gi >= 0)[0]
-    st_a = np.stack([pkg.xorwow_state(1984 + k, 0) for k in range(len(hits))]).astype(np.uint32)
-    st_b = st_a.copy()
-    a = {k: np.zeros((len(hits), 3), np.float32) for k in ("p", "normal", "dir", "atten")}
-    a["scattered"] = np.zeros(len(hits), np.int32)
-    hi, ho, hd, ht = (np.ascontiguousarray(x[hits]) for x in (gi, org, dirs, gt))
-    assert L.rt_scatter_rays(rt._ctx, len(hits), hi.ctypes.data, ho.ctypes.data, hd.ctypes.data, ht.ctypes.data, st_a.ctypes.data,
+    # the hits, then three entries that are not a sphere (scattered = -1: zero outputs, state untouched)
+    hi = np.concatenate([gi[hits], np.array([-1, 8000, 1 << 30], np.int32)])
+    ho, hd, ht = (np.concatenate([x[hits], x[:3]]) for x in (org, dirs, gt))
+    m = len(hi)
+    st0 = np.stack([pkg.xorwow_state(1984 + k, 0) for k in range(m)]).astype(np.uint32)
+    st_a, st_b = st0.copy(), st0.copy()
+    a = {k: np.full((m, 3), 7.0, np.float32) for k in ("p", "normal", "dir", "atten")}
+    a["scattered"] = np.zeros(m, np.int32)
+    assert L.rt_scatter_rays(rt._ctx, m, hi.ctypes.data, ho.ctypes.data, hd.ctypes.data, ht.ctypes.data, st_a.ctypes.data,
                              a["p"].ctypes.data, a["normal"].ctypes.data, a["dir"].ctypes.data, a["atten"].ctypes.data,
                              a["scattered"].ctypes.data) == 0
     b = rt.scatter_rays(hi, ho, hd, ht, st_b, precision=pkg.PREC_FP32)
     assert all(_same(a[k], b[k]) for k in a) and np.array_equal(st_a, st_b)
+    none = a["scattered"] == -1
+    assert np.array_equal(np.nonzero(none)[0], np.arange(len(hits), m)) and np.array_equal(st_a[none], st0[none])
+    assert all((a[k][none] == 0).all() for k in ("p", "normal", "dir", "atten"))
 
 
 # ---- the FP16 Octree export -----------------------------------------------------------------------------------------------------
@@ -427,6 +434,8 @@ def test_fp16_query_errors(rt, pkg):
     assert trace(rt, 0, pkg.PREC_FP16) == 0                              # the flat list needs no tree
     rt.build_octree(30, precision=pkg.PREC_FP16)
     assert trace(rt, 1, pkg.PREC_FP32) == RT_ERR_STATE
+    assert L.rt_trace_rays(rt._ctx, 1, 1, p(one), p(one), p(oi), p(one)) == RT_ERR_STATE        # the entry point without a precision too
+    assert b"other precision" in L.rt_last_error(rt._ctx)
     assert trace(rt, 1, pkg.PREC_FP16) == 0
     with pytest.raises(pkg.RtError, match="other precision"):
         rt.trace_rays(one[:3].reshape(1, 3), one[:3].reshape(1, 3), True)

@@ -134,12 +134,15 @@ def test_stats_null_is_asynchronous_and_reported_afterwards(rt, pkg):
     nx, ny, ns = 64, 32, 2
     pix = torch.from_numpy(pkg.window_pixels(nx, ny, 0, nx, 0, ny).view(np.int32)).cuda()
     out = torch.empty((pix.numel(), 3), dtype=torch.float32, device="cuda")
-    assert rt.render_pixels_device(rt.args(nx, ny, ns, True), pix.data_ptr(), pix.numel(), out.data_ptr(), want_stats=False) is None
-    st = rt.last_render_stats()
-    ref, fst = _frame(rt, rt.args(nx, ny, ns, True), True)
-    assert st["rays"] == fst["rays"] and st["paths"] == fst["paths"] and st["kernel_id"] == fst["kernel_id"]
-    got = out.cpu().numpy()
-    assert np.array_equal(_bits(got), _bits(ref[pix.cpu().numpy().view(np.uint32)]))
+    for seed_mode, launches in ((pkg.SEED_HEAD, 1), (pkg.SEED_UPSTREAM, 2)):      # upstream: the seeding kernel, then the render
+        args = rt.args(nx, ny, ns, True, seed_mode=seed_mode)
+        assert rt.render_pixels_device(args, pix.data_ptr(), pix.numel(), out.data_ptr(), want_stats=False) is None
+        st = rt.last_render_stats()
+        ref, fst = _frame(rt, args, True)
+        assert st["rays"] == fst["rays"] and st["paths"] == fst["paths"] and st["kernel_id"] == fst["kernel_id"]
+        assert st["launches"] == fst["launches"] == launches, seed_mode
+        got = out.cpu().numpy()
+        assert np.array_equal(_bits(got), _bits(ref[pix.cpu().numpy().view(np.uint32)])), seed_mode
 
 
 @gpu
