@@ -7,7 +7,7 @@
 // ~13 references each, 0..75 candidates per ray — and 44 % of the lane-trips of the walk loop doing work.  The exact
 // root evaluation (IEEE sqrt + two divisions) sat in that loop under a branch taken by 3.6 lanes.
 //
-// Here the lanes still own one pixel chain each (ray, RNG and pixel state in registers, shading as in k_render), but the
+// Here the lanes still own one pixel chain each (ray, RNG and pixel state in registers: rt_chain.cuh), but the
 // candidate tests of the warp's 32 rays are pooled:
 //   round   : every walking lane publishes the reference range of its CURRENT voxel; an inclusive warp scan lays the
 //             ranges end to end (a flat list of `total` items of ITEMS consecutive references of one ray);
@@ -302,10 +302,9 @@ __device__ __forceinline__ Hit coop_trace_tree(WarpShared &ws, const SceneView &
     return h;
 }
 
-// The pixel state a lane does not need while its warp traces (RNG stream, attenuation, colour sum, pixel bookkeeping: 21 words)
-// is parked in shared memory during coop_trace instead of being spilled to local memory by the register allocator; that is
-// what lets 8 blocks per SM be resident (-9 % frame time over 6 blocks without parking, profiles r02r-r02t).
-// LIST: pixel-list instances, as k_render's (`pix` is the lane's list slot).
+// The lanes' pixel chains (rt_chain.cuh) are parked in shared memory during coop_trace (Chain::park) instead of being spilled to
+// local memory by the register allocator; that is what lets 8 blocks per SM be resident (-9 % frame time over 6 blocks without
+// parking, profiles r02r-r02t).  LIST: pixel-list instances, as k_render's.
 template <int ITEMS, bool LIST = false>
 __global__ void __launch_bounds__(kRenderThreads, 8) k_render_coop(const __grid_constant__ RenderLaunch p) {
     __shared__ WarpShared wsh[kRenderThreads / 32];
@@ -313,126 +312,18 @@ __global__ void __launch_bounds__(kRenderThreads, 8) k_render_coop(const __grid_
     WarpShared &ws = wsh[threadIdx.x >> 5];
     const SceneView sc = p.scene;
     const unsigned lane = threadIdx.x & 31u;
-    const uint32_t gwarp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
 
-    int pix = -1, pi = 0, pj = 0;
-    int s = 0, depth = 0;
-    xorwow rng;
-    rng.d = rng.v0 = rng.v1 = rng.v2 = rng.v3 = rng.v4 = 0;
-    vec3f o = mk(0, 0, 0), d = mk(0, 0, 1), att = mk(1, 1, 1), col = mk(0, 0, 0);
-    uint32_t nrays = 0, npaths = 0;
     TraceCounters tc;
     tc.sphere_tests = tc.node_tests = tc.voxel_steps = 0;
-    bool exhausted = false;
-    uint32_t stock_next = gwarp * 32u, stock_end = stock_next + 32u;   // the first tile needs no atomic: the queue head starts past the grid
-    const uint32_t batch = claim_batch(p);
-    const float inv_ns = __fdiv_rn(1.0f, (float)p.ns_total);   // vec3.h:137-144: k = 1.0/t
-
-    while (true) {
-        while (true) {      // claim pixels for idle lanes (ballot/popc-compacted queue pop, whole tiles per warp)
-            const bool need = pix < 0 && !exhausted;
-            const unsigned m = __ballot_sync(kFull, need);
-            if (!m) break;
-            const uint32_t item = claim_items(p, m, lane, stock_next, stock_end, batch);
-            if (need) {
-                if (item >= p.total_items) {
-                    exhausted = true;
-                } else if (LIST ? list_to_pixel(p, item, pi, pj) : item_to_pixel(p, item, pi, pj)) {
-                    pix = LIST ? (int)item : pj * p.nx + pi;
-                    s = 0; depth = 0;
-                    col = mk(0, 0, 0);
-                    if (!LIST && p.accumulate) {          // progressive: continue the pixel's sum exactly where the last call left it
-                        const float *acc = p.out + (size_t)pix * 3;
-                        col = mk(acc[0], acc[1], acc[2]);
-                    }
-                    pixel_stream(p, LIST && !p.seed_states ? pj * p.nx + pi : pix, rng);
-                }
-            }
-        }
-        if (!__ballot_sync(kFull, pix >= 0)) break;
-
-        const bool has = pix >= 0;
-        if (has && depth == 0) {   // new sample: main.cu:104-106
-            const float u = div_(add_((float)pi, xorwow_uniform(rng)), (float)p.nx);
-            const float v = div_(add_((float)pj, xorwow_uniform(rng)), (float)p.ny);
-            camera_ray(p.cam, u, v, rng, o, d);
-            att = mk(1.0f, 1.0f, 1.0f);
-            npaths++;
-        }
-        if (has) nrays++;
-        {
-            const unsigned t = threadIdx.x;
-            park[0][t] = rng.d; park[1][t] = rng.v0; park[2][t] = rng.v1; park[3][t] = rng.v2; park[4][t] = rng.v3; park[5][t] = rng.v4;
-            park[6][t] = __float_as_uint(att.x); park[7][t] = __float_as_uint(att.y); park[8][t] = __float_as_uint(att.z);
-            park[9][t] = __float_as_uint(col.x); park[10][t] = __float_as_uint(col.y); park[11][t] = __float_as_uint(col.z);
-            park[12][t] = (uint32_t)pi; park[13][t] = (uint32_t)pj; park[14][t] = (uint32_t)s; park[15][t] = (uint32_t)depth;
-            park[16][t] = (uint32_t)pix; park[17][t] = nrays; park[18][t] = npaths; park[19][t] = stock_next; park[20][t] = stock_end;
-        }
+    run_chains<LIST>(p, ChainF32(p), claim_batch(p), [&](Chain &c, const bool has) {
+        c.park(park, threadIdx.x);
         __syncwarp();
-        const Hit h = coop_trace_tree<ITEMS>(ws, sc, p.tree, &p.tree.planes[0][0], lane, has, o, d, tc);
-        {
-            const unsigned t = threadIdx.x;
-            rng.d = park[0][t]; rng.v0 = park[1][t]; rng.v1 = park[2][t]; rng.v2 = park[3][t]; rng.v3 = park[4][t]; rng.v4 = park[5][t];
-            att = mk(__uint_as_float(park[6][t]), __uint_as_float(park[7][t]), __uint_as_float(park[8][t]));
-            col = mk(__uint_as_float(park[9][t]), __uint_as_float(park[10][t]), __uint_as_float(park[11][t]));
-            pi = (int)park[12][t]; pj = (int)park[13][t]; s = (int)park[14][t]; depth = (int)park[15][t];
-            pix = (int)park[16][t]; nrays = park[17][t]; npaths = park[18][t]; stock_next = park[19][t]; stock_end = park[20][t];
-            const float4 ro = ws.ro[lane], rd = ws.rd[lane];          // the ray itself is still where coop_trace published it
-            o = mk(ro.x, ro.y, ro.z); d = mk(rd.x, rd.y, rd.z);
-        }
-        if (pix >= 0) {   // ---- one iteration of color()'s loop (main.cu:47-73) ----
-            bool sample_done = false;
-            vec3f contrib = mk(0, 0, 0);
-            if (h.idx >= 0) {
-                const float4 g = __ldg(sc.geom + h.idx);
-                const float4 m = __ldg(sc.matl + h.idx);
-                const int tag = __ldg(sc.tag + h.idx);
-                vec3f hp, hn, a, dn;
-                hit_point(g, o, d, h.t, hp, hn);
-                if (scatter(tag, m, d, hp, hn, a, dn, rng)) {
-                    att = mk(mul_(att.x, a.x), mul_(att.y, a.y), mul_(att.z, a.z));
-                    o = hp; d = dn;
-                    depth++;
-                    if (depth >= p.max_depth) sample_done = true;        // main.cu:74: return black
-                } else {
-                    sample_done = true;                                   // absorbed: main.cu:64
-                }
-            } else {
-                const vec3f c = sky(d);
-                contrib = mk(mul_(att.x, c.x), mul_(att.y, c.y), mul_(att.z, c.z));
-                sample_done = true;
-            }
-            if (sample_done) {
-                col = mk(add_(col.x, contrib.x), add_(col.y, contrib.y), add_(col.z, contrib.z));   // main.cu:107
-                depth = 0;
-                s++;
-                if (s >= p.ns_local) {
-                    float *out = p.out + (size_t)pix * 3;
-                    if (p.finalize) {   // main.cu:111-115
-                        out[0] = sqrt_(mul_(col.x, inv_ns));
-                        out[1] = sqrt_(mul_(col.y, inv_ns));
-                        out[2] = sqrt_(mul_(col.z, inv_ns));
-                    } else {
-                        out[0] = col.x; out[1] = col.y; out[2] = col.z;
-                    }
-                    // main.cu:136: rand_state[pixel_index] = local_rand_state
-                    if (!LIST && p.state_out) xorwow_store(p.state_out + (size_t)pix * 6, rng);
-                    pix = -1;
-                }
-            }
-        }
-        __syncwarp();
-    }
-
-    unsigned long long r64 = nrays, p64 = npaths;
-    for (int off = 16; off > 0; off >>= 1) {
-        r64 += __shfl_xor_sync(kFull, r64, off);
-        p64 += __shfl_xor_sync(kFull, p64, off);
-    }
-    if (lane == 0) {
-        atomicAdd(p.counters + 0, r64);
-        atomicAdd(p.counters + 1, p64);
-    }
+        const Hit h = coop_trace_tree<ITEMS>(ws, sc, p.tree, &p.tree.planes[0][0], lane, has, c.o, c.d, tc);
+        c.unpark(park, threadIdx.x);
+        const float4 ro = ws.ro[lane], rd = ws.rd[lane];          // the ray itself is still where coop_trace published it
+        c.o = mk(ro.x, ro.y, ro.z); c.d = mk(rd.x, rd.y, rd.z);
+        return h;
+    });
 #ifdef RT_COUNTERS
     unsigned long long c64[3] = {tc.sphere_tests, tc.node_tests, tc.voxel_steps};
     for (int k = 0; k < 3; k++) {

@@ -3,11 +3,8 @@
 // Reference shape: thread = pixel, 8x8 blocks, each thread runs its ns samples x <=50 bounces serially, so a warp
 // lives as long as its slowest pixel and every bounce pays two virtual calls and an AoS pointer chase.
 // This kernel:
-//   * persistent threads: the grid is sized to what is resident on the SMs; every lane owns one pixel at a time
-//     and runs its sample chain bounce by bounce (the chain is inherently serial: all samples of a pixel draw from
-//     one XORWOW stream, SURVEY D8).  When a lane's pixel is finished it claims the next one from a global queue;
-//     claims are compacted per warp with __ballot_sync/__popc so one atomic serves the whole warp.  Lanes therefore
-//     always have a ray to trace, whatever the path lengths of their neighbours;
+//   * persistent threads: the grid is sized to what is resident on the SMs; every lane owns one pixel chain at a time and
+//     claims the next pixel from a queue when it is done (the lane loop of rt_chain.cuh, shared with k_render_coop);
 //   * pixels are queued in 8x4 tiles so that the 32 lanes of a warp start on neighbouring pixels (coherent rays);
 //   * XORWOW state lives in registers and is seeded in place (render_init fused; no 48-byte state array);
 //   * spheres are SoA float4, materials are tag-dispatched (no device heap, no vtables);
@@ -168,8 +165,9 @@ __device__ __forceinline__ uint32_t claim_batch(const RenderLaunch &p) {   // pi
     return p.total_items / (gridDim.x * blockDim.x) >= 4u ? 32u : 1u;
 }
 
-// LIST: pixel-list instances (rt_render_pixels, list_to_pixel); `pix` is then the lane's list slot.  The whole-frame instances
-// (LIST = false) compile to the same SASS as before the list instances existed.
+#include "rt_chain.cuh"
+
+// LIST: pixel-list instances (rt_render_pixels, list_to_pixel); a chain's `pix` is then the lane's list slot.
 template <bool OCTREE, bool GEOM_SMEM, bool LIST = false>
 __global__ void __launch_bounds__(kRenderThreads, 6) k_render(const __grid_constant__ RenderLaunch p) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -192,115 +190,19 @@ __global__ void __launch_bounds__(kRenderThreads, 6) k_render(const __grid_const
         mbar_wait(&bar, 0);
     }
 
-    const unsigned lane = threadIdx.x & 31u;
-    const uint32_t gwarp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-
-    // per-lane path state
-    int pix = -1, pi = 0, pj = 0;
-    int s = 0, depth = 0;
-    xorwow rng;
-    rng.d = rng.v0 = rng.v1 = rng.v2 = rng.v3 = rng.v4 = 0;
-    vec3f o = mk(0, 0, 0), d = mk(0, 0, 1), att = mk(1, 1, 1), col = mk(0, 0, 0);
-    uint32_t nrays = 0, npaths = 0;
     TraceCounters tc;
     tc.sphere_tests = tc.node_tests = tc.voxel_steps = 0;
-    bool exhausted = false;
-    uint32_t stock_next = gwarp * 32u, stock_end = stock_next + 32u;   // the first tile needs no atomic: the queue head starts past the grid
-    const uint32_t batch = claim_batch(p);
-    const float inv_ns = __fdiv_rn(1.0f, (float)p.ns_total);   // vec3.h:137-144: k = 1.0/t
-
-    while (true) {
-        // ---- claim pixels for idle lanes (ballot/popc-compacted queue pop) ----
-        while (true) {
-            const bool need = pix < 0 && !exhausted;
-            const unsigned m = __ballot_sync(0xffffffffu, need);
-            if (!m) break;
-            const uint32_t item = claim_items(p, m, lane, stock_next, stock_end, batch);
-            if (need) {
-                if (item >= p.total_items) {
-                    exhausted = true;
-                } else if (LIST ? list_to_pixel(p, item, pi, pj) : item_to_pixel(p, item, pi, pj)) {
-                    pix = LIST ? (int)item : pj * p.nx + pi;
-                    s = 0; depth = 0;
-                    col = mk(0, 0, 0);
-                    if (!LIST && p.accumulate) {          // progressive: continue the pixel's sum exactly where the last call left it
-                        const float *acc = p.out + (size_t)pix * 3;
-                        col = mk(acc[0], acc[1], acc[2]);
-                    }
-                    pixel_stream(p, LIST && !p.seed_states ? pj * p.nx + pi : pix, rng);
-                }
-            }
+    run_chains<LIST>(p, ChainF32(p), claim_batch(p), [&](Chain &c, const bool has) {
+        Hit h;
+        if (has) {   // per lane: only the lanes that hold a pixel trace
+            if (OCTREE) h = trace_tree(sc, p.tree, &p.tree.planes[0][0], c.o, c.d, tc);
+            else if (GEOM_SMEM) h = trace_list(geom_s, sc.tag, sc.n, c.o, c.d, tc);
+            else h = trace_list(sc.geom, sc.tag, sc.n, c.o, c.d, tc);
         }
-        if (!__ballot_sync(0xffffffffu, pix >= 0)) break;
-
-        if (pix >= 0) {
-            if (depth == 0) {   // new sample: main.cu:104-106
-                const float u = div_(add_((float)pi, xorwow_uniform(rng)), (float)p.nx);
-                const float v = div_(add_((float)pj, xorwow_uniform(rng)), (float)p.ny);
-                camera_ray(p.cam, u, v, rng, o, d);
-                att = mk(1.0f, 1.0f, 1.0f);
-                npaths++;
-            }
-            // ---- one iteration of color()'s loop (main.cu:47-73) ----
-            nrays++;
-            Hit h;
-            if (OCTREE) h = trace_tree(sc, p.tree, &p.tree.planes[0][0], o, d, tc);
-            else if (GEOM_SMEM) h = trace_list(geom_s, sc.tag, sc.n, o, d, tc);
-            else h = trace_list(sc.geom, sc.tag, sc.n, o, d, tc);
-            bool sample_done = false;
-            vec3f contrib = mk(0, 0, 0);
-            if (h.idx >= 0) {
-                const float4 g = __ldg(sc.geom + h.idx);
-                const float4 m = __ldg(sc.matl + h.idx);
-                const int tag = __ldg(sc.tag + h.idx);
-                vec3f hp, hn, a, dn;
-                hit_point(g, o, d, h.t, hp, hn);
-                if (scatter(tag, m, d, hp, hn, a, dn, rng)) {
-                    att = mk(mul_(att.x, a.x), mul_(att.y, a.y), mul_(att.z, a.z));
-                    o = hp; d = dn;
-                    depth++;
-                    if (depth >= p.max_depth) sample_done = true;        // main.cu:74: return black
-                } else {
-                    sample_done = true;                                   // absorbed: main.cu:64
-                }
-            } else {
-                const vec3f c = sky(d);
-                contrib = mk(mul_(att.x, c.x), mul_(att.y, c.y), mul_(att.z, c.z));
-                sample_done = true;
-            }
-            if (sample_done) {
-                col = mk(add_(col.x, contrib.x), add_(col.y, contrib.y), add_(col.z, contrib.z));   // main.cu:107
-                depth = 0;
-                s++;
-                if (s >= p.ns_local) {
-                    float *out = p.out + (size_t)pix * 3;
-                    if (p.finalize) {   // main.cu:111-115
-                        out[0] = sqrt_(mul_(col.x, inv_ns));
-                        out[1] = sqrt_(mul_(col.y, inv_ns));
-                        out[2] = sqrt_(mul_(col.z, inv_ns));
-                    } else {
-                        out[0] = col.x; out[1] = col.y; out[2] = col.z;
-                    }
-                    // main.cu:136: rand_state[pixel_index] = local_rand_state
-                    if (!LIST && p.state_out) xorwow_store(p.state_out + (size_t)pix * 6, rng);
-                    pix = -1;
-                }
-            }
-        }
-        __syncwarp();
-    }
-
-    // ---- ray / path counters: one atomic per warp ----
-    unsigned long long r64 = nrays, p64 = npaths;
-    for (int off = 16; off > 0; off >>= 1) {
-        r64 += __shfl_xor_sync(0xffffffffu, r64, off);
-        p64 += __shfl_xor_sync(0xffffffffu, p64, off);
-    }
-    if (lane == 0) {
-        atomicAdd(p.counters + 0, r64);
-        atomicAdd(p.counters + 1, p64);
-    }
+        return h;
+    });
 #ifdef RT_COUNTERS
+    const unsigned lane = threadIdx.x & 31u;
     unsigned long long c64[3] = {tc.sphere_tests, tc.node_tests, tc.voxel_steps};
     for (int k = 0; k < 3; k++) {
         for (int off = 16; off > 0; off >>= 1) c64[k] += __shfl_xor_sync(0xffffffffu, c64[k], off);
