@@ -41,6 +41,7 @@ ABI_SYMBOLS = [
     "rt_octree_build", "rt_octree_build_ex", "rt_octree_reference_bytes", "rt_octree_reference_bytes_ex", "rt_octree_export_reference", "rt_octree_debug_read", "rt_xorwow_state", "rt_debug_counters", "rt_trace_rays", "rt_camera_get_rays", "rt_scatter_rays",
     "rt_trace_rays_ex", "rt_camera_get_rays_ex", "rt_scatter_rays_ex",
     "rt_render_accumulate", "rt_last_render_stats", "rt_render_progressive", "rt_finalize", "rt_finalize_n", "rt_finalize_ex", "rt_render", "rt_render_to_host", "rt_render_pixels", "rt_format_ppm",
+    "rt_render_pixels_progressive", "rt_finalize_counts",
     "rt_ppm_format", "rt_ppm_read", "rt_render_to_ppm",
     "rt_ffma_peak", "rt_hfma2_peak", "rt_malloc", "rt_free", "rt_memcpy_to_host", "rt_synchronize", "rt_kernel_name",
     "rt_comm_get_unique_id", "rt_comm_init_rank", "rt_comm_init_all", "rt_comm_attach", "rt_comm_destroy", "rt_comm_rank", "rt_comm_size",
@@ -135,6 +136,8 @@ def load_library(path: str | None = None) -> C.CDLL:
         "rt_render": (i32, [vp, C.POINTER(RenderArgs), vp, C.POINTER(RenderStats)]),
         "rt_render_to_host": (i32, [vp, C.POINTER(RenderArgs), vp, C.POINTER(RenderStats)]),
         "rt_render_pixels": (i32, [vp, C.POINTER(RenderArgs), vp, i32, vp, i32, C.POINTER(RenderStats)]),
+        "rt_render_pixels_progressive": (i32, [vp, C.POINTER(RenderArgs), vp, i32, vp, vp, vp, i32, C.POINTER(RenderStats)]),
+        "rt_finalize_counts": (i32, [vp, vp, vp, vp, sz, i32]),
         "rt_format_ppm": (sz, [vp, i32, i32, vp, sz]),
         "rt_ppm_format": (i32, [vp, vp, i32, i32, C.POINTER(sz)]),
         "rt_ppm_read": (i32, [vp, vp, sz]),
@@ -426,6 +429,18 @@ class RayTracer:
                                               C.byref(st) if want_stats else None), "rt_render_progressive")
         return st.as_dict() if want_stats else None
 
+    def render_pixels_progressive(self, args: RenderArgs, pixels_ptr: int, count: int, accum_ptr: int, state_ptr: int, counts_ptr: int = 0,
+                                  first=False, want_stats=True):
+        """args.ns MORE samples for each distinct pixel of the device list at pixels_ptr (`count` uint32 indices j*nx + i), continuing
+        its sum in the FRAME accum (nx*ny*3 floats) and its stream in the FRAME state buffer (nx*ny*6 words) that
+        render_progressive uses; first=True starts the listed pixels instead.  counts_ptr (nx*ny uint32, optional): the library adds
+        args.ns to each rendered pixel's count (sets it when first).  Unlisted pixels and out-of-frame entries are left untouched."""
+        st = RenderStats()
+        self._ck(self.L.rt_render_pixels_progressive(self._ctx, C.byref(args), C.c_void_p(pixels_ptr), count, C.c_void_p(accum_ptr),
+                                                     C.c_void_p(state_ptr), C.c_void_p(counts_ptr or None), int(bool(first)),
+                                                     C.byref(st) if want_stats else None), "rt_render_pixels_progressive")
+        return st.as_dict() if want_stats else None
+
     def last_render_stats(self) -> dict:
         """Statistics of the last render call made with want_stats=False (waits for the stream)."""
         st = RenderStats()
@@ -442,6 +457,12 @@ class RayTracer:
         """/ns and sqrt on `count` linear sums in the given arithmetic (PREC_FP16: the sums are halves widened to float)."""
         self._ck(self.L.rt_finalize_ex(self._ctx, C.c_void_p(accum_dev_ptr), C.c_void_p(fb_dev_ptr), count, ns, precision),
                  "rt_finalize_ex")
+
+    def finalize_counts(self, accum_ptr: int, counts_ptr: int, fb_ptr: int, npix: int, precision: int = PREC_FP32):
+        """fb = what render() writes for each pixel rendered with counts[pix] samples (count 0: zeros); npix pixels, device
+        pointers, in place allowed."""
+        self._ck(self.L.rt_finalize_counts(self._ctx, C.c_void_p(accum_ptr), C.c_void_p(counts_ptr), C.c_void_p(fb_ptr), npix, precision),
+                 "rt_finalize_counts")
 
     def hfma2_peak_tflops(self) -> float:
         """Measured dense packed-half HFMA2 rate (TFLOP/s, 4 flop per instruction): the USE_FP16 roofline denominator."""

@@ -68,6 +68,9 @@ struct rt_context {
     uint32_t *skip_tables = nullptr;
     uint32_t *seed_states = nullptr;
     size_t seed_states_words = 0;
+    // rt_render_pixels_progressive: the deduplicated pixel list and the one-bit-per-frame-pixel mask that dedupes it
+    uint32_t *list_dedup = nullptr, *list_mask = nullptr;
+    size_t list_dedup_words = 0, list_mask_words = 0;
     // multi-GPU (rt_comm_*): this context's rank in an NCCL communicator
     ncclComm_t comm = nullptr;
     bool comm_owned = false;
@@ -147,6 +150,7 @@ extern "C" void rt_destroy(rt_context *ctx) {
     cudaFree(ctx->geom); cudaFree(ctx->matl); cudaFree(ctx->tag); cudaFree(ctx->cam_dev);
     cudaFree(ctx->work_counter); cudaFree(ctx->counters); cudaFree(ctx->scratch_fb);
     cudaFree(ctx->skip_tables); cudaFree(ctx->seed_states);
+    cudaFree(ctx->list_dedup); cudaFree(ctx->list_mask);
     cudaFree(ctx->geom_h); cudaFree(ctx->matl_h); cudaFree(ctx->cam_h);
     cudaFree(ctx->half_pairs.geom); cudaFree(ctx->half_pairs.idx); cudaFree(ctx->half_pairs.start); cudaFree(ctx->half_pairs.count);
     cudaFree(ctx->half_pairs.nodes); cudaFree(ctx->half_pairs.node_count);
@@ -502,11 +506,21 @@ static int ensure_half(rt_context *ctx, unsigned what, bool octree, const TreeVi
 struct ProgressiveIO {
     uint32_t *state = nullptr;     // 6 words per pixel, device
     bool first = true;
+    uint32_t *counts = nullptr;    // with a pixel list (rt_render_pixels_progressive): samples per frame pixel, or nullptr
 };
 struct PixelList {                 // rt_render_pixels: render these pixels of the frame, results in list order
     const uint32_t *pixels = nullptr;      // device
     int count = 0;
 };
+// A device buffer of the context that holds at least `words` uint32 (grown on demand, contents not kept)
+static int ensure_words(rt_context *ctx, uint32_t *&buf, size_t &cap, size_t words) {
+    if (cap >= words) return RT_OK;
+    cudaFree(buf);
+    buf = nullptr; cap = 0;
+    CK(cudaMalloc(&buf, words * 4));
+    cap = words;
+    return RT_OK;
+}
 // device (or managed) memory of the context's GPU: a kernel may dereference it
 static bool on_device(const rt_context *ctx, const void *ptr) {
     cudaPointerAttributes at;
@@ -535,11 +549,15 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
                      const ProgressiveIO *prog = nullptr, const PixelList *list = nullptr) {
     if (!ctx || !a || !out_dev) return fail(ctx, RT_ERR_INVALID, "render: null argument");
     if (a->nx < 1 || a->ny < 1 || a->ns < 1) return fail(ctx, RT_ERR_INVALID, "render: bad nx/ny/ns");
+    // a pixel list with progressive state: rt_render_pixels_progressive (frame-indexed sums, states and counts)
+    const bool list_prog = list && prog;
     if (list) {
         if (!list->pixels || list->count < 1) return fail(ctx, RT_ERR_INVALID, "rt_render_pixels: null pixel list or count < 1");
         if (a->shard_mode != RT_SHARD_NONE) return fail(ctx, RT_ERR_INVALID, "rt_render_pixels: pixel lists are not sharded (give each GPU its own list)");
         if (!on_device(ctx, list->pixels) || !on_device(ctx, out_dev))
             return fail(ctx, RT_ERR_INVALID, "rt_render_pixels: pixels_dev and out_dev must be device memory of the context's GPU");
+        if (list_prog && (!on_device(ctx, prog->state) || (prog->counts && !on_device(ctx, prog->counts))))
+            return fail(ctx, RT_ERR_INVALID, "rt_render_pixels_progressive: rng_state_dev and counts_dev must be device memory of the context's GPU");
     }
     if (ctx->n < 1) return fail(ctx, RT_ERR_STATE, "render: no scene (rt_scene_generate / rt_scene_upload first)");
     if (a->use_octree && !ctx->octree->built) return fail(ctx, RT_ERR_STATE, "render: USE_OCTREE set but no octree built");
@@ -613,8 +631,14 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
         }
     }
     if (owned * 32 > 0xfffffff0ll) return fail(ctx, RT_ERR_INVALID, "render: image too large for the 32-bit work queue");
+    const size_t npix = (size_t)a->nx * a->ny;
+    if (list_prog) {        // scratch for the preparation pass, before anything is launched
+        int rc = ensure_words(ctx, ctx->list_dedup, ctx->list_dedup_words, (size_t)list->count);
+        if (!rc) rc = ensure_words(ctx, ctx->list_mask, ctx->list_mask_words, (npix + 31) / 32);
+        if (rc) return rc;
+    }
     p.total_items = list ? (uint32_t)list->count : (uint32_t)(owned * 32);
-    if (list) p.pixels = list->pixels;
+    if (list) p.pixels = list_prog ? ctx->list_dedup : list->pixels;
     p.finalize = finalize ? 1 : 0;
     p.variant = a->tune[1] ? a->tune[1] : ctx->default_variant;
     p.out = out_dev;
@@ -623,27 +647,35 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
     CK(cudaMemsetAsync(ctx->counters, 0, 32 * 8, ctx->stream));
     int blocks = 0;
     int launches = 1;
+    const int mode = list_prog ? kModeListProgressive : list ? kModeList : kModeFrame;
     if (a->seed_mode == RT_SEED_UPSTREAM && !continuing) {
-        const size_t npix = list ? (size_t)list->count : (size_t)a->nx * a->ny;      // stream states to seed
         if (!ctx->skip_tables) {
             const std::vector<uint32_t> &t = host_skip_tables();
             CK(cudaMalloc(&ctx->skip_tables, t.size() * 4));
             CK(cudaMemcpyAsync(ctx->skip_tables, t.data(), t.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
         }
-        if (ctx->seed_states_words < npix * 6) {
-            cudaFree(ctx->seed_states);
-            ctx->seed_states = nullptr; ctx->seed_states_words = 0;
-            CK(cudaMalloc(&ctx->seed_states, npix * 6 * 4));
-            ctx->seed_states_words = npix * 6;
+        if (!list_prog) {       // (a progressive list seeds its pixels straight into the caller's state buffer)
+            const size_t nstates = list ? (size_t)list->count : npix;      // stream states to seed
+            if (ctx->seed_states_words < nstates * 6) {
+                cudaFree(ctx->seed_states);
+                ctx->seed_states = nullptr; ctx->seed_states_words = 0;
+                CK(cudaMalloc(&ctx->seed_states, nstates * 6 * 4));
+                ctx->seed_states_words = nstates * 6;
+            }
+            p.seed_states = ctx->seed_states;
         }
-        p.seed_states = ctx->seed_states;
     }
-    if (prog) {
+    if (list_prog) {
+        p.seed_states = prog->state;                  // read and stored back by the list-progressive instances
+        p.accumulate = continuing ? 1 : 0;
+    } else if (prog) {
         p.state_out = prog->state;
         p.accumulate = continuing ? 1 : 0;
     }
     CK(cudaEventRecord(ctx->ev0, ctx->stream));
-    if (continuing) {
+    if (list_prog) {
+        launches = 2;       // the preparation pass, launched right before the render (below)
+    } else if (continuing) {
         p.seed_states = prog->state;                  // every pixel resumes its own stream
     } else if (p.seed_states) {   // render_init (main.cu:424): inside the timed region, as in the reference
         if (list)                 // only the listed pixels' streams
@@ -658,12 +690,19 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
             const int rc = ensure_half(ctx, kHalfPairs | kHalfCamera, a->use_octree != 0, p.tree, a->nx, a->ny);
             if (rc) return rc;
         }
+    }
+    // rt_render_pixels_progressive: dedupe, counts and (first) seeding, inside the timed region as the frames' seeding, and after
+    // the last step that can fail on the context's side, so that an error leaves the caller's buffers untouched
+    if (list_prog)
+        CK(launch_pixels_progressive_prep(list->pixels, list->count, (uint32_t)npix, ctx->list_mask, ctx->list_dedup, prog->counts, (uint32_t)a->ns,
+                                          prog->first, prog->state, a->seed_mode == RT_SEED_UPSTREAM ? ctx->skip_tables : nullptr, ctx->stream));
+    if (fp16) {
         CK(launch_render_half(p, a->use_octree != 0, ctx->geom_h, ctx->matl_h, ctx->cam_h, ctx->half_pairs, ctx->prop.multiProcessorCount,
-                              ctx->stream, &blocks, list != nullptr));
+                              ctx->stream, &blocks, mode));
         ctx->last_kernel = kKernelHalf;
     } else {
         CK(launch_render(p, a->use_octree != 0 || list_grid, ctx->prop.multiProcessorCount, ctx->prop.sharedMemPerBlockOptin, ctx->stream, &blocks,
-                         &ctx->last_kernel, list != nullptr));
+                         &ctx->last_kernel, mode));
     }
     CK(cudaEventRecord(ctx->ev1, ctx->stream));
     ctx->last_launches = launches;
@@ -852,6 +891,19 @@ extern "C" int rt_render_pixels(rt_context *ctx, const rt_render_args *args, con
     return do_render(ctx, args, out_dev, finalize != 0, stats, nullptr, &list);
 }
 
+extern "C" int rt_render_pixels_progressive(rt_context *ctx, const rt_render_args *args, const uint32_t *pixels_dev, int count,
+                                            float *accum_dev, uint32_t *rng_state_dev, uint32_t *counts_dev, int first, rt_render_stats *stats) {
+    if (!rng_state_dev) return fail(ctx, RT_ERR_INVALID, "rt_render_pixels_progressive: null state buffer");
+    PixelList list;
+    list.pixels = pixels_dev;
+    list.count = count;
+    ProgressiveIO io;
+    io.state = rng_state_dev;
+    io.first = first != 0;
+    io.counts = counts_dev;
+    return do_render(ctx, args, accum_dev, false, stats, &io, &list);
+}
+
 extern "C" int rt_render_progressive(rt_context *ctx, const rt_render_args *args, float *accum_dev, uint32_t *rng_state_dev, int first,
                                      rt_render_stats *stats) {
     if (!rng_state_dev) return fail(ctx, RT_ERR_INVALID, "rt_render_progressive: null state buffer");
@@ -877,6 +929,17 @@ extern "C" int rt_finalize_ex(rt_context *ctx, const float *accum_dev, float *fb
     CK(cudaSetDevice(ctx->device));
     CK(precision == RT_PREC_FP16 ? launch_finalize_half(accum_dev, fb_dev, count, ns, ctx->stream)
                                  : launch_finalize_n(accum_dev, fb_dev, count, ns, ctx->stream));
+    return RT_OK;
+}
+
+extern "C" int rt_finalize_counts(rt_context *ctx, const float *accum_dev, const uint32_t *counts_dev, float *fb_dev, size_t npix, int precision) {
+    if (precision != RT_PREC_FP32 && precision != RT_PREC_FP16) return fail(ctx, RT_ERR_INVALID, "rt_finalize_counts: unknown precision");
+    if (!ctx || !accum_dev || !counts_dev || !fb_dev) return fail(ctx, RT_ERR_INVALID, "rt_finalize_counts: null argument");
+    if (npix == 0) return RT_OK;
+    CK(cudaSetDevice(ctx->device));
+    if (!on_device(ctx, accum_dev) || !on_device(ctx, counts_dev) || !on_device(ctx, fb_dev))
+        return fail(ctx, RT_ERR_INVALID, "rt_finalize_counts: accum_dev, counts_dev and fb_dev must be device memory of the context's GPU");
+    CK(launch_finalize_counts(accum_dev, counts_dev, fb_dev, npix, precision == RT_PREC_FP16, ctx->stream));
     return RT_OK;
 }
 

@@ -11,7 +11,7 @@
 // but was scheduled differently and rendered C4 1 % slower (B200 at 1000 W).
 #pragma once
 
-// The per-lane path state.  pix is the lane's pixel (LIST: its list slot), -1 while the lane has none.
+// The per-lane path state.  pix is the lane's pixel (kModeList: its list slot), -1 while the lane has none.
 struct Chain {
     int pix, pi, pj, s, depth;
     xorwow rng;
@@ -76,9 +76,14 @@ struct ChainF32 {
 // Runs the lanes of one warp until the queue is exhausted, then adds their ray and path counts to p.counters[0..1].
 // trace(chain, has) returns the closest hit of the chain's ray (o, d); every lane of the warp calls it, `has` says whether the
 // lane holds a pixel, and it may reload the chain (k_render_coop parks it).  batch: claim_items' tile batch.
-// The progressive branches (p.accumulate: continue the pixel's sum; p.state_out: store its stream) are left out of the LIST
-// instances: a list launch is never progressive, and its list pointer shares state_out's slot.
-template <bool LIST, class Trace>
+// MODE (rt_render.h LaunchMode) says what the queue's items are:
+//   kModeFrame: 8x4 tiles of the frame; progressive calls continue the sum in `out` (p.accumulate) and store the stream to
+//               p.state_out;
+//   kModeList: list entries, each rendered from sample 0 into its list slot (the list pointer shares state_out's slot);
+//   kModeListProgressive: list entries, each a FRAME pixel: its sum continues in out[3 * pixel] (p.accumulate) and its stream is
+//               resumed from and stored back to seed_states[6 * pixel].  The list is deduplicated (k_pixels_progressive_prep),
+//               so no two lanes hold one pixel; an entry outside the frame is skipped and writes nothing.
+template <int MODE, class Trace>
 __device__ __forceinline__ void run_chains(const RenderLaunch &p, const ChainF32 &pol, const uint32_t batch, Trace &&trace) {
     const unsigned lane = threadIdx.x & 31u;
     const uint32_t gwarp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -100,15 +105,15 @@ __device__ __forceinline__ void run_chains(const RenderLaunch &p, const ChainF32
             if (need) {
                 if (item >= p.total_items) {
                     c.exhausted = true;
-                } else if (LIST ? list_to_pixel(p, item, c.pi, c.pj) : item_to_pixel(p, item, c.pi, c.pj)) {
-                    c.pix = LIST ? (int)item : c.pj * p.nx + c.pi;
+                } else if (MODE != kModeFrame ? list_to_pixel(p, item, c.pi, c.pj, MODE == kModeList) : item_to_pixel(p, item, c.pi, c.pj)) {
+                    c.pix = MODE == kModeList ? (int)item : c.pj * p.nx + c.pi;
                     c.s = 0; c.depth = 0;
                     c.col = pol.vec(0.f, 0.f, 0.f);
-                    if (!LIST && p.accumulate) {          // progressive: continue the pixel's sum exactly where the last call left it
+                    if (MODE != kModeList && p.accumulate) {   // progressive: continue the pixel's sum exactly where the last call left it
                         const float *acc = p.out + (size_t)c.pix * 3;
                         c.col = pol.vec(acc[0], acc[1], acc[2]);
                     }
-                    pixel_stream(p, LIST && !p.seed_states ? c.pj * p.nx + c.pi : c.pix, c.rng);
+                    pixel_stream(p, MODE == kModeList && !p.seed_states ? c.pj * p.nx + c.pi : c.pix, c.rng);
                 }
             }
         }
@@ -149,7 +154,8 @@ __device__ __forceinline__ void run_chains(const RenderLaunch &p, const ChainF32
                 if (c.s >= p.ns_local) {
                     pol.write(p.out + (size_t)c.pix * 3, c.col);
                     // main.cu:136: rand_state[pixel_index] = local_rand_state
-                    if (!LIST && p.state_out) xorwow_store(p.state_out + (size_t)c.pix * 6, c.rng);
+                    if (MODE == kModeFrame && p.state_out) xorwow_store(p.state_out + (size_t)c.pix * 6, c.rng);
+                    if (MODE == kModeListProgressive) xorwow_store(const_cast<uint32_t *>(p.seed_states) + (size_t)c.pix * 6, c.rng);
                     c.pix = -1;
                 }
             }

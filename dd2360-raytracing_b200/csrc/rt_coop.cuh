@@ -304,9 +304,9 @@ __device__ __forceinline__ Hit coop_trace_tree(WarpShared &ws, const SceneView &
 
 // The lanes' pixel chains (rt_chain.cuh) are parked in shared memory during coop_trace (Chain::park) instead of being spilled to
 // local memory by the register allocator; that is what lets 8 blocks per SM be resident (-9 % frame time over 6 blocks without
-// parking, profiles r02r-r02t).  LIST: pixel-list instances, as k_render's.
-template <int ITEMS, bool LIST = false>
-__global__ void __launch_bounds__(kRenderThreads, 8) k_render_coop(const __grid_constant__ RenderLaunch p) {
+// parking, profiles r02r-r02t).  The body of k_render_coop and k_render_coop_pixels_progressive; MODE: rt_render.h LaunchMode.
+template <int ITEMS, int MODE>
+__device__ __forceinline__ void render_coop_lanes(const RenderLaunch &p) {
     __shared__ WarpShared wsh[kRenderThreads / 32];
     __shared__ uint32_t park[21][kRenderThreads];
     WarpShared &ws = wsh[threadIdx.x >> 5];
@@ -315,7 +315,7 @@ __global__ void __launch_bounds__(kRenderThreads, 8) k_render_coop(const __grid_
 
     TraceCounters tc;
     tc.sphere_tests = tc.node_tests = tc.voxel_steps = 0;
-    run_chains<LIST>(p, ChainF32(p), claim_batch(p), [&](Chain &c, const bool has) {
+    run_chains<MODE>(p, ChainF32(p), claim_batch(p), [&](Chain &c, const bool has) {
         c.park(park, threadIdx.x);
         __syncwarp();
         const Hit h = coop_trace_tree<ITEMS>(ws, sc, p.tree, &p.tree.planes[0][0], lane, has, c.o, c.d, tc);
@@ -331,6 +331,16 @@ __global__ void __launch_bounds__(kRenderThreads, 8) k_render_coop(const __grid_
         if (lane == 0) atomicAdd(p.counters + 2 + k, c64[k]);
     }
 #endif
+}
+// LIST: pixel-list instances, as k_render's
+template <int ITEMS, bool LIST = false>
+__global__ void __launch_bounds__(kRenderThreads, 8) k_render_coop(const __grid_constant__ RenderLaunch p) {
+    render_coop_lanes<ITEMS, LIST ? kModeList : kModeFrame>(p);
+}
+// progressive pixel lists, as k_render_pixels_progressive
+template <int ITEMS>
+__global__ void __launch_bounds__(kRenderThreads, 8) k_render_coop_pixels_progressive(const __grid_constant__ RenderLaunch p) {
+    render_coop_lanes<ITEMS, kModeListProgressive>(p);
 }
 
 // test hook: closest hit of caller-supplied rays through the cooperative trace (32 rays per warp)

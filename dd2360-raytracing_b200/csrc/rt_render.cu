@@ -109,6 +109,45 @@ cudaError_t launch_seed_upstream_list(uint32_t *states, const uint32_t *pixels, 
     return cudaGetLastError();
 }
 
+// The preparation pass of rt_render_pixels_progressive, one thread per list entry:
+//   * dedupe: the entry that sets its pixel's bit in `mask` (npix bits, zero on entry) keeps the pixel in `filtered`; an entry
+//     outside the frame and every later duplicate become 0xFFFFFFFF there, so the list keeps its order (and its warps their
+//     neighbouring pixels).  Which duplicate wins does not matter: each would do the same work on the same pixel.  Without it two
+//     lanes could hold one pixel, and the one that claims it late would resume the sum and stream the other has advanced;
+//   * counts[pix] += ns (= ns when first) for the pixels kept, if counts is given;
+//   * first: the kept pixels' streams are started in `states` (HEAD: seed 1984 + pix; UPSTREAM: curand_init(1984, pix, 0) with
+//     the skip tables), so the render always resumes from `states`.
+__global__ void k_pixels_progressive_prep(const uint32_t *__restrict__ pixels, int count, uint32_t npix, uint32_t *__restrict__ mask,
+                                          uint32_t *__restrict__ filtered, uint32_t *__restrict__ counts, uint32_t ns, int first,
+                                          uint32_t *__restrict__ states, const uint32_t *__restrict__ tables) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= count) return;
+    const uint32_t e = pixels[k];
+    bool keep = e < npix;
+    if (keep) {
+        const uint32_t bit = 1u << (e & 31u);
+        keep = !(atomicOr(mask + (e >> 5), bit) & bit);
+    }
+    filtered[k] = keep ? e : 0xFFFFFFFFu;
+    if (!keep) return;
+    if (counts) counts[e] = first ? ns : counts[e] + ns;
+    if (first) {
+        xorwow s;
+        if (tables) xorwow_seed_subsequence(s, 1984ull, e, tables);
+        else xorwow_seed(s, 1984ull + e);      // main.cu:93, as pixel_stream
+        xorwow_store(states + (size_t)e * 6, s);
+    }
+}
+
+cudaError_t launch_pixels_progressive_prep(const uint32_t *pixels, int count, uint32_t npix, uint32_t *mask, uint32_t *filtered, uint32_t *counts,
+                                           uint32_t ns, bool first, uint32_t *states, const uint32_t *upstream_tables, cudaStream_t st) {
+    cudaError_t e = cudaMemsetAsync(mask, 0, (size_t)(npix + 31) / 32 * 4, st);
+    if (e != cudaSuccess) return e;
+    k_pixels_progressive_prep<<<(unsigned)((count + 127) / 128), 128, 0, st>>>(pixels, count, npix, mask, filtered, counts, ns, first ? 1 : 0,
+                                                                                states, upstream_tables);
+    return cudaGetLastError();
+}
+
 // item -> pixel.  Items enumerate 8x4 tiles row-major, 32 pixels per tile; `tile_stride/tile_first` select the
 // interleaved tiles a shard owns (RT_SHARD_TILES).
 __device__ __forceinline__ bool item_to_pixel(const RenderLaunch &p, uint32_t item, int &i, int &j) {
@@ -120,14 +159,18 @@ __device__ __forceinline__ bool item_to_pixel(const RenderLaunch &p, uint32_t it
     return i < p.nx && j < p.ny;
 }
 
-// item -> pixel of a pixel-list launch (LIST instances): item k is list entry k, so a warp starts on 32 consecutive entries.
-// The claiming lane keeps k as its slot (result at out[3k], upstream start state at seed_states[6k]); camera u, v and the
-// HEAD seed use the pixel's frame coordinates.  An entry outside the frame gets (0, 0, 0) here and is not traced.
-__device__ __forceinline__ bool list_to_pixel(const RenderLaunch &p, uint32_t item, int &i, int &j) {
+// item -> pixel of a pixel-list launch (kModeList / kModeListProgressive instances): item k is list entry k, so a warp starts on
+// 32 consecutive entries.  kModeList: the claiming lane keeps k as its slot (result at out[3k], upstream start state at
+// seed_states[6k]); camera u, v and the HEAD seed use the pixel's frame coordinates.  An entry outside the frame is not traced;
+// with zero_outside (kModeList, whose `out` is in list order) it gets (0, 0, 0) — kModeListProgressive's `out` is the caller's
+// frame, where such an entry owns nothing.
+__device__ __forceinline__ bool list_to_pixel(const RenderLaunch &p, uint32_t item, int &i, int &j, const bool zero_outside) {
     const uint32_t e = __ldg(p.pixels + item);
     if ((unsigned long long)e >= (unsigned long long)p.nx * (unsigned long long)p.ny) {
-        float *out = p.out + (size_t)item * 3;
-        out[0] = 0.0f; out[1] = 0.0f; out[2] = 0.0f;
+        if (zero_outside) {
+            float *out = p.out + (size_t)item * 3;
+            out[0] = 0.0f; out[1] = 0.0f; out[2] = 0.0f;
+        }
         return false;
     }
     j = (int)(e / (uint32_t)p.nx);
@@ -167,9 +210,9 @@ __device__ __forceinline__ uint32_t claim_batch(const RenderLaunch &p) {   // pi
 
 #include "rt_chain.cuh"
 
-// LIST: pixel-list instances (rt_render_pixels, list_to_pixel); a chain's `pix` is then the lane's list slot.
-template <bool OCTREE, bool GEOM_SMEM, bool LIST = false>
-__global__ void __launch_bounds__(kRenderThreads, 6) k_render(const __grid_constant__ RenderLaunch p) {
+// The body of k_render and k_render_pixels_progressive; MODE: rt_render.h LaunchMode (what the queue's items are, run_chains).
+template <bool OCTREE, bool GEOM_SMEM, int MODE>
+__device__ __forceinline__ void render_lanes(const RenderLaunch &p) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ __align__(8) uint64_t bar;
 
@@ -192,7 +235,7 @@ __global__ void __launch_bounds__(kRenderThreads, 6) k_render(const __grid_const
 
     TraceCounters tc;
     tc.sphere_tests = tc.node_tests = tc.voxel_steps = 0;
-    run_chains<LIST>(p, ChainF32(p), claim_batch(p), [&](Chain &c, const bool has) {
+    run_chains<MODE>(p, ChainF32(p), claim_batch(p), [&](Chain &c, const bool has) {
         Hit h;
         if (has) {   // per lane: only the lanes that hold a pixel trace
             if (OCTREE) h = trace_tree(sc, p.tree, &p.tree.planes[0][0], c.o, c.d, tc);
@@ -209,6 +252,17 @@ __global__ void __launch_bounds__(kRenderThreads, 6) k_render(const __grid_const
         if (lane == 0) atomicAdd(p.counters + 2 + k, c64[k]);
     }
 #endif
+}
+
+// LIST: pixel-list instances (rt_render_pixels, list_to_pixel); a chain's `pix` is then the lane's list slot.
+template <bool OCTREE, bool GEOM_SMEM, bool LIST = false>
+__global__ void __launch_bounds__(kRenderThreads, 6) k_render(const __grid_constant__ RenderLaunch p) {
+    render_lanes<OCTREE, GEOM_SMEM, LIST ? kModeList : kModeFrame>(p);
+}
+// progressive pixel lists (rt_render_pixels_progressive): a chain's `pix` is the frame pixel, its sum and stream the frame's
+template <bool OCTREE, bool GEOM_SMEM>
+__global__ void __launch_bounds__(kRenderThreads, 6) k_render_pixels_progressive(const __grid_constant__ RenderLaunch p) {
+    render_lanes<OCTREE, GEOM_SMEM, kModeListProgressive>(p);
 }
 
 // Persistent grid of a queue-fed render kernel: exactly the blocks that are resident, never more than there is work; the queue
@@ -252,12 +306,13 @@ static void half_views(const HalfPairs &hp, h16::PairView &pv, h16::NodeTab &nt)
     nt.ent = hp.nodes; nt.count = hp.node_count;
 }
 cudaError_t launch_render_half(const RenderLaunch &p, bool octree, const uint2 *geom_h, const uint2 *matl_h, const __half *cam_h,
-                               const HalfPairs &hp, int sm_count, cudaStream_t st, int *blocks_out, bool list) {
+                               const HalfPairs &hp, int sm_count, cudaStream_t st, int *blocks_out, int mode) {
     h16::PairView pv;
     h16::NodeTab nt;
     half_views(hp, pv, nt);
     const bool prog = p.accumulate || p.state_out;
-    auto kern = list ? (octree ? h16::k_render_h<true, false, true> : h16::k_render_h<false, false, true>)
+    auto kern = mode == kModeListProgressive ? (octree ? h16::k_render_h<true, true, true> : h16::k_render_h<false, true, true>)
+              : mode == kModeList ? (octree ? h16::k_render_h<true, false, true> : h16::k_render_h<false, false, true>)
               : octree ? (prog ? h16::k_render_h<true, true> : h16::k_render_h<true, false>)
                        : (prog ? h16::k_render_h<false, true> : h16::k_render_h<false, false>);
     return launch_persistent(kern, 0, p, sm_count, st, blocks_out, p, geom_h, matl_h, cam_h, pv, nt);
@@ -265,6 +320,30 @@ cudaError_t launch_render_half(const RenderLaunch &p, bool octree, const uint2 *
 
 cudaError_t launch_finalize_half(const float *accum, float *fb, size_t count, int ns, cudaStream_t st) {
     h16::k_finalize_h<<<(unsigned)((count + 255) / 256), 256, 0, st>>>(accum, fb, count, ns);
+    return cudaGetLastError();
+}
+
+// fb = sqrt(sum * (1/counts[pix])) with ChainF32's reciprocal (1/S rounded once): what k_render writes for a pixel rendered with
+// ns = counts[pix]; count 0 gives (0, 0, 0)
+__global__ void k_finalize_counts(const float *__restrict__ accum, const uint32_t *__restrict__ counts, float *__restrict__ fb, size_t npix) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= npix) return;
+    const uint32_t c = counts[i];
+    const float a0 = accum[3 * i], a1 = accum[3 * i + 1], a2 = accum[3 * i + 2];
+    if (c == 0) {
+        fb[3 * i] = 0.0f; fb[3 * i + 1] = 0.0f; fb[3 * i + 2] = 0.0f;
+        return;
+    }
+    const float inv_ns = __fdiv_rn(1.0f, (float)c);
+    fb[3 * i] = sqrt_(mul_(a0, inv_ns));
+    fb[3 * i + 1] = sqrt_(mul_(a1, inv_ns));
+    fb[3 * i + 2] = sqrt_(mul_(a2, inv_ns));
+}
+
+cudaError_t launch_finalize_counts(const float *accum, const uint32_t *counts, float *fb, size_t npix, bool fp16, cudaStream_t st) {
+    const unsigned blocks = (unsigned)((npix + 255) / 256);
+    if (fp16) h16::k_finalize_counts_h<<<blocks, 256, 0, st>>>(accum, counts, fb, npix);
+    else k_finalize_counts<<<blocks, 256, 0, st>>>(accum, counts, fb, npix);
     return cudaGetLastError();
 }
 
@@ -418,10 +497,11 @@ cudaError_t launch_finalize_n(const float *accum, float *fb, size_t n3, int ns, 
 }
 
 cudaError_t launch_render(const RenderLaunch &p, bool octree, int sm_count, size_t smem_limit, cudaStream_t st,
-                          int *blocks_out, int *kernel_out, bool list) {
+                          int *blocks_out, int *kernel_out, int mode) {
     int dummy;
     int &which = kernel_out ? *kernel_out : dummy;
-    // a pixel list gets the frame's choice, in its LIST instance
+    const bool list = mode == kModeList, list_prog = mode == kModeListProgressive;
+    // a pixel list gets the frame's choice, in its list (or list-progressive) instance
     if (octree) {
         // automatic choice by scene size (measured on B200, profiles/README.md r02f): the pixel-per-lane walk for small scenes
         // (short candidate lists, many empty voxels: C2 2.3 vs 3.4 ms), the warp-cooperative kernel from kCoopMinSpheres on
@@ -429,18 +509,21 @@ cudaError_t launch_render(const RenderLaunch &p, bool octree, int sm_count, size
         if (p.variant == 40 || (p.variant != 1 && p.scene.n >= kCoopMinSpheres)) {
             which = kKernelCoop;
             // four candidates per lane once voxel lists are long (C5: 71 references per voxel, +4 %; C3: 13 per voxel, -6 %)
-            auto kern = p.coop_items == 4 ? (list ? coop::k_render_coop<4, true> : coop::k_render_coop<4>)
-                                          : (list ? coop::k_render_coop<2, true> : coop::k_render_coop<2>);
+            auto kern = p.coop_items == 4 ? (list_prog ? coop::k_render_coop_pixels_progressive<4> : list ? coop::k_render_coop<4, true> : coop::k_render_coop<4>)
+                                          : (list_prog ? coop::k_render_coop_pixels_progressive<2> : list ? coop::k_render_coop<2, true> : coop::k_render_coop<2>);
             return launch_persistent(kern, 0, p, sm_count, st, blocks_out, p);
         }
         which = kKernelLane;
-        return launch_persistent(list ? k_render<true, false, true> : k_render<true, false>, 0, p, sm_count, st, blocks_out, p);
+        return launch_persistent(list_prog ? k_render_pixels_progressive<true, false> : list ? k_render<true, false, true> : k_render<true, false>, 0, p,
+                                 sm_count, st, blocks_out, p);
     }
     which = kKernelListSweep;
     const size_t geom_bytes = (size_t)p.scene.n * sizeof(float4);
     if (geom_bytes + 1024 <= smem_limit)
-        return launch_persistent(list ? k_render<false, true, true> : k_render<false, true>, geom_bytes, p, sm_count, st, blocks_out, p);
-    return launch_persistent(list ? k_render<false, false, true> : k_render<false, false>, 0, p, sm_count, st, blocks_out, p);
+        return launch_persistent(list_prog ? k_render_pixels_progressive<false, true> : list ? k_render<false, true, true> : k_render<false, true>,
+                                 geom_bytes, p, sm_count, st, blocks_out, p);
+    return launch_persistent(list_prog ? k_render_pixels_progressive<false, false> : list ? k_render<false, false, true> : k_render<false, false>, 0, p,
+                             sm_count, st, blocks_out, p);
 }
 
 }  // namespace rt

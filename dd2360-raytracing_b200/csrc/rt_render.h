@@ -30,24 +30,32 @@ struct RenderLaunch {
     union {
         uint32_t *state_out;          // progressive rendering (main.cu:119-142): every pixel's stream state is stored here when its
                                       // samples of this call are done (same layout); nullptr otherwise
-        const uint32_t *pixels;       // pixel-list launches (rt_render_pixels, never progressive): item k renders pixel pixels[k]
-                                      // into out[3k], seed_states then holds one state per entry.  Sharing the slot keeps the launch
+        const uint32_t *pixels;       // pixel-list launches: item k renders pixel pixels[k].  rt_render_pixels: into out[3k],
+                                      // seed_states then holds one state per entry; rt_render_pixels_progressive: into the frame
+                                      // accum at out[3 * pixels[k]], its stream read from and stored back to seed_states (frame-
+                                      // indexed), so state_out is never needed with a list.  Sharing the slot keeps the launch
                                       // parameters' size, so the parameters after them and the whole-frame instances' SASS stay put
     };
     int accumulate;                   // 1: a pixel's sum CONTINUES from the value in `out` (fb += col, main.cu:141, in one-shot order)
     int coop_items;          // cooperative kernel: candidates per lane and chunk step (2, or 4 for scenes with long voxel lists); 0 = 2
     int variant;             // kernel variant for A/B measurements (rt_render_args.tune[1]); 0 = default
     int finalize;            // 1: write sqrt(sum/ns) (main.cu:111-115); 0: write the linear sum
-    float *out;              // nx*ny*3 floats (pixel lists: count*3, in list order)
+    float *out;              // nx*ny*3 floats (rt_render_pixels: count*3, in list order)
     uint32_t *work_counter;  // queue head
     unsigned long long *counters;   // [0] rays, [1] paths
 };
 
+// what a render launch's queue items are (rt_chain.cuh run_chains): the frame's 8x4 tiles; the entries of a pixel list, each
+// rendered from sample 0 into its list slot (rt_render_pixels); or the entries of a pixel list, each continuing its frame
+// pixel's sum and stream (rt_render_pixels_progressive: out is the frame accum, seed_states the frame's stream states, read
+// and stored back; the list has no pixel twice)
+enum LaunchMode { kModeFrame = 0, kModeList = 1, kModeListProgressive = 2 };
+
 // which kernel a launch used (reported in rt_render_stats::kernel_id; names: rt_kernel_name)
 enum KernelId { kKernelNone = 0, kKernelLane = 1, kKernelListSweep = 2, kKernelCoop = 4, kKernelHalf = 5 };
-// list: p.pixels holds a pixel list (the LIST instance of the kernel the frame would use)
+// mode: LaunchMode; a pixel list (p.pixels) is rendered by the list or list-progressive instance of the kernel the frame would use
 cudaError_t launch_render(const RenderLaunch &p, bool octree, int sm_count, size_t smem_limit, cudaStream_t st,
-                          int *blocks_out, int *kernel_out, bool list = false);
+                          int *blocks_out, int *kernel_out, int mode = kModeFrame);
 cudaError_t launch_trace_rays(const RenderLaunch &p, bool octree, const float *org, const float *dir, int n, int *out_idx,
                               float *out_t, cudaStream_t st);
 cudaError_t launch_camera_rays(const CameraData &cam, int n, const float *s, const float *t, uint32_t *states, float *org, float *dir,
@@ -60,6 +68,13 @@ cudaError_t launch_seed_upstream(uint32_t *states, size_t npix, unsigned long lo
 // the same for a pixel list: states[k] = curand_init(seed, pixels[k], 0) for the entries < npix (the others are never read)
 cudaError_t launch_seed_upstream_list(uint32_t *states, const uint32_t *pixels, int count, size_t npix, unsigned long long seed,
                                       const uint32_t *tables, cudaStream_t st);
+// rt_render_pixels_progressive's preparation pass (k_pixels_progressive_prep): clears the first npix bits of mask, writes the
+// deduplicated list to filtered, adds ns to counts (if given) and, when first, seeds the kept pixels' streams in states
+// (upstream_tables: RT_SEED_UPSTREAM; nullptr: HEAD)
+cudaError_t launch_pixels_progressive_prep(const uint32_t *pixels, int count, uint32_t npix, uint32_t *mask, uint32_t *filtered, uint32_t *counts,
+                                           uint32_t ns, bool first, uint32_t *states, const uint32_t *upstream_tables, cudaStream_t st);
+// fb = sqrt(sum * (1/counts[pix])) per channel for npix pixels, in the FP32 or the USE_FP16 arithmetic; count 0 gives (0, 0, 0)
+cudaError_t launch_finalize_counts(const float *accum, const uint32_t *counts, float *fb, size_t npix, bool fp16, cudaStream_t st);
 // ---- USE_FP16 path (rt_render_half.cuh) ----
 cudaError_t launch_scene_to_half(const float4 *geom, const float4 *matl, int n, uint2 *geom_h, uint2 *matl_h, cudaStream_t st);
 cudaError_t launch_camera_setup_half(const float lookfrom[3], const float lookat[3], const float vup[3], float vfov, int nx, int ny,
@@ -76,7 +91,7 @@ struct HalfPairs {            // candidate lists as transposed sphere pairs (rt_
 };
 cudaError_t build_half_pairs(HalfPairs &hp, const uint2 *geom_h, const int *tag, int n, bool octree, const TreeView &tv, cudaStream_t st);
 cudaError_t launch_render_half(const RenderLaunch &p, bool octree, const uint2 *geom_h, const uint2 *matl_h, const __half *cam_h,
-                               const HalfPairs &hp, int sm_count, cudaStream_t st, int *blocks_out, bool list = false);
+                               const HalfPairs &hp, int sm_count, cudaStream_t st, int *blocks_out, int mode = kModeFrame);
 // fb = the USE_FP16 build's sqrt(accum / ns) on `count` half sums widened to float
 cudaError_t launch_finalize_half(const float *accum, float *fb, size_t count, int ns, cudaStream_t st);
 // per-ray queries of the USE_FP16 build (hitTree / hitable_list::hit, camera::get_ray, material::scatter): float inputs are

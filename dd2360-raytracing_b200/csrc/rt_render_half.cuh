@@ -155,7 +155,9 @@ __global__ void k_camera_setup_h(const float lfx, const float lfy, const float l
 
 // PROG: progressive calls (p.accumulate, p.state_out) get instances of their own: compiled into the whole-frame instances, the
 // two per-pixel branches cost 1.6 % of a C4 frame (2 602 vs 2 559 ms, B200 at 1000 W).
-// LIST: pixel-list instances (with PROG = false), as k_render's (`pix` is the lane's list slot).
+// LIST: pixel-list instances.  With PROG = false they are k_render's kModeList (`pix` is the lane's list slot); with PROG = true
+// kModeListProgressive (`pix` is the frame pixel, whose sum continues in `out` and whose stream is resumed from and stored back
+// to seed_states: the list pointer holds state_out's slot).
 template <bool OCTREE, bool PROG, bool LIST = false>
 __global__ void __launch_bounds__(kRenderThreads, 5)
 k_render_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geom_h, const uint2 *__restrict__ matl_h,
@@ -194,8 +196,8 @@ k_render_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geo
             if (need) {
                 if (item >= p.total_items) {
                     exhausted = true;
-                } else if (LIST ? list_to_pixel(p, item, pi, pj) : item_to_pixel(p, item, pi, pj)) {
-                    pix = LIST ? (int)item : pj * p.nx + pi;
+                } else if (LIST ? list_to_pixel(p, item, pi, pj, !PROG) : item_to_pixel(p, item, pi, pj)) {
+                    pix = LIST && !PROG ? (int)item : pj * p.nx + pi;
                     s = 0; depth = 0;
                     col = mkh(zero, zero, zero);
                     if (PROG && p.accumulate) {  // progressive: the stored sums are halves widened to float, so this is exact
@@ -253,7 +255,8 @@ k_render_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geo
                         out[0] = h2f(vx(col)); out[1] = h2f(vy(col)); out[2] = h2f(col.z);
                     }
                     // main.cu:136: rand_state[pixel_index] = local_rand_state
-                    if (PROG && p.state_out) xorwow_store(p.state_out + (size_t)pix * 6, rng);
+                    if (PROG && !LIST && p.state_out) xorwow_store(p.state_out + (size_t)pix * 6, rng);
+                    if (PROG && LIST) xorwow_store(const_cast<uint32_t *>(p.seed_states) + (size_t)pix * 6, rng);
                     pix = -1;
                 }
             }
@@ -280,6 +283,23 @@ k_render_h(const __grid_constant__ RenderLaunch p, const uint2 *__restrict__ geo
 __global__ void k_finalize_h(const float *__restrict__ accum, float *__restrict__ fb, size_t count, int ns) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < count) fb[i] = h2f(hsqrtf_(hmul_(f2h(accum[i]), inv_ns_h(ns))));
+}
+
+// k_finalize_h with a per-pixel sample count (rt_finalize_counts): what k_render_h writes for a pixel rendered with counts[pix]
+// samples; count 0 gives (0, 0, 0)
+__global__ void k_finalize_counts_h(const float *__restrict__ accum, const uint32_t *__restrict__ counts, float *__restrict__ fb, size_t npix) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= npix) return;
+    const uint32_t c = counts[i];
+    const float a0 = accum[3 * i], a1 = accum[3 * i + 1], a2 = accum[3 * i + 2];
+    if (c == 0) {
+        fb[3 * i] = 0.0f; fb[3 * i + 1] = 0.0f; fb[3 * i + 2] = 0.0f;
+        return;
+    }
+    const hf inv_ns = inv_ns_h((int)c);
+    fb[3 * i] = h2f(hsqrtf_(hmul_(f2h(a0), inv_ns)));
+    fb[3 * i + 1] = h2f(hsqrtf_(hmul_(f2h(a1), inv_ns)));
+    fb[3 * i + 2] = h2f(hsqrtf_(hmul_(f2h(a2), inv_ns)));
 }
 
 // ---- per-ray queries of the USE_FP16 build: hitTree / hitable_list::hit, camera::get_ray, material::scatter -------------------

@@ -222,6 +222,30 @@ int rt_render_to_host(rt_context *ctx, const rt_render_args *args, float *fb_hos
  * pixels next to each other (e.g. in 8x4 tiles, as the frame queue does) for coherent warps. */
 int rt_render_pixels(rt_context *ctx, const rt_render_args *args, const uint32_t *pixels_dev, int count, float *out_dev,
                      int finalize, rt_render_stats *stats);
+/* Progressive rendering of the pixels listed in pixels_dev (device memory: count uint32 pixel indices j*nx + i).  accum_dev
+ * (nx*ny*3 floats) and rng_state_dev (nx*ny*6 words) are FRAME-indexed: the very buffers rt_render_progressive uses, so the
+ * two calls interleave freely.  Each distinct listed pixel gets args->ns MORE samples: its stream resumes from
+ * rng_state_dev[6*pix] and its sum continues from accum_dev[3*pix] (first == 0), or its stream is started with
+ * args->seed_mode and its sum overwritten (first != 0).  A pixel listed more than once in a call is rendered once.  Entries
+ * >= nx*ny and pixels not listed are left untouched in all three buffers.  counts_dev (optional, nx*ny uint32): counts[pix]
+ * += args->ns for every rendered pixel (= args->ns when first != 0).  Any schedule of rt_render_progressive and
+ * rt_render_pixels_progressive calls that gives a pixel S samples in total leaves its sum and state bit-identical to a
+ * one-shot S-sample render of that pixel (rt_render_accumulate / rt_render_progressive(first=1)), in either precision and
+ * seeding.  rt_render_progressive takes no counts: a caller that mixes the two adds the frame call's ns to every pixel's
+ * count.  The kernel is chosen as for the frame; shards are refused; stats as rt_render_pixels (paths = ns x rendered
+ * pixels); stats == NULL is asynchronous (rt_last_render_stats).  A null args / pixels_dev / accum_dev / rng_state_dev,
+ * count < 1, bad nx/ny/ns, args->shard_mode != RT_SHARD_NONE, an unknown seed mode or precision, or a given pointer (counts_dev
+ * included) that is not device (or managed) memory of the context's GPU -> RT_ERR_INVALID; no scene, USE_OCTREE without an
+ * octree, or an octree built for the other precision -> RT_ERR_STATE; nothing is written on an error. */
+int rt_render_pixels_progressive(rt_context *ctx, const rt_render_args *args, const uint32_t *pixels_dev, int count,
+                                 float *accum_dev, uint32_t *rng_state_dev, uint32_t *counts_dev, int first,
+                                 rt_render_stats *stats);
+/* fb = what rt_render writes for a pixel rendered with counts[pix] samples: sqrt(sum * (1/counts[pix])) per channel in the
+ * given precision (RT_PREC_FP16: the USE_FP16 build's finalise, as rt_finalize_ex); counts[pix] == 0 gives (0, 0, 0).
+ * npix pixels (3*npix floats), in place allowed.  A null pointer, a pointer that is not device (or managed) memory of the
+ * context's GPU, or an unknown precision -> RT_ERR_INVALID. */
+int rt_finalize_counts(rt_context *ctx, const float *accum_dev, const uint32_t *counts_dev, float *fb_dev, size_t npix,
+                       int precision);
 
 /* ---- output: replaces output_to_stream (main.cu:321-333) -------------------------------------------------- */
 /* P3 text, byte-identical to the reference writer.  Returns bytes needed when buf == NULL. */
