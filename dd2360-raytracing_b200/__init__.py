@@ -41,7 +41,7 @@ ABI_SYMBOLS = [
     "rt_octree_build", "rt_octree_build_ex", "rt_octree_reference_bytes", "rt_octree_reference_bytes_ex", "rt_octree_export_reference", "rt_octree_debug_read", "rt_xorwow_state", "rt_debug_counters", "rt_trace_rays", "rt_camera_get_rays", "rt_scatter_rays",
     "rt_trace_rays_ex", "rt_camera_get_rays_ex", "rt_scatter_rays_ex",
     "rt_render_accumulate", "rt_last_render_stats", "rt_render_progressive", "rt_finalize", "rt_finalize_n", "rt_finalize_ex", "rt_render", "rt_render_to_host", "rt_render_pixels", "rt_format_ppm",
-    "rt_render_pixels_progressive", "rt_finalize_counts",
+    "rt_render_pixels_progressive", "rt_finalize_counts", "rt_render_adaptive",
     "rt_ppm_format", "rt_ppm_read", "rt_render_to_ppm",
     "rt_ffma_peak", "rt_hfma2_peak", "rt_malloc", "rt_free", "rt_memcpy_to_host", "rt_synchronize", "rt_kernel_name",
     "rt_comm_get_unique_id", "rt_comm_init_rank", "rt_comm_init_all", "rt_comm_attach", "rt_comm_destroy", "rt_comm_rank", "rt_comm_size",
@@ -71,6 +71,20 @@ class RenderStats(C.Structure):
     def as_dict(self):
         d = {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
         d["kernel"] = load_library().rt_kernel_name(self.kernel_id).decode()
+        return d
+
+
+class AdaptiveParams(C.Structure):
+    _fields_ = [("min_spp", C.c_int32), ("threshold", C.c_float), ("reserved", C.c_int32 * 6)]
+
+
+class AdaptiveStats(C.Structure):
+    _fields_ = [("render", RenderStats), ("rounds", C.c_int32), ("reserved", C.c_int32), ("round_pixels", C.c_uint64 * 16)]
+
+    def as_dict(self):
+        d = self.render.as_dict()
+        d["rounds"] = self.rounds
+        d["round_pixels"] = [int(v) for v in self.round_pixels[:self.rounds]]
         return d
 
 
@@ -138,6 +152,7 @@ def load_library(path: str | None = None) -> C.CDLL:
         "rt_render_pixels": (i32, [vp, C.POINTER(RenderArgs), vp, i32, vp, i32, C.POINTER(RenderStats)]),
         "rt_render_pixels_progressive": (i32, [vp, C.POINTER(RenderArgs), vp, i32, vp, vp, vp, i32, C.POINTER(RenderStats)]),
         "rt_finalize_counts": (i32, [vp, vp, vp, vp, sz, i32]),
+        "rt_render_adaptive": (i32, [vp, C.POINTER(RenderArgs), C.POINTER(AdaptiveParams), vp, vp, vp, vp, vp, C.POINTER(AdaptiveStats)]),
         "rt_format_ppm": (sz, [vp, i32, i32, vp, sz]),
         "rt_ppm_format": (i32, [vp, vp, i32, i32, C.POINTER(sz)]),
         "rt_ppm_read": (i32, [vp, vp, sz]),
@@ -439,6 +454,35 @@ class RayTracer:
         self._ck(self.L.rt_render_pixels_progressive(self._ctx, C.byref(args), C.c_void_p(pixels_ptr), count, C.c_void_p(accum_ptr),
                                                      C.c_void_p(state_ptr), C.c_void_p(counts_ptr or None), int(bool(first)),
                                                      C.byref(st) if want_stats else None), "rt_render_pixels_progressive")
+        return st.as_dict() if want_stats else None
+
+    def render_adaptive(self, nx, ny, max_spp, min_spp, threshold, use_octree=True, **kw):
+        """Adaptive sampling (rt_render_adaptive): every 8x4 tile gets between min_spp and max_spp samples, doubling while its noise
+        estimate is above `threshold` (display-space standard error).  Returns host (fb[ny,nx,3] float32, counts[ny,nx] uint32,
+        err[ny,nx] float32, stats); each pixel of fb is bit for bit what render(ns = counts[pixel]) writes for it."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        npix = nx * ny
+        accum = torch.empty(npix * 3, dtype=torch.float32, device=dev)
+        state = torch.empty(npix * 6, dtype=torch.int32, device=dev)
+        counts = torch.empty(npix, dtype=torch.int32, device=dev)
+        fb = torch.empty(npix * 3, dtype=torch.float32, device=dev)
+        err = torch.empty(npix, dtype=torch.float32, device=dev)
+        st = self.render_adaptive_device(self.args(nx, ny, max_spp, use_octree, **kw), min_spp, threshold, accum.data_ptr(), state.data_ptr(),
+                                         counts.data_ptr(), fb.data_ptr(), err.data_ptr())
+        return (fb.cpu().numpy().reshape(ny, nx, 3), counts.cpu().numpy().view(np.uint32).reshape(ny, nx),
+                err.cpu().numpy().reshape(ny, nx), st)
+
+    def render_adaptive_device(self, args: RenderArgs, min_spp: int, threshold: float, accum_ptr: int, state_ptr: int, counts_ptr: int,
+                               fb_ptr: int, err_ptr: int = 0, want_stats=True):
+        """rt_render_adaptive on device pointers: args.ns is max_spp; accum (nx*ny*3 floats), state (nx*ny*6 words) and counts (nx*ny
+        uint32) are the frame-indexed buffers of render_progressive / render_pixels_progressive; fb (nx*ny*3 floats) receives the
+        finalised frame, err (nx*ny floats, optional) every pixel's last estimate."""
+        prm = AdaptiveParams(min_spp, threshold)
+        st = AdaptiveStats()
+        self._ck(self.L.rt_render_adaptive(self._ctx, C.byref(args), C.byref(prm), C.c_void_p(accum_ptr), C.c_void_p(state_ptr),
+                                           C.c_void_p(counts_ptr), C.c_void_p(fb_ptr), C.c_void_p(err_ptr or None),
+                                           C.byref(st) if want_stats else None), "rt_render_adaptive")
         return st.as_dict() if want_stats else None
 
     def last_render_stats(self) -> dict:

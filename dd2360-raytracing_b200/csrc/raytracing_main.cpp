@@ -7,6 +7,9 @@
 // (and RT_SEED_MODE=1 for the upstream per-pixel seeding curand_init(1984, pixel_index, 0), main.cu:90).
 // RT_GPUS=N shards the frame over N GPUs of this box (one context per GPU, rt_comm_* / rt_reduce: NCCL over NVLink);
 // RT_SHARD=tiles (default, bit-identical to one GPU) or spp; USE_FP16 frames shard by tiles only.
+// RT_ADAPTIVE=<threshold>[:<min_spp>] renders an adaptive frame (rt_render_adaptive, one GPU): RT_NS is the per-pixel budget, and
+// every 8x4 tile doubles its samples from min_spp (default 8, capped at RT_NS and rounded down to even) while its display-space
+// standard error is above the threshold.
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -72,6 +75,19 @@ int main(int argc, char **argv) {
     std::cerr << "Output mode: " << output_mode << "\n";
 
     const int gpus = env_int("RT_GPUS", 1);             // > 1: the frame is sharded over that many GPUs of this box (NCCL reduce)
+    const char *adaptive = getenv("RT_ADAPTIVE");
+    rt_adaptive_params ap{};
+    if (adaptive && *adaptive) {
+        ap.min_spp = std::min(8, ns) & ~1;
+        if (sscanf(adaptive, "%f:%d", &ap.threshold, &ap.min_spp) < 1) {
+            std::cerr << "RT_ADAPTIVE=<threshold>[:<min_spp>]: cannot read '" << adaptive << "'\n";
+            exit(99);
+        }
+        if (gpus > 1) {
+            std::cerr << "RT_ADAPTIVE renders on one GPU only (unset RT_GPUS)\n";
+            exit(99);
+        }
+    }
     rt_render_args a{};
     a.nx = nx; a.ny = ny; a.ns = ns; a.max_depth = 50; a.use_octree = use_octree;
     a.precision = precision;
@@ -83,6 +99,9 @@ int main(int argc, char **argv) {
     rt_context *ctx = nullptr;                           // the context that ends up holding the frame (rank 0)
     std::vector<rt_context *> ctxs((size_t)(gpus > 1 ? gpus : 1), nullptr);
     std::vector<float *> bufs(ctxs.size(), nullptr);
+    float *ad_accum = nullptr;                           // RT_ADAPTIVE: the progressive sums, stream states and sample counts
+    uint32_t *ad_state = nullptr, *ad_counts = nullptr;
+    rt_adaptive_stats ast{};
     double secs = 0;
     rt_render_stats st{};
 
@@ -102,6 +121,11 @@ int main(int argc, char **argv) {
         for (auto &t : th) t.join();
         for (size_t g = 0; g < ctxs.size(); g++) { ctx = ctxs[g]; CHECK(rcs[g]); }
         ctx = ctxs[0];
+    }
+    if (adaptive && *adaptive) {
+        CHECK(rt_malloc(ctx, n3 * sizeof(float), reinterpret_cast<void **>(&ad_accum)));
+        CHECK(rt_malloc(ctx, n3 * 2 * sizeof(uint32_t), reinterpret_cast<void **>(&ad_state)));
+        CHECK(rt_malloc(ctx, n3 / 3 * sizeof(uint32_t), reinterpret_cast<void **>(&ad_counts)));
     }
     if (gpus > 1) {
         // RT_SHARD=tiles (default): interleaved 8x4 tiles, the summed frame is bit-identical to the 1-GPU frame;
@@ -142,6 +166,9 @@ int main(int argc, char **argv) {
         CHECK(rt_group_end());
         CHECK(rt_finalize_ex(ctx, bufs[0], bufs[0], n3, ns, precision));     // /ns and sqrt on the sum (main.cu:111-114)
         CHECK(rt_synchronize(ctx));
+    } else if (ad_accum) {
+        CHECK(rt_render_adaptive(ctx, &a, &ap, ad_accum, ad_state, ad_counts, bufs[0], nullptr, &ast));
+        st = ast.render;
     } else {
         CHECK(rt_render(ctx, &a, bufs[0], &st));
     }
@@ -150,6 +177,11 @@ int main(int argc, char **argv) {
     if (getenv("RT_VERBOSE"))
         std::cerr << "rays " << st.rays << ", kernel " << st.kernel_ms << " ms, " << (st.rays / (st.kernel_ms * 1e3)) << " Mrays/s on " << gpus
                   << " GPU(s), " << rt_kernel_name(st.kernel_id) << "\n";
+    if (getenv("RT_VERBOSE") && ad_accum) {
+        std::cerr << "adaptive: threshold " << ap.threshold << ", " << ap.min_spp << ".." << ns << " spp, " << ast.rounds << " rounds (pixels";
+        for (int r = 0; r < ast.rounds; r++) std::cerr << " " << ast.round_pixels[r];
+        std::cerr << "), mean " << (double)st.paths / ((double)nx * ny) << " spp\n";
+    }
 
     // ---- output switch (main.cu:435-453); the frame is quantised and formatted on the GPU, only the text crosses PCIe ----
     if (want_text) {
@@ -163,6 +195,7 @@ int main(int argc, char **argv) {
             out.write(txt.data(), (std::streamsize)need);
         }
     }
+    if (ad_accum) { rt_free(ctx, ad_accum); rt_free(ctx, ad_state); rt_free(ctx, ad_counts); }
     for (size_t g = 0; g < ctxs.size(); g++) { rt_free(ctxs[g], bufs[g]); rt_destroy(ctxs[g]); }
     return 0;
 }

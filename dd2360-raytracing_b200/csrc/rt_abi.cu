@@ -15,6 +15,7 @@
 
 #include "../../include/rt_abi.h"
 #include "rt_math.cuh"
+#include "rt_adaptive.h"
 #include "rt_build.cuh"
 #include "rt_octree.h"
 #include "rt_render.h"
@@ -71,6 +72,11 @@ struct rt_context {
     // rt_render_pixels_progressive: the deduplicated pixel list and the one-bit-per-frame-pixel mask that dedupes it
     uint32_t *list_dedup = nullptr, *list_mask = nullptr;
     size_t list_dedup_words = 0, list_mask_words = 0;
+    // rt_render_adaptive: the snapshot sums (3 floats per pixel), the per-tile words of the selection pass (listed, offset, done),
+    // its pixel list, the scan's temporary storage, and the events that bracket the whole call
+    uint32_t *ad_snap = nullptr, *ad_tiles = nullptr, *ad_list = nullptr, *ad_scan = nullptr;
+    size_t ad_snap_words = 0, ad_tiles_words = 0, ad_list_words = 0, ad_scan_words = 0;
+    cudaEvent_t ad_ev0 = nullptr, ad_ev1 = nullptr;
     // multi-GPU (rt_comm_*): this context's rank in an NCCL communicator
     ncclComm_t comm = nullptr;
     bool comm_owned = false;
@@ -151,6 +157,9 @@ extern "C" void rt_destroy(rt_context *ctx) {
     cudaFree(ctx->work_counter); cudaFree(ctx->counters); cudaFree(ctx->scratch_fb);
     cudaFree(ctx->skip_tables); cudaFree(ctx->seed_states);
     cudaFree(ctx->list_dedup); cudaFree(ctx->list_mask);
+    cudaFree(ctx->ad_snap); cudaFree(ctx->ad_tiles); cudaFree(ctx->ad_list); cudaFree(ctx->ad_scan);
+    if (ctx->ad_ev0) cudaEventDestroy(ctx->ad_ev0);
+    if (ctx->ad_ev1) cudaEventDestroy(ctx->ad_ev1);
     cudaFree(ctx->geom_h); cudaFree(ctx->matl_h); cudaFree(ctx->cam_h);
     cudaFree(ctx->half_pairs.geom); cudaFree(ctx->half_pairs.idx); cudaFree(ctx->half_pairs.start); cudaFree(ctx->half_pairs.count);
     cudaFree(ctx->half_pairs.nodes); cudaFree(ctx->half_pairs.node_count);
@@ -940,6 +949,107 @@ extern "C" int rt_finalize_counts(rt_context *ctx, const float *accum_dev, const
     if (!on_device(ctx, accum_dev) || !on_device(ctx, counts_dev) || !on_device(ctx, fb_dev))
         return fail(ctx, RT_ERR_INVALID, "rt_finalize_counts: accum_dev, counts_dev and fb_dev must be device memory of the context's GPU");
     CK(launch_finalize_counts(accum_dev, counts_dev, fb_dev, npix, precision == RT_PREC_FP16, ctx->stream));
+    return RT_OK;
+}
+
+// Adaptive sampling over the frame queue's 8x4 tiles (rt_adaptive.h, rt_adaptive.cu).  Every round lists whole tiles that all
+// have the same count, so it is one list-progressive render with one ns; the render kernels and their bit-identity guarantee are
+// those of rt_render_progressive and rt_render_pixels_progressive.
+extern "C" int rt_render_adaptive(rt_context *ctx, const rt_render_args *args, const rt_adaptive_params *params, float *accum_dev,
+                                  uint32_t *rng_state_dev, uint32_t *counts_dev, float *fb_dev, float *err_dev, rt_adaptive_stats *stats) {
+    if (!ctx || !args || !params || !accum_dev || !rng_state_dev || !counts_dev || !fb_dev)
+        return fail(ctx, RT_ERR_INVALID, "rt_render_adaptive: null argument");
+    const int min_spp = params->min_spp, max_spp = args->ns;
+    const float threshold = params->threshold;
+    if (args->nx < 1 || args->ny < 1) return fail(ctx, RT_ERR_INVALID, "rt_render_adaptive: bad nx/ny");
+    if (min_spp < 2 || (min_spp & 1)) return fail(ctx, RT_ERR_INVALID, "rt_render_adaptive: min_spp must be even and >= 2");
+    if (max_spp < min_spp || max_spp > 65536) return fail(ctx, RT_ERR_INVALID, "rt_render_adaptive: args->ns (max_spp) must be in [min_spp, 65536]");
+    if (!(threshold >= 0.0f)) return fail(ctx, RT_ERR_INVALID, "rt_render_adaptive: threshold must be >= 0 (and not NaN)");
+    if (args->shard_mode != RT_SHARD_NONE) return fail(ctx, RT_ERR_INVALID, "rt_render_adaptive: adaptive frames are not sharded");
+    if (args->seed_mode != RT_SEED_HEAD && args->seed_mode != RT_SEED_UPSTREAM) return fail(ctx, RT_ERR_INVALID, "rt_render_adaptive: unknown seed_mode");
+    if (args->precision != RT_PREC_FP32 && args->precision != RT_PREC_FP16) return fail(ctx, RT_ERR_INVALID, "rt_render_adaptive: unknown precision");
+    const size_t npix = (size_t)args->nx * args->ny;
+    const uint32_t tiles_x = (uint32_t)(args->nx + 7) / 8;
+    const unsigned long long tiles = (unsigned long long)tiles_x * (unsigned long long)((args->ny + 3) / 4);
+    if (tiles * 32 > 0xfffffff0ull) return fail(ctx, RT_ERR_INVALID, "rt_render_adaptive: image too large for the 32-bit work queue");
+    if (!on_device(ctx, accum_dev) || !on_device(ctx, rng_state_dev) || !on_device(ctx, counts_dev) || !on_device(ctx, fb_dev) ||
+        (err_dev && !on_device(ctx, err_dev)))
+        return fail(ctx, RT_ERR_INVALID, "rt_render_adaptive: accum, state, counts, fb and err must be device memory of the context's GPU");
+    if (ctx->n < 1) return fail(ctx, RT_ERR_STATE, "rt_render_adaptive: no scene (rt_scene_generate / rt_scene_upload first)");
+    if (args->use_octree && !ctx->octree->built) return fail(ctx, RT_ERR_STATE, "rt_render_adaptive: USE_OCTREE set but no octree built");
+    const bool fp16 = args->precision == RT_PREC_FP16;
+    if (args->use_octree && ctx->octree->fp16 != fp16)
+        return fail(ctx, RT_ERR_STATE, "rt_render_adaptive: the octree was built for the other precision (rt_octree_build_ex)");
+    CK(cudaSetDevice(ctx->device));
+    // scratch, before anything is launched: the snapshot, the tile words, the list, the scan's storage, and the rounds' list scratch
+    size_t scan_bytes = 0;
+    CK(adaptive_scan_temp_bytes((uint32_t)tiles, &scan_bytes));
+    int rc = ensure_words(ctx, ctx->ad_snap, ctx->ad_snap_words, npix * 3);
+    if (!rc) rc = ensure_words(ctx, ctx->ad_tiles, ctx->ad_tiles_words, (size_t)tiles * 3);
+    if (!rc) rc = ensure_words(ctx, ctx->ad_list, ctx->ad_list_words, npix);
+    if (!rc) rc = ensure_words(ctx, ctx->ad_scan, ctx->ad_scan_words, scan_bytes / 4 + 1);
+    if (!rc) rc = ensure_words(ctx, ctx->list_dedup, ctx->list_dedup_words, npix);
+    if (!rc) rc = ensure_words(ctx, ctx->list_mask, ctx->list_mask_words, (npix + 31) / 32);
+    if (rc) return rc;
+    if (!ctx->ad_ev0) CK(cudaEventCreate(&ctx->ad_ev0));
+    if (!ctx->ad_ev1) CK(cudaEventCreate(&ctx->ad_ev1));
+
+    rt_render_stats sum, one;
+    memset(&sum, 0, sizeof sum);
+    auto render = [&](rt_render_args &ra, const ProgressiveIO &io, const PixelList *list) {
+        const int r = do_render(ctx, &ra, accum_dev, false, &one, &io, list);
+        sum.rays += one.rays; sum.paths += one.paths; sum.sphere_tests += one.sphere_tests; sum.node_tests += one.node_tests;
+        sum.launches += one.launches; sum.kernel_id = one.kernel_id;
+        return r;
+    };
+    CK(cudaEventRecord(ctx->ad_ev0, ctx->stream));
+    // two whole-frame segments of min_spp/2 samples, the snapshot between them: the first estimate of every pixel
+    rt_render_args ra = *args;
+    ra.ns = min_spp / 2;
+    ProgressiveIO io;
+    io.state = rng_state_dev;
+    io.first = true;
+    if ((rc = render(ra, io, nullptr))) return rc;
+    CK(cudaMemcpyAsync(ctx->ad_snap, accum_dev, npix * 3 * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
+    io.first = false;
+    if ((rc = render(ra, io, nullptr))) return rc;
+    CK(launch_fill_counts(counts_dev, npix, (uint32_t)min_spp, ctx->stream));
+    AdaptiveTiles t;
+    t.listed = ctx->ad_tiles; t.offset = ctx->ad_tiles + tiles; t.done = ctx->ad_tiles + 2 * tiles;
+    t.scan_temp = ctx->ad_scan; t.scan_temp_bytes = ctx->ad_scan_words * 4;
+    CK(cudaMemsetAsync(t.done, 0, (size_t)tiles * 4, ctx->stream));
+    // rounds: the tiles not done all have snapshot count a and count c; a refined tile doubles its count, capped at max_spp, so
+    // there are at most ceil(log2(max_spp / min_spp)) <= 15 rounds
+    io.counts = counts_dev;
+    PixelList list;
+    list.pixels = ctx->ad_list;
+    uint32_t a = (uint32_t)min_spp / 2, c = (uint32_t)min_spp;
+    int rounds = 0;
+    uint64_t round_pixels[16] = {};
+    for (;;) {
+        uint32_t listed = 0;
+        CK(launch_adaptive_select(accum_dev, reinterpret_cast<float *>(ctx->ad_snap), err_dev, args->nx, args->ny, a, c, c < (uint32_t)max_spp,
+                                  threshold, t, ctx->ad_list, &listed, ctx->stream));
+        if (listed == 0) break;
+        const uint32_t more = c < (uint32_t)max_spp - c ? c : (uint32_t)max_spp - c;
+        ra.ns = (int)more;
+        list.count = (int)listed;
+        if ((rc = render(ra, io, &list))) return rc;
+        round_pixels[rounds++] = listed;
+        a = c;
+        c += more;
+    }
+    CK(launch_finalize_counts(accum_dev, counts_dev, fb_dev, npix, fp16, ctx->stream));
+    CK(cudaEventRecord(ctx->ad_ev1, ctx->stream));
+    if (stats) {
+        CK(cudaEventSynchronize(ctx->ad_ev1));
+        memset(stats, 0, sizeof *stats);
+        stats->render = sum;
+        float ms = 0;
+        if (cudaEventElapsedTime(&ms, ctx->ad_ev0, ctx->ad_ev1) == cudaSuccess) stats->render.kernel_ms = ms;
+        stats->rounds = rounds;
+        memcpy(stats->round_pixels, round_pixels, sizeof round_pixels);
+    }
     return RT_OK;
 }
 

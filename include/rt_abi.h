@@ -247,6 +247,40 @@ int rt_render_pixels_progressive(rt_context *ctx, const rt_render_args *args, co
 int rt_finalize_counts(rt_context *ctx, const float *accum_dev, const uint32_t *counts_dev, float *fb_dev, size_t npix,
                        int precision);
 
+/* Adaptive sampling: each 8x4 tile of the frame queue gets as many samples as its noise estimate asks for, between
+ * params->min_spp and args->ns (= max_spp, the per-pixel budget, in [min_spp, 65536]).  The estimate of a pixel compares two
+ * independent segments of its own sample chain, [0, a) and [a, c), in display space, scaled to the standard error of its c-sample
+ * mean (e_p, rt_adaptive.h); a tile's error E_t is the largest e_p of its in-frame pixels (NaN counts as +inf).  The call
+ *   1. renders the whole frame progressively with min_spp/2 samples (first = 1), snapshots the sums, renders min_spp/2 more, and
+ *      sets counts := min_spp;
+ *   2. runs rounds: every tile not yet done with c < max_spp and !(E_t <= threshold) takes its sums as its new snapshot and gets
+ *      min(c, max_spp - c) more samples (one rt_render_pixels_progressive call over those tiles, in tile order); any other tile
+ *      is done and never evaluated again.  The rounds end when a selection lists nothing (at most ceil(log2(max/min)));
+ *   3. finalises the frame from the counts into fb_dev (rt_finalize_counts).
+ * accum_dev (nx*ny*3 floats), rng_state_dev (nx*ny*6 words) and counts_dev (nx*ny uint32) are the frame-indexed buffers of
+ * rt_render_progressive and rt_render_pixels_progressive, so a caller may keep refining with those.  Every pixel ends, bit for
+ * bit, where rt_render(ns = counts[pix]) puts it (fb), and its sum and state where a one-shot counts[pix]-sample progressive render
+ * does, in either precision and seeding.  err_dev (optional, nx*ny floats): e_p of every pixel from its last two segments.
+ * threshold = +inf gives a uniform min_spp frame.  stats (optional): rays, paths and test counters summed over the render calls,
+ * their launches, the render kernel's id, kernel_ms = device time of the whole call, the rounds and the pixels listed in each.  The
+ * call waits for the stream once per round (the list length is read back).  A null args / params / accum_dev / rng_state_dev /
+ * counts_dev / fb_dev, bad nx/ny, an odd min_spp or min_spp < 2, max_spp out of range, a NaN or negative threshold,
+ * args->shard_mode != RT_SHARD_NONE, an unknown seed mode or precision, or a given pointer that is not device (or managed) memory
+ * of the context's GPU -> RT_ERR_INVALID; no scene, USE_OCTREE without an octree, or an octree built for the other precision ->
+ * RT_ERR_STATE; nothing is written on an error. */
+typedef struct rt_adaptive_params {
+    int32_t min_spp;        /* even, >= 2: two whole-frame segments of min_spp/2 give the first estimate */
+    float threshold;        /* display-space standard error a tile must reach; +inf = uniform min_spp frame */
+    int32_t reserved[6];
+} rt_adaptive_params;
+typedef struct rt_adaptive_stats {
+    rt_render_stats render; /* rays/paths summed over all calls; kernel_ms spans the whole call; kernel_id of the render kernel */
+    int32_t rounds, reserved;
+    uint64_t round_pixels[16];   /* pixels listed in round r */
+} rt_adaptive_stats;
+int rt_render_adaptive(rt_context *ctx, const rt_render_args *args, const rt_adaptive_params *params, float *accum_dev,
+                       uint32_t *rng_state_dev, uint32_t *counts_dev, float *fb_dev, float *err_dev, rt_adaptive_stats *stats);
+
 /* ---- output: replaces output_to_stream (main.cu:321-333) -------------------------------------------------- */
 /* P3 text, byte-identical to the reference writer.  Returns bytes needed when buf == NULL. */
 size_t rt_format_ppm(const float *fb_host, int nx, int ny, char *buf, size_t cap);
