@@ -30,52 +30,46 @@ struct rt_context {
     std::string err;
     // scene
     int n = 0;
-    float4 *geom = nullptr, *matl = nullptr;
-    int *tag = nullptr;
-    size_t scene_cap = 0;
+    Buffer<float4> geom, matl;
+    Buffer<int> tag;
     // camera
     bool have_camera = false;
     int cam_nx = 0, cam_ny = 0;
-    CameraData *cam_dev = nullptr;
+    Buffer<CameraData> cam_dev;
     CameraData cam_host{};
     // octree
-    OctreeBuilder *octree = nullptr;
-    OctreeBuilder *list_accel = nullptr;     // USE_OCTREE off: the same grid over ALL spheres answers hitable_list::hit
+    OctreeBuilder octree;
+    OctreeBuilder list_accel;      // USE_OCTREE off: the same grid over ALL spheres answers hitable_list::hit
     bool list_accel_valid = false;
     float grid_density = 4.0f;
     int default_variant = 0;       // RT_RENDER_VARIANT: kernel A/B override for whole test runs (0 = automatic)
     int last_kernel = 0;           // KernelId of the last render launch
     int last_launches = 0;         // kernels the last render call launched (upstream seeding + render)
     // render scratch
-    uint32_t *work_counter = nullptr;
-    unsigned long long *counters = nullptr;
-    float *scratch_fb = nullptr;
-    size_t scratch_fb_bytes = 0;
+    Buffer<uint32_t> work_counter;
+    Buffer<unsigned long long> counters;
+    Buffer<float> scratch_fb;
     PpmWorkspace ppm;
-    float *pinned = nullptr;       // page-locked staging for the scene descriptors
-    size_t pinned_bytes = 0;
-    void *desc_dev = nullptr;      // ... and their raw device copy (split into geom / matl / tag by k_split_scene)
+    Buffer<char, Mem::Pinned> pinned;   // page-locked staging for the scene descriptors
+    Buffer<char> desc_dev;              // ... and their raw device copy (split into geom / matl / tag by k_split_scene)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     // RT_SEED_UPSTREAM: skip-ahead matrices (device copy) and the per-pixel stream states
     // RT_PREC_FP16: the scene rounded to half (8 B geometry + 8 B material per sphere) and the half camera
-    uint2 *geom_h = nullptr, *matl_h = nullptr;
-    size_t half_cap = 0;
+    Buffer<uint2> geom_h, matl_h;
     bool half_valid = false;
     HalfPairs half_pairs;
-    __half *cam_h = nullptr;
+    Buffer<__half> cam_h;
     int cam_h_nx = 0, cam_h_ny = 0;
     rt_camera_desc cam_desc{};
     bool cam_desc_custom = false;
-    uint32_t *skip_tables = nullptr;
-    uint32_t *seed_states = nullptr;
-    size_t seed_states_words = 0;
+    Buffer<uint32_t> skip_tables;
+    Buffer<uint32_t> seed_states;
     // rt_render_pixels_progressive: the deduplicated pixel list and the one-bit-per-frame-pixel mask that dedupes it
-    uint32_t *list_dedup = nullptr, *list_mask = nullptr;
-    size_t list_dedup_words = 0, list_mask_words = 0;
+    Buffer<uint32_t> list_dedup, list_mask;
     // rt_render_adaptive: the snapshot sums (3 floats per pixel), the per-tile words of the selection pass (listed, offset, done),
     // its pixel list, the scan's temporary storage, and the events that bracket the whole call
-    uint32_t *ad_snap = nullptr, *ad_tiles = nullptr, *ad_list = nullptr, *ad_scan = nullptr;
-    size_t ad_snap_words = 0, ad_tiles_words = 0, ad_list_words = 0, ad_scan_words = 0;
+    Buffer<float> ad_snap;
+    Buffer<uint32_t> ad_tiles, ad_list, ad_scan;
     cudaEvent_t ad_ev0 = nullptr, ad_ev1 = nullptr;
     // multi-GPU (rt_comm_*): this context's rank in an NCCL communicator
     ncclComm_t comm = nullptr;
@@ -122,23 +116,22 @@ extern "C" int rt_create(int device, rt_context **out) {
     if ((e = cudaSetDevice(device)) != cudaSuccess || (e = cudaGetDeviceProperties(&ctx->prop, device)) != cudaSuccess ||
         (e = cudaStreamCreateWithFlags(&ctx->own_stream, cudaStreamDefault)) != cudaSuccess ||
         (e = cudaEventCreate(&ctx->ev0)) != cudaSuccess || (e = cudaEventCreate(&ctx->ev1)) != cudaSuccess ||
-        (e = cudaMalloc(&ctx->work_counter, 4)) != cudaSuccess || (e = cudaMalloc(&ctx->counters, 32 * 8)) != cudaSuccess ||
-        (e = cudaMalloc(&ctx->cam_dev, sizeof(CameraData))) != cudaSuccess) {
-        delete ctx;
+        (e = cudaEventCreate(&ctx->ad_ev0)) != cudaSuccess || (e = cudaEventCreate(&ctx->ad_ev1)) != cudaSuccess ||
+        (e = ctx->work_counter.reserve(1)) != cudaSuccess || (e = ctx->counters.reserve(32)) != cudaSuccess ||
+        (e = ctx->cam_dev.reserve(1)) != cudaSuccess) {
+        rt_destroy(ctx);
         return (int)e;
     }
     ctx->stream = ctx->own_stream;
-    ctx->octree = new OctreeBuilder();
-    ctx->list_accel = new OctreeBuilder();
     const char *dens = getenv("RT_GRID_DENSITY");
     if (dens && atof(dens) > 0) ctx->grid_density = (float)atof(dens);
     float flat = 0, wide = 0;
     unsigned flat_min = kFlatVoxelMinSpheres;
     const char *shape = getenv("RT_GRID_SHAPE");        // "flat:wide[:from how many spheres]", e.g. "1:1" for cubes everywhere
     if (shape && sscanf(shape, "%f:%f:%u", &flat, &wide, &flat_min) >= 2 && flat > 0 && wide > 0) {
-        ctx->octree->grid_flat = ctx->list_accel->grid_flat = flat;
-        ctx->octree->grid_wide = ctx->list_accel->grid_wide = wide;
-        ctx->octree->grid_flat_min = ctx->list_accel->grid_flat_min = flat_min;
+        ctx->octree.grid_flat = ctx->list_accel.grid_flat = flat;
+        ctx->octree.grid_wide = ctx->list_accel.grid_wide = wide;
+        ctx->octree.grid_flat_min = ctx->list_accel.grid_flat_min = flat_min;
     }
     const char *var = getenv("RT_RENDER_VARIANT");
     if (var) ctx->default_variant = atoi(var);
@@ -146,27 +139,13 @@ extern "C" int rt_create(int device, rt_context **out) {
     return RT_OK;
 }
 
+// Also the failure path of rt_create, which may leave any of these unset.  The context's buffers free themselves.
 extern "C" void rt_destroy(rt_context *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
-    cudaStreamSynchronize(ctx->stream);
-    delete ctx->octree;
-    delete ctx->list_accel;
-    ppm_free(ctx->ppm);
-    cudaFree(ctx->geom); cudaFree(ctx->matl); cudaFree(ctx->tag); cudaFree(ctx->cam_dev);
-    cudaFree(ctx->work_counter); cudaFree(ctx->counters); cudaFree(ctx->scratch_fb);
-    cudaFree(ctx->skip_tables); cudaFree(ctx->seed_states);
-    cudaFree(ctx->list_dedup); cudaFree(ctx->list_mask);
-    cudaFree(ctx->ad_snap); cudaFree(ctx->ad_tiles); cudaFree(ctx->ad_list); cudaFree(ctx->ad_scan);
-    if (ctx->ad_ev0) cudaEventDestroy(ctx->ad_ev0);
-    if (ctx->ad_ev1) cudaEventDestroy(ctx->ad_ev1);
-    cudaFree(ctx->geom_h); cudaFree(ctx->matl_h); cudaFree(ctx->cam_h);
-    cudaFree(ctx->half_pairs.geom); cudaFree(ctx->half_pairs.idx); cudaFree(ctx->half_pairs.start); cudaFree(ctx->half_pairs.count);
-    cudaFree(ctx->half_pairs.nodes); cudaFree(ctx->half_pairs.node_count);
-    if (ctx->pinned) cudaFreeHost(ctx->pinned);
-    cudaFree(ctx->desc_dev);
-    if (ctx->ev0) cudaEventDestroy(ctx->ev0);
-    if (ctx->ev1) cudaEventDestroy(ctx->ev1);
+    if (ctx->stream) cudaStreamSynchronize(ctx->stream);
+    for (cudaEvent_t ev : {ctx->ev0, ctx->ev1, ctx->ad_ev0, ctx->ad_ev1})
+        if (ev) cudaEventDestroy(ev);
     rt_comm_destroy(ctx);
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
     delete ctx;
@@ -268,34 +247,23 @@ __global__ void k_split_scene(const rt_sphere_desc *__restrict__ d, int n, float
 // buffer is also the context's host copy of the scene (rt_scene_download): `src` is copied ONCE, straight into it.
 static int upload_scene(rt_context *ctx, const rt_sphere_desc *src, bool clamp_fuzz) {
     const int n = ctx->n;
-    if ((size_t)n > ctx->scene_cap) {
-        cudaFree(ctx->geom); cudaFree(ctx->matl); cudaFree(ctx->tag);
-        ctx->geom = ctx->matl = nullptr; ctx->tag = nullptr; ctx->scene_cap = 0;
-        CK(cudaMalloc(&ctx->geom, (size_t)n * sizeof(float4)));
-        CK(cudaMalloc(&ctx->matl, (size_t)n * sizeof(float4)));
-        CK(cudaMalloc(&ctx->tag, (size_t)n * sizeof(int)));
-        ctx->scene_cap = (size_t)n;
-    }
+    CK(ctx->geom.reserve(n));
+    CK(ctx->matl.reserve(n));
+    CK(ctx->tag.reserve(n));
     const size_t bytes = (size_t)n * sizeof(rt_sphere_desc);
     CK(cudaStreamSynchronize(ctx->stream));                      // (an earlier upload may still be reading the staging buffer)
-    if (bytes > ctx->pinned_bytes) {
-        if (ctx->pinned) cudaFreeHost(ctx->pinned);
-        ctx->pinned = nullptr; ctx->pinned_bytes = 0;
-        cudaFree(ctx->desc_dev);
-        ctx->desc_dev = nullptr;
-        CK(cudaMallocHost(reinterpret_cast<void **>(&ctx->pinned), bytes + bytes / 4));
-        ctx->pinned_bytes = bytes + bytes / 4;
-        CK(cudaMalloc(&ctx->desc_dev, bytes + bytes / 4));
-    }
-    rt_sphere_desc *host = reinterpret_cast<rt_sphere_desc *>(ctx->pinned);
+    CK(ctx->pinned.reserve(bytes, bytes / 4));
+    CK(ctx->desc_dev.reserve(bytes, bytes / 4));
+    rt_sphere_desc *host = reinterpret_cast<rt_sphere_desc *>(ctx->pinned.ptr);
     memcpy(host, src, bytes);
     if (clamp_fuzz)
         for (int i = 0; i < n; i++)
             if (host[i].mat == RT_MAT_METAL && !(host[i].param < 1.0f)) host[i].param = 1.0f;   // metal::metal clamps fuzz (material.h:67)
-    CK(cudaMemcpyAsync(ctx->desc_dev, ctx->pinned, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    k_split_scene<<<(n + 255) / 256, 256, 0, ctx->stream>>>(static_cast<const rt_sphere_desc *>(ctx->desc_dev), n, ctx->geom, ctx->matl, ctx->tag);
+    CK(cudaMemcpyAsync(ctx->desc_dev.ptr, ctx->pinned.ptr, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    k_split_scene<<<(n + 255) / 256, 256, 0, ctx->stream>>>(reinterpret_cast<const rt_sphere_desc *>(ctx->desc_dev.ptr), n, ctx->geom.ptr,
+                                                            ctx->matl.ptr, ctx->tag.ptr);
     CK(cudaGetLastError());
-    ctx->octree->built = false;
+    ctx->octree.built = false;
     return RT_OK;
 }
 
@@ -324,7 +292,7 @@ extern "C" int rt_scene_upload(rt_context *ctx, const rt_sphere_desc *spheres, i
 
 extern "C" int rt_scene_download(rt_context *ctx, rt_sphere_desc *out, int n) {
     if (!ctx || !out || n != ctx->n) return fail(ctx, RT_ERR_INVALID, "rt_scene_download: n does not match the scene");
-    memcpy(out, ctx->pinned, (size_t)n * sizeof(rt_sphere_desc));      // the staging buffer of the last upload
+    memcpy(out, ctx->pinned.ptr, (size_t)n * sizeof(rt_sphere_desc));      // the staging buffer of the last upload
     return RT_OK;
 }
 
@@ -388,9 +356,9 @@ extern "C" int rt_camera_set(rt_context *ctx, const rt_camera_desc *desc, int nx
     ctx->cam_desc = c;
     ctx->cam_desc_custom = desc != nullptr;
     ctx->cam_h_nx = ctx->cam_h_ny = 0;          // the half camera is derived on demand
-    k_camera_setup<<<1, 1, 0, ctx->stream>>>(c, ctx->cam_dev);
+    k_camera_setup<<<1, 1, 0, ctx->stream>>>(c, ctx->cam_dev.ptr);
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(&ctx->cam_host, ctx->cam_dev, sizeof(CameraData), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&ctx->cam_host, ctx->cam_dev.ptr, sizeof(CameraData), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     ctx->have_camera = true;
     ctx->cam_nx = nx; ctx->cam_ny = ny;
@@ -408,11 +376,11 @@ static int ensure_half_camera(rt_context *ctx, int nx, int ny) {
         const int rc = rt_camera_set(ctx, nullptr, nx, ny);
         if (rc) return rc;
     }
-    if (!ctx->cam_h) CK(cudaMalloc(&ctx->cam_h, 22 * sizeof(__half)));
+    CK(ctx->cam_h.reserve(22));
     if (ctx->cam_h_nx != nx || ctx->cam_h_ny != ny) {
         const rt_camera_desc &c = ctx->cam_desc;
         CK(launch_camera_setup_half(c.lookfrom, c.lookat, c.vup, c.vfov, nx, ny, ctx->cam_desc_custom ? c.aspect : 0.f, c.aperture,
-                                    c.focus_dist, ctx->cam_h, ctx->stream));
+                                    c.focus_dist, ctx->cam_h.ptr, ctx->stream));
         ctx->cam_h_nx = nx; ctx->cam_h_ny = ny;
     }
     return RT_OK;
@@ -424,7 +392,7 @@ extern "C" int rt_camera_get_half(rt_context *ctx, int nx, int ny, float out22[2
     const int rc = ensure_half_camera(ctx, nx, ny);
     if (rc) return rc;
     __half h[22];
-    CK(cudaMemcpyAsync(h, ctx->cam_h, sizeof h, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(h, ctx->cam_h.ptr, sizeof h, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     for (int k = 0; k < 22; k++) out22[k] = __half2float(h[k]);
     return RT_OK;
@@ -439,7 +407,7 @@ extern "C" int rt_octree_build_ex(rt_context *ctx, int spl, int precision, rt_oc
     if (ctx->n < 1) return fail(ctx, RT_ERR_STATE, "rt_octree_build: no scene");
     CK(cudaSetDevice(ctx->device));
     CK(cudaEventRecord(ctx->ev0, ctx->stream));
-    CK(ctx->octree->build(ctx->stream, ctx->geom, ctx->tag, ctx->n, spl, ctx->grid_density, precision == RT_PREC_FP16));
+    CK(ctx->octree.build(ctx->stream, ctx->geom.ptr, ctx->tag.ptr, ctx->n, spl, ctx->grid_density, precision == RT_PREC_FP16));
     ctx->half_pairs.valid = false;
     CK(cudaEventRecord(ctx->ev1, ctx->stream));
     CK(cudaEventSynchronize(ctx->ev1));
@@ -448,12 +416,12 @@ extern "C" int rt_octree_build_ex(rt_context *ctx, int spl, int precision, rt_oc
         float ms = 0;
         cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
         stats->build_ms = ms;
-        stats->node_count = ctx->octree->counts.node_count;
-        stats->entries = (int64_t)ctx->octree->stats_h[0];
-        stats->dropped_full = (int64_t)ctx->octree->stats_h[1];
-        stats->dropped_outside = (int64_t)ctx->octree->stats_h[2];
-        stats->fine_voxels = ctx->octree->total_voxels;
-        stats->fine_refs = ctx->octree->total_refs;
+        stats->node_count = ctx->octree.counts.node_count;
+        stats->entries = (int64_t)ctx->octree.stats_h[0];
+        stats->dropped_full = (int64_t)ctx->octree.stats_h[1];
+        stats->dropped_outside = (int64_t)ctx->octree.stats_h[2];
+        stats->fine_voxels = ctx->octree.total_voxels;
+        stats->fine_refs = ctx->octree.total_refs;
         stats->leaf_count = 0;   // known once the reference layout is exported
     }
     return RT_OK;
@@ -468,22 +436,22 @@ extern "C" size_t rt_octree_reference_bytes_ex(int spl, int precision) {
 
 extern "C" int rt_octree_export_reference(rt_context *ctx, void *host_blob, size_t bytes) {
     if (!ctx || !host_blob) return RT_ERR_INVALID;
-    if (!ctx->octree->built) return fail(ctx, RT_ERR_STATE, "rt_octree_export_reference: build the octree first");
-    if (ctx->octree->fp16) {      // the USE_FP16 AABB holds the planes as halves: they must be exact there (k_blob_nodes)
-        const float *pl = &ctx->octree->planes.p[0][0];
+    if (!ctx->octree.built) return fail(ctx, RT_ERR_STATE, "rt_octree_export_reference: build the octree first");
+    if (ctx->octree.fp16) {      // the USE_FP16 AABB holds the planes as halves: they must be exact there (k_blob_nodes)
+        const float *pl = &ctx->octree.planes.p[0][0];
         for (int k = 0; k < 3 * kPlanes; k++)
             if (__half2float(__float2half_rn(pl[k])) != pl[k])
                 return fail(ctx, RT_ERR_UNSUPPORTED, "rt_octree_export_reference: box plane %g is not exact in half", (double)pl[k]);
     }
     CK(cudaSetDevice(ctx->device));
-    CK(ctx->octree->export_reference(ctx->stream, host_blob, bytes));
+    CK(ctx->octree.export_reference(ctx->stream, host_blob, bytes));
     return RT_OK;
 }
 
 extern "C" size_t rt_octree_debug_read(rt_context *ctx, int which, void *host, size_t cap) {
     if (!ctx) return 0;
     cudaSetDevice(ctx->device);
-    return ctx->octree->debug_read(ctx->stream, which, host, cap);
+    return ctx->octree.debug_read(ctx->stream, which, host, cap);
 }
 
 // ---- USE_FP16 state -------------------------------------------------------------------------------------------------
@@ -492,21 +460,16 @@ extern "C" size_t rt_octree_debug_read(rt_context *ctx, int which, void *host, s
 // the half camera of an nx x ny frame.  The render and the per-ray entry points share it.
 enum { kHalfPairs = 1, kHalfCamera = 2 };
 static int ensure_half(rt_context *ctx, unsigned what, bool octree, const TreeView &tv, int nx, int ny) {
-    if (ctx->half_cap < (size_t)ctx->n) {
-        cudaFree(ctx->geom_h); cudaFree(ctx->matl_h);
-        ctx->geom_h = ctx->matl_h = nullptr; ctx->half_cap = 0;
-        CK(cudaMalloc(&ctx->geom_h, (size_t)ctx->n * sizeof(uint2)));
-        CK(cudaMalloc(&ctx->matl_h, (size_t)ctx->n * sizeof(uint2)));
-        ctx->half_cap = (size_t)ctx->n;
-        ctx->half_valid = false;
-    }
+    // (a scene change clears half_valid, so the contents a growth drops are never marked valid)
+    CK(ctx->geom_h.reserve(ctx->n));
+    CK(ctx->matl_h.reserve(ctx->n));
     if (!ctx->half_valid) {
-        CK(launch_scene_to_half(ctx->geom, ctx->matl, ctx->n, ctx->geom_h, ctx->matl_h, ctx->stream));
+        CK(launch_scene_to_half(ctx->geom.ptr, ctx->matl.ptr, ctx->n, ctx->geom_h.ptr, ctx->matl_h.ptr, ctx->stream));
         ctx->half_valid = true;
         ctx->half_pairs.valid = false;
     }
     if ((what & kHalfPairs) && (!ctx->half_pairs.valid || ctx->half_pairs.octree != octree))
-        CK(build_half_pairs(ctx->half_pairs, ctx->geom_h, ctx->tag, ctx->n, octree, tv, ctx->stream));
+        CK(build_half_pairs(ctx->half_pairs, ctx->geom_h.ptr, ctx->tag.ptr, ctx->n, octree, tv, ctx->stream));
     if (what & kHalfCamera) return ensure_half_camera(ctx, nx, ny);
     return RT_OK;
 }
@@ -521,15 +484,6 @@ struct PixelList {                 // rt_render_pixels: render these pixels of t
     const uint32_t *pixels = nullptr;      // device
     int count = 0;
 };
-// A device buffer of the context that holds at least `words` uint32 (grown on demand, contents not kept)
-static int ensure_words(rt_context *ctx, uint32_t *&buf, size_t &cap, size_t words) {
-    if (cap >= words) return RT_OK;
-    cudaFree(buf);
-    buf = nullptr; cap = 0;
-    CK(cudaMalloc(&buf, words * 4));
-    cap = words;
-    return RT_OK;
-}
 // device (or managed) memory of the context's GPU: a kernel may dereference it
 static bool on_device(const rt_context *ctx, const void *ptr) {
     cudaPointerAttributes at;
@@ -543,7 +497,7 @@ static bool on_device(const rt_context *ctx, const void *ptr) {
 // for the context's stream.
 static int read_render_stats(rt_context *ctx, rt_render_stats *stats) {
     unsigned long long c[4] = {0, 0, 0, 0};
-    CK(cudaMemcpyAsync(c, ctx->counters, sizeof c, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(c, ctx->counters.ptr, sizeof c, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     memset(stats, 0, sizeof *stats);
     stats->rays = c[0]; stats->paths = c[1];
@@ -569,7 +523,7 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
             return fail(ctx, RT_ERR_INVALID, "rt_render_pixels_progressive: rng_state_dev and counts_dev must be device memory of the context's GPU");
     }
     if (ctx->n < 1) return fail(ctx, RT_ERR_STATE, "render: no scene (rt_scene_generate / rt_scene_upload first)");
-    if (a->use_octree && !ctx->octree->built) return fail(ctx, RT_ERR_STATE, "render: USE_OCTREE set but no octree built");
+    if (a->use_octree && !ctx->octree.built) return fail(ctx, RT_ERR_STATE, "render: USE_OCTREE set but no octree built");
     if (a->seed_mode != RT_SEED_HEAD && a->seed_mode != RT_SEED_UPSTREAM) return fail(ctx, RT_ERR_INVALID, "render: unknown seed_mode");
     if (a->precision != RT_PREC_FP32 && a->precision != RT_PREC_FP16) return fail(ctx, RT_ERR_INVALID, "render: unknown precision");
     const bool fp16 = a->precision == RT_PREC_FP16;
@@ -577,7 +531,7 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
     // samples per rank is a different image from any build of the reference
     if (fp16 && a->shard_mode == RT_SHARD_SPP)
         return fail(ctx, RT_ERR_UNSUPPORTED, "render: USE_FP16 frames shard by tiles only (RT_SHARD_TILES): spp shards' half sums do not add up to the 1-GPU frame");
-    if (a->use_octree && ctx->octree->built && ctx->octree->fp16 != fp16)
+    if (a->use_octree && ctx->octree.built && ctx->octree.fp16 != fp16)
         return fail(ctx, RT_ERR_STATE, "render: the octree was built for the other precision (rt_octree_build_ex)");
     CK(cudaSetDevice(ctx->device));
     if (!ctx->have_camera || ctx->cam_nx != a->nx || ctx->cam_ny != a->ny) {
@@ -594,24 +548,24 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
 
     RenderLaunch p;
     memset(&p, 0, sizeof p);
-    p.scene.geom = ctx->geom; p.scene.matl = ctx->matl; p.scene.tag = ctx->tag; p.scene.n = ctx->n;
-    if (a->use_octree) p.tree = ctx->octree->view();
+    p.scene.geom = ctx->geom.ptr; p.scene.matl = ctx->matl.ptr; p.scene.tag = ctx->tag.ptr; p.scene.n = ctx->n;
+    if (a->use_octree) p.tree = ctx->octree.view();
     // flat-list mode: hitable_list::hit is "closest over all spheres"; above a few hundred spheres the grid answers it
     // with a few dozen tests instead of N (the result is the same minimum; variant 20 forces the N-test sweep)
     bool list_grid = false;
     // (an undefined slot 0 stays unhittable there too: the build sees its tag, TreeView::slot0_none)
     if (!a->use_octree && a->precision == RT_PREC_FP32 && ctx->n >= kListGridMinSpheres && a->tune[1] != 20) {
         if (!ctx->list_accel_valid) {
-            CK(ctx->list_accel->build(ctx->stream, ctx->geom, ctx->tag, ctx->n, 30, ctx->grid_density, false, true));
+            CK(ctx->list_accel.build(ctx->stream, ctx->geom.ptr, ctx->tag.ptr, ctx->n, 30, ctx->grid_density, false, true));
             ctx->list_accel_valid = true;
         }
-        p.tree = ctx->list_accel->view();
+        p.tree = ctx->list_accel.view();
         list_grid = true;
     }
     p.cam = ctx->cam_host;                        // per-context camera, by value in the launch parameters
     {
-        const OctreeBuilder *acc = list_grid ? ctx->list_accel : ctx->octree;
-        p.coop_items = (a->use_octree || list_grid) && acc->total_voxels > 0 && acc->total_refs / acc->total_voxels >= 40 ? 4 : 2;
+        const OctreeBuilder &acc = list_grid ? ctx->list_accel : ctx->octree;
+        p.coop_items = (a->use_octree || list_grid) && acc.total_voxels > 0 && acc.total_refs / acc.total_voxels >= 40 ? 4 : 2;
     }
     p.nx = a->nx; p.ny = a->ny;
     p.ns_total = a->ns;
@@ -642,36 +596,30 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
     if (owned * 32 > 0xfffffff0ll) return fail(ctx, RT_ERR_INVALID, "render: image too large for the 32-bit work queue");
     const size_t npix = (size_t)a->nx * a->ny;
     if (list_prog) {        // scratch for the preparation pass, before anything is launched
-        int rc = ensure_words(ctx, ctx->list_dedup, ctx->list_dedup_words, (size_t)list->count);
-        if (!rc) rc = ensure_words(ctx, ctx->list_mask, ctx->list_mask_words, (npix + 31) / 32);
-        if (rc) return rc;
+        CK(ctx->list_dedup.reserve((size_t)list->count));
+        CK(ctx->list_mask.reserve((npix + 31) / 32));
     }
     p.total_items = list ? (uint32_t)list->count : (uint32_t)(owned * 32);
-    if (list) p.pixels = list_prog ? ctx->list_dedup : list->pixels;
+    if (list) p.pixels = list_prog ? ctx->list_dedup.ptr : list->pixels;
     p.finalize = finalize ? 1 : 0;
     p.variant = a->tune[1] ? a->tune[1] : ctx->default_variant;
     p.out = out_dev;
-    p.work_counter = ctx->work_counter;
-    p.counters = ctx->counters;
-    CK(cudaMemsetAsync(ctx->counters, 0, 32 * 8, ctx->stream));
+    p.work_counter = ctx->work_counter.ptr;
+    p.counters = ctx->counters.ptr;
+    CK(cudaMemsetAsync(ctx->counters.ptr, 0, 32 * 8, ctx->stream));
     int blocks = 0;
     int launches = 1;
     const int mode = list_prog ? kModeListProgressive : list ? kModeList : kModeFrame;
     if (a->seed_mode == RT_SEED_UPSTREAM && !continuing) {
-        if (!ctx->skip_tables) {
+        if (!ctx->skip_tables.ptr) {
             const std::vector<uint32_t> &t = host_skip_tables();
-            CK(cudaMalloc(&ctx->skip_tables, t.size() * 4));
-            CK(cudaMemcpyAsync(ctx->skip_tables, t.data(), t.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+            CK(ctx->skip_tables.reserve(t.size()));
+            CK(cudaMemcpyAsync(ctx->skip_tables.ptr, t.data(), t.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
         }
         if (!list_prog) {       // (a progressive list seeds its pixels straight into the caller's state buffer)
             const size_t nstates = list ? (size_t)list->count : npix;      // stream states to seed
-            if (ctx->seed_states_words < nstates * 6) {
-                cudaFree(ctx->seed_states);
-                ctx->seed_states = nullptr; ctx->seed_states_words = 0;
-                CK(cudaMalloc(&ctx->seed_states, nstates * 6 * 4));
-                ctx->seed_states_words = nstates * 6;
-            }
-            p.seed_states = ctx->seed_states;
+            CK(ctx->seed_states.reserve(nstates * 6));
+            p.seed_states = ctx->seed_states.ptr;
         }
     }
     if (list_prog) {
@@ -688,10 +636,10 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
         p.seed_states = prog->state;                  // every pixel resumes its own stream
     } else if (p.seed_states) {   // render_init (main.cu:424): inside the timed region, as in the reference
         if (list)                 // only the listed pixels' streams
-            CK(launch_seed_upstream_list(ctx->seed_states, list->pixels, list->count, (size_t)a->nx * a->ny, 1984ull, ctx->skip_tables,
+            CK(launch_seed_upstream_list(ctx->seed_states.ptr, list->pixels, list->count, (size_t)a->nx * a->ny, 1984ull, ctx->skip_tables.ptr,
                                          ctx->stream));
         else                      // spp shard g draws from subsequences pixel_index + g * num_pixels (g = 0: the reference's streams)
-            CK(launch_seed_upstream(ctx->seed_states, (size_t)a->nx * a->ny, 1984ull, p.seed_offset, ctx->skip_tables, ctx->stream));
+            CK(launch_seed_upstream(ctx->seed_states.ptr, (size_t)a->nx * a->ny, 1984ull, p.seed_offset, ctx->skip_tables.ptr, ctx->stream));
         launches = 2;
     }
     if (fp16) {
@@ -703,10 +651,11 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
     // rt_render_pixels_progressive: dedupe, counts and (first) seeding, inside the timed region as the frames' seeding, and after
     // the last step that can fail on the context's side, so that an error leaves the caller's buffers untouched
     if (list_prog)
-        CK(launch_pixels_progressive_prep(list->pixels, list->count, (uint32_t)npix, ctx->list_mask, ctx->list_dedup, prog->counts, (uint32_t)a->ns,
-                                          prog->first, prog->state, a->seed_mode == RT_SEED_UPSTREAM ? ctx->skip_tables : nullptr, ctx->stream));
+        CK(launch_pixels_progressive_prep(list->pixels, list->count, (uint32_t)npix, ctx->list_mask.ptr, ctx->list_dedup.ptr, prog->counts,
+                                          (uint32_t)a->ns, prog->first, prog->state, a->seed_mode == RT_SEED_UPSTREAM ? ctx->skip_tables.ptr : nullptr,
+                                          ctx->stream));
     if (fp16) {
-        CK(launch_render_half(p, a->use_octree != 0, ctx->geom_h, ctx->matl_h, ctx->cam_h, ctx->half_pairs, ctx->prop.multiProcessorCount,
+        CK(launch_render_half(p, a->use_octree != 0, ctx->geom_h.ptr, ctx->matl_h.ptr, ctx->cam_h.ptr, ctx->half_pairs, ctx->prop.multiProcessorCount,
                               ctx->stream, &blocks, mode));
         ctx->last_kernel = kKernelHalf;
     } else {
@@ -740,7 +689,7 @@ extern "C" int rt_last_render_stats(rt_context *ctx, rt_render_stats *stats) {
 extern "C" int rt_debug_counters(rt_context *ctx, uint64_t out[32]) {
     if (!ctx || !out) return fail(ctx, RT_ERR_INVALID, "rt_debug_counters: null argument");
     CK(cudaSetDevice(ctx->device));
-    CK(cudaMemcpyAsync(out, ctx->counters, 32 * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(out, ctx->counters.ptr, 32 * 8, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return RT_OK;
 }
@@ -768,12 +717,9 @@ static int run_staged(rt_context *ctx, std::initializer_list<HostArray> arrays, 
     auto padded = [](size_t bytes) { return (bytes + 15) & ~(size_t)15; };
     size_t total = 0;
     for (const HostArray &a : arrays) total += padded(a.bytes);
-    char *base = nullptr;
-    CK(cudaMalloc(&base, total));
-    struct Release {
-        void *p;
-        ~Release() { cudaFree(p); }
-    } release{base};
+    Buffer<char> buf;
+    CK(buf.reserve(total));
+    char *base = buf.ptr;
     std::vector<DevPtr> dev;
     size_t off = 0;
     for (const HostArray &a : arrays) {
@@ -816,15 +762,15 @@ extern "C" int rt_trace_rays_ex(rt_context *ctx, int use_octree, int precision, 
     if (precision != RT_PREC_FP32 && precision != RT_PREC_FP16) return fail(ctx, RT_ERR_INVALID, "rt_trace_rays_ex: unknown precision");
     if (!ctx || n < 1 || !org || !dir || !out_idx || !out_t) return fail(ctx, RT_ERR_INVALID, "rt_trace_rays_ex: bad arguments");
     if (ctx->n < 1) return fail(ctx, RT_ERR_STATE, "rt_trace_rays_ex: no scene");
-    if (use_octree && !ctx->octree->built) return fail(ctx, RT_ERR_STATE, "rt_trace_rays_ex: no octree built");
+    if (use_octree && !ctx->octree.built) return fail(ctx, RT_ERR_STATE, "rt_trace_rays_ex: no octree built");
     const bool fp16 = precision == RT_PREC_FP16;
-    if (use_octree && ctx->octree->fp16 != fp16)
+    if (use_octree && ctx->octree.fp16 != fp16)
         return fail(ctx, RT_ERR_STATE, "rt_trace_rays_ex: the octree was built for the other precision (rt_octree_build_ex)");
     CK(cudaSetDevice(ctx->device));
     RenderLaunch p;
     memset(&p, 0, sizeof p);
-    p.scene.geom = ctx->geom; p.scene.matl = ctx->matl; p.scene.tag = ctx->tag; p.scene.n = ctx->n;
-    if (use_octree) p.tree = ctx->octree->view();
+    p.scene.geom = ctx->geom.ptr; p.scene.matl = ctx->matl.ptr; p.scene.tag = ctx->tag.ptr; p.scene.n = ctx->n;
+    if (use_octree) p.tree = ctx->octree.view();
     if (fp16) {
         const int rc = ensure_half(ctx, kHalfPairs, use_octree != 0, p.tree, 0, 0);
         if (rc) return rc;
@@ -833,7 +779,7 @@ extern "C" int rt_trace_rays_ex(rt_context *ctx, int use_octree, int precision, 
     }
     const size_t N = (size_t)n;
     return run_staged(ctx, {stage_in(org, 3 * N), stage_in(dir, 3 * N), stage_out(out_idx, N), stage_out(out_t, N)}, [&](const DevPtr *d) {
-        return fp16 ? launch_trace_rays_half(p, use_octree != 0, ctx->geom_h, ctx->half_pairs, d[0], d[1], n, d[2], d[3], ctx->stream)
+        return fp16 ? launch_trace_rays_half(p, use_octree != 0, ctx->geom_h.ptr, ctx->half_pairs, d[0], d[1], n, d[2], d[3], ctx->stream)
                     : launch_trace_rays(p, use_octree != 0, d[0], d[1], n, d[2], d[3], ctx->stream);
     });
 }
@@ -852,7 +798,7 @@ extern "C" int rt_camera_get_rays_ex(rt_context *ctx, int precision, int n, cons
     const size_t N = (size_t)n;
     return run_staged(ctx, {stage_in(s, N), stage_in(t, N), stage_inout(states6, 6 * N), stage_out(org, 3 * N), stage_out(dir, 3 * N)},
                       [&](const DevPtr *d) {
-                          return fp16 ? launch_camera_rays_half(ctx->cam_h, n, d[0], d[1], d[2], d[3], d[4], ctx->stream)
+                          return fp16 ? launch_camera_rays_half(ctx->cam_h.ptr, n, d[0], d[1], d[2], d[3], d[4], ctx->stream)
                                       : launch_camera_rays(ctx->cam_host, n, d[0], d[1], d[2], d[3], d[4], ctx->stream);
                       });
 }
@@ -872,13 +818,13 @@ extern "C" int rt_scatter_rays_ex(rt_context *ctx, int precision, int n, const i
         if (rc) return rc;
     }
     SceneView sv;
-    sv.geom = ctx->geom; sv.matl = ctx->matl; sv.tag = ctx->tag; sv.n = ctx->n;
+    sv.geom = ctx->geom.ptr; sv.matl = ctx->matl.ptr; sv.tag = ctx->tag.ptr; sv.n = ctx->n;
     const size_t N = (size_t)n;
     return run_staged(ctx, {stage_in(sphere_idx, N), stage_in(org, 3 * N), stage_in(dir, 3 * N), stage_in(t_hit, N), stage_inout(states6, 6 * N),
                             stage_out(out_p, 3 * N), stage_out(out_normal, 3 * N), stage_out(out_dir, 3 * N), stage_out(out_atten, 3 * N),
                             stage_out(scattered, N)},
                       [&](const DevPtr *d) {
-                          return fp16 ? launch_scatter_rays_half(sv, ctx->geom_h, ctx->matl_h, n, d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7],
+                          return fp16 ? launch_scatter_rays_half(sv, ctx->geom_h.ptr, ctx->matl_h.ptr, n, d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7],
                                                                  d[8], d[9], ctx->stream)
                                       : launch_scatter_rays(sv, n, d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7], d[8], d[9], ctx->stream);
                       });
@@ -976,24 +922,22 @@ extern "C" int rt_render_adaptive(rt_context *ctx, const rt_render_args *args, c
         (err_dev && !on_device(ctx, err_dev)))
         return fail(ctx, RT_ERR_INVALID, "rt_render_adaptive: accum, state, counts, fb and err must be device memory of the context's GPU");
     if (ctx->n < 1) return fail(ctx, RT_ERR_STATE, "rt_render_adaptive: no scene (rt_scene_generate / rt_scene_upload first)");
-    if (args->use_octree && !ctx->octree->built) return fail(ctx, RT_ERR_STATE, "rt_render_adaptive: USE_OCTREE set but no octree built");
+    if (args->use_octree && !ctx->octree.built) return fail(ctx, RT_ERR_STATE, "rt_render_adaptive: USE_OCTREE set but no octree built");
     const bool fp16 = args->precision == RT_PREC_FP16;
-    if (args->use_octree && ctx->octree->fp16 != fp16)
+    if (args->use_octree && ctx->octree.fp16 != fp16)
         return fail(ctx, RT_ERR_STATE, "rt_render_adaptive: the octree was built for the other precision (rt_octree_build_ex)");
     CK(cudaSetDevice(ctx->device));
     // scratch, before anything is launched: the snapshot, the tile words, the list, the scan's storage, and the rounds' list scratch
     size_t scan_bytes = 0;
     CK(adaptive_scan_temp_bytes((uint32_t)tiles, &scan_bytes));
-    int rc = ensure_words(ctx, ctx->ad_snap, ctx->ad_snap_words, npix * 3);
-    if (!rc) rc = ensure_words(ctx, ctx->ad_tiles, ctx->ad_tiles_words, (size_t)tiles * 3);
-    if (!rc) rc = ensure_words(ctx, ctx->ad_list, ctx->ad_list_words, npix);
-    if (!rc) rc = ensure_words(ctx, ctx->ad_scan, ctx->ad_scan_words, scan_bytes / 4 + 1);
-    if (!rc) rc = ensure_words(ctx, ctx->list_dedup, ctx->list_dedup_words, npix);
-    if (!rc) rc = ensure_words(ctx, ctx->list_mask, ctx->list_mask_words, (npix + 31) / 32);
-    if (rc) return rc;
-    if (!ctx->ad_ev0) CK(cudaEventCreate(&ctx->ad_ev0));
-    if (!ctx->ad_ev1) CK(cudaEventCreate(&ctx->ad_ev1));
+    CK(ctx->ad_snap.reserve(npix * 3));
+    CK(ctx->ad_tiles.reserve((size_t)tiles * 3));
+    CK(ctx->ad_list.reserve(npix));
+    CK(ctx->ad_scan.reserve(scan_bytes / 4 + 1));
+    CK(ctx->list_dedup.reserve(npix));
+    CK(ctx->list_mask.reserve((npix + 31) / 32));
 
+    int rc;
     rt_render_stats sum, one;
     memset(&sum, 0, sizeof sum);
     auto render = [&](rt_render_args &ra, const ProgressiveIO &io, const PixelList *list) {
@@ -1010,26 +954,26 @@ extern "C" int rt_render_adaptive(rt_context *ctx, const rt_render_args *args, c
     io.state = rng_state_dev;
     io.first = true;
     if ((rc = render(ra, io, nullptr))) return rc;
-    CK(cudaMemcpyAsync(ctx->ad_snap, accum_dev, npix * 3 * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->ad_snap.ptr, accum_dev, npix * 3 * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
     io.first = false;
     if ((rc = render(ra, io, nullptr))) return rc;
     CK(launch_fill_counts(counts_dev, npix, (uint32_t)min_spp, ctx->stream));
     AdaptiveTiles t;
-    t.listed = ctx->ad_tiles; t.offset = ctx->ad_tiles + tiles; t.done = ctx->ad_tiles + 2 * tiles;
-    t.scan_temp = ctx->ad_scan; t.scan_temp_bytes = ctx->ad_scan_words * 4;
+    t.listed = ctx->ad_tiles.ptr; t.offset = ctx->ad_tiles.ptr + tiles; t.done = ctx->ad_tiles.ptr + 2 * tiles;
+    t.scan_temp = ctx->ad_scan.ptr; t.scan_temp_bytes = ctx->ad_scan.cap * 4;
     CK(cudaMemsetAsync(t.done, 0, (size_t)tiles * 4, ctx->stream));
     // rounds: the tiles not done all have snapshot count a and count c; a refined tile doubles its count, capped at max_spp, so
     // there are at most ceil(log2(max_spp / min_spp)) <= 15 rounds
     io.counts = counts_dev;
     PixelList list;
-    list.pixels = ctx->ad_list;
+    list.pixels = ctx->ad_list.ptr;
     uint32_t a = (uint32_t)min_spp / 2, c = (uint32_t)min_spp;
     int rounds = 0;
     uint64_t round_pixels[16] = {};
     for (;;) {
         uint32_t listed = 0;
-        CK(launch_adaptive_select(accum_dev, reinterpret_cast<float *>(ctx->ad_snap), err_dev, args->nx, args->ny, a, c, c < (uint32_t)max_spp,
-                                  threshold, t, ctx->ad_list, &listed, ctx->stream));
+        CK(launch_adaptive_select(accum_dev, ctx->ad_snap.ptr, err_dev, args->nx, args->ny, a, c, c < (uint32_t)max_spp, threshold, t,
+                                  ctx->ad_list.ptr, &listed, ctx->stream));
         if (listed == 0) break;
         const uint32_t more = c < (uint32_t)max_spp - c ? c : (uint32_t)max_spp - c;
         ra.ns = (int)more;
@@ -1056,21 +1000,15 @@ extern "C" int rt_render_adaptive(rt_context *ctx, const rt_render_args *args, c
 // rt_render into the context's scratch frame, grown to the frame's size: the device frame of the host and PPM outputs
 static int render_to_scratch(rt_context *ctx, const rt_render_args *args, rt_render_stats *stats) {
     CK(cudaSetDevice(ctx->device));
-    const size_t bytes = (size_t)args->nx * args->ny * 3 * sizeof(float);
-    if (bytes > ctx->scratch_fb_bytes) {
-        cudaFree(ctx->scratch_fb);
-        ctx->scratch_fb = nullptr; ctx->scratch_fb_bytes = 0;
-        CK(cudaMalloc(&ctx->scratch_fb, bytes));
-        ctx->scratch_fb_bytes = bytes;
-    }
-    return do_render(ctx, args, ctx->scratch_fb, true, stats);
+    CK(ctx->scratch_fb.reserve((size_t)args->nx * args->ny * 3));
+    return do_render(ctx, args, ctx->scratch_fb.ptr, true, stats);
 }
 
 extern "C" int rt_render_to_host(rt_context *ctx, const rt_render_args *args, float *fb_host, rt_render_stats *stats) {
     if (!ctx || !args || !fb_host) return fail(ctx, RT_ERR_INVALID, "rt_render_to_host: null argument");
     const int rc = render_to_scratch(ctx, args, stats);
     if (rc) return rc;
-    CK(cudaMemcpyAsync(fb_host, ctx->scratch_fb, (size_t)args->nx * args->ny * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(fb_host, ctx->scratch_fb.ptr, (size_t)args->nx * args->ny * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return RT_OK;
 }
@@ -1085,9 +1023,9 @@ extern "C" int rt_ppm_format(rt_context *ctx, const float *fb_dev, int nx, int n
 
 extern "C" int rt_ppm_read(rt_context *ctx, char *buf_host, size_t cap) {
     if (!ctx || !buf_host) return fail(ctx, RT_ERR_INVALID, "rt_ppm_read: null argument");
-    if (!ctx->ppm.text || cap < ctx->ppm.text_len) return fail(ctx, RT_ERR_INVALID, "rt_ppm_read: no formatted frame, or the buffer is smaller than its text");
+    if (!ctx->ppm.text.ptr || cap < ctx->ppm.text_len) return fail(ctx, RT_ERR_INVALID, "rt_ppm_read: no formatted frame, or the buffer is smaller than its text");
     CK(cudaSetDevice(ctx->device));
-    CK(cudaMemcpyAsync(buf_host, ctx->ppm.text, ctx->ppm.text_len, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(buf_host, ctx->ppm.text.ptr, ctx->ppm.text_len, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return RT_OK;
 }
@@ -1096,7 +1034,7 @@ extern "C" int rt_render_to_ppm(rt_context *ctx, const rt_render_args *args, rt_
     if (!ctx || !args) return fail(ctx, RT_ERR_INVALID, "rt_render_to_ppm: null argument");
     const int rc = render_to_scratch(ctx, args, stats);
     if (rc) return rc;
-    CK(ppm_format_device(ctx->ppm, ctx->scratch_fb, args->nx, args->ny, ctx->stream, len_out));
+    CK(ppm_format_device(ctx->ppm, ctx->scratch_fb.ptr, args->nx, args->ny, ctx->stream, len_out));
     return RT_OK;
 }
 
@@ -1169,7 +1107,7 @@ static int peak_rate(rt_context *ctx, double iter_flops, float *tflops, float *m
 
 extern "C" int rt_ffma_peak(rt_context *ctx, float *tflops, float *ms_out) {
     return peak_rate(ctx, 2.0 * 8 * 16, tflops, ms_out, [&](int blocks, int threads, int iters) {
-        k_ffma_peak<<<blocks, threads, 0, ctx->stream>>>(reinterpret_cast<float *>(ctx->counters), iters, 1.000001f, 1e-7f);
+        k_ffma_peak<<<blocks, threads, 0, ctx->stream>>>(reinterpret_cast<float *>(ctx->counters.ptr), iters, 1.000001f, 1e-7f);
     });
 }
 
@@ -1194,7 +1132,7 @@ __global__ void __launch_bounds__(256) k_hfma2_peak(float *out, int iters, float
 
 extern "C" int rt_hfma2_peak(rt_context *ctx, float *tflops, float *ms_out) {
     return peak_rate(ctx, 4.0 * 8 * 16, tflops, ms_out, [&](int blocks, int threads, int iters) {
-        k_hfma2_peak<<<blocks, threads, 0, ctx->stream>>>(reinterpret_cast<float *>(ctx->counters), iters, 0.999f, 1e-3f);
+        k_hfma2_peak<<<blocks, threads, 0, ctx->stream>>>(reinterpret_cast<float *>(ctx->counters.ptr), iters, 0.999f, 1e-3f);
     });
 }
 

@@ -390,27 +390,14 @@ static void make_planes(BuildPlanes &P) {
     }
 }
 
+// the arrays sized by the scene grow with headroom, so that rebuilds of slightly larger scenes reuse them
 template <typename T>
-static cudaError_t ensure(T *&ptr, size_t &cap, size_t need) {
-    if (need <= cap) return cudaSuccess;
-    if (ptr) cudaFree(ptr);
-    ptr = nullptr;
-    cap = 0;
-    size_t want = need + need / 4 + 256;
-    cudaError_t e = cudaMalloc(reinterpret_cast<void **>(&ptr), want * sizeof(T));
-    if (e == cudaSuccess) cap = want;
-    return e;
+static cudaError_t ensure(Buffer<T> &b, size_t need) {
+    return b.reserve(need, need / 4 + 256);
 }
 
 OctreeBuilder::OctreeBuilder() : grid_flat(kGridFlat), grid_wide(kGridWide), grid_flat_min(kFlatVoxelMinSpheres) {
-    memset(&d, 0, sizeof d); memset(&cap, 0, sizeof cap); memset(&grid, 0, sizeof grid); make_planes(planes);
-}
-
-OctreeBuilder::~OctreeBuilder() {
-    void *ptrs[] = {d.ranges, d.ent_count, d.ent_off, d.keys, d.vals, d.keys_sorted, d.vals_sorted, d.cell_count,
-                    d.cell_start, d.ent_cell, d.sph_flag, d.stats, d.node_of_potential, d.counts, d.prep, d.big_refs,
-                    d.vox_count, d.vox_start, d.vox_refs, d.vox, d.cub_tmp, d.leaf_index, d.blob, d.ref_geom, d.prolog_geom};
-    for (void *p : ptrs) if (p) cudaFree(p);
+    memset(&grid, 0, sizeof grid); make_planes(planes);
 }
 
 // RT_BUILD_TRACE=1: host wall clock at the build's synchronisation points (diagnostic, stderr)
@@ -433,65 +420,63 @@ cudaError_t OctreeBuilder::build(cudaStream_t st, const float4 *geom, const int 
     all_spheres = all_spheres_;
     built = false;
     blob_valid = false;
-    RT_CUDA(ensure(d.ranges, cap.ranges, (size_t)n + 1));
-    RT_CUDA(ensure(d.ent_count, cap.ent_count, (size_t)n + 1));
-    RT_CUDA(ensure(d.ent_off, cap.ent_off, (size_t)n + 1));
-    RT_CUDA(ensure(d.sph_flag, cap.sph_flag, (size_t)n + 1));
-    if (!d.cell_count) {
-        RT_CUDA(cudaMalloc(&d.cell_count, kCells * 4));
-        RT_CUDA(cudaMalloc(&d.cell_start, (kCells + 1) * 4));
-        RT_CUDA(cudaMalloc(&d.stats, 4 * 8));
-        RT_CUDA(cudaMalloc(&d.node_of_potential, kNumberNodes * 4));
-        RT_CUDA(cudaMalloc(&d.counts, sizeof(BuildCounts)));
-        RT_CUDA(cudaMalloc(&d.prep, sizeof(GridPrep)));
-        RT_CUDA(cudaMalloc(&d.big_refs, (kMaxBig + 1) * 4));   // [0] = ground sphere, then the big spheres
-        RT_CUDA(cudaMalloc(&d.leaf_index, kCells * 8 * 4 + 4));
-    }
-    RT_CUDA(cudaMemsetAsync(d.cell_count, 0, kCells * 4, st));
-    RT_CUDA(cudaMemsetAsync(d.stats, 0, 4 * 8, st));
-    RT_CUDA(cudaMemsetAsync(d.ent_count + n, 0, 4, st));
-    RT_CUDA(cudaMemsetAsync(d.sph_flag, 0, (size_t)n + 1, st));
+    RT_CUDA(ensure(d.ranges, (size_t)n + 1));
+    RT_CUDA(ensure(d.ent_count, (size_t)n + 1));
+    RT_CUDA(ensure(d.ent_off, (size_t)n + 1));
+    RT_CUDA(ensure(d.sph_flag, (size_t)n + 1));
+    RT_CUDA(d.cell_count.reserve(kCells));
+    RT_CUDA(d.cell_start.reserve(kCells + 1));
+    RT_CUDA(d.stats.reserve(4));
+    RT_CUDA(d.node_of_potential.reserve(kNumberNodes));
+    RT_CUDA(d.counts.reserve(1));
+    RT_CUDA(d.prep.reserve(1));
+    RT_CUDA(d.big_refs.reserve(kMaxBig + 1));   // [0] = ground sphere, then the big spheres
+    RT_CUDA(d.leaf_index.reserve(kCells * 8 + 1));
+    RT_CUDA(cudaMemsetAsync(d.cell_count.ptr, 0, kCells * 4, st));
+    RT_CUDA(cudaMemsetAsync(d.stats.ptr, 0, 4 * 8, st));
+    RT_CUDA(cudaMemsetAsync(d.ent_count.ptr + n, 0, 4, st));
+    RT_CUDA(cudaMemsetAsync(d.sph_flag.ptr, 0, (size_t)n + 1, st));
     const int tb = 256;
-    k_classify<<<(n + tb - 1) / tb, tb, 0, st>>>(geom, n, planes, fp16 ? 1 : 0, d.ranges, d.ent_count, d.cell_count, d.stats + 2);
+    k_classify<<<(n + tb - 1) / tb, tb, 0, st>>>(geom, n, planes, fp16 ? 1 : 0, d.ranges.ptr, d.ent_count.ptr, d.cell_count.ptr, d.stats.ptr + 2);
     size_t tmp = 0;
-    cub::DeviceScan::ExclusiveSum(nullptr, tmp, d.ent_count, d.ent_off, n + 1, st);
-    RT_CUDA(ensure(d.cub_tmp, cap.cub, tmp));
-    cub::DeviceScan::ExclusiveSum(d.cub_tmp, tmp, d.ent_count, d.ent_off, n + 1, st);
+    cub::DeviceScan::ExclusiveSum(nullptr, tmp, d.ent_count.ptr, d.ent_off.ptr, n + 1, st);
+    RT_CUDA(ensure(d.cub_tmp, tmp));
+    cub::DeviceScan::ExclusiveSum(d.cub_tmp.ptr, tmp, d.ent_count.ptr, d.ent_off.ptr, n + 1, st);
     uint32_t E_h = 0;
-    RT_CUDA(cudaMemcpyAsync(&E_h, d.ent_off + n, 4, cudaMemcpyDeviceToHost, st));
+    RT_CUDA(cudaMemcpyAsync(&E_h, d.ent_off.ptr + n, 4, cudaMemcpyDeviceToHost, st));
     trace.mark("classify+scan issued");
     RT_CUDA(cudaStreamSynchronize(st));
     trace.mark("sync 1 (entry count)");
     E = E_h;
-    RT_CUDA(ensure(d.keys, cap.keys, (size_t)E + 1));
-    RT_CUDA(ensure(d.vals, cap.vals, (size_t)E + 1));
-    RT_CUDA(ensure(d.keys_sorted, cap.keys_sorted, (size_t)E + 1));
-    RT_CUDA(ensure(d.vals_sorted, cap.vals_sorted, (size_t)E + 1));
-    RT_CUDA(ensure(d.ent_cell, cap.ent_cell, (size_t)E + 2));
-    k_emit<<<(n + tb - 1) / tb, tb, 0, st>>>(d.ranges, d.ent_off, n, d.keys, d.vals, d.ent_cell);
+    RT_CUDA(ensure(d.keys, (size_t)E + 1));
+    RT_CUDA(ensure(d.vals, (size_t)E + 1));
+    RT_CUDA(ensure(d.keys_sorted, (size_t)E + 1));
+    RT_CUDA(ensure(d.vals_sorted, (size_t)E + 1));
+    RT_CUDA(ensure(d.ent_cell, (size_t)E + 2));
+    k_emit<<<(n + tb - 1) / tb, tb, 0, st>>>(d.ranges.ptr, d.ent_off.ptr, n, d.keys.ptr, d.vals.ptr, d.ent_cell.ptr);
     if (E > 0) {
         tmp = 0;
-        cub::DeviceRadixSort::SortPairs(nullptr, tmp, d.keys, d.keys_sorted, d.vals, d.vals_sorted, (int)E, 0, 9, st);
-        RT_CUDA(ensure(d.cub_tmp, cap.cub, tmp));
-        cub::DeviceRadixSort::SortPairs(d.cub_tmp, tmp, d.keys, d.keys_sorted, d.vals, d.vals_sorted, (int)E, 0, 9, st);
+        cub::DeviceRadixSort::SortPairs(nullptr, tmp, d.keys.ptr, d.keys_sorted.ptr, d.vals.ptr, d.vals_sorted.ptr, (int)E, 0, 9, st);
+        RT_CUDA(ensure(d.cub_tmp, tmp));
+        cub::DeviceRadixSort::SortPairs(d.cub_tmp.ptr, tmp, d.keys.ptr, d.keys_sorted.ptr, d.vals.ptr, d.vals_sorted.ptr, (int)E, 0, 9, st);
     }
-    k_cell_scan<<<1, kCells, 0, st>>>(d.cell_count, d.cell_start);
+    k_cell_scan<<<1, kCells, 0, st>>>(d.cell_count.ptr, d.cell_start.ptr);
     if (E > 0)
-        k_mark_entries<<<(E + tb - 1) / tb, tb, 0, st>>>(d.keys_sorted, d.vals_sorted, d.cell_start, E, spl, d.ranges, d.ent_off,
-                                                        d.ent_cell, d.sph_flag, d.stats);
-    k_number_nodes<<<1, 1024, 0, st>>>(d.vals_sorted, d.cell_start, d.node_of_potential, d.counts);
+        k_mark_entries<<<(E + tb - 1) / tb, tb, 0, st>>>(d.keys_sorted.ptr, d.vals_sorted.ptr, d.cell_start.ptr, E, spl, d.ranges.ptr,
+                                                        d.ent_off.ptr, d.ent_cell.ptr, d.sph_flag.ptr, d.stats.ptr);
+    k_number_nodes<<<1, 1024, 0, st>>>(d.vals_sorted.ptr, d.cell_start.ptr, d.node_of_potential.ptr, d.counts.ptr);
     // grid over the small stored spheres
     GridPrep init;
     memset(&init, 0, sizeof init);
     for (int k = 0; k < 3; k++) { init.lo[k] = 0xffffffffu; init.hi[k] = 0u; }
-    RT_CUDA(cudaMemcpyAsync(d.prep, &init, sizeof init, cudaMemcpyHostToDevice, st));
+    RT_CUDA(cudaMemcpyAsync(d.prep.ptr, &init, sizeof init, cudaMemcpyHostToDevice, st));
     const float big_r = kBigRadiusFrac * fmaxf(planes.p[0][1] - planes.p[0][0], fmaxf(planes.p[1][1] - planes.p[1][0], planes.p[2][1] - planes.p[2][0]));
-    if (all_spheres) RT_CUDA(cudaMemsetAsync(d.sph_flag + 1, 1, (size_t)n - 1, st));     // every sphere but the ground (prolog[0])
-    k_grid_prep<<<(n + tb - 1) / tb, tb, 0, st>>>(geom, tag, n, big_r, d.sph_flag, d.prep);
+    if (all_spheres) RT_CUDA(cudaMemsetAsync(d.sph_flag.ptr + 1, 1, (size_t)n - 1, st));     // every sphere but the ground (prolog[0])
+    k_grid_prep<<<(n + tb - 1) / tb, tb, 0, st>>>(geom, tag, n, big_r, d.sph_flag.ptr, d.prep.ptr);
     GridPrep prep;
-    RT_CUDA(cudaMemcpyAsync(&prep, d.prep, sizeof prep, cudaMemcpyDeviceToHost, st));
-    RT_CUDA(cudaMemcpyAsync(&counts, d.counts, sizeof counts, cudaMemcpyDeviceToHost, st));
-    RT_CUDA(cudaMemcpyAsync(stats_h, d.stats, 4 * 8, cudaMemcpyDeviceToHost, st));
+    RT_CUDA(cudaMemcpyAsync(&prep, d.prep.ptr, sizeof prep, cudaMemcpyDeviceToHost, st));
+    RT_CUDA(cudaMemcpyAsync(&counts, d.counts.ptr, sizeof counts, cudaMemcpyDeviceToHost, st));
+    RT_CUDA(cudaMemcpyAsync(stats_h, d.stats.ptr, 4 * 8, cudaMemcpyDeviceToHost, st));
     trace.mark("sort..grid_prep issued");
     RT_CUDA(cudaStreamSynchronize(st));
     trace.mark("sync 2 (counts, grid box)");
@@ -500,42 +485,43 @@ cudaError_t OctreeBuilder::build(cudaStream_t st, const float4 *geom, const int 
     std::sort(prep.big, prep.big + nbig);       // ascending: deterministic traversal order
     prolog_h[0] = 0;
     memcpy(prolog_h + 1, prep.big, kMaxBig * 4);
-    RT_CUDA(cudaMemcpyAsync(d.big_refs, prolog_h, (kMaxBig + 1) * 4, cudaMemcpyHostToDevice, st));
+    RT_CUDA(cudaMemcpyAsync(d.big_refs.ptr, prolog_h, (kMaxBig + 1) * 4, cudaMemcpyHostToDevice, st));
     float lo[3], hi[3];
     for (int k = 0; k < 3; k++) { lo[k] = ord2f(prep.lo[k]); hi[k] = ord2f(prep.hi[k]); }
     memset(&grid, 0, sizeof grid);
     const uint32_t V = choose_grid(lo, hi, prep.live, density, grid, grid_flat, grid_wide, grid_flat_min);
     total_voxels = V;
     total_refs = 0;
-    RT_CUDA(ensure(d.vox_count, cap.vox_count, (size_t)V + 2));
-    RT_CUDA(ensure(d.vox_start, cap.vox_start, (size_t)V + 2));
-    RT_CUDA(ensure(d.vox, cap.vox, (size_t)V + 1));
+    RT_CUDA(ensure(d.vox_count, (size_t)V + 2));
+    RT_CUDA(ensure(d.vox_start, (size_t)V + 2));
+    RT_CUDA(ensure(d.vox, (size_t)V + 1));
     if (V > 0) {
-        RT_CUDA(cudaMemsetAsync(d.vox_count, 0, ((size_t)V + 2) * 4, st));
-        k_vox_pass<false><<<(n + tb - 1) / tb, tb, 0, st>>>(geom, d.sph_flag, n, grid, d.vox_count, nullptr, nullptr);
+        RT_CUDA(cudaMemsetAsync(d.vox_count.ptr, 0, ((size_t)V + 2) * 4, st));
+        k_vox_pass<false><<<(n + tb - 1) / tb, tb, 0, st>>>(geom, d.sph_flag.ptr, n, grid, d.vox_count.ptr, nullptr, nullptr);
         tmp = 0;
-        cub::DeviceScan::ExclusiveSum(nullptr, tmp, d.vox_count, d.vox_start, (int)V + 1, st);
-        RT_CUDA(ensure(d.cub_tmp, cap.cub, tmp));
-        cub::DeviceScan::ExclusiveSum(d.cub_tmp, tmp, d.vox_count, d.vox_start, (int)V + 1, st);
+        cub::DeviceScan::ExclusiveSum(nullptr, tmp, d.vox_count.ptr, d.vox_start.ptr, (int)V + 1, st);
+        RT_CUDA(ensure(d.cub_tmp, tmp));
+        cub::DeviceScan::ExclusiveSum(d.cub_tmp.ptr, tmp, d.vox_count.ptr, d.vox_start.ptr, (int)V + 1, st);
         uint32_t R_h = 0;
-        RT_CUDA(cudaMemcpyAsync(&R_h, d.vox_start + V, 4, cudaMemcpyDeviceToHost, st));
+        RT_CUDA(cudaMemcpyAsync(&R_h, d.vox_start.ptr + V, 4, cudaMemcpyDeviceToHost, st));
         trace.mark("vox count pass issued");
         RT_CUDA(cudaStreamSynchronize(st));
         trace.mark("sync 3 (reference count)");
         total_refs = R_h;
-        RT_CUDA(ensure(d.vox_refs, cap.vox_refs, (size_t)total_refs + 1));
-        RT_CUDA(cudaMemsetAsync(d.vox_count, 0, ((size_t)V + 2) * 4, st));
-        k_vox_pass<true><<<(n + tb - 1) / tb, tb, 0, st>>>(geom, d.sph_flag, n, grid, d.vox_count, d.vox_start, d.vox_refs);
-        k_vox_finish<<<(V + tb - 1) / tb, tb, 0, st>>>(d.vox_start, V, d.vox_refs, d.vox);
-        RT_CUDA(ensure(d.ref_geom, cap.ref_geom, (size_t)total_refs + 4));   // (the cooperative kernel loads up to 3 entries past a list)
-        if (total_refs) k_gather_geom<<<(unsigned)(((size_t)total_refs + tb - 1) / tb), tb, 0, st>>>(geom, d.vox_refs, total_refs, d.ref_geom);
+        RT_CUDA(ensure(d.vox_refs, (size_t)total_refs + 1));
+        RT_CUDA(cudaMemsetAsync(d.vox_count.ptr, 0, ((size_t)V + 2) * 4, st));
+        k_vox_pass<true><<<(n + tb - 1) / tb, tb, 0, st>>>(geom, d.sph_flag.ptr, n, grid, d.vox_count.ptr, d.vox_start.ptr, d.vox_refs.ptr);
+        k_vox_finish<<<(V + tb - 1) / tb, tb, 0, st>>>(d.vox_start.ptr, V, d.vox_refs.ptr, d.vox.ptr);
+        RT_CUDA(ensure(d.ref_geom, (size_t)total_refs + 4));   // (the cooperative kernel loads up to 3 entries past a list)
+        if (total_refs)
+            k_gather_geom<<<(unsigned)(((size_t)total_refs + tb - 1) / tb), tb, 0, st>>>(geom, d.vox_refs.ptr, total_refs, d.ref_geom.ptr);
     }
-    if (!d.prolog_geom) RT_CUDA(cudaMalloc(&d.prolog_geom, (kMaxBig + 1) * sizeof(float4)));
-    k_gather_geom<<<1, kMaxBig + 1, 0, st>>>(geom, d.big_refs, (size_t)(1 + nbig), d.prolog_geom);
+    RT_CUDA(d.prolog_geom.reserve(kMaxBig + 1));
+    k_gather_geom<<<1, kMaxBig + 1, 0, st>>>(geom, d.big_refs.ptr, (size_t)(1 + nbig), d.prolog_geom.ptr);
     RT_CUDA(cudaGetLastError());
-    grid.vox = d.vox;
-    grid.refs = d.vox_refs;
-    grid.ref_geom = d.ref_geom;
+    grid.vox = d.vox.ptr;
+    grid.refs = d.vox_refs.ptr;
+    grid.ref_geom = d.ref_geom.ptr;
     built = true;
     n_spheres = n;
     trace.mark("fill passes issued (async)");
@@ -550,24 +536,24 @@ cudaError_t OctreeBuilder::export_reference(cudaStream_t st, void *host_blob, si
     if (!built) return cudaErrorNotReady;
     const size_t need = reference_bytes(spl, fp16);
     if (bytes < need) return cudaErrorInvalidValue;
-    RT_CUDA(ensure(d.blob, cap.blob, need));
-    RT_CUDA(cudaMemsetAsync(d.blob, 0, need, st));          // `new Octree()` value-initialises
-    int *leaf_count = d.leaf_index + kCells * 8;
+    RT_CUDA(ensure(d.blob, need));
+    RT_CUDA(cudaMemsetAsync(d.blob.ptr, 0, need, st));          // `new Octree()` value-initialises
+    int *leaf_count = d.leaf_index.ptr + kCells * 8;
     RT_CUDA(cudaMemsetAsync(leaf_count, 0, 4, st));
-    k_leaf_number<<<(kCells * 8 + 255) / 256, 256, 0, st>>>(d.vals_sorted, d.cell_start, spl, d.leaf_index, leaf_count);
+    k_leaf_number<<<(kCells * 8 + 255) / 256, 256, 0, st>>>(d.vals_sorted.ptr, d.cell_start.ptr, spl, d.leaf_index.ptr, leaf_count);
     // the leaves follow the nodes: OctLeaf is all ints in both layouts, and the buckets of an FP16 build are its own memberships
-    int32_t *leaves = reinterpret_cast<int32_t *>(d.blob + (size_t)kNumberNodes * (fp16 ? kNodeBytesHalf : kNodeInts * 4));
-    if (fp16) k_blob_nodes<true><<<(kNumberNodes + 255) / 256, 256, 0, st>>>(d.node_of_potential, d.leaf_index, planes, d.blob);
-    else k_blob_nodes<false><<<(kNumberNodes + 255) / 256, 256, 0, st>>>(d.node_of_potential, d.leaf_index, planes, d.blob);
+    int32_t *leaves = reinterpret_cast<int32_t *>(d.blob.ptr + (size_t)kNumberNodes * (fp16 ? kNodeBytesHalf : kNodeInts * 4));
+    if (fp16) k_blob_nodes<true><<<(kNumberNodes + 255) / 256, 256, 0, st>>>(d.node_of_potential.ptr, d.leaf_index.ptr, planes, d.blob.ptr);
+    else k_blob_nodes<false><<<(kNumberNodes + 255) / 256, 256, 0, st>>>(d.node_of_potential.ptr, d.leaf_index.ptr, planes, d.blob.ptr);
     if (E > 0)
-        k_blob_leaves<<<(E + 255) / 256, 256, 0, st>>>(d.keys_sorted, d.vals_sorted, d.cell_start, E, spl, d.leaf_index, leaves);
+        k_blob_leaves<<<(E + 255) / 256, 256, 0, st>>>(d.keys_sorted.ptr, d.vals_sorted.ptr, d.cell_start.ptr, E, spl, d.leaf_index.ptr, leaves);
     int lc = 0;
     RT_CUDA(cudaMemcpyAsync(&lc, leaf_count, 4, cudaMemcpyDeviceToHost, st));
     RT_CUDA(cudaStreamSynchronize(st));
     leaf_count_h = lc + 1;                                   // leafCount starts at 1 (:60)
     const int32_t tail[2] = {counts.node_count, leaf_count_h};
-    RT_CUDA(cudaMemcpyAsync(d.blob + need - 8, tail, 8, cudaMemcpyHostToDevice, st));
-    RT_CUDA(cudaMemcpyAsync(host_blob, d.blob, need, cudaMemcpyDeviceToHost, st));
+    RT_CUDA(cudaMemcpyAsync(d.blob.ptr + need - 8, tail, 8, cudaMemcpyHostToDevice, st));
+    RT_CUDA(cudaMemcpyAsync(host_blob, d.blob.ptr, need, cudaMemcpyDeviceToHost, st));
     RT_CUDA(cudaStreamSynchronize(st));
     blob_valid = true;
     return cudaGetLastError();
@@ -584,14 +570,14 @@ size_t OctreeBuilder::debug_read(cudaStream_t st, int which, void *host, size_t 
             memcpy(desc + 12, &grid.nx, 4); memcpy(desc + 13, &grid.ny, 4); memcpy(desc + 14, &grid.nz, 4);
             if (host && cap_bytes >= sizeof desc) memcpy(host, desc, sizeof desc);
             return sizeof desc;
-        case 1: src = d.vox; bytes = (size_t)total_voxels * sizeof(uint2); break;
-        case 2: src = d.vox_refs; bytes = (size_t)total_refs * 4; break;
-        case 3: src = d.ent_off; bytes = ((size_t)n_spheres + 1) * 4; break;
-        case 4: src = d.ent_cell; bytes = (size_t)E * 2; break;
-        case 5: src = d.big_refs + 1; bytes = (size_t)nbig * 4; break;
-        case 6: src = d.sph_flag; bytes = (size_t)n_spheres; break;
-        case 7: src = d.cell_start; bytes = (size_t)(kCells + 1) * 4; break;
-        case 8: src = d.vals_sorted; bytes = (size_t)E * 4; break;
+        case 1: src = d.vox.ptr; bytes = (size_t)total_voxels * sizeof(uint2); break;
+        case 2: src = d.vox_refs.ptr; bytes = (size_t)total_refs * 4; break;
+        case 3: src = d.ent_off.ptr; bytes = ((size_t)n_spheres + 1) * 4; break;
+        case 4: src = d.ent_cell.ptr; bytes = (size_t)E * 2; break;
+        case 5: src = d.big_refs.ptr + 1; bytes = (size_t)nbig * 4; break;
+        case 6: src = d.sph_flag.ptr; bytes = (size_t)n_spheres; break;
+        case 7: src = d.cell_start.ptr; bytes = (size_t)(kCells + 1) * 4; break;
+        case 8: src = d.vals_sorted.ptr; bytes = (size_t)E * 4; break;
         default: return 0;
     }
     if (!host) return bytes;
@@ -605,14 +591,14 @@ TreeView OctreeBuilder::view() const {
     TreeView v;
     memset(&v, 0, sizeof v);
     v.grid = grid;
-    v.vis.ent_off = d.ent_off;
-    v.vis.ent_cell = d.ent_cell;
-    v.cell_list = d.vals_sorted;
-    v.cell_start = d.cell_start;
+    v.vis.ent_off = d.ent_off.ptr;
+    v.vis.ent_cell = d.ent_cell.ptr;
+    v.cell_list = d.vals_sorted.ptr;
+    v.cell_start = d.cell_start.ptr;
     v.cell_cap = 8 * spl;
     v.check_visibility = all_spheres ? 0 : 1;
-    v.prolog = d.big_refs;
-    v.prolog_geom = d.prolog_geom;
+    v.prolog = d.big_refs.ptr;
+    v.prolog_geom = d.prolog_geom.ptr;
     v.nprolog = 1 + nbig;
     v.slot0_none = slot0_none;
     for (int a = 0; a < 3; a++) for (int i = 0; i < kPlanes; i++) v.planes[a][i] = planes.p[a][i];

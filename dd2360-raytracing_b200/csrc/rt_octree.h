@@ -4,6 +4,7 @@
 #include <stddef.h>
 #include <stdint.h>
 
+#include "rt_buffer.h"
 #include "rt_types.h"
 
 namespace rt {
@@ -24,9 +25,6 @@ struct GridPrep {                 // k_grid_prep output: bounding box (order-pre
 class OctreeBuilder {
 public:
     OctreeBuilder();
-    ~OctreeBuilder();
-    OctreeBuilder(const OctreeBuilder &) = delete;
-    OctreeBuilder &operator=(const OctreeBuilder &) = delete;
 
     // replaces D2H(spheres) + buildOctree + H2D(Octree), main.cu:405-415
     // fp16: the USE_FP16 build of the reference (half-rounded scene, half arithmetic in `intersects`)
@@ -59,25 +57,21 @@ public:
 
 private:
     struct {
-        uint32_t *ranges, *ent_count, *ent_off, *keys, *vals, *keys_sorted, *vals_sorted, *cell_count, *cell_start;
-        uint16_t *ent_cell;
-        uint8_t *sph_flag;
-        unsigned long long *stats;
-        int *node_of_potential;
-        BuildCounts *counts;
-        GridPrep *prep;
-        uint32_t *big_refs;
-        uint32_t *vox_count, *vox_start, *vox_refs;
-        float4 *ref_geom, *prolog_geom;
-        uint2 *vox;
-        uint8_t *cub_tmp;
-        int *leaf_index;
-        uint8_t *blob;
+        Buffer<uint32_t> ranges, ent_count, ent_off, keys, vals, keys_sorted, vals_sorted, cell_count, cell_start;
+        Buffer<uint16_t> ent_cell;
+        Buffer<uint8_t> sph_flag;
+        Buffer<unsigned long long> stats;
+        Buffer<int> node_of_potential;
+        Buffer<BuildCounts> counts;
+        Buffer<GridPrep> prep;
+        Buffer<uint32_t> big_refs;
+        Buffer<uint32_t> vox_count, vox_start, vox_refs;
+        Buffer<float4> ref_geom, prolog_geom;
+        Buffer<uint2> vox;
+        Buffer<uint8_t> cub_tmp;
+        Buffer<int> leaf_index;
+        Buffer<uint8_t> blob;
     } d;
-    struct {
-        size_t ranges, ent_count, ent_off, keys, vals, keys_sorted, vals_sorted, ent_cell, sph_flag, vox_count, vox_start,
-            vox_refs, vox, cub, blob, ref_geom;
-    } cap;
 };
 
 }  // namespace rt

@@ -161,40 +161,24 @@ cudaError_t ppm_format_device(PpmWorkspace &ws, const float *fb, int nx, int ny,
     const size_t npix = (size_t)nx * ny;
     const size_t blocks = (npix + kPpmThreads - 1) / kPpmThreads;
     cudaError_t e;
-    if (blocks + 1 > ws.block_cap) {
-        cudaFree(ws.block_len); cudaFree(ws.block_off);
-        ws.block_len = nullptr; ws.block_off = nullptr; ws.block_cap = 0;
-        if ((e = cudaMalloc(&ws.block_len, (blocks + 1) * sizeof(uint32_t))) != cudaSuccess) return e;
-        if ((e = cudaMalloc(&ws.block_off, (blocks + 1) * sizeof(unsigned long long))) != cudaSuccess) return e;
-        ws.block_cap = blocks + 1;
-    }
+    if ((e = ws.block_len.reserve(blocks + 1)) != cudaSuccess || (e = ws.block_off.reserve(blocks + 1)) != cudaSuccess) return e;
     PpmHead head;
     head.len = snprintf(head.text, sizeof head.text, "P3\n%d %d\n255\n", nx, ny);
-    if (blocks) k_ppm_len<<<(unsigned)blocks, kPpmThreads, 0, st>>>(fb, nx, ny, npix, ws.block_len);
-    k_ppm_scan<<<1, 1024, 0, st>>>(ws.block_len, blocks, (unsigned long long)head.len, ws.block_off);
+    if (blocks) k_ppm_len<<<(unsigned)blocks, kPpmThreads, 0, st>>>(fb, nx, ny, npix, ws.block_len.ptr);
+    k_ppm_scan<<<1, 1024, 0, st>>>(ws.block_len.ptr, blocks, (unsigned long long)head.len, ws.block_off.ptr);
     unsigned long long total = 0;
-    if ((e = cudaMemcpyAsync(&total, ws.block_off + blocks, sizeof total, cudaMemcpyDeviceToHost, st)) != cudaSuccess) return e;
+    if ((e = cudaMemcpyAsync(&total, ws.block_off.ptr + blocks, sizeof total, cudaMemcpyDeviceToHost, st)) != cudaSuccess) return e;
     if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return e;
-    if (total + 16 > ws.text_cap) {
-        cudaFree(ws.text);
-        ws.text = nullptr; ws.text_cap = 0;
-        if ((e = cudaMalloc(&ws.text, total + 16)) != cudaSuccess) return e;
-        ws.text_cap = total + 16;
-    }
+    if ((e = ws.text.reserve(total + 16)) != cudaSuccess) return e;
     if (blocks) {
-        k_ppm_write<<<(unsigned)blocks, kPpmThreads, 0, st>>>(fb, nx, ny, npix, ws.block_off, head, ws.text);
+        k_ppm_write<<<(unsigned)blocks, kPpmThreads, 0, st>>>(fb, nx, ny, npix, ws.block_off.ptr, head, ws.text.ptr);
     } else {
-        if ((e = cudaMemcpyAsync(ws.text, head.text, (size_t)head.len, cudaMemcpyHostToDevice, st)) != cudaSuccess) return e;
+        if ((e = cudaMemcpyAsync(ws.text.ptr, head.text, (size_t)head.len, cudaMemcpyHostToDevice, st)) != cudaSuccess) return e;
         if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return e;
     }
     ws.text_len = (size_t)total;
     if (len_out) *len_out = (size_t)total;
     return cudaGetLastError();
-}
-
-void ppm_free(PpmWorkspace &ws) {
-    cudaFree(ws.block_len); cudaFree(ws.block_off); cudaFree(ws.text);
-    ws = PpmWorkspace();
 }
 
 }  // namespace rt

@@ -302,8 +302,8 @@ cudaError_t launch_camera_setup_half(const float lookfrom[3], const float lookat
 }
 // the half kernels' views of the context's USE_FP16 pair lists and node tables
 static void half_views(const HalfPairs &hp, h16::PairView &pv, h16::NodeTab &nt) {
-    pv.geom = hp.geom; pv.idx = hp.idx; pv.start = hp.start;
-    nt.ent = hp.nodes; nt.count = hp.node_count;
+    pv.geom = hp.geom.ptr; pv.idx = hp.idx.ptr; pv.start = hp.start.ptr;
+    nt.ent = hp.nodes.ptr; nt.count = hp.node_count.ptr;
 }
 cudaError_t launch_render_half(const RenderLaunch &p, bool octree, const uint2 *geom_h, const uint2 *matl_h, const __half *cam_h,
                                const HalfPairs &hp, int sm_count, cudaStream_t st, int *blocks_out, int mode) {
@@ -375,36 +375,19 @@ cudaError_t launch_scatter_rays_half(const SceneView &sc, const uint2 *geom_h, c
 cudaError_t build_half_pairs(HalfPairs &hp, const uint2 *geom_h, const int *tag, int n, bool octree, const TreeView &tv, cudaStream_t st) {
     const int lists = octree ? kCells : 1;
     cudaError_t e;
-    if (!hp.count || !hp.start || !hp.nodes || !hp.node_count) {      // all four or none: a partial failure is rolled back
-        cudaFree(hp.count); cudaFree(hp.start); cudaFree(hp.nodes); cudaFree(hp.node_count);
-        hp.count = hp.start = nullptr; hp.nodes = nullptr; hp.node_count = nullptr;
-        if ((e = cudaMalloc(&hp.count, (kCells + 1) * 4)) != cudaSuccess || (e = cudaMalloc(&hp.start, (kCells + 2) * 4)) != cudaSuccess ||
-            (e = cudaMalloc(&hp.nodes, (8 + 64 + 512) * sizeof(uint2))) != cudaSuccess ||
-            (e = cudaMalloc(&hp.node_count, (4 + 64 + 8) * 4)) != cudaSuccess) {
-            cudaFree(hp.count); cudaFree(hp.start); cudaFree(hp.nodes); cudaFree(hp.node_count);
-            hp.count = hp.start = nullptr; hp.nodes = nullptr; hp.node_count = nullptr;
-            return e;
-        }
-    }
-    if (octree) h16::k_fp16_nodes<<<1, 1, 0, st>>>(tv.cell_start, hp.nodes, hp.node_count);
-    h16::k_pairs_count<<<(lists + 127) / 128, 128, 0, st>>>(tag, n, lists, tv.cell_start, tv.cell_list, tv.cell_cap, hp.count);
-    h16::k_pairs_scan<<<1, 32, 0, st>>>(hp.count, lists, hp.start);
+    if ((e = hp.count.reserve(kCells + 1)) != cudaSuccess || (e = hp.start.reserve(kCells + 2)) != cudaSuccess ||
+        (e = hp.nodes.reserve(8 + 64 + 512)) != cudaSuccess || (e = hp.node_count.reserve(4 + 64 + 8)) != cudaSuccess)
+        return e;
+    if (octree) h16::k_fp16_nodes<<<1, 1, 0, st>>>(tv.cell_start, hp.nodes.ptr, hp.node_count.ptr);
+    h16::k_pairs_count<<<(lists + 127) / 128, 128, 0, st>>>(tag, n, lists, tv.cell_start, tv.cell_list, tv.cell_cap, hp.count.ptr);
+    h16::k_pairs_scan<<<1, 32, 0, st>>>(hp.count.ptr, lists, hp.start.ptr);
     uint32_t total = 0;
-    if ((e = cudaMemcpyAsync(&total, hp.start + lists, 4, cudaMemcpyDeviceToHost, st)) != cudaSuccess) return e;
+    if ((e = cudaMemcpyAsync(&total, hp.start.ptr + lists, 4, cudaMemcpyDeviceToHost, st)) != cudaSuccess) return e;
     if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return e;
     hp.valid = false;                           // until the lists are rebuilt: a failure below must not leave stale lists marked usable
-    if (total + 1 > hp.cap) {
-        cudaFree(hp.geom); cudaFree(hp.idx);
-        hp.geom = nullptr; hp.idx = nullptr; hp.cap = 0;
-        if ((e = cudaMalloc(&hp.geom, ((size_t)total + 1) * sizeof(uint4))) != cudaSuccess) return e;
-        if ((e = cudaMalloc(&hp.idx, ((size_t)total + 1) * sizeof(int2))) != cudaSuccess) {
-            cudaFree(hp.geom);
-            hp.geom = nullptr;
-            return e;
-        }
-        hp.cap = (size_t)total + 1;
-    }
-    h16::k_pairs_fill<<<(lists + 127) / 128, 128, 0, st>>>(geom_h, tag, n, lists, tv.cell_start, tv.cell_list, tv.cell_cap, hp.start, hp.geom, hp.idx);
+    if ((e = hp.geom.reserve((size_t)total + 1)) != cudaSuccess || (e = hp.idx.reserve((size_t)total + 1)) != cudaSuccess) return e;
+    h16::k_pairs_fill<<<(lists + 127) / 128, 128, 0, st>>>(geom_h, tag, n, lists, tv.cell_start, tv.cell_list, tv.cell_cap, hp.start.ptr,
+                                                           hp.geom.ptr, hp.idx.ptr);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
     hp.pairs = total;
     hp.octree = octree;

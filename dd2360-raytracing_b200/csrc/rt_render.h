@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "rt_buffer.h"
 #include "rt_types.h"
 
 namespace rt {
@@ -80,12 +81,11 @@ cudaError_t launch_scene_to_half(const float4 *geom, const float4 *matl, int n, 
 cudaError_t launch_camera_setup_half(const float lookfrom[3], const float lookat[3], const float vup[3], float vfov, int nx, int ny,
                                      float aspect_override, float aperture, float focus_dist, __half *cam_h, cudaStream_t st);
 struct HalfPairs {            // candidate lists as transposed sphere pairs (rt_half.cuh PairView), owned by the context
-    uint4 *geom = nullptr;
-    int2 *idx = nullptr;
-    uint32_t *start = nullptr, *count = nullptr;
-    uint2 *nodes = nullptr;          // compact per-level tables of the existing octree nodes (rt_half.cuh NodeTab)
-    uint32_t *node_count = nullptr;
-    size_t cap = 0;
+    Buffer<uint4> geom;
+    Buffer<int2> idx;
+    Buffer<uint32_t> start, count;
+    Buffer<uint2> nodes;             // compact per-level tables of the existing octree nodes (rt_half.cuh NodeTab)
+    Buffer<uint32_t> node_count;
     uint32_t pairs = 0;
     bool valid = false, octree = false;
 };
@@ -105,14 +105,12 @@ cudaError_t launch_scatter_rays_half(const SceneView &sc, const uint2 *geom_h, c
                                      float *out_att, int *scattered, cudaStream_t st);
 // ---- output_to_stream on the device (rt_ppm.cu) ----
 struct PpmWorkspace {
-    uint32_t *block_len = nullptr;
-    unsigned long long *block_off = nullptr;
-    size_t block_cap = 0;
-    char *text = nullptr;
-    size_t text_cap = 0, text_len = 0;
+    Buffer<uint32_t> block_len;
+    Buffer<unsigned long long> block_off;
+    Buffer<char> text;
+    size_t text_len = 0;
 };
 cudaError_t ppm_format_device(PpmWorkspace &ws, const float *fb, int nx, int ny, cudaStream_t st, size_t *len_out);
-void ppm_free(PpmWorkspace &ws);
 cudaError_t launch_finalize_n(const float *accum, float *fb, size_t count, int ns, cudaStream_t st);
 
 }  // namespace rt

@@ -1,5 +1,5 @@
-"""Compiler output of rt_render.cu at two source trees: ptxas registers, spills and stack per kernel, and which kernels compile
-to the same SASS.  Host only (nvcc + cuobjdump, no GPU): the check a refactor of the render kernels owes before any run.
+"""Compiler output of the library's CUDA sources (build.SOURCES) at two source trees: ptxas registers, spills and stack per kernel,
+and which kernels compile to the same SASS.  Host only (nvcc + cuobjdump, no GPU): the check a refactor owes before any run.
 
     python profiles/compare_render_ptxas.py BASE_CSRC NEW_CSRC [--out FILE]
 
@@ -25,10 +25,10 @@ STACK = re.compile(r"(\d+) bytes stack frame, (\d+) bytes spill stores, (\d+) by
 REGS = re.compile(r"Used (\d+) registers")
 
 
-def compile_tree(csrc: str, extra: list[str], tmp: str) -> tuple[dict, dict]:
-    """-> ({kernel: (regs, spill stores, spill loads, stack)}, {kernel: [SASS lines without addresses]})"""
-    obj = os.path.join(tmp, "rt_render.o")
-    cmd = [rt_build._nvcc(), *rt_build.NVCC_FLAGS, *extra, "-Xptxas", "-v", "-c", os.path.join(csrc, "rt_render.cu"), "-o", obj]
+def compile_source(csrc: str, src: str, extra: list[str], tmp: str) -> tuple[dict, dict]:
+    """-> ({kernel: (regs, spill stores, spill loads, stack)}, {kernel: [SASS lines without addresses]}) of one source"""
+    obj = os.path.join(tmp, src.replace(".cu", ".o"))
+    cmd = [rt_build._nvcc(), *rt_build.NVCC_FLAGS, *extra, "-Xptxas", "-v", "-c", os.path.join(csrc, src), "-o", obj]
     log = subprocess.run(cmd, check=True, capture_output=True, text=True).stderr
     res, cur, stack = {}, None, (0, 0, 0)
     for line in log.splitlines():
@@ -63,25 +63,27 @@ def main() -> int:
     a = ap.parse_args()
     lines, worse = [], False
     for label, extra in (("plain build", []), ("-DRT_COUNTERS build", ["-DRT_COUNTERS"])):
-        with tempfile.TemporaryDirectory() as t0, tempfile.TemporaryDirectory() as t1, ThreadPoolExecutor(2) as ex:
-            f0, f1 = ex.submit(compile_tree, a.base, extra, t0), ex.submit(compile_tree, a.new, extra, t1)
-            (r0, s0), (r1, s1) = f0.result(), f1.result()
-        names = sorted(set(r0) | set(r1))
-        dm = demangle(names)
-        same = [n for n in names if n in s0 and n in s1 and s0[n] == s1[n]]
-        lines.append(f"{label}: {len(same)} of {len(r0)} kernels SASS-identical")
-        lines.append(f"  {'kernel':58s} {'regs':>9s} {'spill st':>11s} {'spill ld':>11s} {'stack':>11s}   (base -> new)")
-        for n in names:
-            if n in same:
-                continue
-            b, c = r0.get(n), r1.get(n)
-            cells = [f"{'-' if b is None else b[k]:>4} -> {'-' if c is None else c[k]:<4}" for k in range(4)]
-            flag = ""
-            if b and c and any(c[k] > b[k] for k in range(4)):
-                flag, worse = "  WORSE", True
-            lines.append(f"  {dm[n]:58s} {cells[0]:>9s} {cells[1]:>11s} {cells[2]:>11s} {cells[3]:>11s}{flag}")
-        lines.append("  SASS-identical: " + ", ".join(dm[n] for n in same))
-        lines.append("")
+        with tempfile.TemporaryDirectory() as t0, tempfile.TemporaryDirectory() as t1, ThreadPoolExecutor() as ex:
+            jobs = [(src, ex.submit(compile_source, a.base, src, extra, t0), ex.submit(compile_source, a.new, src, extra, t1))
+                    for src in rt_build.SOURCES]
+            results = [(src, f0.result(), f1.result()) for src, f0, f1 in jobs]
+        for src, (r0, s0), (r1, s1) in results:
+            names = sorted(set(r0) | set(r1))
+            dm = demangle(names)
+            same = [n for n in names if n in s0 and n in s1 and s0[n] == s1[n]]
+            lines.append(f"{label}, {src}: {len(same)} of {len(r0)} kernels SASS-identical")
+            differ = [n for n in names if n not in same]
+            if differ:
+                lines.append(f"  {'kernel':58s} {'regs':>9s} {'spill st':>11s} {'spill ld':>11s} {'stack':>11s}   (base -> new)")
+            for n in differ:
+                b, c = r0.get(n), r1.get(n)
+                cells = [f"{'-' if b is None else b[k]:>4} -> {'-' if c is None else c[k]:<4}" for k in range(4)]
+                flag = ""
+                if b and c and any(c[k] > b[k] for k in range(4)):
+                    flag, worse = "  WORSE", True
+                lines.append(f"  {dm[n]:58s} {cells[0]:>9s} {cells[1]:>11s} {cells[2]:>11s} {cells[3]:>11s}{flag}")
+            lines.append("  SASS-identical: " + ", ".join(dm[n] for n in same))
+            lines.append("")
     text = "\n".join(lines)
     print(text)
     if a.out:
