@@ -474,6 +474,26 @@ static int ensure_half(rt_context *ctx, unsigned what, bool octree, const TreeVi
     return RT_OK;
 }
 
+// The structure a render or a per-ray query walks, shared by both so that rt_trace_rays answers a ray as the render's kernels do.
+// Octree mode: the octree's grid.  Flat-list mode: hitable_list::hit is "closest over all spheres"; in FP32 from kListGridMinSpheres
+// spheres on the grid over ALL spheres answers it with a few dozen tests instead of N (the same minimum; variant 20 forces the N-test
+// sweep), built on first use (an undefined slot 0 stays unhittable there too: the build sees its tag, TreeView::slot0_none).
+// p.coop_items: four candidates per lane for the cooperative walk once voxel lists are long.
+static int select_walk(rt_context *ctx, const bool use_octree, const int precision, const int variant, RenderLaunch &p, bool &list_grid) {
+    list_grid = !use_octree && precision == RT_PREC_FP32 && ctx->n >= kListGridMinSpheres && variant != 20;
+    if (use_octree) p.tree = ctx->octree.view();
+    if (list_grid) {
+        if (!ctx->list_accel_valid) {
+            CK(ctx->list_accel.build(ctx->stream, ctx->geom.ptr, ctx->tag.ptr, ctx->n, 30, ctx->grid_density, false, true));
+            ctx->list_accel_valid = true;
+        }
+        p.tree = ctx->list_accel.view();
+    }
+    const OctreeBuilder &acc = list_grid ? ctx->list_accel : ctx->octree;
+    p.coop_items = (use_octree || list_grid) && acc.total_voxels > 0 && acc.total_refs / acc.total_voxels >= 40 ? 4 : 2;
+    return RT_OK;
+}
+
 // ---- render -----------------------------------------------------------------------------------------------------
 struct ProgressiveIO {
     uint32_t *state = nullptr;     // 6 words per pixel, device
@@ -549,24 +569,12 @@ static int do_render(rt_context *ctx, const rt_render_args *a, float *out_dev, b
     RenderLaunch p;
     memset(&p, 0, sizeof p);
     p.scene.geom = ctx->geom.ptr; p.scene.matl = ctx->matl.ptr; p.scene.tag = ctx->tag.ptr; p.scene.n = ctx->n;
-    if (a->use_octree) p.tree = ctx->octree.view();
-    // flat-list mode: hitable_list::hit is "closest over all spheres"; above a few hundred spheres the grid answers it
-    // with a few dozen tests instead of N (the result is the same minimum; variant 20 forces the N-test sweep)
     bool list_grid = false;
-    // (an undefined slot 0 stays unhittable there too: the build sees its tag, TreeView::slot0_none)
-    if (!a->use_octree && a->precision == RT_PREC_FP32 && ctx->n >= kListGridMinSpheres && a->tune[1] != 20) {
-        if (!ctx->list_accel_valid) {
-            CK(ctx->list_accel.build(ctx->stream, ctx->geom.ptr, ctx->tag.ptr, ctx->n, 30, ctx->grid_density, false, true));
-            ctx->list_accel_valid = true;
-        }
-        p.tree = ctx->list_accel.view();
-        list_grid = true;
+    {
+        const int rc = select_walk(ctx, a->use_octree != 0, a->precision, a->tune[1], p, list_grid);
+        if (rc) return rc;
     }
     p.cam = ctx->cam_host;                        // per-context camera, by value in the launch parameters
-    {
-        const OctreeBuilder &acc = list_grid ? ctx->list_accel : ctx->octree;
-        p.coop_items = (a->use_octree || list_grid) && acc.total_voxels > 0 && acc.total_refs / acc.total_voxels >= 40 ? 4 : 2;
-    }
     p.nx = a->nx; p.ny = a->ny;
     p.ns_total = a->ns;
     p.ns_local = a->ns;
@@ -738,7 +746,8 @@ static int run_staged(rt_context *ctx, std::initializer_list<HostArray> arrays, 
     return RT_OK;
 }
 
-// test hook: closest hit of caller-supplied rays (host arrays of 3 floats per ray)
+// test hook: closest hit of caller-supplied rays (host arrays of 3 floats per ray), by the walk the render would use for the scene
+// (select_walk; RT_RENDER_VARIANT picks another: launch_trace_rays)
 extern "C" int rt_trace_rays(rt_context *ctx, int use_octree, int n, const float *org, const float *dir, int *out_idx, float *out_t) {
     return rt_trace_rays_ex(ctx, use_octree, RT_PREC_FP32, n, org, dir, out_idx, out_t);
 }
@@ -770,17 +779,20 @@ extern "C" int rt_trace_rays_ex(rt_context *ctx, int use_octree, int precision, 
     RenderLaunch p;
     memset(&p, 0, sizeof p);
     p.scene.geom = ctx->geom.ptr; p.scene.matl = ctx->matl.ptr; p.scene.tag = ctx->tag.ptr; p.scene.n = ctx->n;
-    if (use_octree) p.tree = ctx->octree.view();
+    p.variant = fp16 ? 0 : ctx->default_variant;     // RT_RENDER_VARIANT selects the FP32 walk (launch_trace_rays)
+    bool list_grid = false;
+    {
+        const int rc = select_walk(ctx, use_octree != 0, precision, p.variant, p, list_grid);
+        if (rc) return rc;
+    }
     if (fp16) {
         const int rc = ensure_half(ctx, kHalfPairs, use_octree != 0, p.tree, 0, 0);
         if (rc) return rc;
-    } else {
-        p.variant = ctx->default_variant;          // RT_RENDER_VARIANT=1: the per-lane walk
     }
     const size_t N = (size_t)n;
     return run_staged(ctx, {stage_in(org, 3 * N), stage_in(dir, 3 * N), stage_out(out_idx, N), stage_out(out_t, N)}, [&](const DevPtr *d) {
         return fp16 ? launch_trace_rays_half(p, use_octree != 0, ctx->geom_h.ptr, ctx->half_pairs, d[0], d[1], n, d[2], d[3], ctx->stream)
-                    : launch_trace_rays(p, use_octree != 0, d[0], d[1], n, d[2], d[3], ctx->stream);
+                    : launch_trace_rays(p, use_octree != 0 || list_grid, d[0], d[1], n, d[2], d[3], ctx->stream);
     });
 }
 

@@ -192,9 +192,9 @@ __device__ __forceinline__ Hit coop_trace(WarpShared &ws, const SceneView &sc, c
             ix = imin(imax(ix, 0), g.nx - 1);
             iy = imin(imax(iy, 0), g.ny - 1);
             iz = imin(imax(iz, 0), g.nz - 1);
-            if (fabsf(d.x) > 0.0f) tmx = (g.org[0] + (float)(ix + (sx > 0)) * g.vs[0] - o.x) * r.inv.x;
-            if (fabsf(d.y) > 0.0f) tmy = (g.org[1] + (float)(iy + (sy > 0)) * g.vs[1] - o.y) * r.inv.y;
-            if (fabsf(d.z) > 0.0f) tmz = (g.org[2] + (float)(iz + (sz > 0)) * g.vs[2] - o.z) * r.inv.z;
+            if (fabsf(d.x) >= kDdaMinDir) tmx = (g.org[0] + (float)(ix + (sx > 0)) * g.vs[0] - o.x) * r.inv.x;
+            if (fabsf(d.y) >= kDdaMinDir) tmy = (g.org[1] + (float)(iy + (sy > 0)) * g.vs[1] - o.y) * r.inv.y;
+            if (fabsf(d.z) >= kDdaMinDir) tmz = (g.org[2] + (float)(iz + (sz > 0)) * g.vs[2] - o.z) * r.inv.z;
             dtx = fabsf(g.vs[0] * r.inv.x); dty = fabsf(g.vs[1] * r.inv.y); dtz = fabsf(g.vs[2] * r.inv.z);
             RT_COUNT(voxel_steps);
             const uint2 v = __ldg(g.vox + ((size_t)(iz * g.ny + iy) * g.nx + ix));
@@ -343,8 +343,10 @@ __global__ void __launch_bounds__(kRenderThreads, 8) k_render_coop_pixels_progre
     render_coop_lanes<ITEMS, kModeListProgressive>(p);
 }
 
-// test hook: closest hit of caller-supplied rays through the cooperative trace (32 rays per warp)
-__global__ void __launch_bounds__(kRenderThreads) k_trace_rays_coop(const __grid_constant__ RenderLaunch p, const float *__restrict__ org,
+// test hook: closest hit of caller-supplied rays through the cooperative trace (32 rays per warp, ITEMS candidates per lane; launched
+// with kRenderThreads per block).  The register cap replaces __launch_bounds__: under it ptxas spills (ITEMS 4: 24 B) at 64 registers.
+template <int ITEMS>
+__global__ void __maxnreg__(128) k_trace_rays_coop(const __grid_constant__ RenderLaunch p, const float *__restrict__ org,
                                                                    const float *__restrict__ dir, int n, int *__restrict__ out_idx,
                                                                    float *__restrict__ out_t) {
     __shared__ WarpShared wsh[kRenderThreads / 32];
@@ -354,7 +356,7 @@ __global__ void __launch_bounds__(kRenderThreads) k_trace_rays_coop(const __grid
     const vec3f d = has ? mk(dir[3 * i], dir[3 * i + 1], dir[3 * i + 2]) : mk(0, 0, 1);
     TraceCounters tc;
     tc.sphere_tests = tc.node_tests = tc.voxel_steps = 0;
-    const Hit h = coop_trace_tree<2>(wsh[threadIdx.x >> 5], p.scene, p.tree, &p.tree.planes[0][0], threadIdx.x & 31u, has, o, d, tc);
+    const Hit h = coop_trace_tree<ITEMS>(wsh[threadIdx.x >> 5], p.scene, p.tree, &p.tree.planes[0][0], threadIdx.x & 31u, has, o, d, tc);
     if (has) { out_idx[i] = h.idx; out_t[i] = h.t; }
 }
 

@@ -409,10 +409,15 @@ __global__ void k_trace_rays(const __grid_constant__ RenderLaunch p, int octree,
     out_t[i] = h.t;
 }
 
+// octree: the octree's grid, or the flat-list mode's grid over all spheres (p.tree); otherwise the N-test sweep
 cudaError_t launch_trace_rays(const RenderLaunch &p, bool octree, const float *org, const float *dir, int n, int *out_idx,
                               float *out_t, cudaStream_t st) {
-    if (octree && p.variant != 1)     // the render kernels' default trace: warp-cooperative (rt_coop.cuh); variant 1 = the per-lane walk
-        coop::k_trace_rays_coop<<<(n + kRenderThreads - 1) / kRenderThreads, kRenderThreads, 0, st>>>(p, org, dir, n, out_idx, out_t);
+    const unsigned blocks = (unsigned)((n + kRenderThreads - 1) / kRenderThreads);
+    // the render kernels' default trace: warp-cooperative (rt_coop.cuh) at p.coop_items candidates per lane; variant 1 = the per-lane walk
+    if (octree && p.variant != 1 && p.coop_items == 4)
+        coop::k_trace_rays_coop<4><<<blocks, kRenderThreads, 0, st>>>(p, org, dir, n, out_idx, out_t);
+    else if (octree && p.variant != 1)
+        coop::k_trace_rays_coop<2><<<blocks, kRenderThreads, 0, st>>>(p, org, dir, n, out_idx, out_t);
     else
         k_trace_rays<<<(n + 127) / 128, 128, 0, st>>>(p, octree ? 1 : 0, org, dir, n, out_idx, out_t);
     return cudaGetLastError();

@@ -162,13 +162,19 @@ RT_HD bool maybe_hit_ub(const float4 s, const vec3f o, const vec3f d, const floa
     return pass;
 }
 
+// Smallest direction component the 3D-DDA steps along (FLT_MIN): below it the ray moves less than 1e-35 per unit of t, far
+// inside the voxel lists' padding, and the walk treats the axis as fixed.
+constexpr float kDdaMinDir = 1.17549435e-38f;
+
 struct RayPre {
     vec3f o, d, inv;    // inv = 1/d (IEEE; +-inf for zero components)
     float a;            // dot(d,d)
 };
 
 // Conservative ray/box interval: returns false when the ray cannot be inside [lo,hi] for any t in
-// (kTMin, t_far].  fminf/fmaxf drop NaNs (0*inf), which only ever widens the interval.
+// (kTMin, t_far].  A zero direction component with the origin exactly on that face gives a NaN slab bound (0*inf), and
+// fminf/fmaxf pick the other bound: fminf(NaN, +inf) = +inf, so such a ray skips the box.  Harmless for the grid box: it holds
+// every padded sphere, so no hit lies in its faces.
 RT_HD bool ray_box(const RayPre &r, const float *lo, const float *hi, const float t_far, float &t_enter, float &t_exit) {
     const float tx0 = (lo[0] - r.o.x) * r.inv.x, tx1 = (hi[0] - r.o.x) * r.inv.x;
     const float ty0 = (lo[1] - r.o.y) * r.inv.y, ty1 = (hi[1] - r.o.y) * r.inv.y;
@@ -336,10 +342,11 @@ RT_HD Hit trace_walk(const SceneView &sc, const TreeView &tv, const float *plane
     iz = imin(imax(iz, 0), g.nz - 1);
     const int sx = d.x >= 0.0f ? 1 : -1, sy = d.y >= 0.0f ? 1 : -1, sz = d.z >= 0.0f ? 1 : -1;
     // ray parameter at which the ray leaves the current voxel along each axis; an axis the ray does not move along
-    // never advances
-    float tmx = fabsf(d.x) > 0.0f ? (g.org[0] + (float)(ix + (sx > 0)) * g.vs[0] - o.x) * r.inv.x : kTMax;
-    float tmy = fabsf(d.y) > 0.0f ? (g.org[1] + (float)(iy + (sy > 0)) * g.vs[1] - o.y) * r.inv.y : kTMax;
-    float tmz = fabsf(d.z) > 0.0f ? (g.org[2] + (float)(iz + (sz > 0)) * g.vs[2] - o.z) * r.inv.z : kTMax;
+    // never advances.  A subnormal component counts as not moving (kDdaMinDir): its reciprocal is infinite, and with the origin
+    // on a voxel plane of that axis 0 * inf would make tm NaN, every step comparison false and the walk lose its other axes
+    float tmx = fabsf(d.x) >= kDdaMinDir ? (g.org[0] + (float)(ix + (sx > 0)) * g.vs[0] - o.x) * r.inv.x : kTMax;
+    float tmy = fabsf(d.y) >= kDdaMinDir ? (g.org[1] + (float)(iy + (sy > 0)) * g.vs[1] - o.y) * r.inv.y : kTMax;
+    float tmz = fabsf(d.z) >= kDdaMinDir ? (g.org[2] + (float)(iz + (sz > 0)) * g.vs[2] - o.z) * r.inv.z : kTMax;
     const float dtx = fabsf(g.vs[0] * r.inv.x), dty = fabsf(g.vs[1] * r.inv.y), dtz = fabsf(g.vs[2] * r.inv.z);
     uint32_t k, e;
     {

@@ -152,8 +152,16 @@ int rt_xorwow_state(unsigned long long seed, unsigned long long subsequence, uin
  * [3] visibility line tests and [4] voxel steps. */
 int rt_debug_counters(rt_context *ctx, uint64_t out[32]);
 
-/* test hook: closest hit (sphere index or -1, and t) of n caller-supplied rays — hitTree / hitable_list::hit per ray.  An octree
- * query on a tree built for RT_PREC_FP16 is RT_ERR_STATE ("other precision"), as in rt_trace_rays_ex. */
+/* test hook: closest hit (sphere index or -1, and t) of n caller-supplied rays — hitTree / hitable_list::hit per ray, answered by
+ * the walk the FP32 render kernels use for the same scene, so that each of them can be held to a reference ray by ray:
+ *   octree            : the warp-cooperative walk (two candidates per lane, four once voxel lists average 40 or more references);
+ *   flat list         : below 256 spheres the N-test sweep; from 256 on the same walks over the grid of all spheres the render
+ *                       builds for that mode (built here on first use);
+ * the environment variable RT_RENDER_VARIANT, read by rt_create, selects another walk: 1 the per-lane grid walk, 20 the N-test
+ * sweep (flat list), 40 the cooperative walk.  Every walk returns the same index and t.  Outside the contract (the answer may differ
+ * from the reference's): in octree mode, a zero direction component with the origin exactly on one of the reference's level-3 cell
+ * planes of that axis (x, z = -11 + 2.75k, y = 0.25k), where the reference's own slab test divides 0 by 0.  An octree query on a tree built for RT_PREC_FP16 is RT_ERR_STATE
+ * ("other precision"), as in rt_trace_rays_ex. */
 int rt_trace_rays(rt_context *ctx, int use_octree, int n, const float *org, const float *dir, int *out_idx, float *out_t);
 
 /* camera::get_ray(s, t, &rand_state) (camera.h:45-49) for n (s, t) pairs, each drawing its lens sample from its own XORWOW

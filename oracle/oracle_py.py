@@ -98,6 +98,9 @@ def lib() -> C.CDLL:
         L.rto_closest_hit.restype = C.c_int
         L.rto_closest_hit.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                       C.c_void_p, C.c_void_p, C.POINTER(C.c_float)]
+        L.rto_closest_hits.restype = None
+        L.rto_closest_hits.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.rto_version.restype = C.c_char_p
         _lib = L
     return _lib
@@ -194,6 +197,18 @@ def closest_hit(spheres, o, d, blob=None, spl=30, use_octree=False, arith=ARITH_
     t = C.c_float(0)
     idx = lib().rto_closest_hit(_p(spheres), len(spheres), _p(blob), spl, int(use_octree), arith, _p(o), _p(d), C.byref(t))
     return idx, t.value
+
+
+def closest_hits(spheres, org, dirs, blob=None, spl=30, use_octree=False, arith=ARITH_DEVICE):
+    """closest_hit for every row of org / dirs ([R, 3]), OpenMP over the rays: (index int32[R], t float32[R])."""
+    org = np.ascontiguousarray(org, dtype=np.float32).reshape(-1, 3)
+    dirs = np.ascontiguousarray(dirs, dtype=np.float32).reshape(-1, 3)
+    assert org.shape == dirs.shape
+    idx = np.zeros(len(org), np.int32)
+    t = np.zeros(len(org), np.float32)
+    lib().rto_closest_hits(_p(spheres), len(spheres), _p(blob), spl, int(use_octree), arith, len(org), _p(org), _p(dirs),
+                           _p(idx), _p(t))
+    return idx, t
 
 
 # ---------------------------------------------------------------------------------------------------------

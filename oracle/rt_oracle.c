@@ -373,6 +373,13 @@ int rto_closest_hit(const rto_sphere *sph, int n, const void *blob, int spl, int
                                      : closest_hit_host(sph, n, &ov, use_octree, O, D, t_out);
 }
 
+void rto_closest_hits(const rto_sphere *sph, int n, const void *blob, int spl, int use_octree, int arith, int nrays,
+                      const float *org, const float *dir, int *out_idx, float *out_t) {
+#pragma omp parallel for schedule(dynamic, 64)
+    for (int k = 0; k < nrays; k++)
+        out_idx[k] = rto_closest_hit(sph, n, blob, spl, use_octree, arith, org + 3 * (size_t)k, dir + 3 * (size_t)k, out_t + k);
+}
+
 /* main.cu:321-333 */
 void rto_quantise(const float *fb, int nx, int ny, uint8_t *out) {
     for (int j = ny - 1; j >= 0; j--)

@@ -105,6 +105,9 @@ int rto_xorwow_skip_tables(uint32_t *out, int max_bits);
 /* Single-ray closest hit (for per-ray parity tests): returns sphere index or -1; t/normal out. */
 int rto_closest_hit(const rto_sphere *spheres, int n, const void *octree_blob, int spl, int use_octree,
                     int arith, const float origin[3], const float dir[3], float *t_out);
+/* rto_closest_hit for nrays rays (origins and directions: 3 floats each), OpenMP over the rays: out_idx[k], out_t[k]. */
+void rto_closest_hits(const rto_sphere *spheres, int n, const void *octree_blob, int spl, int use_octree, int arith, int nrays,
+                      const float *origins, const float *dirs, int *out_idx, float *out_t);
 
 const char *rto_version(void);
 

@@ -208,9 +208,9 @@ static CoopHit coop_walk_host(const SceneView &sc, const TreeView &tv, const vec
         int iz = (int)floorf((o.z + d.z * te - g.org[2]) * g.inv_vs[2]);
         ix = imin(imax(ix, 0), g.nx - 1); iy = imin(imax(iy, 0), g.ny - 1); iz = imin(imax(iz, 0), g.nz - 1);
         const int sx = d.x >= 0.0f ? 1 : -1, sy = d.y >= 0.0f ? 1 : -1, sz = d.z >= 0.0f ? 1 : -1;
-        float tmx = fabsf(d.x) > 0.0f ? (g.org[0] + (float)(ix + (sx > 0)) * g.vs[0] - o.x) * r.inv.x : kTMax;
-        float tmy = fabsf(d.y) > 0.0f ? (g.org[1] + (float)(iy + (sy > 0)) * g.vs[1] - o.y) * r.inv.y : kTMax;
-        float tmz = fabsf(d.z) > 0.0f ? (g.org[2] + (float)(iz + (sz > 0)) * g.vs[2] - o.z) * r.inv.z : kTMax;
+        float tmx = fabsf(d.x) >= kDdaMinDir ? (g.org[0] + (float)(ix + (sx > 0)) * g.vs[0] - o.x) * r.inv.x : kTMax;
+        float tmy = fabsf(d.y) >= kDdaMinDir ? (g.org[1] + (float)(iy + (sy > 0)) * g.vs[1] - o.y) * r.inv.y : kTMax;
+        float tmz = fabsf(d.z) >= kDdaMinDir ? (g.org[2] + (float)(iz + (sz > 0)) * g.vs[2] - o.z) * r.inv.z : kTMax;
         const float dtx = fabsf(g.vs[0] * r.inv.x), dty = fabsf(g.vs[1] * r.inv.y), dtz = fabsf(g.vs[2] * r.inv.z);
         int budget = g.nx + g.ny + g.nz + 4;
         bool walking = true;
@@ -391,6 +391,68 @@ int hs_render_with_tree(const hs_sphere *sph, int n, const float *camera22, cons
     tv.no_drops = 1;
     for (uint32_t k = 0, e = tv.vis.ent_off[n]; k < e; k++) if (tv.vis.ent_cell[k] & kEntDropped) tv.no_drops = 0;
     return render_core(sph, n, camera22, nullptr, p, 0.f, fb_gamma, nullptr, ctr_out, nullptr, &tv);
+}
+
+// The traversal structure of the scene: the octree's grid (use_octree, from the reference-layout blob) or the flat-list mode's grid
+// over all spheres, and its view.
+struct HostScene {
+    std::vector<float4> geom;
+    std::vector<int> tag;
+    HostTree T;
+    TreeView tv;
+    SceneView sc;
+};
+static void host_scene(const hs_sphere *sph, int n, const void *blob, int spl, int use_octree, float density, HostScene &S) {
+    S.geom.resize((size_t)n);
+    S.tag.resize((size_t)n);
+    for (int i = 0; i < n; i++) { S.geom[(size_t)i] = make_float4(sph[i].cx, sph[i].cy, sph[i].cz, sph[i].radius); S.tag[(size_t)i] = sph[i].mat; }
+    if (use_octree) build_host_tree(S.geom, S.tag, static_cast<const int32_t *>(blob), spl, density, S.T);
+    else build_list_grid(S.geom, S.tag, density, S.T);
+    view_of(S.T, S.tv, S.tag[0] < 0, use_octree != 0);
+    memset(&S.sc, 0, sizeof S.sc);
+    S.sc.geom = S.geom.data(); S.sc.tag = S.tag.data(); S.sc.n = n;
+}
+
+// Closest hit of caller rays (3 floats each) by the product's walks compiled for the host, over the octree's grid (use_octree) or
+// the flat-list mode's grid: walk 0 trace_tree (k_trace_rays), 1 / 2 the cooperative candidate rule (coop_walk_host, eager / lazy
+// schedule) followed by finish_hit, as coop_trace_tree.  out_idx = -1 on a miss.
+int hs_trace_rays(const hs_sphere *sph, int n, const void *blob, int spl, int use_octree, float density, int walk, int nrays,
+                  const float *org, const float *dir, int *out_idx, float *out_t) {
+    if (walk < 0 || walk > 2 || (use_octree && !blob) || n < 1) return -1;
+    HostScene S;
+    host_scene(sph, n, blob, spl, use_octree, density, S);
+    const float *planes = &S.tv.planes[0][0];
+#pragma omp parallel for schedule(dynamic, 64)
+    for (int k = 0; k < nrays; k++) {
+        const vec3f o = mk(org[3 * (size_t)k], org[3 * (size_t)k + 1], org[3 * (size_t)k + 2]);
+        const vec3f d = mk(dir[3 * (size_t)k], dir[3 * (size_t)k + 1], dir[3 * (size_t)k + 2]);
+        TraceCounters tc{};
+        Hit h;
+        if (walk == 0) {
+            h = trace_tree(S.sc, S.tv, planes, o, d, tc);
+        } else {
+            const CoopHit c = coop_walk_host(S.sc, S.tv, o, d, walk == 1);
+            h.t = c.t; h.idx = c.idx;
+            h = finish_hit(S.sc, S.tv, planes, o, d, h, c.tie, tc);
+        }
+        out_idx[k] = h.idx;
+        out_t[k] = h.t;
+    }
+    return 0;
+}
+
+// The voxel grid the build makes for the scene (as hs_trace_rays): out9 = origin, voxel size, far corner; dims = nx, ny, nz;
+// counts = voxels, references (the library's coop_items rule reads their ratio).
+int hs_grid_geometry(const hs_sphere *sph, int n, const void *blob, int spl, int use_octree, float density, float *out9, int *dims,
+                     uint64_t *counts) {
+    if ((use_octree && !blob) || n < 1) return -1;
+    HostScene S;
+    host_scene(sph, n, blob, spl, use_octree, density, S);
+    const GridView &g = S.T.grid;
+    for (int k = 0; k < 3; k++) { out9[k] = g.org[k]; out9[3 + k] = g.vs[k]; out9[6 + k] = g.hi[k]; }
+    dims[0] = g.nx; dims[1] = g.ny; dims[2] = g.nz;
+    counts[0] = S.T.vox.size(); counts[1] = S.T.refs.size();
+    return 0;
 }
 
 // Soundness of visible_fast (rt_trace.cuh) against the rule it short-cuts: for `nrays` pseudo-random rays — aimed at sphere

@@ -9,6 +9,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
+import ray_families as F
 import test_caller_worlds_host as W
 
 pytestmark = pytest.mark.gpu
@@ -126,21 +127,6 @@ def test_dense_list_world_four_candidates_per_lane(rt, pkg, O):
     _check_frames(rt, pkg, O, sph, None, False, ["wide_aperture", "in_glass"], 64, 48, 2, (40, 1, 20))
 
 
-def _rays_on_and_in(sph, rng, idx):
-    """Rays from the surfaces (|r| out from the centre) and from inside (|r| / 2) of the spheres idx, outwards, inwards and at random."""
-    c = np.stack([sph["cx"][idx], sph["cy"][idx], sph["cz"][idx]], 1).astype(np.float64)
-    r = np.abs(sph["radius"][idx]).astype(np.float64)[:, None]
-    u = rng.normal(size=(len(idx), 3))
-    u /= np.linalg.norm(u, axis=1, keepdims=True)
-    org, dirs = [], []
-    for depth in (1.0, 0.5):
-        o = c + depth * r * u
-        for d in (u, -u, rng.normal(size=u.shape)):
-            org.append(o)
-            dirs.append(d)
-    return np.concatenate(org).astype(np.float32), np.concatenate(dirs).astype(np.float32)
-
-
 @pytest.mark.parametrize("octree", [True, False], ids=["octree", "list"])
 @pytest.mark.parametrize("world", ["hollow", "duplicates"])
 def test_closest_hit_from_on_and_inside_spheres(rt, O, world, octree):
@@ -155,7 +141,7 @@ def test_closest_hit_from_on_and_inside_spheres(rt, O, world, octree):
     else:
         idx = rng.choice(np.arange(len(sph) // 2 + 1, len(sph)), 150, replace=False)    # the duplicates
     idx = rng.choice(idx, min(len(idx), 150), replace=False)
-    org, dirs = _rays_on_and_in(sph, rng, idx)
+    org, dirs = F.on_and_in(sph, rng, idx)
     gi, gt = rt.trace_rays(org, dirs, octree)
     hits = 0
     for k in range(len(org)):
